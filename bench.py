@@ -100,6 +100,15 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
+def dump_outputs(out_dir, fields):
+    """One DIR/<name>.npy per result field: float32 fields stay float32, every other field (indices and counts included,
+    all exact below 2^53) is written as float64."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in fields.items():
+        np.save(d / f"{name}.npy", np.asarray(a, dtype=np.float32 if a.dtype == np.float32 else np.float64))
+
+
 # ---- clocks ----------------------------------------------------------------------------------------
 class ClockSampler:
     Q = ("clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.hw_slowdown,"
@@ -171,14 +180,19 @@ def run_reference(args):
     t_off, r_off = toff[:sample_units + 1], roff[:sample_units + 1]
     ncand = len(ora.search_grid(STEP_DEG, RANGE_DEG, None, RANGE_DEG)[0])
 
+    last = {}
+
     def step():
         t0 = time.perf_counter()
-        ora.sweep_batch(txy[sl], t_off, rxy[sl], r_off, cen[:sample_units], 0, STEP_DEG, RANGE_DEG, RANGE_DEG, threads=cores)
+        last["best_idx"], last["best_dist"] = ora.sweep_batch(txy[sl], t_off, rxy[sl], r_off, cen[:sample_units], 0, STEP_DEG,
+                                                              RANGE_DEG, RANGE_DEG, threads=cores)
         return time.perf_counter() - t0
 
     for _ in range(min(args.warmup, 1)):
         step()
     times = [step() for _ in range(args.steps)]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
     evals = sample_units * ncand
     v = evals * len(times) / sum(times)
     sample = (f"per step {sample_units} of the {398 * N_PAIRS} frame-pair units x {ncand} candidates (N=M={n}), {cores} host "
@@ -218,7 +232,12 @@ def main():
     ap.add_argument("--no-api", action="store_true", help="skip the public-API wall-time legs (e2e_api, full_mode)")
     ap.add_argument("--no-tc", action="store_true", help="skip the opt-in tier legs (tensor-core prefilter, pruning)")
     ap.add_argument("--write-golden", action="store_true", help="N = 1 only: (re)write tests/golden/bench_units.npz")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the per-unit results of the last timed step as DIR/<field>.npy, so that two builds can be "
+                         "compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -296,6 +315,8 @@ def main():
     clk = clocks.stop()
     total_ms = max_over_ranks(sum(dev_ms))
     value = evals * K / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:   # every rank holds the whole merged result
+        dump_outputs(args.dump_outputs, {f: res[f] for f in res.dtype.names})
 
     # ---- every rank holds the whole result: identical across ranks, equal to the committed 1-GPU result -------------
     digest = sha(np.stack([res["best_idx"].astype(np.float64), res["best_angle"], res["best_dist"],

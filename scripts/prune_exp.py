@@ -1,5 +1,7 @@
 import sys
-sys.path[:0]=['/root/repo','/root/repo/multimoda-rs_b200']
+from pathlib import Path
+ROOT = Path(__file__).resolve().parents[1]
+sys.path[:0] = [str(ROOT), str(ROOT / 'multimoda-rs_b200')]
 sys.argv=['x','none','--no-tc']
 from scripts import tc_bench as T
 from multimodars import _native as nat

@@ -1,6 +1,8 @@
 """Experiment: which 32 rows make the tightest lower bound (MMRS_LB_PICK = 0 strided, 1 alternating far/near, 2 far)."""
 import sys
-sys.path[:0] = ['/root/repo', '/root/repo/multimoda-rs_b200']
+from pathlib import Path
+ROOT = Path(__file__).resolve().parents[1]
+sys.path[:0] = [str(ROOT), str(ROOT / 'multimoda-rs_b200')]
 import numpy as np
 import bench
 from multimodars import _native as nat

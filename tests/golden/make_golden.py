@@ -1,10 +1,10 @@
-"""Generates tests/golden/*.npz. Run HERE (the container that has /root/reference):
+"""Generates tests/golden/*.npz. Run with a checkout of the reference:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <reference checkout>
 
 Inputs: the reference's example / fixture pullbacks, re-encoded as (N,4) [frame, x, y, z]
-arrays (+ reference point, + records) so they can travel to the GPU box, where
-/root/reference does not exist. Outputs: what the CPU ORACLE (oracle/, a restatement pinned on
+arrays (+ reference point, + records) so the tests run without the
+reference. Outputs: what the CPU ORACLE (oracle/, a restatement pinned on
 the reference's Rust KATs — the reference itself cannot be built here) returns for the
 reference's own configurations. These are oracle-generated goldens, not reference-generated."""
 import hashlib
@@ -17,7 +17,7 @@ ROOT = Path(__file__).resolve().parents[2]
 sys.path[:0] = [str(ROOT)]
 from oracle import oracle_py as ora  # noqa: E402
 
-REF = Path("/root/reference")
+REF = Path(sys.argv[1])
 OUT = Path(__file__).resolve().parent
 
 

@@ -1,15 +1,16 @@
-"""Generates tests/golden/reference_signatures.json. Run HERE (the container that has /root/reference):
+"""Generates tests/golden/reference_signatures.json. Run with a checkout of the reference:
 
-    python tests/golden/make_signature_golden.py
+    python tests/golden/make_signature_golden.py <reference checkout>
 
 Parameter names, order and default values of the reference's public Python surface, read with `ast` from
 multimodars/_processing.py, multimodars/_converters.py (functions) and multimodars/multimodars.pyi (classes, methods,
 properties) — the names a user's code depends on. tests/test_signatures_cpu.py holds this package against it."""
 import ast
 import json
+import sys
 from pathlib import Path
 
-REF = Path("/root/reference/multimodars")
+REF = Path(sys.argv[1]) / "multimodars"
 OUT = Path(__file__).resolve().parent / "reference_signatures.json"
 
 

@@ -22,8 +22,8 @@ def oracle_outputs():
 
 def phase_arrays(pack, name, diastole):
     ph = "diastolic" if diastole else "systolic"
-    g = lambda k: pack[f"{name}__{ph}_{k}"] if f"{name}__{ph}_{k}" in pack.files else None  # noqa: E731
-    rec = pack[f"{name}__records"] if f"{name}__records" in pack.files else None
+    g = lambda k: pack[f"{name}__{ph}_{k}"] if f"{name}__{ph}_{k}" in pack else None  # noqa: E731
+    rec = pack[f"{name}__records"] if f"{name}__records" in pack else None
     return dict(lumen=g("lumen"), ref_point=g("ref"), eem=g("eem"), calc=g("calc"), side=g("side"), records=rec)
 
 

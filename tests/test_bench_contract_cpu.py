@@ -5,7 +5,7 @@ import subprocess
 import sys
 from pathlib import Path
 
-import numpy as np  # noqa: F401
+import numpy as np
 
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
@@ -22,9 +22,9 @@ def test_workload_shape_is_baseline_config_2():
     assert bench.flops_per_eval(520, 520) == 10 * 520 * 520 + 6 * 520
 
 
-def test_reference_arm_prints_one_json_line():
-    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
-                       capture_output=True, text=True, timeout=600)
+def test_reference_arm_prints_one_json_line(tmp_path):
+    r = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -40,3 +40,8 @@ def test_reference_arm_prints_one_json_line():
     # ... key for key: both arms build it with the same function for the same N
     assert d["config"] == bench.base_config(398 * bench.N_PAIRS, 36000, bench.N_POINTS + bench.N_CATH, 1)
     assert "host threads" in d["cpu_baseline"]["parallelism"]
+    # --dump-outputs: what the last timed step computed, unit 0 of the committed 1-GPU result
+    g = np.load(bench.GOLDEN)
+    idx, dist = np.load(tmp_path / "out" / "best_idx.npy"), np.load(tmp_path / "out" / "best_dist.npy")
+    assert idx.dtype == dist.dtype == np.float64 and idx.shape == dist.shape == (1,)
+    assert idx[0] == g["best_idx"][0] and dist[0] == g["best_dist"][0]
