@@ -198,7 +198,9 @@ int mmrs_ctx_set_prune(mmrs_ctx* ctx, int32_t on);
  * scoring in ms, [3] candidates scored exactly (survivors, all units).
  * Tensor-core prefilter of the last run: [0] 1 if it ran, [1] K1t device time in ms, [2] tier-1 window +
  * tier-2 exact FP32 re-scoring time in ms, [3] candidates re-scored in FP32 (all units), [4] largest observed
- * |d_tc^2 - d_fp32^2| / Rmax^2 over them, [5] the window prefilter_abs in force.                              */
+ * |d_tc^2 - d_fp32^2| / Rmax^2 over them, [5] the window prefilter_abs in force.
+ * When no tier ran ([0] == 0) and the dense sweep ran the early-break kernel K1e: [3] pair distances it evaluated,
+ * [4] candidates it scored (divide for pairs per candidate; K1 evaluates N M).                                */
 int mmrs_sweep_prefilter_info(mmrs_ctx* ctx, double out[6]);
 
 /* Reference-arithmetic f64 cost of an explicit list of angles for one unit

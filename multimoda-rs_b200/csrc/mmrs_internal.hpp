@@ -75,6 +75,9 @@ struct mmrs_ctx {
         size_t smem = 0;
         size_t work_begin = 0, work_count = 0;  // range of h_work / d_work
         long long cost = 0;                     // padded pair evaluations per candidate, summed over the class
+        size_t smem_eb = 0;                     // shared memory of a K1e CTA (k_sweep_eb) of this class
+        bool eb = false;                        // the dense sweep of this class runs K1e (decided per grid set)
+        long long live = 0;                     // candidates of this class swept by this rank
     };
     std::vector<SweepClass> classes;
     std::vector<int> class_of_unit;
@@ -126,6 +129,12 @@ struct mmrs_ctx {
     std::vector<mmrs::UnitDesc> h_units_lb;   // [2 U]: pass A (test rows) then pass B (reference rows)
     std::vector<mmrs::WorkItem> h_work_lb;
     mmrs::DevBuf d_units_lb, d_lay_lb, d_work_lb;
+
+    // early-break dense sweep K1e (k_sweep_eb, sweep_kernels.cuh)
+    int eb_env = -1;            // MMRS_EARLY_BREAK at upload: -1 unset (K1e where 3 CTAs fit per SM), 0 K1 everywhere, 1 K1e wherever it fits
+    bool eb_ran = false;
+    long long eb_cands = 0;     // candidates K1e scored in the last run
+    mmrs::DevBuf d_eb_pairs;    // pair distances K1e evaluated in the last run (one 64-bit counter)
 
     // partition of every batched sweep across ranks (mmrs_ctx_comm_init / mmrs_ctx_set_shard / mmrs_ctx_set_partition)
     int shard_rank = 0, shard_world = 1;

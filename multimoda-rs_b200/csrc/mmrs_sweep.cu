@@ -204,7 +204,7 @@ void mmrs_ctx::free_all() {
     for (DevBuf* b : {&d_test, &d_ref, &d_units, &d_work, &d_lay, &d_cs64, &d_cs32, &d_zero, &d_dist32, &d_key,
                       &d_rmax, &d_sl_base, &d_sl_dist, &d_sl_count, &d_items, &d_nitems, &d_res, &d_tmp, &d_work_tc,
                       &d_work_list, &d_key_tc, &d_l1_items, &d_l1_count, &d_l1_base, &d_l1_n, &d_units_lb, &d_lay_lb,
-                      &d_work_lb, &d_res_all, &d_cnt, &d_bcast, &d_big_rows, &d_exact_scratch}) {
+                      &d_work_lb, &d_res_all, &d_cnt, &d_bcast, &d_big_rows, &d_exact_scratch, &d_eb_pairs}) {
         if (b->p) cudaFree(b->p);
         b->p = nullptr;
         b->cap = 0;
@@ -234,6 +234,12 @@ static int ensure(mmrs_ctx* ctx, DevBuf& b, size_t bytes) {
     } while (0)
 
 constexpr bool kXfDefault = false;   // what mmrs_sweep_opts.prefilter = 0 (auto) resolves to for large batches
+
+// Early-break dense sweep K1e (k_sweep_eb). A warp walks a contiguous run of candidates and carries its hints from one
+// candidate to the next. Measured on B200 (profiles/r03_early_break_bench.json) it beats K1 on every grid tried, from
+// 0.01 deg (7.3x) to 1 deg steps (1.05x) and 41-candidate sweeps (1.9x), so the rule is only that a CTA fits 3 per SM.
+constexpr size_t kEbAutoSmem = 72 * 1024;
+constexpr long long kEbMinRun = 32, kEbMaxRun = 256;   // candidates per warp run
 
 // ---- kernel dispatch over TA ----------------------------------------------------------
 struct ListArgs {  // LIST arguments of k_sweep; all null for the dense sweep
@@ -449,6 +455,9 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
                 ctx->classes.push_back(c);
             }
             ctx->classes[k].smem = std::max(ctx->classes[k].smem, smem);
+            if (!big)   // K1e: the same staging image plus, per warp, A' and the row / column hints
+                ctx->classes[k].smem_eb = std::max(ctx->classes[k].smem_eb, 16 + (size_t)(a_elems + b_elems + nb_elems + t_elems) * 16 +
+                                                                              (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m));
             ctx->classes[k].cost += (long long)d.n_chunks * 32 * d.ta * d.m;
             ctx->class_of_unit[u] = k;
         }
@@ -664,9 +673,18 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             }
         }
     }
+    for (auto& cl : ctx->classes) cl.live = 0;
     for (int64_t u = 0; u < U; ++u)
-        if (!units[u].flags) live += units[u].c_hi - units[u].c_lo;
-    // work list: one CTA = one unit x one tile of candidates (8 warps, one candidate per warp per pass)
+        if (!units[u].flags) {
+            live += units[u].c_hi - units[u].c_lo;
+            ctx->classes[ctx->class_of_unit[u]].live += units[u].c_hi - units[u].c_lo;
+        }
+    // K1e per size class (MMRS_EARLY_BREAK: 0 = K1 everywhere, 1 = K1e wherever its shared memory fits). A class beyond
+    // the per-warp A' and hints (sets above ~1 000 points, the chunked 2 020-point units among them) keeps K1.
+    for (auto& cl : ctx->classes)
+        cl.eb = ctx->eb_env != 0 && !cl.big && cl.smem_eb <= (ctx->eb_env == 1 ? (size_t)kMaxDynSmem : kEbAutoSmem);
+    // work list: one CTA = one unit x one tile of candidates (8 warps, one candidate per warp per pass; K1e: one
+    // contiguous run per warp, as long as the batch still gives ~4 waves of 3 CTAs per SM)
     {
         const long long slots = (long long)ctx->n_sm * 2 * 4;  // CTAs for ~4 waves at 2 CTAs/SM
         long long per_warp = (live + slots * kWarpsPerCta - 1) / (slots * kWarpsPerCta);
@@ -679,11 +697,14 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         for (size_t k = 0; k < ctx->classes.size(); ++k) {   // one contiguous range of the work list per size class
             auto& cl = ctx->classes[k];
             cl.work_begin = ctx->h_work.size();
+            const long long eb_slots = (long long)ctx->n_sm * 3 * 4 * kWarpsPerCta;
+            const int tile_k = cl.eb ? (int)(kWarpsPerCta * std::max(kEbMinRun, std::min(kEbMaxRun, (cl.live + eb_slots - 1) / eb_slots)))
+                                     : tile;
             for (int64_t u = 0; u < U; ++u) {
                 const UnitDesc& d = units[u];
                 if (d.flags || ctx->class_of_unit[u] != (int)k) continue;
-                for (int c0 = d.c_lo; c0 < d.c_hi; c0 += tile)
-                    ctx->h_work.push_back(WorkItem{(int)u, c0, std::min(tile, d.c_hi - c0), 0});
+                for (int c0 = d.c_lo; c0 < d.c_hi; c0 += tile_k)
+                    ctx->h_work.push_back(WorkItem{(int)u, c0, std::min(tile_k, d.c_hi - c0), 0});
             }
             cl.work_count = ctx->h_work.size() - cl.work_begin;
         }
@@ -833,6 +854,10 @@ extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const
     ctx->ran = false;
     ctx->n_units = b->n_units;
     ctx->mode = b->mode;
+    {
+        const char* env = std::getenv("MMRS_EARLY_BREAK");   // A/B runs and tests: 0 = K1 everywhere, 1 = K1e wherever it fits
+        ctx->eb_env = (env && *env) ? (*env == '0' ? 0 : 1) : -1;
+    }
     ctx->opt_rel = (o && o->shortlist_rel > 0) ? o->shortlist_rel : 2e-6;
     ctx->opt_abs = (o && o->shortlist_abs > 0) ? o->shortlist_abs : 2e-6;
     ctx->cap = (o && o->shortlist_cap > 0) ? o->shortlist_cap : 64;
@@ -956,6 +981,8 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     const bool tc = ctx->use_tc && !ctx->h_work_tc.empty();
     const bool xf = !tc && ctx->use_xf && !ctx->h_work.empty();
     const bool prune = !tc && !xf && ctx->use_prune && !ctx->h_work_lb.empty();
+    ctx->eb_ran = false;
+    ctx->eb_cands = 0;
     ctx->xf_ran = xf;
     ctx->tc_ran = tc || xf;
     ctx->prune_ran = prune;
@@ -1131,6 +1158,22 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
                                                       (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
                                                       (float*)ctx->d_big_rows.p, ctx->big_scratch_per_warp);
                 CUDA_TRY(ctx, cudaGetLastError());
+                ctx->launches += 1;
+                continue;
+            }
+            if (cl.eb) {
+                if (!ctx->eb_ran) {
+                    ENSURE(ctx->d_eb_pairs, 8);
+                    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
+                    ctx->eb_ran = true;
+                }
+                CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb));
+                k_sweep_eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(
+                    units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
+                    (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
+                    (unsigned long long*)ctx->d_eb_pairs.p);
+                CUDA_TRY(ctx, cudaGetLastError());
+                ctx->eb_cands += cl.live;
                 ctx->launches += 1;
                 continue;
             }
@@ -1451,6 +1494,15 @@ extern "C" int mmrs_sweep_prefilter_info(mmrs_ctx* ctx, double out[6]) {
     if (!ctx->ran) return set_err(ctx, MMRS_ERR_STATE, "mmrs_sweep_prefilter_info: nothing has been run");
     for (int i = 0; i < 6; ++i) out[i] = 0.0;
     out[5] = ctx->tc_abs;
+    if (!ctx->tc_ran && !ctx->prune_ran && ctx->eb_ran) {   // the dense sweep ran K1e: [3] pairs evaluated, [4] candidates
+        ENTER_DEVICE(ctx);
+        CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev[3]));
+        unsigned long long pairs = 0;
+        CUDA_TRY(ctx, cudaMemcpy(&pairs, ctx->d_eb_pairs.p, 8, cudaMemcpyDeviceToHost));
+        out[3] = (double)pairs;
+        out[4] = (double)ctx->eb_cands;
+        return MMRS_OK;
+    }
     if ((!ctx->tc_ran && !ctx->prune_ran) || ctx->n_units == 0) return MMRS_OK;
     ENTER_DEVICE(ctx);
     CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev[3]));

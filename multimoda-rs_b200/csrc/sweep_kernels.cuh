@@ -10,6 +10,8 @@
 //                     f32x2 arithmetic (FADD2/FMUL2/FFMA2), 3-input FMNMX and
 //                     warp REDUX; fused per-unit arg-min on a packed
 //                     (distance, index) 64-bit key with atomicMin.
+//   K1e k_sweep_eb    the dense sweep with early-break directed passes: every candidate's FP32 distance,
+//                     bit-identical to K1, from ~1 % of the pair distances (default wherever it fits)
 //   K2  k_shortlist   candidates within the FP32 error window of the minimum
 //   K3  k_exact       the reference's f64 arithmetic, literally, on those
 //   K4  k_select      leftmost f64 arg-min + tie count per unit
@@ -543,6 +545,212 @@ __global__ void __launch_bounds__(kThreads, 2)
     if (g_pos >= g_hi) break;
     __syncthreads();  // every warp is done with the staged unit and s_key before the next run re-stages
     }
+}
+
+// =============================================================================
+// K1e: the dense sweep with EARLY-BREAK directed passes. Same work items, staging image (one TMA bulk copy) and outputs
+// (dist32, the packed (distance, index) key) as K1, but a candidate no longer costs all N M pair distances:
+//     H^2 = max( max_a min_b d^2 , max_b min_a d^2 ),
+// and once L, an exactly computed row or column minimum of THIS candidate, is known, a row that meets one b with
+// d^2 <= L cannot raise the maximum and stops there. Per warp, over a contiguous run of the tile's candidates:
+//   rotate  the N test points into a per-warp shared-memory row A'[N];
+//   seed    L = max(exact minimum of row ra, exact minimum of column cb), where ra / cb defined the previous
+//           candidate's maximum (the warp's first candidate: the points farthest from the rotation centre);
+//   rows    lane l takes rows l, l + 32, ...: kEbTries positions of a zig-zag scan around the row's hint (the index
+//           where it stopped for the previous candidate); rows still open are then finished one at a time by the
+//           whole warp (32 positions per round, one REDUX.MIN), stopping at the first round whose minimum is <= L;
+//           a row that runs to its end has an exact minimum > L, which becomes L;
+//   columns the same with the reference points as rows and A' as the set.
+// Every pair distance is K1's operation sequence (x' = fma(y, -s, x c), y' = fma(x, s, y c), d^2 = fma(dx, dx, dy dy)),
+// pinned against contraction; the column pass reads the same A' (|a - b|^2 and |b - a|^2 round alike). L only ever
+// holds exact minima of the current candidate: earlier candidates decide the ORDER of the scans, never a threshold. So
+// the final L is max over every row and column minimum, and dist32 is bit-identical to K1's. An overflowed d^2 = inf
+// never passes <= L: that row scans to its exact minimum, as K1 computes it.
+// =============================================================================
+constexpr int kEbTries = 4;   // zig-zag positions a lane tries on its own before the warp takes its row over
+
+// per-warp shared memory of K1e: A'[n] (float2), then the row hints [n] and column hints [m] (16-bit indices)
+__host__ __device__ constexpr int eb_warp_bytes(int n, int m) { return (8 * n + 2 * (n + m) + 15) & ~15; }
+
+__device__ __forceinline__ float eb_d2(float2 a, float2 b) {
+    const float dx = __fsub_rn(a.x, b.x), dy = __fsub_rn(a.y, b.y);
+    return __fmaf_rn(dx, dx, __fmul_rn(dy, dy));
+}
+// t-th position (t < n: every index exactly once) of a scan over n points that starts at h and zig-zags outward:
+// h, h + 1, h - 1, h + 2, ... modulo n (contours are closed)
+__device__ __forceinline__ int eb_zig(int h, int t, int n) {
+    int j = h + ((t & 1) ? (t + 1) >> 1 : -(t >> 1));
+    j = j < 0 ? j + n : j;
+    return j >= n ? j - n : j;
+}
+// Minimum of d^2(a, P[j]) over the n points of P, the whole warp together along the zig-zag from h (call it with the
+// full warp, warp-uniform arguments). early: stop after the first round whose running minimum is <= L. Returns the bit
+// pattern of the minimum found (the exact minimum whenever it is > L) and, in arg, where it was found.
+__device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a, int h, unsigned L, bool early, int lane,
+                                                int& arg, unsigned& pairs) {
+    unsigned best = ~0u, m = ~0u;
+    int bj = h;
+    for (int t0 = 0; t0 < n; t0 += 32) {
+        const int t = t0 + lane;
+        if (t < n) {
+            const int j = eb_zig(h, t, n);
+            const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+            if (d < best) best = d, bj = j;
+            ++pairs;
+        }
+        m = __reduce_min_sync(0xffffffffu, best);
+        if (early && m <= L) break;
+    }
+    arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
+    return m;
+}
+// Index of the largest v over the warp (v: non-negative float bits; ties -> lowest lane).
+__device__ __forceinline__ int eb_warp_argmax(unsigned v, int idx) {
+    const unsigned m = __reduce_max_sync(0xffffffffu, v);
+    return __shfl_sync(0xffffffffu, idx, __ffs(__ballot_sync(0xffffffffu, v == m)) - 1);
+}
+
+__global__ void __launch_bounds__(kThreads, 3)
+    k_sweep_eb(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
+               const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
+               unsigned long long* __restrict__ pairs_out) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
+    unsigned long long* s_key = reinterpret_cast<unsigned long long*>(smem_raw + 8);
+    float4* sA = reinterpret_cast<float4*>(smem_raw + 16);
+    const WorkItem w = work[blockIdx.x];
+    const UnitDesc ud = units[w.unit];
+    const int lane = threadIdx.x & 31, wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+    const int TA = ud.ta, S = (TA + 1) / 2, N = ud.n, M = ud.m, n_main = N - ud.n_tail;
+    const int a_elems = ud.n_chunks * S * 32;
+    const int b_elems = ud.n_tail > 0 ? 16 * (TA + 1) : ud.m_pairs;
+    const int nb_elems = (b_elems + 1) / 2, t_elems = (ud.n_tail + 1) / 2;
+    const float4* sB4 = sA + a_elems;
+    const float2* sB = reinterpret_cast<const float2*>(sB4);                              // reference point j
+    const float2* sT = reinterpret_cast<const float2*>(sB4 + b_elems + nb_elems);         // tail point t
+    unsigned char* my = reinterpret_cast<unsigned char*>(sA + a_elems + b_elems + nb_elems + t_elems) + wid * eb_warp_bytes(N, M);
+    float2* sR = reinterpret_cast<float2*>(my);                                           // A': rotated test points
+    unsigned short* hr = reinterpret_cast<unsigned short*>(sR + N);                       // row hints
+    unsigned short* hc = hr + N;                                                          // column hints
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        *s_key = ~0ull;
+        const uint32_t bytes = (uint32_t)(a_elems + b_elems + nb_elems + t_elems) * 16u;
+        mbar_expect_tx(bar, bytes);
+        tma_bulk_g2s(sA, lay + ud.lay_off, bytes, bar);
+    }
+    __syncthreads();
+    mbar_wait(bar, 0);
+
+    // test point i of the staging image (K0's layout: register slots, then the exact-tiling tail block)
+    auto test_pt = [&](int i) -> float2 {
+        if (i >= n_main) return sT[i - n_main];
+        const int c = i / (32 * TA), r = i - c * 32 * TA;
+        const float4 v = sA[(c * S + (r >> 6)) * 32 + (r & 31)];
+        return (r & 32) ? make_float2(v.y, v.w) : make_float2(v.x, v.z);
+    };
+    // this warp's contiguous run of candidates: neighbouring angles keep the hints valid
+    const int per = (w.count + kWarpsPerCta - 1) / kWarpsPerCta;
+    const int c_begin = w.begin + min(w.count, wid * per), c_end = w.begin + min(w.count, (wid + 1) * per);
+    unsigned long long best = ~0ull;
+    unsigned pairs = 0;
+    if (c_begin < c_end) {
+        // first candidate: hints on the index diagonal, seeds at the points farthest from the rotation centre
+        unsigned far_a = 0u, far_b = 0u;
+        int ia = 0, ib = 0;
+        for (int i = lane; i < N; i += 32) {
+            const float2 p = test_pt(i);
+            const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
+            if (r2 > far_a) far_a = r2, ia = i;
+            hr[i] = (unsigned short)(((long long)i * M) / N);
+        }
+        for (int j = lane; j < M; j += 32) {
+            const float2 p = sB[j];
+            const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
+            if (r2 > far_b) far_b = r2, ib = j;
+            hc[j] = (unsigned short)(((long long)j * N) / M);
+        }
+        int ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
+        for (int c = c_begin; c < c_end; ++c) {
+            const float2 cs = __ldg(&cs32[ud.cand_off + c]);
+            __syncwarp();   // the previous candidate is done with A' and the hints
+            for (int i = lane; i < N; i += 32) {
+                const float2 p = test_pt(i);
+                sR[i] = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
+            }
+            __syncwarp();
+            int arg;
+            unsigned L = eb_warp_min(sB, M, sR[ra], hr[ra], 0u, false, lane, arg, pairs);
+            const int h_ra = arg;
+            const unsigned lc = eb_warp_min(sR, N, sB[cb], hc[cb], 0u, false, lane, arg, pairs);
+            __syncwarp();
+            if (lane == 0) hr[ra] = (unsigned short)h_ra, hc[cb] = (unsigned short)arg;
+            L = max(L, lc);
+            __syncwarp();
+            // rows: test point i against the reference points
+            for (int g = 0; g < N; g += 32) {
+                const int i = g + lane;
+                bool open = false;
+                if (i < N) {
+                    const float2 a = sR[i];
+                    const int h = hr[i];
+                    open = true;
+                    for (int t = 0; t < kEbTries && t < M; ++t) {
+                        const int j = eb_zig(h, t, M);
+                        ++pairs;
+                        if (__float_as_uint(eb_d2(a, sB[j])) <= L) {
+                            hr[i] = (unsigned short)j;
+                            open = false;
+                            break;
+                        }
+                    }
+                }
+                for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
+                    const int ii = g + __ffs(open_mask) - 1;
+                    const unsigned mn = eb_warp_min(sB, M, sR[ii], hr[ii], L, true, lane, arg, pairs);
+                    if (mn > L) L = mn, ra = ii;
+                    __syncwarp();
+                    if (lane == 0) hr[ii] = (unsigned short)arg;
+                }
+            }
+            // columns: reference point j against A'
+            for (int g = 0; g < M; g += 32) {
+                const int j = g + lane;
+                bool open = false;
+                if (j < M) {
+                    const float2 b = sB[j];
+                    const int h = hc[j];
+                    open = true;
+                    for (int t = 0; t < kEbTries && t < N; ++t) {
+                        const int i = eb_zig(h, t, N);
+                        ++pairs;
+                        if (__float_as_uint(eb_d2(sR[i], b)) <= L) {
+                            hc[j] = (unsigned short)i;
+                            open = false;
+                            break;
+                        }
+                    }
+                }
+                for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
+                    const int jj = g + __ffs(open_mask) - 1;
+                    const unsigned mn = eb_warp_min(sR, N, sB[jj], hc[jj], L, true, lane, arg, pairs);
+                    if (mn > L) L = mn, cb = jj;
+                    __syncwarp();
+                    if (lane == 0) hc[jj] = (unsigned short)arg;
+                }
+            }
+            const float d = sqrtf(__uint_as_float(L));
+            if (lane == 0) {
+                dist32[ud.dist_off + c] = d;
+                best = min(best, ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)c);
+            }
+        }
+    }
+    const unsigned warp_pairs = __reduce_add_sync(0xffffffffu, pairs);
+    if (lane == 0 && pairs_out && warp_pairs) atomicAdd(pairs_out, (unsigned long long)warp_pairs);
+    if (lane == 0 && best != ~0ull) atomicMin(s_key, best);
+    __syncthreads();
+    if (threadIdx.x == 0 && *s_key != ~0ull) atomicMin(&key[w.unit], *s_key);
 }
 
 // =============================================================================

@@ -264,8 +264,11 @@ class Context:
         o = (C.c_double * 6)()
         lib().mmrs_sweep_prefilter_info.argtypes = [C.c_void_p, c_dp]
         self._check(lib().mmrs_sweep_prefilter_info(self._p, o))
-        return dict(ran=bool(o[0]), kind={0: None, 1: "tensor-core prefilter", 2: "lower-bound pruning", 3: "expanded-form tier"}[int(o[0])],
-                    tc_ms=o[1], rescore_ms=o[2], rescored=int(o[3]), max_err=o[4], window=o[5])
+        ran = bool(o[0])
+        # when no tier ran, [3] / [4] count the early-break dense sweep (K1e): pair distances evaluated, candidates scored
+        return dict(ran=ran, kind={0: None, 1: "tensor-core prefilter", 2: "lower-bound pruning", 3: "expanded-form tier"}[int(o[0])],
+                    tc_ms=o[1], rescore_ms=o[2], rescored=int(o[3]) if ran else 0, max_err=o[4] if ran else 0.0, window=o[5],
+                    eb_pairs=0 if ran else int(o[3]), eb_candidates=0 if ran else int(o[4]))
 
     def eval_exact(self, test_xy, ref_xy, centre, mode, angles):
         t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
