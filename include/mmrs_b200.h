@@ -182,9 +182,11 @@ int mmrs_sweep_download(mmrs_ctx* ctx, mmrs_unit_result* out);
 int mmrs_sweep_plan(mmrs_ctx* ctx, int64_t plan_out[5]);
 
 /* Diagnostics on the last run (valid until the next upload).                 */
-/* FP32 distance of every candidate of `unit` (needs opts.keep_dist32).       */
+/* FP32 distance of every candidate of `unit` (needs opts.keep_dist32). After a
+ * rigid run, in flattened candidate order c = i*T + j (see mmrs_tgrid).      */
 int mmrs_sweep_get_dist32(mmrs_ctx* ctx, int64_t unit, float* out, int64_t cap);
-/* Rechecked candidates of `unit`: indices and their f64 distances.           */
+/* Rechecked candidates of `unit`: indices and their f64 distances (flattened
+ * candidate indices c = i*T + j after a rigid run).                          */
 int mmrs_sweep_get_shortlist(mmrs_ctx* ctx, int64_t unit, int64_t* idx_out, double* dist_out, int32_t cap,
                              int32_t* n_out);
 /* Device time of the last run in ms: [0] FP32 sweep kernel, [1] shortlist,
@@ -212,6 +214,59 @@ int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const 
 /* Pure-FFMA FP32 throughput probe (denominator check for the roofline): runs
  * `iters` dependent FFMA chains on every SM, returns achieved TFLOP/s.        */
 int mmrs_fp32_probe(mmrs_ctx* ctx, int32_t iters, double* tflops_out);
+
+/* ---- rigid candidates: rotation grid x translation grid (opt-in) -------------------------------------------
+ * Searches the best rigid transform (theta, tx, ty) instead of the best theta about a fixed offset. The reference
+ * has no counterpart (it always aligns centroids, align_within.rs:84-90, align_between.rs:33-40); the semantics
+ * below are this library's own and are restated by the test oracle.
+ *
+ * Translation grid: T = (2 half_n + 1)^2 offsets; translation j = jy (2 half_n + 1) + jx, jx, jy in [0, 2 half_n],
+ *   tx = t0x + (double)(jx - half_n) * step,   ty = t0y + (double)(jy - half_n) * step   (host f64, as written).
+ * Candidate c = i T + j: angle i of the unit's mmrs_grid, translation j of its mmrs_tgrid. With half_n = 0 and
+ * t0 = (0, 0), c == i.
+ * Cost (f64): the rotation of the batch's mode (0 / 1, same operation order, same angle == 0.0 identity in mode 0,
+ *   same host cos / sin), then x' = rx + tx, y' = ry + ty (one rounding each; + 0.0 is exact, so a zero translation
+ *   gives the rotation-only cost bit for bit), then hausdorff_distance(reference, transformed).
+ * Selection: leftmost arg-min over c (strict <): ties go to the lowest angle index, then the lowest jy, then jx.
+ * n_ties: 1 + rechecked candidates within tie_margin * max(1, R_eff) whose TRANSFORM differs from the winner's
+ *   (a different (cos, sin) or a different (tx, ty)); R_eff = Rmax + max_j |t_j| replaces Rmax in the FP32
+ *   shortlist window as well.
+ * Execution: the dense FP32 sweep on this context's device alone (no lower-bound pruning, no prefilter tier, no
+ * partition across ranks: a bound communicator or shard transport is not used). opts.prune > 0 or
+ * opts.prefilter 2 / 3 is an error; the context's prune default is ignored.
+ * Edge cases: degenerate angle grid -> best_idx = -1, best_angle = fallback, angle_idx = trans_idx = -1,
+ *   (best_tx, best_ty) = (t0x, t0y); an empty set -> every candidate costs 0, candidate 0 wins; non-finite points
+ *   are dropped as in the rotation-only sweep. half_n < 0, a non-finite t0 / step, step <= 0 with half_n > 0, or
+ *   more than INT32_MAX candidates (angles x translations) in one unit is MMRS_ERR_ARG.                     */
+typedef struct mmrs_tgrid {
+    double t0x, t0y; /* centre of the grid                 */
+    double step;     /* spacing (same unit as the points)  */
+    int32_t half_n;  /* 2 half_n + 1 offsets per axis      */
+} mmrs_tgrid;
+
+typedef struct mmrs_rigid_result {
+    mmrs_unit_result r;  /* r.best_idx = flattened candidate index, r.best_angle = its (wrapped) angle */
+    int64_t angle_idx;   /* best_idx / T (-1 if degenerate)                                          */
+    int32_t trans_idx;   /* best_idx % T (-1 if degenerate)                                          */
+    int32_t pad;
+    double best_tx, best_ty;
+} mmrs_rigid_result;
+
+/* mmrs_sweep_batched with a translation grid per unit: `tgrid_of_unit` == NULL -> every unit uses tgrids[0]. */
+int mmrs_rigid_sweep_batched(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_tgrid* tgrids, int64_t n_tgrids,
+                             const int32_t* tgrid_of_unit, const mmrs_sweep_opts* opts, mmrs_rigid_result* out);
+/* The same in steps: upload, regrid (new angle and translation grids on the uploaded points), mmrs_sweep_run,
+ * download. mmrs_sweep_download after a rigid run returns the mmrs_unit_result part.                          */
+int mmrs_rigid_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_tgrid* tgrids, int64_t n_tgrids,
+                            const int32_t* tgrid_of_unit, const mmrs_sweep_opts* opts);
+int mmrs_rigid_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
+                            const mmrs_tgrid* tgrids, int64_t n_tgrids, const int32_t* tgrid_of_unit, double tie_margin);
+int mmrs_rigid_sweep_download(mmrs_ctx* ctx, mmrs_rigid_result* out);
+/* f64 cost of explicit rigid candidates k = (angles[k], txy[2k], txy[2k+1]) for one unit (mmrs_eval_exact plus the
+ * translation).                                                                                                */
+int mmrs_eval_exact_rigid(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
+                          double cx, double cy, int32_t mode, const double* angles, const double* txy, int64_t n_cand,
+                          double* dist_out);
 
 /* ---- geometry blob -------------------------------------------------------------
  * Geometries cross the boundary as one f64 stream (u32 ids are exact in f64):

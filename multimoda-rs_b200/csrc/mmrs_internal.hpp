@@ -26,6 +26,9 @@ struct UnitDesc {
     int c_lo, c_hi;               // candidates [c_lo, c_hi) are swept by THIS rank (all of them unless the batch is
                                   // partitioned across ranks: whole units -> empty range on the other ranks, candidate
                                   // axis -> one contiguous sub-range per rank, global indices kept)
+    long long t_off;              // rigid runs: offset of this unit's translation grid in the t64 / t32 tables
+    int n_trans;                  // translations per angle (1 without a translation grid): candidate c = i n_trans + j
+    int t_pad;
 };
 constexpr int kFlagRemote = 0x400;  // internal UnitDesc.flags bit: another rank owns this unit (never leaves the library)
 
@@ -135,6 +138,14 @@ struct mmrs_ctx {
     bool eb_ran = false;
     long long eb_cands = 0;     // candidates K1e scored in the last run
     mmrs::DevBuf d_eb_pairs;    // pair distances K1e evaluated in the last run (one 64-bit counter)
+
+    // rigid candidates (mmrs_rigid_sweep_*): a translation grid per unit on top of its angle grid
+    bool rigid = false;                     // the uploaded grids carry translation grids
+    std::vector<mmrs_tgrid> tgrids;
+    std::vector<int> tgrid_of_unit;
+    std::vector<double> h_t;                // (tx, ty) of every translation of every translation grid
+    std::vector<double> h_tmax;             // per unit: largest |t| of its translation grid
+    mmrs::DevBuf d_t64, d_t32, d_tmax, d_reff;   // translation tables; per unit R_eff = Rmax + max |t| (float bits)
 
     // partition of every batched sweep across ranks (mmrs_ctx_comm_init / mmrs_ctx_set_shard / mmrs_ctx_set_partition)
     int shard_rank = 0, shard_world = 1;

@@ -266,22 +266,35 @@ static cudaError_t raise_smem_once(K kernel, std::once_flag& once, cudaError_t& 
         return raise_smem_once(kernel, once, result);            \
     }())
 
-template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF>
+template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false>
 static void launch_sweep_k(int grid, size_t smem, cudaStream_t s, const UnitDesc* units, const WorkItem* work,
                            const float4* lay, const float2* cs32, float* dist32, unsigned long long* key,
-                           const ListArgs& l) {
-    RAISE_SMEM((k_sweep<TA, MULTI, LIST, TAILP, XF>));
-    k_sweep<TA, MULTI, LIST, TAILP, XF><<<grid, kThreads, smem, s>>>(units, work, lay, cs32, dist32, key, l.items,
-                                                                     l.n_items, l.cap, l.chunk, l.rmax, l.diag);
+                           const ListArgs& l, const float2* t32 = nullptr) {
+    RAISE_SMEM((k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID>));
+    k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID><<<grid, kThreads, smem, s>>>(units, work, lay, cs32, dist32, key, l.items,
+                                                                            l.n_items, l.cap, l.chunk, l.rmax, l.diag, t32);
 }
 // xf: the expanded-form tier K1x (dense launches only; a list is always re-scored in direct form)
+// t32 != NULL: rigid candidates (dense direct-form launches only)
 template <int TA>
 static void launch_sweep_ta(bool multi, bool tailp, bool xf, int grid, size_t smem, cudaStream_t s, const UnitDesc* units,
                             const WorkItem* work, const float4* lay, const float2* cs32, float* dist32,
-                            unsigned long long* key, const ListArgs* l) {
+                            unsigned long long* key, const ListArgs* l, const float2* t32) {
     const ListArgs none{};
     const ListArgs& la = l ? *l : none;
 #define GO(M, L, T, X) launch_sweep_k<TA, M, L, T, X>(grid, smem, s, units, work, lay, cs32, dist32, key, la)
+#define GO_RIGID(M, T) launch_sweep_k<TA, M, false, T, false, true>(grid, smem, s, units, work, lay, cs32, dist32, key, la, t32)
+    if (t32) {
+        if constexpr (TA % 2 == 0 && TA >= 4) {
+            if (tailp) {
+                GO_RIGID(false, true);
+                return;
+            }
+        }
+        if (multi) GO_RIGID(true, false);
+        else GO_RIGID(false, false);
+        return;
+    }
     if constexpr (TA % 2 == 0 && TA >= 4) {   // exact tiling is instantiated for even register tiles
         if (tailp) {
             if (l) GO(false, true, true, false);
@@ -301,14 +314,15 @@ static void launch_sweep_ta(bool multi, bool tailp, bool xf, int grid, size_t sm
         else GO(false, false, false, false);
     }
 #undef GO
+#undef GO_RIGID
 }
 static bool launch_sweep(int TA, bool multi, bool tailp, int grid, size_t smem, cudaStream_t s, const UnitDesc* units,
                          const WorkItem* work, const float4* lay, const float2* cs32, float* dist32,
-                         unsigned long long* key, const ListArgs* l = nullptr, bool xf = false) {
+                         unsigned long long* key, const ListArgs* l = nullptr, bool xf = false, const float2* t32 = nullptr) {
     switch (TA) {
-#define CASE(T)                                                                                   \
-    case T:                                                                                       \
-        launch_sweep_ta<T>(multi, tailp, xf, grid, smem, s, units, work, lay, cs32, dist32, key, l); \
+#define CASE(T)                                                                                        \
+    case T:                                                                                            \
+        launch_sweep_ta<T>(multi, tailp, xf, grid, smem, s, units, work, lay, cs32, dist32, key, l, t32); \
         return true;
         CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9) CASE(10) CASE(11) CASE(12) CASE(13) CASE(14)
             CASE(15) CASE(16) CASE(17) CASE(18)
@@ -490,7 +504,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
         ctx->lb_R = biggest >= 1024 ? 128 : 32;  // rows per lower-bound pass: k_lb<1,8> or k_lb<4,2>
         // the bound tier's staging images are only built for a batch that may use it (opts / context default / MMRS_PRUNE)
         const char* prune_env = std::getenv("MMRS_PRUNE");
-        const bool may_prune = (prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1;
+        const bool may_prune = !ctx->rigid && ((prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1);
         ctx->lb_shape_ok = ok && biggest > 0 && may_prune;
         ctx->h_units_lb.assign(2 * (size_t)U, UnitDesc{});
         long long off = 0;
@@ -558,8 +572,28 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
     return MMRS_OK;
 }
 
+// Translation grid checks of mmrs_tgrid (include/mmrs_b200.h).
+static int check_tgrid(mmrs_ctx* ctx, const mmrs_tgrid& t) {
+    if (t.half_n < 0) return set_err(ctx, MMRS_ERR_ARG, "translation grid: half_n must be >= 0");
+    if (!std::isfinite(t.t0x) || !std::isfinite(t.t0y) || !std::isfinite(t.step))
+        return set_err(ctx, MMRS_ERR_ARG, "translation grid: t0 and step must be finite");
+    if (t.half_n > 0 && !(t.step > 0.0)) return set_err(ctx, MMRS_ERR_ARG, "translation grid: step must be > 0 when half_n > 0");
+    if (t.half_n > 23169) return set_err(ctx, MMRS_ERR_ARG, "translation grid: more than INT32_MAX translations");
+    return MMRS_OK;
+}
+// Translation j = jy (2 half_n + 1) + jx of a translation grid, evaluated in f64 exactly as the header states.
+static inline void tgrid_offset(const mmrs_tgrid& t, int64_t j, double* tx, double* ty) {
+    const int64_t w = 2 * (int64_t)t.half_n + 1, jy = j / w, jx = j - jy * w;
+    *tx = t.t0x + (double)(jx - t.half_n) * t.step;
+    *ty = t.t0y + (double)(jy - t.half_n) * t.step;
+}
+
 // Grid part: candidate tables (host glibc cos/sin), per-unit candidate ranges, the CTA work list.
-static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit) {
+// tgrids == NULL: rotation-only candidates (every unit has one translation, none applied). Otherwise rigid candidates:
+// unit u sweeps grid x tgrids[tgrid_of_unit[u]], candidate c = i T + j (angle i, translation j), densely and on this
+// rank alone (no pruning / prefilter tier, no partition).
+static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
+                       const mmrs_tgrid* tgrids = nullptr, int64_t n_tgrids = 0, const int32_t* tgrid_of_unit = nullptr) {
     const int64_t U = ctx->n_units;
     ctx->grids.assign(grids, grids + n_grids);
     ctx->grid_of_unit.resize(U);
@@ -567,6 +601,44 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         const int g = grid_of_unit ? grid_of_unit[u] : 0;
         if (g < 0 || g >= n_grids) return set_err(ctx, MMRS_ERR_ARG, "grid_of_unit out of range");
         ctx->grid_of_unit[u] = g;
+    }
+    ctx->rigid = tgrids != nullptr;
+    std::vector<long long> tgrid_off(1, 0);
+    if (ctx->rigid) {
+        if (n_tgrids < 1) return set_err(ctx, MMRS_ERR_ARG, "rigid sweep: n_tgrids must be >= 1");
+        ctx->tgrids.assign(tgrids, tgrids + n_tgrids);
+        ctx->tgrid_of_unit.resize(U);
+        for (int64_t u = 0; u < U; ++u) {
+            const int g = tgrid_of_unit ? tgrid_of_unit[u] : 0;
+            if (g < 0 || g >= n_tgrids) return set_err(ctx, MMRS_ERR_ARG, "tgrid_of_unit out of range");
+            ctx->tgrid_of_unit[u] = g;
+        }
+        tgrid_off.assign(n_tgrids + 1, 0);
+        for (int64_t g = 0; g < n_tgrids; ++g) {
+            if (int rc = check_tgrid(ctx, tgrids[g])) return rc;
+            const long long w = 2LL * tgrids[g].half_n + 1;
+            tgrid_off[g + 1] = tgrid_off[g] + w * w;
+        }
+        for (int64_t u = 0; u < U; ++u) {
+            const mmrs_grid& gr = grids[ctx->grid_of_unit[u]];
+            const long long T = tgrid_off[ctx->tgrid_of_unit[u] + 1] - tgrid_off[ctx->tgrid_of_unit[u]];
+            if (!gr.degenerate && (double)gr.n_cand * (double)T > 2147483646.0)
+                return set_err(ctx, MMRS_ERR_ARG,
+                               "rigid sweep: angles x translations of unit " + std::to_string(u) + " exceed INT32_MAX candidates");
+        }
+        ctx->h_t.resize(2 * (size_t)tgrid_off[n_tgrids]);
+        std::vector<double> tmax_of_grid(n_tgrids, 0.0);
+        for (int64_t g = 0; g < n_tgrids; ++g)
+            for (long long j = 0; j < tgrid_off[g + 1] - tgrid_off[g]; ++j) {
+                double* t = &ctx->h_t[2 * (tgrid_off[g] + j)];
+                tgrid_offset(tgrids[g], j, &t[0], &t[1]);
+                tmax_of_grid[g] = std::max(tmax_of_grid[g], std::hypot(t[0], t[1]));
+            }
+        ctx->h_tmax.resize(U);
+        for (int64_t u = 0; u < U; ++u) ctx->h_tmax[u] = tmax_of_grid[ctx->tgrid_of_unit[u]];
+    } else {
+        ctx->tgrids.clear();
+        ctx->tgrid_of_unit.clear();
     }
     // cos/sin tables: HOST glibc (bit-identical to Rust's f64::sin/cos), one per grid.
     std::vector<long long> grid_off(n_grids + 1, 0);
@@ -607,7 +679,9 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         UnitDesc& d = units[u];
         const mmrs_grid& gr = grids[ctx->grid_of_unit[u]];
         d.cand_off = grid_off[ctx->grid_of_unit[u]];
-        d.n_cand = gr.degenerate ? 0 : (int)gr.n_cand;
+        d.t_off = ctx->rigid ? tgrid_off[ctx->tgrid_of_unit[u]] : 0;
+        d.n_trans = ctx->rigid ? (int)(tgrid_off[ctx->tgrid_of_unit[u] + 1] - d.t_off) : 1;
+        d.n_cand = gr.degenerate ? 0 : (int)(gr.n_cand * d.n_trans);
         d.flags = 0;
         if (gr.degenerate) d.flags |= MMRS_FLAG_DEGENERATE;
         if (d.n == 0 || d.m == 0) d.flags |= MMRS_FLAG_EMPTY;
@@ -621,7 +695,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
     {
         const int world = ctx->shard_world, rank = ctx->shard_rank;
         int axis = ctx->opt_partition == 0 ? ctx->part_axis : ctx->opt_partition;
-        if (world <= 1 || (!ctx->comm && !ctx->exchange) || axis < 1 || axis > 2) axis = 0;
+        if (world <= 1 || (!ctx->comm && !ctx->exchange) || axis < 1 || axis > 2 || ctx->rigid) axis = 0;
         if (axis == 1 && ctx->opt_partition == 0) {
             // The context's default axis is a POLICY, decided from the shape of the batch alone (so every rank decides
             // alike): whole units where they balance; candidate sub-ranges where a handful of large units cannot be
@@ -716,11 +790,11 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             if (!d.flags) ++live_units;
         const char* env = std::getenv("MMRS_PREFILTER");  // experiments: 0 = off, 1 = on where the shapes allow
         int mode = ctx->opt_prefilter;
-        if (env && *env) mode = (*env == '0') ? 1 : 2;
+        if (env && *env && !ctx->rigid) mode = (*env == '0') ? 1 : 2;
         // auto (0) currently resolves to the dense FP32 sweep: on B200 the prefilter's per-tile TMEM hand-shakes and
         // the FMNMX-bound epilogue make K1t slower than K1 (17 vs 24 M evaluations/s, DESIGN.md §4).
-        ctx->use_tc = mode == 2 && ctx->tc_shape_ok && live_units > 0 && ctx->part_active != 2;
-        if (mode == 2 && !ctx->use_tc && ctx->opt_prefilter == 2)
+        ctx->use_tc = !ctx->rigid && mode == 2 && ctx->tc_shape_ok && live_units > 0 && ctx->part_active != 2;
+        if (mode == 2 && !ctx->use_tc && ctx->opt_prefilter == 2 && !ctx->rigid)
             return set_err(ctx, MMRS_ERR_ARG,
                            "prefilter required but the batch does not fit the tensor-core operand layout (64 <= points "
                            "per set <= 2048)");
@@ -752,12 +826,12 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
     {
         const char* env = std::getenv("MMRS_XF");   // experiments: 1 = on for every batch that qualifies, 0 = off
         int mode = ctx->opt_prefilter;
-        if (env && *env && mode == 0) mode = (*env == '0') ? 1 : 3;
+        if (env && *env && mode == 0 && !ctx->rigid) mode = (*env == '0') ? 1 : 3;
         if (mode == 0) mode = kXfDefault ? 3 : 1;
         // worth it when the sweep is long enough to pay for two extra launches (window + re-scoring)
         bool any_big = false;
         for (const auto& cl : ctx->classes) any_big = any_big || cl.big;
-        ctx->use_xf = mode == 3 && !ctx->use_tc && !any_big && ctx->part_active != 2 &&
+        ctx->use_xf = !ctx->rigid && mode == 3 && !ctx->use_tc && !any_big && ctx->part_active != 2 &&
                       live >= (ctx->opt_prefilter == 3 ? 1 : (1 << 20));
         if (ctx->use_xf) {
             ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>({(long long)U * 64, 65536LL, live / 32}),
@@ -776,8 +850,8 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             if (!d.flags) ++live_units;
         const char* env = std::getenv("MMRS_PRUNE");
         int mode = ctx->opt_prune;
-        if (env && *env) mode = (*env == '0') ? 0 : 1;
-        ctx->use_prune = mode == 1 && !ctx->use_tc && !ctx->use_xf && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units &&
+        if (env && *env && !ctx->rigid) mode = (*env == '0') ? 0 : 1;
+        ctx->use_prune = !ctx->rigid && mode == 1 && !ctx->use_tc && !ctx->use_xf && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units &&
                          ctx->part_active != 2;
         ctx->h_work_lb.clear();
         if (ctx->use_prune) {
@@ -840,18 +914,53 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         CUDA_TRY(ctx, cudaGetLastError());
         ctx->upload_launches += 1;
     }
+    if (ctx->rigid) {   // translation tables (f64 for K3 / K4, rounded once to FP32 for the sweep) and R_eff per unit
+        const long long n_t = (long long)ctx->h_t.size() / 2;
+        ENSURE(ctx->d_t64, (size_t)n_t * 16);
+        ENSURE(ctx->d_t32, (size_t)n_t * 8);
+        ENSURE(ctx->d_tmax, (size_t)U * 8);
+        ENSURE(ctx->d_reff, (size_t)U * 4);
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_t64.p, ctx->h_t.data(), (size_t)n_t * 16, cudaMemcpyHostToDevice, s));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_tmax.p, ctx->h_tmax.data(), (size_t)U * 8, cudaMemcpyHostToDevice, s));
+        k_cs32<<<(unsigned)((n_t + 255) / 256), 256, 0, s>>>((const double2*)ctx->d_t64.p, (float2*)ctx->d_t32.p, n_t);
+        CUDA_TRY(ctx, cudaGetLastError());
+        k_reff<<<(unsigned)((U + 255) / 256), 256, 0, s>>>((const unsigned*)ctx->d_rmax.p, (const double*)ctx->d_tmax.p,
+                                                           (unsigned*)ctx->d_reff.p, (int)U);
+        CUDA_TRY(ctx, cudaGetLastError());
+        ctx->upload_launches += 2;
+    }
     return MMRS_OK;
 }
 
-extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_sweep_opts* o) {
-    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_sweep_upload: ctx is NULL");
+// Translation grids of a rigid upload / regrid, checked before any device work.
+static int check_tgrids(mmrs_ctx* ctx, const char* fn, int64_t n_units, const mmrs_tgrid* tgrids, int64_t n_tgrids,
+                        const int32_t* tgrid_of_unit) {
+    if (!tgrids || n_tgrids < 1) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad translation grids");
+    for (int64_t g = 0; g < n_tgrids; ++g)
+        if (int rc = check_tgrid(ctx, tgrids[g])) return rc;
+    for (int64_t u = 0; tgrid_of_unit && u < n_units; ++u)
+        if (tgrid_of_unit[u] < 0 || tgrid_of_unit[u] >= n_tgrids) return set_err(ctx, MMRS_ERR_ARG, "tgrid_of_unit out of range");
+    return MMRS_OK;
+}
+
+// Upload of a rotation-only batch (tgrids == NULL) or of a rigid one.
+static int upload_impl(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_sweep_opts* o, const mmrs_tgrid* tgrids,
+                       int64_t n_tgrids, const int32_t* tgrid_of_unit, const char* fn) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (!b || b->n_units < 0 || (b->n_units > 0 && (!b->test_off || !b->ref_off || !b->centre_xy || !b->grids)) ||
         (b->n_grids < 1 && b->n_units > 0))
-        return set_err(ctx, MMRS_ERR_ARG, "mmrs_sweep_upload: bad batch");
-    if (b->mode != 0 && b->mode != 1) return set_err(ctx, MMRS_ERR_ARG, "mmrs_sweep_upload: mode must be 0 or 1");
+        return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad batch");
+    if (b->mode != 0 && b->mode != 1) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": mode must be 0 or 1");
+    if (tgrids || n_tgrids) {
+        if (int rc = check_tgrids(ctx, fn, b->n_units, tgrids, n_tgrids, tgrid_of_unit)) return rc;
+        if (o && o->prune > 0) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prune is not supported with a translation grid");
+        if (o && (o->prefilter == 2 || o->prefilter == 3))
+            return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3 is not supported with a translation grid");
+    }
     ENTER_DEVICE(ctx);
     ctx->ready = false;
     ctx->ran = false;
+    ctx->rigid = tgrids != nullptr;
     ctx->n_units = b->n_units;
     ctx->mode = b->mode;
     {
@@ -877,6 +986,8 @@ extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const
     if (b->n_units == 0) {
         ctx->grids.clear();
         ctx->grid_of_unit.clear();
+        ctx->tgrids.clear();
+        ctx->tgrid_of_unit.clear();
         ctx->h_units.clear();
         ctx->h_work.clear();
         ctx->total_cands = 0;
@@ -885,7 +996,7 @@ extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const
     }
     int rc = upload_points(ctx, b);
     if (rc != MMRS_OK) return rc;
-    rc = apply_grids(ctx, b->grids, b->n_grids, b->grid_of_unit);
+    rc = apply_grids(ctx, b->grids, b->n_grids, b->grid_of_unit, tgrids, n_tgrids, tgrid_of_unit);
     if (rc != MMRS_OK) return rc;
     // The host arrays (and our own staging vectors) must outlive the async copies.
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -893,22 +1004,48 @@ extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const
     return MMRS_OK;
 }
 
-extern "C" int mmrs_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
-                                 double tie_margin) {
-    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_sweep_regrid: ctx is NULL");
-    if (!ctx->ready) return set_err(ctx, MMRS_ERR_STATE, "mmrs_sweep_regrid: no batch uploaded");
+extern "C" int mmrs_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_sweep_opts* o) {
+    return upload_impl(ctx, b, o, nullptr, 0, nullptr, "mmrs_sweep_upload");
+}
+
+extern "C" int mmrs_rigid_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_tgrid* tgrids, int64_t n_tgrids,
+                                       const int32_t* tgrid_of_unit, const mmrs_sweep_opts* o) {
+    if (!tgrids && ctx) return set_err(ctx, MMRS_ERR_ARG, "mmrs_rigid_sweep_upload: bad translation grids");
+    return upload_impl(ctx, b, o, tgrids, n_tgrids, tgrid_of_unit, "mmrs_rigid_sweep_upload");
+}
+
+static int regrid_impl(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
+                       const mmrs_tgrid* tgrids, int64_t n_tgrids, const int32_t* tgrid_of_unit, double tie_margin,
+                       const char* fn) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
+    if (!ctx->ready) return set_err(ctx, MMRS_ERR_STATE, std::string(fn) + ": no batch uploaded");
+    if (tgrids || n_tgrids)
+        if (int rc = check_tgrids(ctx, fn, ctx->n_units, tgrids, n_tgrids, tgrid_of_unit)) return rc;
     if (ctx->n_units == 0) return MMRS_OK;
-    if (!grids || n_grids < 1) return set_err(ctx, MMRS_ERR_ARG, "mmrs_sweep_regrid: bad grids");
+    if (!grids || n_grids < 1) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad grids");
     ENTER_DEVICE(ctx);
     ctx->ready = false;
     ctx->ran = false;
     ctx->tie_margin = tie_margin > 0 ? tie_margin : 0.0;
     ctx->upload_launches = 0;
-    int rc = apply_grids(ctx, grids, n_grids, grid_of_unit);
+    int rc = apply_grids(ctx, grids, n_grids, grid_of_unit, tgrids, n_tgrids, tgrid_of_unit);
     if (rc != MMRS_OK) return rc;
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     ctx->ready = true;
     return MMRS_OK;
+}
+
+extern "C" int mmrs_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
+                                 double tie_margin) {
+    return regrid_impl(ctx, grids, n_grids, grid_of_unit, nullptr, 0, nullptr, tie_margin, "mmrs_sweep_regrid");
+}
+
+extern "C" int mmrs_rigid_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
+                                       const mmrs_tgrid* tgrids, int64_t n_tgrids, const int32_t* tgrid_of_unit,
+                                       double tie_margin) {
+    if (!tgrids) return set_err(ctx, MMRS_ERR_ARG, "mmrs_rigid_sweep_regrid: bad translation grids");
+    return regrid_impl(ctx, grids, n_grids, grid_of_unit, tgrids, n_tgrids, tgrid_of_unit, tie_margin,
+                       "mmrs_rigid_sweep_regrid");
 }
 
 // ---- run ------------------------------------------------------------------------------
@@ -941,7 +1078,8 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     k_exact_dense<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u,
                                                           (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
                                                           (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
-                                                          d.cand_off, d.n_cand, (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch);
+                                                          d.cand_off, d.n_cand, (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch,
+                                                          ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
     CUDA_TRY(ctx, cudaGetLastError());
     std::vector<double> h(d.n_cand);
     CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), ctx->d_tmp.p, (size_t)d.n_cand * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -953,8 +1091,16 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     const double lim = h[best] + ctx->tie_margin * std::fmax(1.0, (double)ctx->h_rmax[u]);
     int ties = 1;
     const double* cs = ctx->h_cs.data() + 2 * d.cand_off;
-    for (int c = 0; c < d.n_cand; ++c)
-        if (c != best && h[c] <= lim && (cs[2 * c] != cs[2 * best] || cs[2 * c + 1] != cs[2 * best + 1])) ++ties;
+    const int T = d.n_trans;   // rigid candidates: a tie is a different (cos, sin) or a different (tx, ty)
+    const double* tt = ctx->rigid ? ctx->h_t.data() + 2 * d.t_off : nullptr;
+    const int bi = best / T, bj = best % T;
+    for (int c = 0; c < d.n_cand; ++c) {
+        if (c == best || h[c] > lim) continue;
+        const int i = c / T, j = c % T;
+        bool differs = cs[2 * i] != cs[2 * bi] || cs[2 * i + 1] != cs[2 * bi + 1];
+        if (tt) differs = differs || tt[2 * j] != tt[2 * bj] || tt[2 * j + 1] != tt[2 * bj + 1];
+        if (differs) ++ties;
+    }
     r.best_idx = best;
     r.best_dist = h[best];
     r.n_shortlist = d.n_cand;
@@ -975,6 +1121,10 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     if (U == 0) return MMRS_OK;
     cudaStream_t s = ctx->stream;
     const UnitDesc* units = (const UnitDesc*)ctx->d_units.p;
+    // rigid candidates: translation tables, and R_eff in place of Rmax wherever the FP32 error bound enters
+    const float2* t32 = ctx->rigid ? (const float2*)ctx->d_t32.p : nullptr;
+    const double2* t64 = ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr;
+    const unsigned* rbits = (const unsigned*)(ctx->rigid ? ctx->d_reff.p : ctx->d_rmax.p);
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key.p, 0xff, U * 8, s));
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_nitems.p, 0, 16, s));
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[0], s));
@@ -1153,10 +1303,11 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
             if (cl.big) {
                 const int grid = (int)std::min<size_t>(cl.work_count, (size_t)ctx->n_sm * 2);
                 ENSURE(ctx->d_big_rows, (size_t)grid * kWarpsPerCta * ctx->big_scratch_per_warp * 4);
-                k_sweep_big<<<grid, kThreads, 0, s>>>(units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (int)cl.work_count,
-                                                      (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p,
-                                                      (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                                                      (float*)ctx->d_big_rows.p, ctx->big_scratch_per_warp);
+                auto big = t32 ? k_sweep_big<true> : k_sweep_big<false>;
+                big<<<grid, kThreads, 0, s>>>(units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (int)cl.work_count,
+                                              (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p,
+                                              (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
+                                              (float*)ctx->d_big_rows.p, ctx->big_scratch_per_warp, t32);
                 CUDA_TRY(ctx, cudaGetLastError());
                 ctx->launches += 1;
                 continue;
@@ -1167,11 +1318,13 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
                     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
                     ctx->eb_ran = true;
                 }
-                CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb));
-                k_sweep_eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(
+                if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<true>));
+                else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<false>));
+                auto eb = t32 ? k_sweep_eb<true> : k_sweep_eb<false>;
+                eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(
                     units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
                     (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                    (unsigned long long*)ctx->d_eb_pairs.p);
+                    (unsigned long long*)ctx->d_eb_pairs.p, t32);
                 CUDA_TRY(ctx, cudaGetLastError());
                 ctx->eb_cands += cl.live;
                 ctx->launches += 1;
@@ -1179,7 +1332,8 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
             }
             if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units,
                               (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
-                              (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p))
+                              (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
+                              nullptr, false, t32))
                 return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
             CUDA_TRY(ctx, cudaGetLastError());
             ctx->launches += 1;
@@ -1194,7 +1348,7 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     }
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[1], s));
     k_shortlist<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p,
-                                            (const unsigned long long*)ctx->d_key.p, (const unsigned*)ctx->d_rmax.p,
+                                            (const unsigned long long*)ctx->d_key.p, rbits,
                                             (float)ctx->opt_rel, (float)ctx->opt_abs, ctx->pool_cap,
                                             (int*)ctx->d_sl_count.p, (unsigned*)ctx->d_sl_base.p, (int2*)ctx->d_items.p,
                                             (unsigned*)ctx->d_nitems.p, 0, (tc || xf) ? (const int*)ctx->d_l1_count.p : nullptr);
@@ -1207,15 +1361,14 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
         k_exact<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
                                               (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
                                               (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
-                                              (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch);
+                                              (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, t64);
         CUDA_TRY(ctx, cudaGetLastError());
         k_select<<<(unsigned)((U + 7) / 8), 256, 0, s>>>(units, (int)U, (const double2*)ctx->d_cs64.p,
                                                          (const int2*)ctx->d_items.p,
                                                          (const double*)ctx->d_sl_dist.p, (const int*)ctx->d_sl_count.p,
                                                          (const unsigned*)ctx->d_sl_base.p,
-                                                         (const unsigned long long*)ctx->d_key.p,
-                                                         (const unsigned*)ctx->d_rmax.p, ctx->tie_margin,
-                                                         (UnitResultDev*)ctx->d_res.p);
+                                                         (const unsigned long long*)ctx->d_key.p, rbits,
+                                                         ctx->tie_margin, (UnitResultDev*)ctx->d_res.p, t64);
         CUDA_TRY(ctx, cudaGetLastError());
     }
     ctx->launches += 3;
@@ -1253,12 +1406,14 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
 }
 
 // ---- download ------------------------------------------------------------------------
-extern "C" int mmrs_sweep_download(mmrs_ctx* ctx, mmrs_unit_result* out) {
-    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_sweep_download: ctx is NULL");
-    if (!ctx->ready || !ctx->ran) return set_err(ctx, MMRS_ERR_STATE, "mmrs_sweep_download: nothing has been run");
+// out: the per-unit results (best_idx = the flattened candidate index i T + j of a rigid run, best_angle = angle i);
+// rout (rigid download): the same plus the angle / translation indices and the translation of the winner.
+static int download_impl(mmrs_ctx* ctx, mmrs_unit_result* out, mmrs_rigid_result* rout, const char* fn) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
+    if (!ctx->ready || !ctx->ran) return set_err(ctx, MMRS_ERR_STATE, std::string(fn) + ": nothing has been run");
     const int64_t U = ctx->n_units;
     if (U == 0) return MMRS_OK;
-    if (!out) return set_err(ctx, MMRS_ERR_ARG, "mmrs_sweep_download: out is NULL");
+    if (!out && !rout) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": out is NULL");
     ENTER_DEVICE(ctx);
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_res, ctx->d_res.p, U * sizeof(UnitResultDev), cudaMemcpyDeviceToHost,
                                   ctx->stream));
@@ -1294,35 +1449,67 @@ extern "C" int mmrs_sweep_download(mmrs_ctx* ctx, mmrs_unit_result* out) {
     bool need_rmax = false;
     for (int64_t u = 0; u < U; ++u)
         if (hr[u].n_shortlist < 0) need_rmax = true;
-    if (need_rmax) {
+    if (need_rmax) {   // tie margin of the full f64 recheck: R_eff for rigid candidates
         ctx->h_rmax.resize(U);
-        CUDA_TRY(ctx, cudaMemcpy(ctx->h_rmax.data(), ctx->d_rmax.p, U * 4, cudaMemcpyDeviceToHost));
+        CUDA_TRY(ctx, cudaMemcpy(ctx->h_rmax.data(), ctx->rigid ? ctx->d_reff.p : ctx->d_rmax.p, U * 4, cudaMemcpyDeviceToHost));
     }
     for (int64_t u = 0; u < U; ++u) {
         UnitResultDev r = hr[u];
         const mmrs_grid& g = ctx->grids[ctx->grid_of_unit[u]];
-        mmrs_unit_result& o = out[u];
+        const int T = ctx->h_units[u].n_trans;
+        mmrs_unit_result o;
         if (r.flags & MMRS_FLAG_DEGENERATE) {
             o = mmrs_unit_result{-1, g.fallback, 0.0, 0.0f, 0, 0, r.flags};
-            continue;
+        } else if (r.flags & MMRS_FLAG_EMPTY) {  // every candidate costs 0.0 -> leftmost wins (process_utils.rs:86-88)
+            o = mmrs_unit_result{0, mmrs_grid_angle(&g, 0), 0.0, 0.0f, 0, (int32_t)(g.n_cand * T), r.flags};
+        } else {
+            if (r.n_shortlist < 0) {
+                int rc = full_f64_unit(ctx, u, r);
+                if (rc != MMRS_OK) return rc;
+            }
+            o.best_idx = r.best_idx;
+            o.best_angle = mmrs_grid_angle(&g, r.best_idx / T);
+            o.best_dist = r.best_dist;
+            o.best_dist_f32 = r.best_d32;
+            o.n_shortlist = r.n_shortlist;
+            o.n_ties = r.n_ties;
+            o.flags = r.flags;
         }
-        if (r.flags & MMRS_FLAG_EMPTY) {  // every candidate costs 0.0 -> leftmost wins (process_utils.rs:86-88)
-            o = mmrs_unit_result{0, mmrs_grid_angle(&g, 0), 0.0, 0.0f, 0, (int32_t)g.n_cand, r.flags};
-            continue;
+        if (out) out[u] = o;
+        if (rout) {
+            mmrs_rigid_result& q = rout[u];
+            q.r = o;
+            q.pad = 0;
+            if (o.best_idx < 0) {   // degenerate angle grid: the fallback angle at the translation grid's centre
+                q.angle_idx = -1, q.trans_idx = -1;
+                q.best_tx = ctx->rigid ? ctx->tgrids[ctx->tgrid_of_unit[u]].t0x : 0.0;
+                q.best_ty = ctx->rigid ? ctx->tgrids[ctx->tgrid_of_unit[u]].t0y : 0.0;
+            } else {
+                q.angle_idx = o.best_idx / T, q.trans_idx = (int32_t)(o.best_idx % T);
+                q.best_tx = ctx->rigid ? ctx->h_t[2 * (ctx->h_units[u].t_off + q.trans_idx)] : 0.0;
+                q.best_ty = ctx->rigid ? ctx->h_t[2 * (ctx->h_units[u].t_off + q.trans_idx) + 1] : 0.0;
+            }
         }
-        if (r.n_shortlist < 0) {
-            int rc = full_f64_unit(ctx, u, r);
-            if (rc != MMRS_OK) return rc;
-        }
-        o.best_idx = r.best_idx;
-        o.best_angle = mmrs_grid_angle(&g, r.best_idx);
-        o.best_dist = r.best_dist;
-        o.best_dist_f32 = r.best_d32;
-        o.n_shortlist = r.n_shortlist;
-        o.n_ties = r.n_ties;
-        o.flags = r.flags;
     }
     return MMRS_OK;
+}
+
+extern "C" int mmrs_sweep_download(mmrs_ctx* ctx, mmrs_unit_result* out) {
+    return download_impl(ctx, out, nullptr, "mmrs_sweep_download");
+}
+
+extern "C" int mmrs_rigid_sweep_download(mmrs_ctx* ctx, mmrs_rigid_result* out) {
+    return download_impl(ctx, nullptr, out, "mmrs_rigid_sweep_download");
+}
+
+extern "C" int mmrs_rigid_sweep_batched(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_tgrid* tgrids,
+                                        int64_t n_tgrids, const int32_t* tgrid_of_unit, const mmrs_sweep_opts* opts,
+                                        mmrs_rigid_result* out) {
+    int rc = mmrs_rigid_sweep_upload(ctx, batch, tgrids, n_tgrids, tgrid_of_unit, opts);
+    if (rc != MMRS_OK) return rc;
+    rc = mmrs_sweep_run(ctx);
+    if (rc != MMRS_OK) return rc;
+    return mmrs_rigid_sweep_download(ctx, out);
 }
 
 extern "C" int mmrs_sweep_batched(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_sweep_opts* opts,
@@ -1411,12 +1598,13 @@ extern "C" int mmrs_last_timings(mmrs_ctx* ctx, float ms_out[4], int32_t* launch
 }
 
 // ---- explicit-angle exact evaluation ----------------------------------------------------
-extern "C" int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy,
-                               int64_t n_ref, double cx, double cy, int32_t mode, const double* angles,
-                               int64_t n_angles, double* dist_out) {
-    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_eval_exact: ctx is NULL");
+// txy == NULL: rotation only; otherwise candidate k is (angles[k], txy[2k], txy[2k+1]).
+static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
+                           double cx, double cy, int32_t mode, const double* angles, const double* txy, int64_t n_angles,
+                           double* dist_out, const char* fn) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (n_test < 0 || n_ref < 0 || n_angles < 0 || (n_angles > 0 && (!angles || !dist_out)))
-        return set_err(ctx, MMRS_ERR_ARG, "mmrs_eval_exact: bad arguments");
+        return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad arguments");
     if (n_angles == 0) return MMRS_OK;
     if (n_test == 0 || n_ref == 0) {  // process_utils.rs:86-88
         for (int64_t i = 0; i < n_angles; ++i) dist_out[i] = 0.0;
@@ -1434,8 +1622,9 @@ extern "C" int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_t
     // private scratch (does not disturb an uploaded batch)
     const size_t b_pts = (size_t)(n_test + n_ref) * 16, b_cs = (size_t)n_angles * 16, b_out = (size_t)n_angles * 8;
     const size_t o_cs = (b_pts + 255) / 256 * 256, o_zero = o_cs + (b_cs + 255) / 256 * 256,
-                 o_out = o_zero + ((size_t)n_angles + 255) / 256 * 256, o_unit = o_out + (b_out + 255) / 256 * 256;
-    ENSURE(ctx->d_tmp, o_unit + sizeof(UnitDesc));
+                 o_out = o_zero + ((size_t)n_angles + 255) / 256 * 256, o_unit = o_out + (b_out + 255) / 256 * 256,
+                 o_t = o_unit + 256;
+    ENSURE(ctx->d_tmp, o_t + (txy ? b_cs : 0));
     unsigned char* base = (unsigned char*)ctx->d_tmp.p;
     UnitDesc d{};
     d.test_off = 0;
@@ -1444,6 +1633,8 @@ extern "C" int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_t
     d.m = (int)n_ref;
     d.cx = cx;
     d.cy = cy;
+    d.n_trans = 1;
+    if (txy) CUDA_TRY(ctx, cudaMemcpyAsync(base + o_t, txy, b_cs, cudaMemcpyHostToDevice, s));
     CUDA_TRY(ctx, cudaMemcpyAsync(base, test_xy, (size_t)n_test * 16, cudaMemcpyHostToDevice, s));
     CUDA_TRY(ctx, cudaMemcpyAsync(base + (size_t)n_test * 16, ref_xy, (size_t)n_ref * 16, cudaMemcpyHostToDevice, s));
     CUDA_TRY(ctx, cudaMemcpyAsync(base + o_cs, cs.data(), b_cs, cudaMemcpyHostToDevice, s));
@@ -1456,12 +1647,28 @@ extern "C" int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_t
     k_exact_dense<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
                                                 (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
                                                 (const unsigned char*)(base + o_zero), 0, (int)n_angles,
-                                                (double*)(base + o_out), max_n, ep.scratch);
+                                                (double*)(base + o_out), max_n, ep.scratch,
+                                                txy ? (const double2*)(base + o_t) : nullptr, true);
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(dist_out, base + o_out, b_out, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
     ctx->eval_launches += 1;
     return MMRS_OK;
+}
+
+extern "C" int mmrs_eval_exact(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy,
+                               int64_t n_ref, double cx, double cy, int32_t mode, const double* angles,
+                               int64_t n_angles, double* dist_out) {
+    return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, nullptr, n_angles, dist_out,
+                           "mmrs_eval_exact");
+}
+
+extern "C" int mmrs_eval_exact_rigid(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy,
+                                     int64_t n_ref, double cx, double cy, int32_t mode, const double* angles,
+                                     const double* txy, int64_t n_cand, double* dist_out) {
+    if (n_cand > 0 && !txy) return set_err(ctx, MMRS_ERR_ARG, "mmrs_eval_exact_rigid: txy is NULL");
+    return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, txy, n_cand, dist_out,
+                           "mmrs_eval_exact_rigid");
 }
 
 // ---- FP32 peak probe ------------------------------------------------------------------------

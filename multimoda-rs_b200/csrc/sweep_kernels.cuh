@@ -216,15 +216,19 @@ __global__ void k_cs32(const double2* __restrict__ cs64, float2* __restrict__ cs
 //               of the minimum are re-scored by the direct-form kernel (LIST), and K2/K3/K4 run unchanged on exact
 //               FP32 values — the selection is bit-identical to the dense direct path. The tail pass and the odd
 //               scalar slot stay in direct form (their values are exact, the seeds and minima mix freely).
-template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF>
+// RIGID = true: rigid candidates (dense launches, direct form). Candidate c = i n_trans + j is angle i of the unit's
+//               grid and translation j of its translation grid (t32, FP32); every rotated test point gets the
+//               translation added once (one FADD2 per packed pair and coordinate, one FADD for the unpaired point).
+template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false>
 __global__ void __launch_bounds__(kThreads, 2)
     k_sweep(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
             const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
             const int2* __restrict__ l_items, const unsigned* __restrict__ l_nitems, unsigned l_cap, int l_chunk,
-            const unsigned* __restrict__ rmax_bits, unsigned* __restrict__ diag) {
+            const unsigned* __restrict__ rmax_bits, unsigned* __restrict__ diag, const float2* __restrict__ t32) {
     static_assert(TA >= 2 && TA <= 18, "register tile out of range");
     static_assert(!(TAILP && MULTI), "the tail pass is for single-chunk units");
     static_assert(!(XF && LIST), "the expanded form is a dense tier; lists are re-scored in direct form");
+    static_assert(!(RIGID && (XF || LIST)), "rigid candidates run the dense direct-form sweep");
     constexpr int SB = TA + 1;         // TAILP: reference points per lane of the tail pass (M <= 32 SB)
     constexpr int H = TA / 2;          // packed pairs of test points per lane
     constexpr bool TAIL = (TA & 1);    // plus one unpaired point when TA is odd
@@ -306,8 +310,15 @@ __global__ void __launch_bounds__(kThreads, 2)
 
     for (int ci = wid; ci < total; ci += kWarpsPerCta) {
         const int c = LIST ? my_items[ci].y : w.begin + ci;
-        const float2 cs = __ldg(&cs32[ud.cand_off + c]);
+        float2 tr = make_float2(0.f, 0.f);   // RIGID: translation of this candidate
+        int ia = c;                          // RIGID: its angle index
+        if (RIGID) {
+            ia = c / ud.n_trans;
+            tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
+        }
+        const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
         const uint64_t C2 = pk(cs.x, cs.x), S2 = pk(cs.y, cs.y), NS2 = pk(-cs.y, -cs.y);
+        const uint64_t TX2 = pk(tr.x, tr.x), TY2 = pk(tr.y, tr.y);
         unsigned rowmax = 0u, colmax = 0u;  // bit patterns of non-negative floats order like unsigned ints
         bool gave_up = false;
 
@@ -331,7 +342,8 @@ __global__ void __launch_bounds__(kThreads, 2)
 #endif
                 const float4 a = sT[t];  // (x0, y0, x1, y1): broadcast
                 const uint64_t X2 = pk(a.x, a.z), Y2 = pk(a.y, a.w);
-                const uint64_t PX = fma2(Y2, NS2, mul2(X2, C2)), PY = fma2(X2, S2, mul2(Y2, C2));
+                uint64_t PX = fma2(Y2, NS2, mul2(X2, C2)), PY = fma2(X2, S2, mul2(Y2, C2));
+                if (RIGID) PX = add2(PX, TX2), PY = add2(PY, TY2);
                 float r0 = INF, r1 = INF;   // row minima of the two tail points over this lane's reference points
 #pragma unroll
                 for (int q = 0; q < SB; q += 2) {
@@ -372,6 +384,7 @@ __global__ void __launch_bounds__(kThreads, 2)
                 const float4 a = sA[(ch * S + H) * 32 + lane];
                 tx = fmaf(a.z, -cs.y, a.x * cs.x);
                 ty = fmaf(a.x, cs.y, a.z * cs.x);
+                if (RIGID) tx = __fadd_rn(tx, tr.x), ty = __fadd_rn(ty, tr.y);
                 row[TA - 1] = INF;
             }
 #pragma unroll
@@ -380,6 +393,10 @@ __global__ void __launch_bounds__(kThreads, 2)
                 const uint64_t X2 = pk(a.x, a.y), Y2 = pk(a.z, a.w);
                 AX[k] = fma2(Y2, NS2, mul2(X2, C2));  // x' = x cos - y sin
                 AY[k] = fma2(X2, S2, mul2(Y2, C2));   // y' = x sin + y cos
+                if (RIGID) {                          // + t, rounded once
+                    AX[k] = add2(AX[k], TX2);
+                    AY[k] = add2(AY[k], TY2);
+                }
                 if (XF) {
                     NA[k] = fma2(AX[k], AX[k], mul2(AY[k], AY[k]));
                     const uint64_t M2 = pk(-2.f, -2.f);
@@ -610,10 +627,13 @@ __device__ __forceinline__ int eb_warp_argmax(unsigned v, int idx) {
     return __shfl_sync(0xffffffffu, idx, __ffs(__ballot_sync(0xffffffffu, v == m)) - 1);
 }
 
+// RIGID = true: rigid candidates, c = i n_trans + j (see k_sweep): A'[k] = R a_k + t, the translation added once with
+// __fadd_rn when the row is materialised; the column pass reads the same A', so K1e stays bit-identical to K1.
+template <bool RIGID = false>
 __global__ void __launch_bounds__(kThreads, 3)
     k_sweep_eb(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
                const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
-               unsigned long long* __restrict__ pairs_out) {
+               unsigned long long* __restrict__ pairs_out, const float2* __restrict__ t32) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
     unsigned long long* s_key = reinterpret_cast<unsigned long long*>(smem_raw + 8);
@@ -672,11 +692,19 @@ __global__ void __launch_bounds__(kThreads, 3)
         }
         int ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
         for (int c = c_begin; c < c_end; ++c) {
-            const float2 cs = __ldg(&cs32[ud.cand_off + c]);
+            float2 tr = make_float2(0.f, 0.f);
+            int ia = c;
+            if (RIGID) {
+                ia = c / ud.n_trans;
+                tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
+            }
+            const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
             __syncwarp();   // the previous candidate is done with A' and the hints
             for (int i = lane; i < N; i += 32) {
                 const float2 p = test_pt(i);
-                sR[i] = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
+                float2 r = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
+                if (RIGID) r = make_float2(__fadd_rn(r.x, tr.x), __fadd_rn(r.y, tr.y));
+                sR[i] = r;
             }
             __syncwarp();
             int arg;
@@ -767,10 +795,13 @@ __global__ void __launch_bounds__(kThreads, 3)
 constexpr int kBigBlock = 1024;   // reference points per shared-memory block
 constexpr int kBigTA = 16;
 
+// RIGID = true: rigid candidates, c = i n_trans + j (see k_sweep).
+template <bool RIGID = false>
 __global__ void __launch_bounds__(kThreads, 2)
     k_sweep_big(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, int n_work,
                 const float4* __restrict__ lay, const float2* __restrict__ cs32, float* __restrict__ dist32,
-                unsigned long long* __restrict__ key, float* __restrict__ row_scratch, long long scratch_per_warp) {
+                unsigned long long* __restrict__ key, float* __restrict__ row_scratch, long long scratch_per_warp,
+                const float2* __restrict__ t32) {
     constexpr int TA = kBigTA, H = TA / 2;
     __shared__ __align__(16) float4 sB[kBigBlock / 2];
     __shared__ unsigned s_col[kWarpsPerCta][kBigBlock];
@@ -787,8 +818,15 @@ __global__ void __launch_bounds__(kThreads, 2)
         for (int c0 = 0; c0 < w.count; c0 += kWarpsPerCta) {   // one candidate per warp and round; every warp walks the blocks
             const bool live = c0 + wid < w.count;
             const int c = w.begin + min(c0 + wid, w.count - 1);
-            const float2 cs = __ldg(&cs32[ud.cand_off + c]);
+            float2 tr = make_float2(0.f, 0.f);
+            int ia = c;
+            if (RIGID) {
+                ia = c / ud.n_trans;
+                tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
+            }
+            const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
             const uint64_t C2 = pk(cs.x, cs.x), S2 = pk(cs.y, cs.y), NS2 = pk(-cs.y, -cs.y);
+            const uint64_t TX2 = pk(tr.x, tr.x), TY2 = pk(tr.y, tr.y);
             unsigned rowmax = 0u, colmax = 0u;
             for (int bb = 0; bb < n_blocks; ++bb) {
                 const int j0 = bb * (kBigBlock / 2), jn = min(kBigBlock / 2, ud.m_pairs - j0);
@@ -805,6 +843,10 @@ __global__ void __launch_bounds__(kThreads, 2)
                         const uint64_t X2 = pk(a.x, a.y), Y2 = pk(a.z, a.w);
                         AX[k] = fma2(Y2, NS2, mul2(X2, C2));
                         AY[k] = fma2(X2, S2, mul2(Y2, C2));
+                        if (RIGID) {
+                            AX[k] = add2(AX[k], TX2);
+                            AY[k] = add2(AY[k], TY2);
+                        }
                         if (bb == 0) {
                             row[2 * k] = INF;
                             row[2 * k + 1] = INF;
@@ -1129,8 +1171,11 @@ __global__ void k_shortlist(const UnitDesc* __restrict__ units, const float* __r
 // sin/cos are not bit-identical to glibc's.
 //   rotate     : contour_point.rs:38-52 (mode 0, identity iff angle == 0.0) /
 //                align_between.rs:193-209 (mode 1)
+//   translate  : rigid candidates only: x' = rx + tx, y' = ry + ty (__dadd_rn; + 0.0 is exact, so a zero translation
+//                is the rotation-only cost bit for bit)
 //   distances  : process_utils.rs:84-121, both directions, sqrt, max
 // One CTA per (unit, candidate) item; grid-stride over the item list.
+// t64 != NULL: rigid candidates, c = i n_trans + j -> angle i of the unit's grid, translation j of its translation grid.
 // =============================================================================
 __device__ __forceinline__ double block_max(double v, double* s_red) {
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
@@ -1146,7 +1191,8 @@ __device__ __forceinline__ double block_max(double v, double* s_red) {
 // it) a per-CTA scratch row in global memory for the rotated points and the caller's reference array itself (copy_ref = false).
 __device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* __restrict__ test_xy,
                                              const double* __restrict__ ref_xy, double cosv, double sinv, bool identity,
-                                             double2* s_rot, const double2* s_ref_in, double* s_red, bool copy_ref = true) {
+                                             double2* s_rot, const double2* s_ref_in, double* s_red, bool copy_ref = true,
+                                             bool rigid = false, double2 t = double2{0.0, 0.0}) {
     double2* s_ref_w = const_cast<double2*>(s_ref_in);
     const double2* s_ref = copy_ref ? s_ref_in : reinterpret_cast<const double2*>(ref_xy + 2 * ud.ref_off);
     for (int i = threadIdx.x; i < ud.n; i += blockDim.x) {
@@ -1157,6 +1203,7 @@ __device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* _
             rx = __dadd_rn(__dsub_rn(__dmul_rn(x, cosv), __dmul_rn(y, sinv)), ud.cx);
             ry = __dadd_rn(__dadd_rn(__dmul_rn(x, sinv), __dmul_rn(y, cosv)), ud.cy);
         }
+        if (rigid) rx = __dadd_rn(rx, t.x), ry = __dadd_rn(ry, t.y);
         s_rot[i] = make_double2(rx, ry);
     }
     if (copy_ref)
@@ -1199,7 +1246,7 @@ __global__ void __launch_bounds__(256)
     k_exact(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
             const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
             const int2* __restrict__ items, const unsigned* __restrict__ n_items, unsigned pool_cap,
-            double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch) {
+            double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch, const double2* __restrict__ t64) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* s_red = reinterpret_cast<double*>(smem_raw);
     // g_scratch != NULL: the point sets do not fit shared memory — rotated points in this CTA's global scratch row
@@ -1211,30 +1258,37 @@ __global__ void __launch_bounds__(256)
         if (item.x < 0) continue;  // uniform per CTA
         const UnitDesc ud = units[item.x];
         const int c = item.y;
-        const double2 cs = cs64[ud.cand_off + c];
-        const bool identity = zero_flag[ud.cand_off + c] != 0;
-        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr);
+        const int i = t64 ? c / ud.n_trans : c;
+        const double2 cs = cs64[ud.cand_off + i];
+        const bool identity = zero_flag[ud.cand_off + i] != 0;
+        const double2 t = t64 ? t64[ud.t_off + (c - i * ud.n_trans)] : make_double2(0.0, 0.0);
+        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr,
+                                    t64 != nullptr, t);
         if (threadIdx.x == 0) sl_dist[it] = d;
         __syncthreads();
     }
 }
 
 // Dense variant: every candidate [c0, c0+count) of one unit (shortlist overflow
-// path and mmrs_eval_exact).
+// path and mmrs_eval_exact). t64 != NULL: rigid candidates; paired = true (mmrs_eval_exact_rigid): candidate c takes
+// angle c and translation t64[c] instead of the grid product.
 __global__ void __launch_bounds__(256)
     k_exact_dense(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
                   const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
                   const unsigned char* __restrict__ zero_flag, long long cs_off, int count, double* __restrict__ out,
-                  int max_n, double2* __restrict__ g_scratch) {
+                  int max_n, double2* __restrict__ g_scratch, const double2* __restrict__ t64, bool paired) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* s_red = reinterpret_cast<double*>(smem_raw);
     double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
     double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
     const UnitDesc ud = units[unit];
     for (int c = blockIdx.x; c < count; c += gridDim.x) {
-        const double2 cs = cs64[cs_off + c];
-        const bool identity = zero_flag[cs_off + c] != 0;
-        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr);
+        const int i = (t64 && !paired) ? c / ud.n_trans : c;
+        const double2 cs = cs64[cs_off + i];
+        const bool identity = zero_flag[cs_off + i] != 0;
+        const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
+        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr,
+                                    t64 != nullptr, t);
         if (threadIdx.x == 0) out[c] = d;
         __syncthreads();
     }
@@ -1249,7 +1303,8 @@ __global__ void k_select(const UnitDesc* __restrict__ units, int n_units, const 
                          const int2* __restrict__ items, const double* __restrict__ sl_dist,
                          const int* __restrict__ sl_count,
                          const unsigned* __restrict__ sl_base, const unsigned long long* __restrict__ key,
-                         const unsigned* __restrict__ rmax_bits, double tie_margin, UnitResultDev* __restrict__ res) {
+                         const unsigned* __restrict__ rmax_bits, double tie_margin, UnitResultDev* __restrict__ res,
+                         const double2* __restrict__ t64) {
     const int u = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (u >= n_units) return;
@@ -1291,15 +1346,23 @@ __global__ void k_select(const UnitDesc* __restrict__ units, int n_units, const 
         // Tie count: rechecked candidates within the margin whose ANGLE differs from the winner's. A candidate
         // with the winner's own angle (the -pi / +pi wrap duplicates of a +-180 deg grid) has the winner's cost
         // in any arithmetic, so the lowest index wins there regardless and it is not an ambiguity.
+        // Rigid candidates (t64 != NULL): whose TRANSFORM differs, i.e. a different (cos, sin) or a different (tx, ty).
         const double lim = bd + tie_margin * fmax(1.0, (double)__uint_as_float(rmax_bits[u]));
-        const long long co = units[u].cand_off;
-        const double2 wcs = cs64[co + bi];
+        const long long co = units[u].cand_off, to = units[u].t_off;
+        const int nt = t64 ? units[u].n_trans : 1;
+        const double2 wcs = cs64[co + bi / nt];
+        const double2 wt = t64 ? t64[to + bi % nt] : make_double2(0.0, 0.0);
         int ties = 0;
         for (int k = lane; k < n; k += 32) {
             const int i = items[base + k].y;
             if (i == bi || sl_dist[base + k] > lim) continue;
-            const double2 c = cs64[co + i];
-            ties += (c.x != wcs.x || c.y != wcs.y) ? 1 : 0;
+            const double2 c = cs64[co + i / nt];
+            bool differs = c.x != wcs.x || c.y != wcs.y;
+            if (t64) {
+                const double2 t = t64[to + i % nt];
+                differs = differs || t.x != wt.x || t.y != wt.y;
+            }
+            ties += differs ? 1 : 0;
         }
         for (int o = 16; o > 0; o >>= 1) ties += __shfl_xor_sync(0xffffffffu, ties, o);
         r.best_idx = bi;
@@ -1371,6 +1434,14 @@ __global__ void k_finish_angle(int n_units, const int4* __restrict__ cnt, UnitRe
     // a pool overflow on any rank: every rank rechecks ALL candidates of the unit in f64 at download (negative count)
     res[u].n_shortlist = c.z ? -1 : c.x;
     res[u].n_ties = res[u].best_idx >= 0 ? c.y + 1 : 0;
+}
+
+// Rigid runs: R_eff = Rmax + max_j |t_j| per unit (the coordinate magnitude the FP32 error bound scales with), rounded
+// up to FP32 bits; used wherever the rotation-only sweep uses Rmax (K2 window, tie margin).
+__global__ void k_reff(const unsigned* __restrict__ rmax_bits, const double* __restrict__ tmax, unsigned* __restrict__ reff,
+                       int n_units) {
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u < n_units) reff[u] = __float_as_uint(__double2float_ru((double)__uint_as_float(rmax_bits[u]) + tmax[u]));
 }
 
 // =============================================================================

@@ -7,6 +7,7 @@ from ._processing import (align_combined, align_manual, align_three_point, to_ob
                           from_array_singlepair, from_file_doublepair, from_file_full, from_file_single,
                           from_file_singlepair, get_context)
 from ._native import MmrsError
+from ._rigid import find_best_rigid_transform
 from ._vtp import read_centerline_vtp
 from ._centerline import load_centerline, prepare_centerline
 

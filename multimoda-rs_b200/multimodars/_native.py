@@ -48,6 +48,16 @@ class UnitResult(C.Structure):
                 ("flags", C.c_int32)]
 
 
+class TGrid(C.Structure):
+    """mmrs_tgrid: (2 half_n + 1)^2 translations t0 + (jx - half_n, jy - half_n) * step."""
+    _fields_ = [("t0x", C.c_double), ("t0y", C.c_double), ("step", C.c_double), ("half_n", C.c_int32)]
+
+
+class RigidResult(C.Structure):
+    _fields_ = [("r", UnitResult), ("angle_idx", C.c_int64), ("trans_idx", C.c_int32), ("pad", C.c_int32),
+                ("best_tx", C.c_double), ("best_ty", C.c_double)]
+
+
 class AlignParams(C.Structure):
     _fields_ = [("step_deg", C.c_double), ("range_deg", C.c_double), ("sample_size", C.c_int64),
                 ("smooth", C.c_int32), ("bruteforce", C.c_int32), ("postprocessing", C.c_int32)]
@@ -63,6 +73,11 @@ class CenterlineParams(C.Structure):
 RESULT_DTYPE = np.dtype([("best_idx", "<i8"), ("best_angle", "<f8"), ("best_dist", "<f8"), ("best_dist_f32", "<f4"),
                          ("n_shortlist", "<i4"), ("n_ties", "<i4"), ("flags", "<i4")], align=True)
 assert RESULT_DTYPE.itemsize == C.sizeof(UnitResult)
+# mmrs_rigid_result: the unit result (best_idx = flattened candidate i T + j) plus the angle / translation indices
+RIGID_RESULT_DTYPE = np.dtype([("best_idx", "<i8"), ("best_angle", "<f8"), ("best_dist", "<f8"), ("best_dist_f32", "<f4"),
+                               ("n_shortlist", "<i4"), ("n_ties", "<i4"), ("flags", "<i4"), ("angle_idx", "<i8"),
+                               ("trans_idx", "<i4"), ("pad", "<i4"), ("best_tx", "<f8"), ("best_ty", "<f8")], align=True)
+assert RIGID_RESULT_DTYPE.itemsize == C.sizeof(RigidResult)
 
 FLAG_DEGENERATE, FLAG_FULL_F64, FLAG_EMPTY = 1, 2, 4
 
@@ -77,6 +92,8 @@ EXPORTS = [
     "mmrs_process_cases", "mmrs_process_stats", "mmrs_ctx_set_shard", "mmrs_export_pair", "mmrs_export_single",
     "mmrs_align_centerline", "mmrs_sweep_prefilter_info", "mmrs_ctx_set_prune", "mmrs_contour_metrics",
     "mmrs_comm_unique_id", "mmrs_ctx_comm_init", "mmrs_ctx_set_partition", "mmrs_ctx_comm_info",
+    "mmrs_rigid_sweep_batched", "mmrs_rigid_sweep_upload", "mmrs_rigid_sweep_regrid", "mmrs_rigid_sweep_download",
+    "mmrs_eval_exact_rigid",
 ]
 
 _lib = None
@@ -115,6 +132,15 @@ def lib():
         L.mmrs_fp32_probe.argtypes = [C.c_void_p, C.c_int32, c_dp]
         L.mmrs_process_stats.argtypes = [C.c_void_p, c_i64p]
         L.mmrs_ctx_set_shard.argtypes = [C.c_void_p, C.c_int32, C.c_int32, EXCHANGE_FN, C.c_void_p]
+        L.mmrs_rigid_sweep_batched.argtypes = [C.c_void_p, C.POINTER(SweepBatch), C.POINTER(TGrid), C.c_int64, c_i32p,
+                                               C.POINTER(SweepOpts), C.c_void_p]
+        L.mmrs_rigid_sweep_upload.argtypes = [C.c_void_p, C.POINTER(SweepBatch), C.POINTER(TGrid), C.c_int64, c_i32p,
+                                              C.POINTER(SweepOpts)]
+        L.mmrs_rigid_sweep_regrid.argtypes = [C.c_void_p, C.POINTER(Grid), C.c_int64, c_i32p, C.POINTER(TGrid), C.c_int64,
+                                              c_i32p, C.c_double]
+        L.mmrs_rigid_sweep_download.argtypes = [C.c_void_p, C.c_void_p]
+        L.mmrs_eval_exact_rigid.argtypes = [C.c_void_p, c_dp, C.c_int64, c_dp, C.c_int64, C.c_double, C.c_double,
+                                            C.c_int32, c_dp, c_dp, C.c_int64, c_dp]
         _lib = L
     return _lib
 
@@ -136,6 +162,11 @@ def make_grid(step_deg, range_deg, center=None, limes_deg=None) -> Grid:
 
 def grid_angle(g: Grid, i: int) -> float:
     return lib().mmrs_grid_angle(C.byref(g), int(i))
+
+
+def make_tgrid(step, half_n, t0=(0.0, 0.0)) -> TGrid:
+    """Translation grid of (2 half_n + 1)^2 offsets t0 + ((jx - half_n) step, (jy - half_n) step), j = jy (2 half_n + 1) + jx."""
+    return TGrid(float(t0[0]), float(t0[1]), float(step), int(half_n))
 
 
 def stage_plan(step_deg, range_deg):
@@ -231,6 +262,57 @@ class Context:
     def sweep_download(self):
         out = np.zeros(self._n_units, dtype=RESULT_DTYPE)
         self._check(lib().mmrs_sweep_download(self._p, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    # -- rigid candidates (angle grid x translation grid, mmrs_b200.h "rigid candidates") -------------------------
+    @staticmethod
+    def _tgrids(tgrids, tgrid_of_unit):
+        tarr = (TGrid * max(len(tgrids), 1))(*tgrids)
+        tou = None if tgrid_of_unit is None else np.ascontiguousarray(tgrid_of_unit, dtype=np.int32)
+        return tarr, tou, None if tou is None else tou.ctypes.data_as(c_i32p)
+
+    def rigid_sweep_batched(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids, grid_of_unit=None,
+                            tgrid_of_unit=None, mode=0, **opts):
+        """mmrs_rigid_sweep_batched: host arrays in, structured result array (RIGID_RESULT_DTYPE) out."""
+        b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
+        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        o = self._opts(**opts)
+        out = np.zeros(U, dtype=RIGID_RESULT_DTYPE)
+        self._check(lib().mmrs_rigid_sweep_batched(self._p, C.byref(b), tarr, len(tgrids), ptou, C.byref(o),
+                                                   out.ctypes.data_as(C.c_void_p)))
+        self._n_units = U
+        return out
+
+    def rigid_upload(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids, grid_of_unit=None,
+                     tgrid_of_unit=None, mode=0, **opts):
+        b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
+        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        o = self._opts(**opts)
+        self._check(lib().mmrs_rigid_sweep_upload(self._p, C.byref(b), tarr, len(tgrids), ptou, C.byref(o)))
+        self._n_units = U
+
+    def rigid_regrid(self, grids, tgrids, grid_of_unit=None, tgrid_of_unit=None, tie_margin=0.0):
+        garr = (Grid * max(len(grids), 1))(*grids)
+        gou = None if grid_of_unit is None else np.ascontiguousarray(grid_of_unit, dtype=np.int32)
+        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        self._check(lib().mmrs_rigid_sweep_regrid(self._p, garr, len(grids), None if gou is None else gou.ctypes.data_as(c_i32p),
+                                                  tarr, len(tgrids), ptou, float(tie_margin)))
+
+    def rigid_download(self):
+        out = np.zeros(self._n_units, dtype=RIGID_RESULT_DTYPE)
+        self._check(lib().mmrs_rigid_sweep_download(self._p, out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def eval_exact_rigid(self, test_xy, ref_xy, centre, mode, angles, txy):
+        """f64 cost of the rigid candidates (angles[k], txy[k]) (mmrs_eval_exact_rigid)."""
+        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
+        tt = _f64(txy).reshape(-1, 2)
+        if len(tt) != len(a):
+            raise ValueError("eval_exact_rigid: angles and txy differ in length")
+        out = np.empty(len(a), dtype=np.float64)
+        self._check(lib().mmrs_eval_exact_rigid(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r),
+                                                float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
+                                                tt.ctypes.data_as(c_dp), len(a), out.ctypes.data_as(c_dp)))
         return out
 
     def plan(self):
