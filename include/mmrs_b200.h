@@ -268,6 +268,40 @@ int mmrs_eval_exact_rigid(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, 
                           double cx, double cy, int32_t mode, const double* angles, const double* txy, int64_t n_cand,
                           double* dist_out);
 
+/* ---- partial cost: rank-K Hausdorff distance, a set fraction of outlier points ignored (opt-in) ---------------
+ * The symmetric Hausdorff distance is a maximum, so one artefact (a side-branch bulge, a calcification, a catheter
+ * shadow) decides every candidate's cost. The partial distance (Huttenlocher, Klanderman and Rucklidge, IEEE TPAMI
+ * 1993) takes, in each direction, the K-th smallest point minimum instead of the largest, so the worst n - K points
+ * of each set do not count. Like the rigid candidates, this is this library's own extension, restated by the tests.
+ *
+ * One inlier_fraction f, finite, 0 < f <= 1, for both directions. For a set of n finite points (non-finite points
+ *   are dropped, as everywhere): K(n) = max(1, ceil(f * n)) (host f64, as written); q(n) = n - K(n) points do not count.
+ * Row value of a point p against a set Q: v(p) = min_{x in Q} d^2(p, x); a non-finite minimum counts as 0.
+ * Directed partial value: the (q + 1)-th largest v(p) over the set, duplicates counted. Cost (f64):
+ *   fmax(sqrt(fwd), sqrt(bwd)), fwd: the reference points against the transformed test set, q = q(m);
+ *   bwd: the transformed test points against the reference set, q = q(n).
+ * The transform (mode 0 / 1 rotation, plus the optional translation grid) and the selection (leftmost arg-min, tie
+ *   margin, R_eff for rigid runs) are those of the rotation-only and rigid sweeps. f = 1 gives q = 0: today's cost.
+ *   An empty set still costs 0.
+ * Limits (MMRS_ERR_ARG, checked before any device work): q <= 255 per direction and unit; no unit beyond the
+ *   shared-memory staging (more than ~4 000 points per set); opts.prune > 0 or opts.prefilter 2 / 3. The context's
+ *   prune default and any partition across ranks are not used, as for rigid runs.
+ * Exactness: the FP32 sweep computes each candidate's partial FP32 distance exactly (an early-break kernel whose
+ *   threshold only holds exact minima of the current candidate); MMRS_EARLY_BREAK=0 at upload switches the early
+ *   break off in the same kernel. The FP32 -> f64 window is that of the full cost.                               */
+
+/* mmrs_sweep_upload (tgrids == NULL) or mmrs_rigid_sweep_upload with the partial cost. inlier_fraction == 1.0 is
+ * exactly the plain upload with the same opts. The fraction stays with the uploaded points: mmrs_sweep_regrid /
+ * mmrs_rigid_sweep_regrid, mmrs_sweep_run and the download calls work on it unchanged; a later plain upload clears it. */
+int mmrs_partial_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_tgrid* tgrids /* NULL: rotation only */,
+                              int64_t n_tgrids, const int32_t* tgrid_of_unit, double inlier_fraction,
+                              const mmrs_sweep_opts* opts);
+/* f64 partial cost of explicit candidates k = (angles[k], txy[2k], txy[2k+1]) for one unit (txy == NULL: no
+ * translation), on the finite points of each set.                                                              */
+int mmrs_eval_exact_partial(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
+                            double cx, double cy, int32_t mode, const double* angles, const double* txy /* NULL: none */,
+                            int64_t n_cand, double inlier_fraction, double* dist_out);
+
 /* ---- geometry blob -------------------------------------------------------------
  * Geometries cross the boundary as one f64 stream (u32 ids are exact in f64):
  *   n_frames,

@@ -28,7 +28,7 @@ struct UnitDesc {
                                   // axis -> one contiguous sub-range per rank, global indices kept)
     long long t_off;              // rigid runs: offset of this unit's translation grid in the t64 / t32 tables
     int n_trans;                  // translations per angle (1 without a translation grid): candidate c = i n_trans + j
-    int t_pad;
+    short q_fwd, q_bwd;           // partial cost: points that do not count, reference -> test (q(m)) / test -> reference (q(n))
 };
 constexpr int kFlagRemote = 0x400;  // internal UnitDesc.flags bit: another rank owns this unit (never leaves the library)
 
@@ -81,6 +81,9 @@ struct mmrs_ctx {
         size_t smem_eb = 0;                     // shared memory of a K1e CTA (k_sweep_eb) of this class
         bool eb = false;                        // the dense sweep of this class runs K1e (decided per grid set)
         long long live = 0;                     // candidates of this class swept by this rank
+        size_t stage = 0, ebp_warp = 0;         // partial cost: largest staging image / per-warp block of the class
+        int ebp_warps = 0;                      // warps per CTA of the partial kernel (8, 4, 2 or 1)
+        size_t smem_ebp = 0;
     };
     std::vector<SweepClass> classes;
     std::vector<int> class_of_unit;
@@ -146,6 +149,10 @@ struct mmrs_ctx {
     std::vector<double> h_t;                // (tx, ty) of every translation of every translation grid
     std::vector<double> h_tmax;             // per unit: largest |t| of its translation grid
     mmrs::DevBuf d_t64, d_t32, d_tmax, d_reff;   // translation tables; per unit R_eff = Rmax + max |t| (float bits)
+
+    // partial (rank-K) cost (mmrs_partial_sweep_upload): set with the points, kept across regrids
+    bool partial = false;
+    double inlier_fraction = 1.0;
 
     // partition of every batched sweep across ranks (mmrs_ctx_comm_init / mmrs_ctx_set_shard / mmrs_ctx_set_partition)
     int shard_rank = 0, shard_world = 1;

@@ -359,6 +359,12 @@ static ClassChoice choose_class(int n, int m) {
     return best;
 }
 
+// Partial cost: points of an n-point set that do not count, q(n) = n - K(n), K(n) = max(1, ceil(f n)) in f64.
+static int partial_q(double f, int n) {
+    if (n <= 0) return 0;
+    return n - (int)std::max(1.0, std::ceil(f * (double)n));
+}
+
 // ---- upload ----------------------------------------------------------------------------
 // Points part of an upload: validates the offsets, chooses the register tile, lays every unit out in the
 // staging image (k_prep) and keeps the f64 points on the device. Grid-independent.
@@ -428,6 +434,14 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
         d.cx = b->centre_xy[2 * u];
         d.cy = b->centre_xy[2 * u + 1];
         d.lay_off = lay_off;
+        if (ctx->partial) {
+            const int q_f = partial_q(ctx->inlier_fraction, d.m), q_b = partial_q(ctx->inlier_fraction, d.n);
+            if (q_f > kPartialMaxQ || q_b > kPartialMaxQ)
+                return set_err(ctx, MMRS_ERR_ARG, "partial cost: unit " + std::to_string(u) + " leaves out " +
+                                                      std::to_string(std::max(q_f, q_b)) +
+                                                      " points in one direction; at most q = 255 per direction and unit");
+            d.q_fwd = (short)q_f, d.q_bwd = (short)q_b;
+        }
         d.ta = 2;
         if (d.n > 0 && d.m > 0) {
             const ClassChoice cc = choose_class(d.n, d.m);
@@ -474,6 +488,26 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
                                                                               (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m));
             ctx->classes[k].cost += (long long)d.n_chunks * 32 * d.ta * d.m;
             ctx->class_of_unit[u] = k;
+            if (ctx->partial && big)
+                return set_err(ctx, MMRS_ERR_ARG, "partial cost: unit " + std::to_string(u) +
+                                                      " is beyond the shared-memory staging (more than ~4 000 points per set)");
+            if (ctx->partial) {
+                auto& cl = ctx->classes[k];
+                cl.stage = std::max(cl.stage, 16 + (size_t)(a_elems + b_elems + nb_elems + t_elems) * 16);
+                cl.ebp_warp = std::max(cl.ebp_warp, (size_t)ebp_warp_bytes(d.n, d.m, d.q_bwd, d.q_fwd));
+            }
+        }
+    }
+    if (ctx->partial) {
+        // K1e-partial: 8 warps per CTA where the staging image and 8 per-warp blocks fit the 227 KB a CTA may have,
+        // else 4, 2 or 1 (the chunked 2 020-point units take 4)
+        for (auto& cl : ctx->classes) {
+            cl.ebp_warps = 0;
+            for (int wp = kWarpsPerCta; wp >= 1 && !cl.ebp_warps; wp /= 2)
+                if (cl.stage + wp * cl.ebp_warp <= (size_t)kMaxDynSmem) cl.ebp_warps = wp;
+            if (!cl.ebp_warps)
+                return set_err(ctx, MMRS_ERR_ARG, "partial cost: a unit does not fit the shared memory of one warp");
+            cl.smem_ebp = cl.stage + cl.ebp_warps * cl.ebp_warp;
         }
     }
     {   // tensor-core prefilter: every non-empty unit must fit its operand layout
@@ -504,7 +538,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
         ctx->lb_R = biggest >= 1024 ? 128 : 32;  // rows per lower-bound pass: k_lb<1,8> or k_lb<4,2>
         // the bound tier's staging images are only built for a batch that may use it (opts / context default / MMRS_PRUNE)
         const char* prune_env = std::getenv("MMRS_PRUNE");
-        const bool may_prune = !ctx->rigid && ((prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1);
+        const bool may_prune = !ctx->rigid && !ctx->partial && ((prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1);
         ctx->lb_shape_ok = ok && biggest > 0 && may_prune;
         ctx->h_units_lb.assign(2 * (size_t)U, UnitDesc{});
         long long off = 0;
@@ -603,6 +637,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         ctx->grid_of_unit[u] = g;
     }
     ctx->rigid = tgrids != nullptr;
+    const bool solo = ctx->rigid || ctx->partial;   // the dense sweep on this device alone: no tier, no partition
     std::vector<long long> tgrid_off(1, 0);
     if (ctx->rigid) {
         if (n_tgrids < 1) return set_err(ctx, MMRS_ERR_ARG, "rigid sweep: n_tgrids must be >= 1");
@@ -695,7 +730,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
     {
         const int world = ctx->shard_world, rank = ctx->shard_rank;
         int axis = ctx->opt_partition == 0 ? ctx->part_axis : ctx->opt_partition;
-        if (world <= 1 || (!ctx->comm && !ctx->exchange) || axis < 1 || axis > 2 || ctx->rigid) axis = 0;
+        if (world <= 1 || (!ctx->comm && !ctx->exchange) || axis < 1 || axis > 2 || solo) axis = 0;
         if (axis == 1 && ctx->opt_partition == 0) {
             // The context's default axis is a POLICY, decided from the shape of the batch alone (so every rank decides
             // alike): whole units where they balance; candidate sub-ranges where a handful of large units cannot be
@@ -755,8 +790,9 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         }
     // K1e per size class (MMRS_EARLY_BREAK: 0 = K1 everywhere, 1 = K1e wherever its shared memory fits). A class beyond
     // the per-warp A' and hints (sets above ~1 000 points, the chunked 2 020-point units among them) keeps K1.
+    // A partial run takes K1e-partial in every class (MMRS_EARLY_BREAK=0 only switches its early break off).
     for (auto& cl : ctx->classes)
-        cl.eb = ctx->eb_env != 0 && !cl.big && cl.smem_eb <= (ctx->eb_env == 1 ? (size_t)kMaxDynSmem : kEbAutoSmem);
+        cl.eb = !ctx->partial && ctx->eb_env != 0 && !cl.big && cl.smem_eb <= (ctx->eb_env == 1 ? (size_t)kMaxDynSmem : kEbAutoSmem);
     // work list: one CTA = one unit x one tile of candidates (8 warps, one candidate per warp per pass; K1e: one
     // contiguous run per warp, as long as the batch still gives ~4 waves of 3 CTAs per SM)
     {
@@ -772,8 +808,9 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             auto& cl = ctx->classes[k];
             cl.work_begin = ctx->h_work.size();
             const long long eb_slots = (long long)ctx->n_sm * 3 * 4 * kWarpsPerCta;
-            const int tile_k = cl.eb ? (int)(kWarpsPerCta * std::max(kEbMinRun, std::min(kEbMaxRun, (cl.live + eb_slots - 1) / eb_slots)))
-                                     : tile;
+            const long long run = std::max(kEbMinRun, std::min(kEbMaxRun, (cl.live + eb_slots - 1) / eb_slots));
+            // K1e-partial: K1e's run per warp, ebp_warps warps per CTA
+            const int tile_k = ctx->partial ? (int)(cl.ebp_warps * run) : cl.eb ? (int)(kWarpsPerCta * run) : tile;
             for (int64_t u = 0; u < U; ++u) {
                 const UnitDesc& d = units[u];
                 if (d.flags || ctx->class_of_unit[u] != (int)k) continue;
@@ -790,11 +827,11 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             if (!d.flags) ++live_units;
         const char* env = std::getenv("MMRS_PREFILTER");  // experiments: 0 = off, 1 = on where the shapes allow
         int mode = ctx->opt_prefilter;
-        if (env && *env && !ctx->rigid) mode = (*env == '0') ? 1 : 2;
+        if (env && *env && !solo) mode = (*env == '0') ? 1 : 2;
         // auto (0) currently resolves to the dense FP32 sweep: on B200 the prefilter's per-tile TMEM hand-shakes and
         // the FMNMX-bound epilogue make K1t slower than K1 (17 vs 24 M evaluations/s, DESIGN.md §4).
-        ctx->use_tc = !ctx->rigid && mode == 2 && ctx->tc_shape_ok && live_units > 0 && ctx->part_active != 2;
-        if (mode == 2 && !ctx->use_tc && ctx->opt_prefilter == 2 && !ctx->rigid)
+        ctx->use_tc = !solo && mode == 2 && ctx->tc_shape_ok && live_units > 0 && ctx->part_active != 2;
+        if (mode == 2 && !ctx->use_tc && ctx->opt_prefilter == 2 && !solo)
             return set_err(ctx, MMRS_ERR_ARG,
                            "prefilter required but the batch does not fit the tensor-core operand layout (64 <= points "
                            "per set <= 2048)");
@@ -826,12 +863,12 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
     {
         const char* env = std::getenv("MMRS_XF");   // experiments: 1 = on for every batch that qualifies, 0 = off
         int mode = ctx->opt_prefilter;
-        if (env && *env && mode == 0 && !ctx->rigid) mode = (*env == '0') ? 1 : 3;
+        if (env && *env && mode == 0 && !solo) mode = (*env == '0') ? 1 : 3;
         if (mode == 0) mode = kXfDefault ? 3 : 1;
         // worth it when the sweep is long enough to pay for two extra launches (window + re-scoring)
         bool any_big = false;
         for (const auto& cl : ctx->classes) any_big = any_big || cl.big;
-        ctx->use_xf = !ctx->rigid && mode == 3 && !ctx->use_tc && !any_big && ctx->part_active != 2 &&
+        ctx->use_xf = !solo && mode == 3 && !ctx->use_tc && !any_big && ctx->part_active != 2 &&
                       live >= (ctx->opt_prefilter == 3 ? 1 : (1 << 20));
         if (ctx->use_xf) {
             ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>({(long long)U * 64, 65536LL, live / 32}),
@@ -850,8 +887,8 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             if (!d.flags) ++live_units;
         const char* env = std::getenv("MMRS_PRUNE");
         int mode = ctx->opt_prune;
-        if (env && *env && !ctx->rigid) mode = (*env == '0') ? 0 : 1;
-        ctx->use_prune = !ctx->rigid && mode == 1 && !ctx->use_tc && !ctx->use_xf && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units &&
+        if (env && *env && !solo) mode = (*env == '0') ? 0 : 1;
+        ctx->use_prune = !solo && mode == 1 && !ctx->use_tc && !ctx->use_xf && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units &&
                          ctx->part_active != 2;
         ctx->h_work_lb.clear();
         if (ctx->use_prune) {
@@ -943,9 +980,9 @@ static int check_tgrids(mmrs_ctx* ctx, const char* fn, int64_t n_units, const mm
     return MMRS_OK;
 }
 
-// Upload of a rotation-only batch (tgrids == NULL) or of a rigid one.
+// Upload of a rotation-only batch (tgrids == NULL) or of a rigid one; inlier_fraction < 1: the partial cost.
 static int upload_impl(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_sweep_opts* o, const mmrs_tgrid* tgrids,
-                       int64_t n_tgrids, const int32_t* tgrid_of_unit, const char* fn) {
+                       int64_t n_tgrids, const int32_t* tgrid_of_unit, const char* fn, double inlier_fraction = 1.0) {
     if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (!b || b->n_units < 0 || (b->n_units > 0 && (!b->test_off || !b->ref_off || !b->centre_xy || !b->grids)) ||
         (b->n_grids < 1 && b->n_units > 0))
@@ -957,10 +994,18 @@ static int upload_impl(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_swee
         if (o && (o->prefilter == 2 || o->prefilter == 3))
             return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3 is not supported with a translation grid");
     }
+    const bool partial = inlier_fraction < 1.0;
+    if (partial) {
+        if (o && o->prune > 0) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prune is not supported with the partial cost");
+        if (o && (o->prefilter == 2 || o->prefilter == 3))
+            return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3 is not supported with the partial cost");
+    }
     ENTER_DEVICE(ctx);
     ctx->ready = false;
     ctx->ran = false;
     ctx->rigid = tgrids != nullptr;
+    ctx->partial = partial;
+    ctx->inlier_fraction = inlier_fraction;
     ctx->n_units = b->n_units;
     ctx->mode = b->mode;
     {
@@ -1014,6 +1059,20 @@ extern "C" int mmrs_rigid_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b,
     return upload_impl(ctx, b, o, tgrids, n_tgrids, tgrid_of_unit, "mmrs_rigid_sweep_upload");
 }
 
+extern "C" int mmrs_partial_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_tgrid* tgrids,
+                                         int64_t n_tgrids, const int32_t* tgrid_of_unit, double inlier_fraction,
+                                         const mmrs_sweep_opts* o) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_partial_sweep_upload: ctx is NULL");
+    if (!std::isfinite(inlier_fraction) || !(inlier_fraction > 0.0) || inlier_fraction > 1.0)
+        return set_err(ctx, MMRS_ERR_ARG, "mmrs_partial_sweep_upload: inlier_fraction must be finite with 0 < f <= 1");
+    if (!tgrids && (n_tgrids || tgrid_of_unit)) return set_err(ctx, MMRS_ERR_ARG, "mmrs_partial_sweep_upload: bad translation grids");
+    return upload_impl(ctx, b, o, tgrids, n_tgrids, tgrid_of_unit,
+                       inlier_fraction < 1.0 ? "mmrs_partial_sweep_upload"
+                       : tgrids              ? "mmrs_rigid_sweep_upload"
+                                             : "mmrs_sweep_upload",
+                       inlier_fraction);
+}
+
 static int regrid_impl(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
                        const mmrs_tgrid* tgrids, int64_t n_tgrids, const int32_t* tgrid_of_unit, double tie_margin,
                        const char* fn) {
@@ -1054,6 +1113,7 @@ extern "C" int mmrs_rigid_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, in
 struct ExactPlan {
     int smem, grid;
     double2* scratch;
+    double* mins = nullptr;   // partial cost: the CTAs' row minima in global memory (with scratch)
 };
 static int exact_plan(mmrs_ctx* ctx, int max_pts, int want_grid, ExactPlan* p) {
     const long long smem = 64 + 2LL * max_pts * 16;
@@ -1066,6 +1126,19 @@ static int exact_plan(mmrs_ctx* ctx, int max_pts, int want_grid, ExactPlan* p) {
     *p = ExactPlan{64, grid, (double2*)ctx->d_exact_scratch.p};
     return MMRS_OK;
 }
+// The same for the partial cost, which also keeps the row minima of one direction (max_pts doubles per CTA).
+static int exact_plan_partial(mmrs_ctx* ctx, int max_pts, int want_grid, ExactPlan* p) {
+    const long long smem = 64 + 2LL * max_pts * 16 + (long long)max_pts * 8;
+    if (smem <= kMaxDynSmem) {
+        *p = ExactPlan{(int)smem, want_grid, nullptr};
+        return MMRS_OK;
+    }
+    const int grid = std::max(1, std::min(want_grid, ctx->n_sm * 2));
+    ENSURE(ctx->d_exact_scratch, (size_t)grid * max_pts * 24);
+    *p = ExactPlan{64, grid, (double2*)ctx->d_exact_scratch.p,
+                   (double*)((char*)ctx->d_exact_scratch.p + (size_t)grid * max_pts * 16)};
+    return MMRS_OK;
+}
 
 // f64 recheck of every candidate of `unit` (shortlist overflow): leftmost arg-min on the host
 // over device-computed reference-arithmetic distances.
@@ -1073,13 +1146,22 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     const UnitDesc& d = ctx->h_units[u];
     ENSURE(ctx->d_tmp, (size_t)d.n_cand * 8);
     ExactPlan ep;
-    if (int rc = exact_plan(ctx, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
-    CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
-    k_exact_dense<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u,
-                                                          (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-                                                          (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
-                                                          d.cand_off, d.n_cand, (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch,
-                                                          ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
+    if (ctx->partial) {
+        if (int rc = exact_plan_partial(ctx, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
+        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense_partial));
+        k_exact_dense_partial<<<ep.grid, 256, ep.smem, ctx->stream>>>(
+            (const UnitDesc*)ctx->d_units.p, (int)u, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
+            (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p, d.cand_off, d.n_cand, (double*)ctx->d_tmp.p,
+            ctx->max_pts, ep.scratch, ep.mins, ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
+    } else {
+        if (int rc = exact_plan(ctx, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
+        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
+        k_exact_dense<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u,
+                                                              (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
+                                                              (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
+                                                              d.cand_off, d.n_cand, (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch,
+                                                              ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
+    }
     CUDA_TRY(ctx, cudaGetLastError());
     std::vector<double> h(d.n_cand);
     CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), ctx->d_tmp.p, (size_t)d.n_cand * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1312,6 +1394,24 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
                 ctx->launches += 1;
                 continue;
             }
+            if (ctx->partial) {   // K1e-partial (every class: big units are refused at upload)
+                if (!ctx->eb_ran) {
+                    ENSURE(ctx->d_eb_pairs, 8);
+                    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
+                    ctx->eb_ran = true;
+                }
+                if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<true>));
+                else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<false>));
+                auto ebp = t32 ? k_sweep_ebp<true> : k_sweep_ebp<false>;
+                ebp<<<(unsigned)cl.work_count, cl.ebp_warps * 32, cl.smem_ebp, s>>>(
+                    units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
+                    (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
+                    (unsigned long long*)ctx->d_eb_pairs.p, t32, ctx->eb_env != 0 ? 1 : 0);
+                CUDA_TRY(ctx, cudaGetLastError());
+                ctx->eb_cands += cl.live;
+                ctx->launches += 1;
+                continue;
+            }
             if (cl.eb) {
                 if (!ctx->eb_ran) {
                     ENSURE(ctx->d_eb_pairs, 8);
@@ -1356,12 +1456,21 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
     {
         ExactPlan ep;
-        if (int rc = exact_plan(ctx, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
-        CUDA_TRY(ctx, RAISE_SMEM(k_exact));
-        k_exact<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-                                              (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
-                                              (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
-                                              (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, t64);
+        if (ctx->partial) {
+            if (int rc = exact_plan_partial(ctx, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
+            CUDA_TRY(ctx, RAISE_SMEM(k_exact_partial));
+            k_exact_partial<<<ep.grid, 256, ep.smem, s>>>(
+                units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p, (const double2*)ctx->d_cs64.p,
+                (const unsigned char*)ctx->d_zero.p, (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p,
+                ctx->pool_cap, (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, ep.mins, t64);
+        } else {
+            if (int rc = exact_plan(ctx, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
+            CUDA_TRY(ctx, RAISE_SMEM(k_exact));
+            k_exact<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
+                                                  (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
+                                                  (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
+                                                  (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, t64);
+        }
         CUDA_TRY(ctx, cudaGetLastError());
         k_select<<<(unsigned)((U + 7) / 8), 256, 0, s>>>(units, (int)U, (const double2*)ctx->d_cs64.p,
                                                          (const int2*)ctx->d_items.p,
@@ -1599,12 +1708,27 @@ extern "C" int mmrs_last_timings(mmrs_ctx* ctx, float ms_out[4], int32_t* launch
 
 // ---- explicit-angle exact evaluation ----------------------------------------------------
 // txy == NULL: rotation only; otherwise candidate k is (angles[k], txy[2k], txy[2k+1]).
+// inlier_fraction < 1: the partial cost, on the finite points of each set (as the sweep uploads them).
 static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
                            double cx, double cy, int32_t mode, const double* angles, const double* txy, int64_t n_angles,
-                           double* dist_out, const char* fn) {
+                           double* dist_out, const char* fn, double inlier_fraction = 1.0) {
     if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (n_test < 0 || n_ref < 0 || n_angles < 0 || (n_angles > 0 && (!angles || !dist_out)))
         return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad arguments");
+    const bool partial = inlier_fraction < 1.0;
+    std::vector<double> f_test, f_ref;
+    if (partial) {
+        if ((n_test > 0 && !test_xy) || (n_ref > 0 && !ref_xy)) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad arguments");
+        auto finite = [](const double* xy, int64_t n, std::vector<double>& out) {
+            for (int64_t i = 0; i < n; ++i)
+                if (std::isfinite(xy[2 * i]) && std::isfinite(xy[2 * i + 1])) out.push_back(xy[2 * i]), out.push_back(xy[2 * i + 1]);
+        };
+        finite(test_xy, n_test, f_test);
+        finite(ref_xy, n_ref, f_ref);
+        test_xy = f_test.data(), n_test = (int64_t)f_test.size() / 2;
+        ref_xy = f_ref.data(), n_ref = (int64_t)f_ref.size() / 2;
+        if (n_test > (1 << 24) || n_ref > (1 << 24)) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": too many points");
+    }
     if (n_angles == 0) return MMRS_OK;
     if (n_test == 0 || n_ref == 0) {  // process_utils.rs:86-88
         for (int64_t i = 0; i < n_angles; ++i) dist_out[i] = 0.0;
@@ -1634,6 +1758,8 @@ static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test,
     d.cx = cx;
     d.cy = cy;
     d.n_trans = 1;
+    d.q_fwd = (short)partial_q(inlier_fraction, d.m);
+    d.q_bwd = (short)partial_q(inlier_fraction, d.n);
     if (txy) CUDA_TRY(ctx, cudaMemcpyAsync(base + o_t, txy, b_cs, cudaMemcpyHostToDevice, s));
     CUDA_TRY(ctx, cudaMemcpyAsync(base, test_xy, (size_t)n_test * 16, cudaMemcpyHostToDevice, s));
     CUDA_TRY(ctx, cudaMemcpyAsync(base + (size_t)n_test * 16, ref_xy, (size_t)n_ref * 16, cudaMemcpyHostToDevice, s));
@@ -1642,13 +1768,23 @@ static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test,
     CUDA_TRY(ctx, cudaMemcpyAsync(base + o_unit, &d, sizeof(UnitDesc), cudaMemcpyHostToDevice, s));
     const int max_n = (int)std::max(n_test, n_ref);
     ExactPlan ep;
-    if (int rc = exact_plan(ctx, max_n, (int)std::min<int64_t>(n_angles, (int64_t)ctx->n_sm * 8), &ep)) return rc;
-    CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
-    k_exact_dense<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
-                                                (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
-                                                (const unsigned char*)(base + o_zero), 0, (int)n_angles,
-                                                (double*)(base + o_out), max_n, ep.scratch,
-                                                txy ? (const double2*)(base + o_t) : nullptr, true);
+    const int want_grid = (int)std::min<int64_t>(n_angles, (int64_t)ctx->n_sm * 8);
+    if (partial) {
+        if (int rc = exact_plan_partial(ctx, max_n, want_grid, &ep)) return rc;
+        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense_partial));
+        k_exact_dense_partial<<<ep.grid, 256, ep.smem, s>>>(
+            (const UnitDesc*)(base + o_unit), 0, (const double*)base, (const double*)(base + (size_t)n_test * 16),
+            (const double2*)(base + o_cs), (const unsigned char*)(base + o_zero), 0, (int)n_angles, (double*)(base + o_out),
+            max_n, ep.scratch, ep.mins, txy ? (const double2*)(base + o_t) : nullptr, true);
+    } else {
+        if (int rc = exact_plan(ctx, max_n, want_grid, &ep)) return rc;
+        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
+        k_exact_dense<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
+                                                    (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
+                                                    (const unsigned char*)(base + o_zero), 0, (int)n_angles,
+                                                    (double*)(base + o_out), max_n, ep.scratch,
+                                                    txy ? (const double2*)(base + o_t) : nullptr, true);
+    }
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(dist_out, base + o_out, b_out, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1669,6 +1805,15 @@ extern "C" int mmrs_eval_exact_rigid(mmrs_ctx* ctx, const double* test_xy, int64
     if (n_cand > 0 && !txy) return set_err(ctx, MMRS_ERR_ARG, "mmrs_eval_exact_rigid: txy is NULL");
     return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, txy, n_cand, dist_out,
                            "mmrs_eval_exact_rigid");
+}
+
+extern "C" int mmrs_eval_exact_partial(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy,
+                                       int64_t n_ref, double cx, double cy, int32_t mode, const double* angles,
+                                       const double* txy, int64_t n_cand, double inlier_fraction, double* dist_out) {
+    if (!std::isfinite(inlier_fraction) || !(inlier_fraction > 0.0) || inlier_fraction > 1.0)
+        return set_err(ctx, MMRS_ERR_ARG, "mmrs_eval_exact_partial: inlier_fraction must be finite with 0 < f <= 1");
+    return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, txy, n_cand, dist_out,
+                           "mmrs_eval_exact_partial", inlier_fraction);
 }
 
 // ---- FP32 peak probe ------------------------------------------------------------------------

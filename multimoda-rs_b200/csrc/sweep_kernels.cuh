@@ -782,6 +782,274 @@ __global__ void __launch_bounds__(kThreads, 3)
 }
 
 // =============================================================================
+// K1e-partial (k_sweep_ebp): the early-break sweep for the PARTIAL cost (include/mmrs_b200.h "partial cost"). In each
+// direction the directed value is the (q + 1)-th largest row minimum instead of the largest, so the q worst points of
+// each set do not count. Same work items, staging image and outputs as K1e; per warp, over its contiguous run:
+//   lists   per direction the q + 1 largest EXACT minima found so far (float bits + point index) in per-warp shared
+//           memory; kth = the smallest of them when the list is full, else 0; L = max(kth_rows, kth_cols);
+//   seed    the rows of the previous candidate's list in the direction that defined its value (the run's first
+//           candidate: the q + 1 points farthest from the centre, both directions), each scanned to its end by one
+//           lane; they enter the list and are marked so that the main pass skips them;
+//   rows    exactly K1e's passes: zig-zag tries from the hints, then the warp finishes the open rows; a row stops at
+//           the first d^2 <= L; a row that scans to its end has an exact minimum > L and enters its list (replacing
+//           the smallest entry when full); L is recomputed;
+//   columns the same with the reference points as rows.
+// Exactness (F = max(V_r, V_c), V the true (q + 1)-th largest FP32 minimum of a direction): L is always the (q + 1)-th
+// largest of a subset of exact minima, so L <= F; a row that was not collected has a minimum <= L at that time <=
+// L_final; if V_r > L_final, all q + 1 rows of the true top q + 1 were collected and the list's kth is V_r; otherwise
+// kth_r <= V_r <= L_final. Hence L_final = F, bit for bit, and with q = 0 this is K1e. early = 0 (MMRS_EARLY_BREAK=0):
+// no row stops early (every row is scanned to its end by one lane), the bit-for-bit test partner.
+// =============================================================================
+constexpr int kPartialMaxQ = 255;   // points per direction and unit that may be left out (the list holds q + 1 <= 256)
+
+// per-warp shared memory of K1e-partial: K1e's block (A', row / column hints), then for rows and for columns the list
+// (q + 1 float bits, q + 1 indices) and a bit set of the seeded points
+__host__ __device__ constexpr int ebp_warp_bytes(int n, int m, int q_r, int q_c) {
+    return (eb_warp_bytes(n, m) + 8 * (q_r + 1) + 8 * (q_c + 1) + 4 * ((n + 31) / 32 + (m + 31) / 32) + 15) & ~15;
+}
+
+// The q + 1 largest exact minima of one direction found so far. cnt, kth and at are warp-uniform.
+struct EbList {
+    unsigned* val;
+    int* idx;
+    int cap, cnt;
+    unsigned kth;   // smallest entry when the list is full, else 0
+    int at;         // its slot
+};
+__device__ __forceinline__ void ebl_refresh(EbList& l, int lane) {
+    __syncwarp();
+    if (l.cnt < l.cap) {
+        l.kth = 0u;
+        return;
+    }
+    unsigned mn = ~0u;
+    int at = 0;
+    for (int k = lane; k < l.cap; k += 32)
+        if (l.val[k] < mn) mn = l.val[k], at = k;
+    const unsigned m = __reduce_min_sync(0xffffffffu, mn);
+    l.at = __shfl_sync(0xffffffffu, at, __ffs(__ballot_sync(0xffffffffu, mn == m)) - 1);
+    l.kth = m;
+}
+// v: an exact minimum > kth (warp-uniform arguments)
+__device__ __forceinline__ void ebl_insert(EbList& l, unsigned v, int i, int lane) {
+    const int k = l.cnt < l.cap ? l.cnt++ : l.at;
+    if (lane == 0) l.val[k] = v, l.idx[k] = i;
+    ebl_refresh(l, lane);
+}
+// Exact minimum of d^2(a, P[j]) over the n points of P by ONE lane, in index order (the warp's lanes read the same P[j]:
+// a broadcast); arg = where it was first found.
+__device__ __forceinline__ unsigned eb_lane_min(const float2* P, int n, float2 a, int& arg, unsigned& pairs) {
+    unsigned best = ~0u;
+    int bj = 0;
+    for (int j = 0; j < n; ++j) {
+        const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+        if (d < best) best = d, bj = j;
+    }
+    pairs += (unsigned)n;
+    arg = bj;
+    return best;
+}
+
+// RIGID: as in k_sweep_eb. Warps per CTA = blockDim.x / 32 (the host picks 8, 4, 2 or 1 per size class).
+template <bool RIGID>
+__global__ void __launch_bounds__(kThreads, 2)
+    k_sweep_ebp(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
+                const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
+                unsigned long long* __restrict__ pairs_out, const float2* __restrict__ t32, int early) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
+    unsigned long long* s_key = reinterpret_cast<unsigned long long*>(smem_raw + 8);
+    float4* sA = reinterpret_cast<float4*>(smem_raw + 16);
+    const WorkItem w = work[blockIdx.x];
+    const UnitDesc ud = units[w.unit];
+    const int n_warps = blockDim.x >> 5;
+    const int lane = threadIdx.x & 31, wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
+    const int TA = ud.ta, S = (TA + 1) / 2, N = ud.n, M = ud.m, n_main = N - ud.n_tail;
+    const int a_elems = ud.n_chunks * S * 32;
+    const int b_elems = ud.n_tail > 0 ? 16 * (TA + 1) : ud.m_pairs;
+    const int nb_elems = (b_elems + 1) / 2, t_elems = (ud.n_tail + 1) / 2;
+    const float4* sB4 = sA + a_elems;
+    const float2* sB = reinterpret_cast<const float2*>(sB4);
+    const float2* sT = reinterpret_cast<const float2*>(sB4 + b_elems + nb_elems);
+    unsigned char* my = reinterpret_cast<unsigned char*>(sA + a_elems + b_elems + nb_elems + t_elems) +
+                        wid * ebp_warp_bytes(N, M, ud.q_bwd, ud.q_fwd);
+    float2* sR = reinterpret_cast<float2*>(my);
+    unsigned short* hint[2];
+    hint[0] = reinterpret_cast<unsigned short*>(sR + N);   // rows: test point i against the reference points
+    hint[1] = hint[0] + N;                                 // columns: reference point j against A'
+    unsigned* lp = reinterpret_cast<unsigned*>(my + eb_warp_bytes(N, M));
+    EbList lst[2];
+    lst[0].cap = ud.q_bwd + 1, lst[1].cap = ud.q_fwd + 1;
+    lst[0].val = lp;
+    lst[0].idx = reinterpret_cast<int*>(lp + lst[0].cap);
+    lst[1].val = lp + 2 * lst[0].cap;
+    lst[1].idx = reinterpret_cast<int*>(lst[1].val + lst[1].cap);
+    unsigned* bits[2];
+    bits[0] = lp + 2 * (lst[0].cap + lst[1].cap);
+    bits[1] = bits[0] + (N + 31) / 32;
+    const int n_rows[2] = {N, M};
+    if (threadIdx.x == 0) {
+        mbar_init(bar, 1);
+        *s_key = ~0ull;
+        const uint32_t bytes = (uint32_t)(a_elems + b_elems + nb_elems + t_elems) * 16u;
+        mbar_expect_tx(bar, bytes);
+        tma_bulk_g2s(sA, lay + ud.lay_off, bytes, bar);
+    }
+    __syncthreads();
+    mbar_wait(bar, 0);
+
+    auto test_pt = [&](int i) -> float2 {
+        if (i >= n_main) return sT[i - n_main];
+        const int c = i / (32 * TA), r = i - c * 32 * TA;
+        const float4 v = sA[(c * S + (r >> 6)) * 32 + (r & 31)];
+        return (r & 32) ? make_float2(v.y, v.w) : make_float2(v.x, v.z);
+    };
+    // direction 0: rows = A' against the reference points; direction 1: columns = reference points against A'
+    auto row_pt = [&](int dir, int r) -> float2 { return dir ? sB[r] : sR[r]; };
+    auto set_of = [&](int dir) -> const float2* { return dir ? sR : sB; };
+    const int per = (w.count + n_warps - 1) / n_warps;
+    const int c_begin = w.begin + min(w.count, wid * per), c_end = w.begin + min(w.count, (wid + 1) * per);
+    unsigned long long best = ~0ull;
+    unsigned pairs = 0;
+    if (c_begin < c_end) {
+        bool seed[2] = {true, true};
+#pragma unroll
+        for (int dir = 0; dir < 2; ++dir) {
+            const int n = n_rows[dir];
+            for (int k = lane; k < (n + 31) / 32; k += 32) bits[dir][k] = 0u;
+            for (int r = lane; r < n; r += 32)
+                hint[dir][r] = (unsigned short)(((long long)r * n_rows[1 - dir]) / n);
+            __syncwarp();
+            // first candidate's seeds: the q + 1 points farthest from the rotation centre (unrotated)
+            EbList& l = lst[dir];
+            for (int k = 0; k < l.cap; ++k) {
+                unsigned far = 0u;
+                int at = 0;
+                for (int r = lane; r < n; r += 32) {
+                    if ((bits[dir][r >> 5] >> (r & 31)) & 1u) continue;
+                    const float2 p = dir ? sB[r] : test_pt(r);
+                    const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y) + 1u;   // > 0: not yet taken
+                    if (r2 > far) far = r2, at = r;
+                }
+                const int r = eb_warp_argmax(far, at);
+                if (lane == 0) {
+                    l.idx[k] = r;
+                    bits[dir][r >> 5] |= 1u << (r & 31);
+                }
+                __syncwarp();
+            }
+            l.cnt = l.cap;
+        }
+        for (int c = c_begin; c < c_end; ++c) {
+            float2 tr = make_float2(0.f, 0.f);
+            int ia = c;
+            if (RIGID) {
+                ia = c / ud.n_trans;
+                tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
+            }
+            const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
+            __syncwarp();   // the previous candidate is done with A', the hints and the lists
+            for (int i = lane; i < N; i += 32) {
+                const float2 p = test_pt(i);
+                float2 r = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
+                if (RIGID) r = make_float2(__fadd_rn(r.x, tr.x), __fadd_rn(r.y, tr.y));
+                sR[i] = r;
+            }
+            __syncwarp();
+            // seeds: the listed rows of the seeded directions, one lane each, scanned to the end
+#pragma unroll
+            for (int dir = 0; dir < 2; ++dir) {
+                EbList& l = lst[dir];
+                if (!seed[dir]) {
+                    l.cnt = 0;
+                    l.kth = 0u;
+                    continue;
+                }
+                for (int k = lane; k < l.cnt; k += 32) {
+                    const int r = l.idx[k];
+                    int arg;
+                    l.val[k] = eb_lane_min(set_of(dir), n_rows[1 - dir], row_pt(dir, r), arg, pairs);
+                    hint[dir][r] = (unsigned short)arg;
+                    atomicOr(&bits[dir][r >> 5], 1u << (r & 31));
+                }
+                ebl_refresh(l, lane);
+            }
+            unsigned L = max(lst[0].kth, lst[1].kth);
+#pragma unroll
+            for (int dir = 0; dir < 2; ++dir) {
+                const int n = n_rows[dir], n_set = n_rows[1 - dir];
+                const float2* P = set_of(dir);
+                unsigned short* h = hint[dir];
+                EbList& l = lst[dir];
+                for (int g = 0; g < n; g += 32) {
+                    const int i = g + lane;
+                    bool open = i < n && !((bits[dir][i >> 5] >> (i & 31)) & 1u);
+                    if (!early) {
+                        // every open row scanned to its end by its lane; the exact minima > L enter the list in lane order
+                        unsigned mn = ~0u;
+                        if (open) {
+                            int arg;
+                            mn = eb_lane_min(P, n_set, row_pt(dir, i), arg, pairs);
+                            h[i] = (unsigned short)arg;
+                        }
+                        for (unsigned m = __ballot_sync(0xffffffffu, open); m; m &= m - 1) {
+                            const int src = __ffs(m) - 1;
+                            const unsigned v = __shfl_sync(0xffffffffu, mn, src);
+                            if (v > L) {
+                                ebl_insert(l, v, g + src, lane);
+                                L = max(lst[0].kth, lst[1].kth);
+                            }
+                        }
+                        continue;
+                    }
+                    if (open) {
+                        const float2 a = row_pt(dir, i);
+                        const int h0 = h[i];
+                        for (int t = 0; t < kEbTries && t < n_set; ++t) {
+                            const int j = eb_zig(h0, t, n_set);
+                            ++pairs;
+                            if (__float_as_uint(eb_d2(a, P[j])) <= L) {
+                                h[i] = (unsigned short)j;
+                                open = false;
+                                break;
+                            }
+                        }
+                    }
+                    for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
+                        const int ii = g + __ffs(open_mask) - 1;
+                        int arg;
+                        const unsigned mn = eb_warp_min(P, n_set, row_pt(dir, ii), h[ii], L, true, lane, arg, pairs);
+                        __syncwarp();
+                        if (lane == 0) h[ii] = (unsigned short)arg;
+                        if (mn > L) {
+                            ebl_insert(l, mn, ii, lane);
+                            L = max(lst[0].kth, lst[1].kth);
+                        }
+                    }
+                }
+            }
+            const float d = sqrtf(__uint_as_float(L));
+            if (lane == 0) {
+                dist32[ud.dist_off + c] = d;
+                best = min(best, ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)c);
+            }
+            // the next candidate seeds the direction that defined this value (ties: rows) from this list
+            seed[0] = lst[0].kth >= lst[1].kth;
+            seed[1] = !seed[0];
+            __syncwarp();
+#pragma unroll
+            for (int dir = 0; dir < 2; ++dir)
+                for (int k = lane; k < (n_rows[dir] + 31) / 32; k += 32) bits[dir][k] = 0u;
+        }
+    }
+    const unsigned warp_pairs = __reduce_add_sync(0xffffffffu, pairs);
+    if (lane == 0 && pairs_out && warp_pairs) atomicAdd(pairs_out, (unsigned long long)warp_pairs);
+    if (lane == 0 && best != ~0ull) atomicMin(s_key, best);
+    __syncthreads();
+    if (threadIdx.x == 0 && *s_key != ~0ull) atomicMin(&key[w.unit], *s_key);
+}
+
+// =============================================================================
 // K1b: the FP32 sweep for units that do not fit K1's shared-memory staging (more than ~4 000 points per set; the
 // reference has no size limit, process_utils.rs:84-121). Same arithmetic as K1's chunked flavour (one warp = one
 // candidate, TA = 16 test points per lane and chunk, packed f32x2, 3-input minima, one REDUX per reference point), but
@@ -1289,6 +1557,123 @@ __global__ void __launch_bounds__(256)
         const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
         const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr,
                                     t64 != nullptr, t);
+        if (threadIdx.x == 0) out[c] = d;
+        __syncthreads();
+    }
+}
+
+// ---- K3 for the partial cost --------------------------------------------------------------------------------------
+// (q + 1)-th largest of the n non-negative values v (duplicates counted), by the whole CTA: the v_i with
+// #{v_j > v_i} <= q < #{v_j >= v_i}. Every i that satisfies this holds the same value, so the result does not depend
+// on the order of the threads.
+__device__ __forceinline__ double block_kth_largest(const double* v, int n, int q, double* s_red) {
+    double sel = 0.0;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const double x = v[i];
+        int gt = 0, ge = 0;
+        for (int j = 0; j < n && gt <= q; ++j) {
+            const double y = v[j];
+            gt += y > x ? 1 : 0;
+            ge += y >= x ? 1 : 0;
+        }
+        if (gt <= q && q < ge) sel = x;
+    }
+    return block_max(sel, s_red);
+}
+
+// exact_cost with the partial cost: each directed value is the (q + 1)-th largest row minimum (a non-finite minimum
+// counts as 0) instead of the largest. s_min: n (or m) doubles of the CTA (shared memory or a global scratch row).
+__device__ __forceinline__ double exact_cost_partial(const UnitDesc& ud, const double* __restrict__ test_xy,
+                                                     const double* __restrict__ ref_xy, double cosv, double sinv,
+                                                     bool identity, double2* s_rot, const double2* s_ref_in, double* s_red,
+                                                     double* s_min, bool copy_ref, bool rigid, double2 t) {
+    double2* s_ref_w = const_cast<double2*>(s_ref_in);
+    const double2* s_ref = copy_ref ? s_ref_in : reinterpret_cast<const double2*>(ref_xy + 2 * ud.ref_off);
+    for (int i = threadIdx.x; i < ud.n; i += blockDim.x) {
+        const double px = test_xy[2 * (ud.test_off + i)], py = test_xy[2 * (ud.test_off + i) + 1];
+        double rx = px, ry = py;
+        if (!identity) {
+            const double x = __dsub_rn(px, ud.cx), y = __dsub_rn(py, ud.cy);
+            rx = __dadd_rn(__dsub_rn(__dmul_rn(x, cosv), __dmul_rn(y, sinv)), ud.cx);
+            ry = __dadd_rn(__dadd_rn(__dmul_rn(x, sinv), __dmul_rn(y, cosv)), ud.cy);
+        }
+        if (rigid) rx = __dadd_rn(rx, t.x), ry = __dadd_rn(ry, t.y);
+        s_rot[i] = make_double2(rx, ry);
+    }
+    if (copy_ref)
+        for (int j = threadIdx.x; j < ud.m; j += blockDim.x)
+            s_ref_w[j] = make_double2(ref_xy[2 * (ud.ref_off + j)], ref_xy[2 * (ud.ref_off + j) + 1]);
+    __syncthreads();
+    const double INF = __longlong_as_double(0x7ff0000000000000LL);
+    auto directed = [&](const double2* rows, int nr, const double2* set, int ns, int q) {
+        for (int i = threadIdx.x; i < nr; i += blockDim.x) {
+            const double2 a = rows[i];
+            double mn = INF;
+            for (int j = 0; j < ns; ++j) {
+                const double2 b = set[j];
+                const double dx = __dsub_rn(a.x, b.x), dy = __dsub_rn(a.y, b.y);
+                const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
+                if (d2 < mn) mn = d2;
+            }
+            s_min[i] = isfinite(mn) ? mn : 0.0;
+        }
+        __syncthreads();
+        return block_kth_largest(s_min, nr, q, s_red);   // ends with a barrier: s_min may be reused
+    };
+    const double fwd = directed(s_ref, ud.m, s_rot, ud.n, ud.q_fwd);   // reference -> transformed
+    const double bwd = directed(s_rot, ud.n, s_ref, ud.m, ud.q_bwd);   // transformed -> reference
+    return fmax(__dsqrt_rn(fwd), __dsqrt_rn(bwd));
+}
+
+// k_exact / k_exact_dense for the partial cost; g_min != NULL: the CTA's row minima in a global scratch row (with
+// g_scratch), else shared memory after the two staged sets.
+__global__ void __launch_bounds__(256)
+    k_exact_partial(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
+                    const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
+                    const int2* __restrict__ items, const unsigned* __restrict__ n_items, unsigned pool_cap,
+                    double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min,
+                    const double2* __restrict__ t64) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    double* s_red = reinterpret_cast<double*>(smem_raw);
+    double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
+    double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
+    double* s_min = g_min ? g_min + (size_t)blockIdx.x * max_n : reinterpret_cast<double*>(s_ref + max_n);
+    const unsigned total = min(*n_items, pool_cap);
+    for (unsigned it = blockIdx.x; it < total; it += gridDim.x) {
+        const int2 item = items[it];
+        if (item.x < 0) continue;  // uniform per CTA
+        const UnitDesc ud = units[item.x];
+        const int c = item.y;
+        const int i = t64 ? c / ud.n_trans : c;
+        const double2 cs = cs64[ud.cand_off + i];
+        const bool identity = zero_flag[ud.cand_off + i] != 0;
+        const double2 t = t64 ? t64[ud.t_off + (c - i * ud.n_trans)] : make_double2(0.0, 0.0);
+        const double d = exact_cost_partial(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+                                            g_scratch == nullptr, t64 != nullptr, t);
+        if (threadIdx.x == 0) sl_dist[it] = d;
+        __syncthreads();
+    }
+}
+
+__global__ void __launch_bounds__(256)
+    k_exact_dense_partial(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
+                          const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
+                          const unsigned char* __restrict__ zero_flag, long long cs_off, int count, double* __restrict__ out,
+                          int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min,
+                          const double2* __restrict__ t64, bool paired) {
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    double* s_red = reinterpret_cast<double*>(smem_raw);
+    double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
+    double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
+    double* s_min = g_min ? g_min + (size_t)blockIdx.x * max_n : reinterpret_cast<double*>(s_ref + max_n);
+    const UnitDesc ud = units[unit];
+    for (int c = blockIdx.x; c < count; c += gridDim.x) {
+        const int i = (t64 && !paired) ? c / ud.n_trans : c;
+        const double2 cs = cs64[cs_off + i];
+        const bool identity = zero_flag[cs_off + i] != 0;
+        const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
+        const double d = exact_cost_partial(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+                                            g_scratch == nullptr, t64 != nullptr, t);
         if (threadIdx.x == 0) out[c] = d;
         __syncthreads();
     }

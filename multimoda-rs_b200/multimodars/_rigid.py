@@ -8,6 +8,7 @@ include/mmrs_b200.h "rigid candidates"). This has no reference counterpart; test
 from __future__ import annotations
 
 import math
+import numbers
 
 import numpy as np
 
@@ -55,7 +56,7 @@ def _finite_number(v, name):
 
 
 def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rotation_deg=90.0, step_translation=0.05,
-                              range_translation=0.25, centre=None, bruteforce=False):
+                              range_translation=0.25, centre=None, bruteforce=False, inlier_fraction=1.0):
     """Best rigid transform (rotation about `centre`, then translation) of `test` onto `reference`.
 
     Candidates: rotations on the grid of the rotation sweep (coarse-to-fine like find_best_rotation, or one stage
@@ -66,6 +67,9 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
 
     test, reference: one (N, >=2) array each (only x, y are used), or equal-length sequences of them; all pairs run
     as one batched sweep per stage. `centre`: one (x, y) for every pair, or one per pair.
+    inlier_fraction: f < 1 scores the partial (rank-K) Hausdorff distance instead (include/mmrs_b200.h "partial
+    cost"): in each direction the worst n - max(1, ceil(f n)) points of a set do not count, so a few artefact points
+    (a side-branch bulge, a calcification) do not decide the transform. 1.0 is the full distance.
     Returns a structured array, one row per pair: angle_rad, rotation_deg, tx, ty, distance, n_ties."""
     tests, refs = _as_sets(test, "test"), _as_sets(reference, "reference")
     if len(tests) != len(refs):
@@ -84,6 +88,11 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
         raise ValueError("step_translation must be > 0")
     if range_t < 0.0:
         raise ValueError("range_translation must be >= 0")
+    if isinstance(inlier_fraction, bool) or not isinstance(inlier_fraction, numbers.Real):
+        raise TypeError("inlier_fraction must be a number")
+    frac = _finite_number(inlier_fraction, "inlier_fraction")
+    if not 0.0 < frac <= 1.0:
+        raise ValueError("inlier_fraction must satisfy 0 < inlier_fraction <= 1")
     half_n = int(math.floor(range_t / step_t + 1e-9))
     if half_n > 1000:
         raise ValueError(f"range_translation / step_translation = {half_n} translations per side; at most 1000")
@@ -110,7 +119,10 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
     ctx = get_context()
     res = None
     for k, (step, window) in enumerate(stages):
-        if k == 0:   # stage 0 centred on 0; stage k > 0 on the previous stage's angle, clipped to +-range_rotation_deg
+        if k == 0 and frac < 1.0:
+            ctx.partial_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
+                               mode=1, inlier_fraction=frac)
+        elif k == 0:   # stage 0 centred on 0; stage k > 0 on the previous stage's angle, clipped to +-range_rotation_deg
             ctx.rigid_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
                              mode=1)
         else:
