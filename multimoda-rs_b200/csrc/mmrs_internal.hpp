@@ -32,6 +32,10 @@ struct UnitDesc {
 };
 constexpr int kFlagRemote = 0x400;  // internal UnitDesc.flags bit: another rank owns this unit (never leaves the library)
 
+// How a run scores its candidates: the dense sweep, or a tier that scores them approximately (or bounds them) and
+// re-scores a list with the exact FP32 sweep. The values are the codes mmrs_sweep_prefilter_info reports in out[0].
+enum Tier : int { kTierDense = 0, kTierTc = 1, kTierPrune = 2, kTierXf = 3 };
+
 struct WorkItem {
     int unit;
     int begin;  // first candidate
@@ -112,24 +116,24 @@ struct mmrs_ctx {
     mmrs::DevBuf d_test, d_ref, d_units, d_work, d_lay, d_cs64, d_cs32, d_zero, d_dist32, d_key, d_rmax, d_sl_base,
         d_sl_dist, d_sl_count, d_items, d_nitems, d_res, d_tmp;
 
+    // sweep tiers: K1t, K1x (expanded form, k_sweep<.., XF>) and K1p (lower-bound pruning)
+    mmrs::Tier tier = mmrs::kTierDense;       // decided per grid set (apply_grids)
+    mmrs::Tier tier_ran = mmrs::kTierDense;   // the last run's: the planned tier, or dense when it had no work
+
     // tensor-core prefilter tier (tc_kernels.cuh)
     int opt_prefilter = 0;      // mmrs_sweep_opts.prefilter: 0 auto, 1 off, 2 required
     bool tc_shape_ok = false;   // every live unit has kTcMinPts <= n, m <= kTcMaxPts (decided at upload)
-    bool use_tc = false;        // decided per grid set (apply_grids)
-    bool tc_ran = false;
-    bool use_xf = false, xf_ran = false;   // expanded-form tier K1x (k_sweep<.., XF>)
     double xf_abs = 8e-6;       // its tier-1 window: d^2 <= dmin^2 + xf_abs * Rmax^2 (>= 4.8x the proven error bound)
     double tc_abs = 4e-6;       // tier-1 window: d^2 <= dmin^2 + tc_abs * Rmax^2
     unsigned l1_cap = 0;
     size_t smem_tc = 0;
-    std::vector<mmrs::WorkItem> h_work_tc, h_work_list;
-    mmrs::DevBuf d_work_tc, d_work_list, d_key_tc, d_l1_items, d_l1_count, d_l1_base, d_l1_n;
+    std::vector<mmrs::WorkItem> h_work_tc;
+    mmrs::DevBuf d_work_tc, d_key_tc, d_l1_items, d_l1_count, d_l1_base, d_l1_n;
 
     // exact lower-bound pruning tier (k_lb, sweep_kernels.cuh)
     int opt_prune = 0;          // mmrs_sweep_opts.prune / mmrs_ctx_set_prune: 0 off, 1 on where the batch qualifies
     int ctx_prune = 0;          // context-wide default used when the opts do not say
     bool lb_shape_ok = false;   // every live unit has >= 128 points per set (decided at upload)
-    bool use_prune = false, prune_ran = false;
     int lb_R = 64;              // rows of a lower-bound unit (32 * TA_lb)
     size_t smem_lb = 0;
     std::vector<mmrs::UnitDesc> h_units_lb;   // [2 U]: pass A (test rows) then pass B (reference rows)

@@ -203,7 +203,7 @@ extern "C" void mmrs_ctx_destroy(mmrs_ctx* ctx) {
 void mmrs_ctx::free_all() {
     for (DevBuf* b : {&d_test, &d_ref, &d_units, &d_work, &d_lay, &d_cs64, &d_cs32, &d_zero, &d_dist32, &d_key,
                       &d_rmax, &d_sl_base, &d_sl_dist, &d_sl_count, &d_items, &d_nitems, &d_res, &d_tmp, &d_work_tc,
-                      &d_work_list, &d_key_tc, &d_l1_items, &d_l1_count, &d_l1_base, &d_l1_n, &d_units_lb, &d_lay_lb,
+                      &d_key_tc, &d_l1_items, &d_l1_count, &d_l1_base, &d_l1_n, &d_units_lb, &d_lay_lb,
                       &d_work_lb, &d_res_all, &d_cnt, &d_bcast, &d_big_rows, &d_exact_scratch, &d_eb_pairs}) {
         if (b->p) cudaFree(b->p);
         b->p = nullptr;
@@ -622,6 +622,97 @@ static inline void tgrid_offset(const mmrs_tgrid& t, int64_t j, double* tx, doub
     *ty = t.t0y + (double)(jy - t.half_n) * t.step;
 }
 
+// The tier of the uploaded grids, in order of precedence: the tensor-core prefilter K1t, the expanded form K1x, then
+// lower-bound pruning K1p. solo (rigid or partial candidates) and the candidate-axis partition take the dense sweep.
+// Sizes the tier's candidate list and builds its work list.
+static int plan_tier(mmrs_ctx* ctx, bool solo, long long live) {
+    const int64_t U = ctx->n_units;
+    const std::vector<UnitDesc>& units = ctx->h_units;
+    long long live_units = 0;
+    for (auto& d : units)
+        if (!d.flags) ++live_units;
+    bool any_big = false;
+    for (const auto& cl : ctx->classes) any_big = any_big || cl.big;
+    ctx->tier = kTierDense;
+    ctx->h_work_tc.clear();
+    ctx->h_work_lb.clear();
+    if (solo) return MMRS_OK;
+    const bool part2 = ctx->part_active == 2;
+    // Tensor-core prefilter: worth it when the units carry enough candidates to amortise the per-CTA operand set-up.
+    const char* env = std::getenv("MMRS_PREFILTER");  // experiments: 0 = off, 1 = on where the shapes allow
+    int tc_mode = ctx->opt_prefilter;
+    if (env && *env) tc_mode = (*env == '0') ? 1 : 2;
+    // auto (0) currently resolves to the dense FP32 sweep: on B200 the prefilter's per-tile TMEM hand-shakes and
+    // the FMNMX-bound epilogue make K1t slower than K1 (17 vs 24 M evaluations/s, DESIGN.md §4).
+    const bool tc = tc_mode == 2 && ctx->tc_shape_ok && live_units > 0 && !part2;
+    if (tc_mode == 2 && !tc && ctx->opt_prefilter == 2)
+        return set_err(ctx, MMRS_ERR_ARG,
+                       "prefilter required but the batch does not fit the tensor-core operand layout (64 <= points "
+                       "per set <= 2048)");
+    // Expanded-form tier K1x (k_sweep<.., XF>): the same work list and size classes as the dense sweep, 6 instead of 8
+    // packed FP32 instructions per 2 x 2 block; candidates inside its error window are re-scored in direct form.
+    env = std::getenv("MMRS_XF");   // experiments: 1 = on for every batch that qualifies, 0 = off
+    int xf_mode = ctx->opt_prefilter;
+    if (env && *env && xf_mode == 0) xf_mode = (*env == '0') ? 1 : 3;
+    if (xf_mode == 0) xf_mode = kXfDefault ? 3 : 1;
+    // worth it when the sweep is long enough to pay for two extra launches (window + re-scoring)
+    const bool xf = xf_mode == 3 && !any_big && !part2 && live >= (ctx->opt_prefilter == 3 ? 1 : (1 << 20));
+    // Lower-bound pruning: worth it when a unit carries enough candidates for the two extra passes to pay off.
+    env = std::getenv("MMRS_PRUNE");
+    int prune_mode = ctx->opt_prune;
+    if (env && *env) prune_mode = (*env == '0') ? 0 : 1;
+    const bool prune = prune_mode == 1 && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units && !part2;
+    ctx->tier = tc ? kTierTc : xf ? kTierXf : prune ? kTierPrune : kTierDense;
+    if (ctx->tier == kTierTc) {
+        long long tile = (live + (long long)ctx->n_sm * 6 - 1) / ((long long)ctx->n_sm * 6);
+        tile = std::max<long long>(64, std::min<long long>(tile, 512));
+        for (int64_t u = 0; u < U; ++u) {
+            const UnitDesc& d = units[u];
+            if (d.flags) continue;
+            const int parts = (int)((d.n_cand + tile - 1) / tile);
+            const int per = (d.n_cand + parts - 1) / parts;
+            for (int c0 = 0; c0 < d.n_cand; c0 += per)
+                ctx->h_work_tc.push_back(WorkItem{(int)u, c0, std::min(per, d.n_cand - c0), 0});
+        }
+        ctx->l1_cap = (unsigned)std::min<unsigned long long>(
+            std::max<unsigned long long>((unsigned long long)U * 256, 1ull << 20), 0x7fffffffull);
+        ENSURE(ctx->d_work_tc, ctx->h_work_tc.size() * sizeof(WorkItem));
+        ENSURE(ctx->d_key_tc, U * 8);
+    } else if (ctx->tier == kTierXf) {
+        ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>({(long long)U * 64, 65536LL, live / 32}),
+                                                    std::max<long long>(live, 1));
+        ENSURE(ctx->d_key_tc, U * 8);
+    } else if (ctx->tier == kTierPrune) {
+        for (int pass = 0; pass < 2; ++pass)
+            for (int64_t u = 0; u < U; ++u) {
+                UnitDesc& l = ctx->h_units_lb[u + pass * U];
+                const UnitDesc& d = units[u];
+                l.cand_off = d.cand_off, l.n_cand = d.n_cand, l.dist_off = d.dist_off;
+                l.flags = d.flags | (pass == 1 ? kLbNegSin : 0);
+            }
+        const long long slots = (long long)ctx->n_sm * 2 * 4;
+        long long per_warp = (2 * live + slots * kWarpsPerCta - 1) / (slots * kWarpsPerCta);
+        per_warp = std::max<long long>(8, std::min<long long>((per_warp + 7) / 8 * 8, 64));  // k_lb: 8 candidates per warp pass
+        const int tile = (int)per_warp * kWarpsPerCta;
+        for (int pass = 0; pass < 2; ++pass)
+            for (int64_t u = 0; u < U; ++u) {
+                const UnitDesc& d = units[u];
+                if (d.flags) continue;
+                for (int c0 = 0; c0 < d.n_cand; c0 += tile)
+                    ctx->h_work_lb.push_back(WorkItem{(int)(u + pass * U), c0, std::min(tile, d.n_cand - c0), 0});
+            }
+        ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>(ctx->total_cands, 1), 0x7fffffffLL);
+        ENSURE(ctx->d_work_lb, ctx->h_work_lb.size() * sizeof(WorkItem));
+    } else {
+        return MMRS_OK;
+    }
+    ENSURE(ctx->d_l1_items, (size_t)ctx->l1_cap * 8);
+    ENSURE(ctx->d_l1_count, U * 4);
+    ENSURE(ctx->d_l1_base, U * 4);
+    ENSURE(ctx->d_l1_n, 16);
+    return MMRS_OK;
+}
+
 // Grid part: candidate tables (host glibc cos/sin), per-unit candidate ranges, the CTA work list.
 // tgrids == NULL: rotation-only candidates (every unit has one translation, none applied). Otherwise rigid candidates:
 // unit u sweeps grid x tgrids[tgrid_of_unit[u]], candidate c = i T + j (angle i, translation j), densely and on this
@@ -820,104 +911,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             cl.work_count = ctx->h_work.size() - cl.work_begin;
         }
     }
-    // Tensor-core prefilter: worth it when the units carry enough candidates to amortise the per-CTA operand set-up.
-    {
-        long long live_units = 0;
-        for (auto& d : units)
-            if (!d.flags) ++live_units;
-        const char* env = std::getenv("MMRS_PREFILTER");  // experiments: 0 = off, 1 = on where the shapes allow
-        int mode = ctx->opt_prefilter;
-        if (env && *env && !solo) mode = (*env == '0') ? 1 : 2;
-        // auto (0) currently resolves to the dense FP32 sweep: on B200 the prefilter's per-tile TMEM hand-shakes and
-        // the FMNMX-bound epilogue make K1t slower than K1 (17 vs 24 M evaluations/s, DESIGN.md §4).
-        ctx->use_tc = !solo && mode == 2 && ctx->tc_shape_ok && live_units > 0 && ctx->part_active != 2;
-        if (mode == 2 && !ctx->use_tc && ctx->opt_prefilter == 2 && !solo)
-            return set_err(ctx, MMRS_ERR_ARG,
-                           "prefilter required but the batch does not fit the tensor-core operand layout (64 <= points "
-                           "per set <= 2048)");
-        ctx->h_work_tc.clear();
-        ctx->h_work_list.clear();
-        if (ctx->use_tc) {
-            long long tile = (live + (long long)ctx->n_sm * 6 - 1) / ((long long)ctx->n_sm * 6);
-            tile = std::max<long long>(64, std::min<long long>(tile, 512));
-            for (int64_t u = 0; u < U; ++u) {
-                const UnitDesc& d = units[u];
-                if (d.flags) continue;
-                const int parts = (int)((d.n_cand + tile - 1) / tile);
-                const int per = (d.n_cand + parts - 1) / parts;
-                for (int c0 = 0; c0 < d.n_cand; c0 += per)
-                    ctx->h_work_tc.push_back(WorkItem{(int)u, c0, std::min(per, d.n_cand - c0), 0});
-            }
-            ctx->l1_cap = (unsigned)std::min<unsigned long long>(
-                std::max<unsigned long long>((unsigned long long)U * 256, 1ull << 20), 0x7fffffffull);
-            ENSURE(ctx->d_work_tc, ctx->h_work_tc.size() * sizeof(WorkItem));
-            ENSURE(ctx->d_key_tc, U * 8);
-            ENSURE(ctx->d_l1_items, (size_t)ctx->l1_cap * 8);
-            ENSURE(ctx->d_l1_count, U * 4);
-            ENSURE(ctx->d_l1_base, U * 4);
-            ENSURE(ctx->d_l1_n, 16);
-        }
-    }
-    // Expanded-form tier K1x (k_sweep<.., XF>): the same work list and size classes as the dense sweep, 6 instead of 8
-    // packed FP32 instructions per 2 x 2 block; candidates inside its error window are re-scored in direct form.
-    {
-        const char* env = std::getenv("MMRS_XF");   // experiments: 1 = on for every batch that qualifies, 0 = off
-        int mode = ctx->opt_prefilter;
-        if (env && *env && mode == 0 && !solo) mode = (*env == '0') ? 1 : 3;
-        if (mode == 0) mode = kXfDefault ? 3 : 1;
-        // worth it when the sweep is long enough to pay for two extra launches (window + re-scoring)
-        bool any_big = false;
-        for (const auto& cl : ctx->classes) any_big = any_big || cl.big;
-        ctx->use_xf = !solo && mode == 3 && !ctx->use_tc && !any_big && ctx->part_active != 2 &&
-                      live >= (ctx->opt_prefilter == 3 ? 1 : (1 << 20));
-        if (ctx->use_xf) {
-            ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>({(long long)U * 64, 65536LL, live / 32}),
-                                                        std::max<long long>(live, 1));
-            ENSURE(ctx->d_key_tc, U * 8);
-            ENSURE(ctx->d_l1_items, (size_t)ctx->l1_cap * 8);
-            ENSURE(ctx->d_l1_count, U * 4);
-            ENSURE(ctx->d_l1_base, U * 4);
-            ENSURE(ctx->d_l1_n, 16);
-        }
-    }
-    // Lower-bound pruning: worth it when a unit carries enough candidates for the two extra passes to pay off.
-    {
-        long long live_units = 0;
-        for (auto& d : units)
-            if (!d.flags) ++live_units;
-        const char* env = std::getenv("MMRS_PRUNE");
-        int mode = ctx->opt_prune;
-        if (env && *env && !solo) mode = (*env == '0') ? 0 : 1;
-        ctx->use_prune = !solo && mode == 1 && !ctx->use_tc && !ctx->use_xf && ctx->lb_shape_ok && live_units > 0 && live >= 256 * live_units &&
-                         ctx->part_active != 2;
-        ctx->h_work_lb.clear();
-        if (ctx->use_prune) {
-            for (int pass = 0; pass < 2; ++pass)
-                for (int64_t u = 0; u < U; ++u) {
-                    UnitDesc& l = ctx->h_units_lb[u + pass * U];
-                    const UnitDesc& d = units[u];
-                    l.cand_off = d.cand_off, l.n_cand = d.n_cand, l.dist_off = d.dist_off;
-                    l.flags = d.flags | (pass == 1 ? kLbNegSin : 0);
-                }
-            const long long slots = (long long)ctx->n_sm * 2 * 4;
-            long long per_warp = (2 * live + slots * kWarpsPerCta - 1) / (slots * kWarpsPerCta);
-            per_warp = std::max<long long>(8, std::min<long long>((per_warp + 7) / 8 * 8, 64));  // k_lb: 8 candidates per warp pass
-            const int tile = (int)per_warp * kWarpsPerCta;
-            for (int pass = 0; pass < 2; ++pass)
-                for (int64_t u = 0; u < U; ++u) {
-                    const UnitDesc& d = units[u];
-                    if (d.flags) continue;
-                    for (int c0 = 0; c0 < d.n_cand; c0 += tile)
-                        ctx->h_work_lb.push_back(WorkItem{(int)(u + pass * U), c0, std::min(tile, d.n_cand - c0), 0});
-                }
-            ctx->l1_cap = (unsigned)std::min<long long>(std::max<long long>(dist_off, 1), 0x7fffffffLL);
-            ENSURE(ctx->d_work_lb, ctx->h_work_lb.size() * sizeof(WorkItem));
-            ENSURE(ctx->d_l1_items, (size_t)ctx->l1_cap * 8);
-            ENSURE(ctx->d_l1_count, U * 4);
-            ENSURE(ctx->d_l1_base, U * 4);
-            ENSURE(ctx->d_l1_n, 16);
-        }
-    }
+    if (int rc = plan_tier(ctx, solo, live)) return rc;
     ENSURE(ctx->d_work, ctx->h_work.size() * sizeof(WorkItem));
     ENSURE(ctx->d_cs64, (size_t)n_cs * 16);
     ENSURE(ctx->d_cs32, (size_t)n_cs * 8);
@@ -933,13 +927,13 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
     if (!ctx->h_work.empty())
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_work.p, ctx->h_work.data(), ctx->h_work.size() * sizeof(WorkItem),
                                       cudaMemcpyHostToDevice, s));
-    if (ctx->use_prune && !ctx->h_work_lb.empty()) {
+    if (ctx->tier == kTierPrune && !ctx->h_work_lb.empty()) {
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_units_lb.p, ctx->h_units_lb.data(), 2 * U * sizeof(UnitDesc),
                                       cudaMemcpyHostToDevice, s));
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_work_lb.p, ctx->h_work_lb.data(), ctx->h_work_lb.size() * sizeof(WorkItem),
                                       cudaMemcpyHostToDevice, s));
     }
-    if (ctx->use_tc && !ctx->h_work_tc.empty()) {
+    if (ctx->tier == kTierTc && !ctx->h_work_tc.empty()) {
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_work_tc.p, ctx->h_work_tc.data(), ctx->h_work_tc.size() * sizeof(WorkItem),
                                       cudaMemcpyHostToDevice, s));
     }
@@ -1115,28 +1109,18 @@ struct ExactPlan {
     double2* scratch;
     double* mins = nullptr;   // partial cost: the CTAs' row minima in global memory (with scratch)
 };
-static int exact_plan(mmrs_ctx* ctx, int max_pts, int want_grid, ExactPlan* p) {
-    const long long smem = 64 + 2LL * max_pts * 16;
+// The partial cost also keeps the row minima of one direction (max_pts doubles per CTA).
+static int exact_plan(mmrs_ctx* ctx, bool partial, int max_pts, int want_grid, ExactPlan* p) {
+    const long long smem = 64 + 2LL * max_pts * 16 + (partial ? (long long)max_pts * 8 : 0);
     if (smem <= kMaxDynSmem) {
         *p = ExactPlan{(int)smem, want_grid, nullptr};
         return MMRS_OK;
     }
     const int grid = std::max(1, std::min(want_grid, ctx->n_sm * 2));
-    ENSURE(ctx->d_exact_scratch, (size_t)grid * max_pts * 16);
-    *p = ExactPlan{64, grid, (double2*)ctx->d_exact_scratch.p};
-    return MMRS_OK;
-}
-// The same for the partial cost, which also keeps the row minima of one direction (max_pts doubles per CTA).
-static int exact_plan_partial(mmrs_ctx* ctx, int max_pts, int want_grid, ExactPlan* p) {
-    const long long smem = 64 + 2LL * max_pts * 16 + (long long)max_pts * 8;
-    if (smem <= kMaxDynSmem) {
-        *p = ExactPlan{(int)smem, want_grid, nullptr};
-        return MMRS_OK;
-    }
-    const int grid = std::max(1, std::min(want_grid, ctx->n_sm * 2));
-    ENSURE(ctx->d_exact_scratch, (size_t)grid * max_pts * 24);
-    *p = ExactPlan{64, grid, (double2*)ctx->d_exact_scratch.p,
-                   (double*)((char*)ctx->d_exact_scratch.p + (size_t)grid * max_pts * 16)};
+    const size_t rot = (size_t)grid * max_pts * 16;
+    ENSURE(ctx->d_exact_scratch, partial ? (size_t)grid * max_pts * 24 : rot);
+    char* base = (char*)ctx->d_exact_scratch.p;
+    *p = ExactPlan{64, grid, (double2*)base, partial ? (double*)(base + rot) : nullptr};
     return MMRS_OK;
 }
 
@@ -1146,22 +1130,14 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     const UnitDesc& d = ctx->h_units[u];
     ENSURE(ctx->d_tmp, (size_t)d.n_cand * 8);
     ExactPlan ep;
-    if (ctx->partial) {
-        if (int rc = exact_plan_partial(ctx, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
-        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense_partial));
-        k_exact_dense_partial<<<ep.grid, 256, ep.smem, ctx->stream>>>(
-            (const UnitDesc*)ctx->d_units.p, (int)u, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-            (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p, d.cand_off, d.n_cand, (double*)ctx->d_tmp.p,
-            ctx->max_pts, ep.scratch, ep.mins, ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
-    } else {
-        if (int rc = exact_plan(ctx, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
-        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
-        k_exact_dense<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u,
-                                                              (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-                                                              (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
-                                                              d.cand_off, d.n_cand, (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch,
-                                                              ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
-    }
+    if (int rc = exact_plan(ctx, ctx->partial, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
+    CUDA_TRY(ctx, ctx->partial ? RAISE_SMEM(k_exact_dense<true>) : RAISE_SMEM(k_exact_dense<false>));
+    auto k3 = ctx->partial ? k_exact_dense<true> : k_exact_dense<false>;
+    k3<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u, (const double*)ctx->d_test.p,
+                                               (const double*)ctx->d_ref.p, (const double2*)ctx->d_cs64.p,
+                                               (const unsigned char*)ctx->d_zero.p, d.cand_off, d.n_cand,
+                                               (double*)ctx->d_tmp.p, ctx->max_pts, ep.scratch, ep.mins,
+                                               ctx->rigid ? (const double2*)ctx->d_t64.p : nullptr, false);
     CUDA_TRY(ctx, cudaGetLastError());
     std::vector<double> h(d.n_cand);
     CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), ctx->d_tmp.p, (size_t)d.n_cand * 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1192,6 +1168,191 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     return MMRS_OK;
 }
 
+// Re-scores a candidate list (in d_l1_items) with the exact FP32 sweep: one launch per size class, each scoring the list
+// items of its own units. n_items: the list's device counter (NULL: exactly `cap` items); diag: slot of d_l1_n that
+// receives the kernel's diagnostic.
+static int rescore_list(mmrs_ctx* ctx, const unsigned* n_items, unsigned cap, int chunk, int diag) {
+    const ListArgs la{(const int2*)ctx->d_l1_items.p, n_items, cap, chunk, (const unsigned*)ctx->d_rmax.p,
+                      (unsigned*)ctx->d_l1_n.p + diag};
+    const int grid = (int)(((long long)la.cap + la.chunk - 1) / la.chunk);
+    for (const auto& cl : ctx->classes) {
+        if (!launch_sweep(cl.ta, cl.multi, cl.tailp, grid, cl.smem, ctx->stream, (const UnitDesc*)ctx->d_units.p, nullptr,
+                          (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p,
+                          (unsigned long long*)ctx->d_key.p, &la))
+            return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
+        ctx->launches += 1;
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
+    return MMRS_OK;
+}
+
+// Tier 1 and 2 of every tier: the candidates inside the window (rel, abs, k_shortlist `mode`) of each unit's minimum in
+// `key` go to the list, which is re-scored with the exact FP32 sweep.
+static int rescore_window(mmrs_ctx* ctx, const unsigned long long* key, float rel, float abs, int mode, int chunk, int diag) {
+    cudaStream_t s = ctx->stream;
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[1], s));
+    k_shortlist<<<(unsigned)ctx->n_units, 256, 0, s>>>((const UnitDesc*)ctx->d_units.p, (const float*)ctx->d_dist32.p, key,
+                                                       (const unsigned*)ctx->d_rmax.p, rel, abs, ctx->l1_cap,
+                                                       (int*)ctx->d_l1_count.p, (unsigned*)ctx->d_l1_base.p,
+                                                       (int2*)ctx->d_l1_items.p, (unsigned*)ctx->d_l1_n.p, mode, nullptr);
+    CUDA_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    if (int rc = rescore_list(ctx, (const unsigned*)ctx->d_l1_n.p, ctx->l1_cap, chunk, diag)) return rc;
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[2], s));
+    return MMRS_OK;
+}
+
+// Lower-bound pruning (K1p): bounds of every candidate; the candidate with the smallest bound is scored first, and only
+// the candidates whose bound is within the window of that exact distance are scored after it.
+static int run_prune(mmrs_ctx* ctx) {
+    const int64_t U = ctx->n_units;
+    cudaStream_t s = ctx->stream;
+    const UnitDesc* units = (const UnitDesc*)ctx->d_units.p;
+    // tier 0: lower bounds of every candidate (rows-only passes over R strided points of each set)
+    const UnitDesc* lbu = (const UnitDesc*)ctx->d_units_lb.p;
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_dist32.p, 0, (size_t)ctx->total_cands * 4, s));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
+    if (ctx->lb_R == 128) {
+        CUDA_TRY(ctx, RAISE_SMEM((k_lb<4, 2>)));
+        k_lb<4, 2><<<(unsigned)ctx->h_work_lb.size(), kThreads, ctx->smem_lb, s>>>(
+            lbu, (const WorkItem*)ctx->d_work_lb.p, (const float4*)ctx->d_lay_lb.p, (const float2*)ctx->d_cs32.p,
+            (float*)ctx->d_dist32.p);
+    } else {
+        CUDA_TRY(ctx, RAISE_SMEM((k_lb<1, 8>)));
+        k_lb<1, 8><<<(unsigned)ctx->h_work_lb.size(), kThreads, ctx->smem_lb, s>>>(
+            lbu, (const WorkItem*)ctx->d_work_lb.p, (const float4*)ctx->d_lay_lb.p, (const float2*)ctx->d_cs32.p,
+            (float*)ctx->d_dist32.p);
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
+    // the candidate with the smallest bound is scored first: its exact FP32 distance bounds the minimum from above
+    k_lb_argmin<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p, (int*)ctx->d_l1_count.p,
+                                            (unsigned*)ctx->d_l1_base.p, (int2*)ctx->d_l1_items.p);
+    CUDA_TRY(ctx, cudaGetLastError());
+    ctx->launches += 2;
+    if (int rc = rescore_list(ctx, nullptr, (unsigned)U, 1, 2)) return rc;   // k_lb_argmin's list: one item per unit
+    // survivors: bound <= that distance + twice the FP32 window; everything else cannot be the arg-min
+    return rescore_window(ctx, (const unsigned long long*)ctx->d_key.p, 4e-6f, 4e-6f, 0, 32, 2);
+}
+
+// MMRS_TC_TRACE (experiments): the per-tile clock stamps of K1t's CTA 0, as a text file at `path`.
+static int dump_tc_trace(mmrs_ctx* ctx, const long long* d_trace, const char* path) {
+    cudaStream_t s = ctx->stream;
+    std::vector<long long> h(8 * 256 + 64 * 8);
+    CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), d_trace, h.size() * 8, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s));
+    if (FILE* f = std::fopen(path, "w")) {
+        std::fprintf(f, "tile wg issuer_ready issuer_committed epi_woken epi_released\n");
+        for (int g = 0; g < 2; ++g)
+            for (int t = 0; t < 256; ++t)
+                std::fprintf(f, "%d %d %lld %lld %lld %lld\n", t, g, h[(g * 4 + 0) * 256 + t], h[(g * 4 + 1) * 256 + t],
+                             h[(g * 4 + 2) * 256 + t], h[(g * 4 + 3) * 256 + t]);
+        std::fprintf(f, "fine stamps (wg 0, quarter 0): tile start ld0_done fold0_done wait1_done wait3_done fold3_done fenced\n");
+        for (int t = 0; t < 64; ++t) {
+            std::fprintf(f, "%d", t);
+            for (int k = 0; k < 7; ++k) std::fprintf(f, " %lld", h[2048 + t * 8 + k] - h[2048 + t * 8]);
+            std::fprintf(f, " | woken->start %lld, fenced->released %lld\n", h[2048 + t * 8] - h[(0 * 4 + 2) * 256 + t],
+                         h[(0 * 4 + 3) * 256 + t] - h[2048 + t * 8 + 6]);
+        }
+        std::fclose(f);
+    }
+    return MMRS_OK;
+}
+
+// Tensor-core prefilter (K1t): every candidate on the tensor cores, then the candidates inside its window re-scored.
+static int run_tc(mmrs_ctx* ctx) {
+    const int64_t U = ctx->n_units;
+    cudaStream_t s = ctx->stream;
+    // tier 0: every candidate on the tensor cores (bf16x3, FP32 accumulate) -> approximate dist32 + per-unit minimum
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key_tc.p, 0xff, U * 8, s));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
+    CUDA_TRY(ctx, RAISE_SMEM(k_tc_sweep));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
+    const char* trace_path = std::getenv("MMRS_TC_TRACE");  // experiments: per-tile clock stamps of CTA 0
+    long long* d_trace = nullptr;
+    if (trace_path && *trace_path) {
+        ENSURE(ctx->d_tmp, (8 * 256 + 64 * 8) * 8);
+        d_trace = (long long*)ctx->d_tmp.p;
+        CUDA_TRY(ctx, cudaMemsetAsync(d_trace, 0, (8 * 256 + 64 * 8) * 8, s));
+    }
+    k_tc_sweep<<<(unsigned)ctx->h_work_tc.size(), kTcThreads, ctx->smem_tc, s>>>(
+        (const UnitDesc*)ctx->d_units.p, (const WorkItem*)ctx->d_work_tc.p, (const double*)ctx->d_test.p,
+        (const double*)ctx->d_ref.p, (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p,
+        (unsigned long long*)ctx->d_key_tc.p, d_trace);
+    CUDA_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    if (d_trace)
+        if (int rc = dump_tc_trace(ctx, d_trace, trace_path)) return rc;
+    return rescore_window(ctx, (const unsigned long long*)ctx->d_key_tc.p, 1e-6f, (float)ctx->tc_abs, 1, 8, 1);
+}
+
+// Expanded-form tier (K1x): every candidate in the expanded form, then the candidates inside its window re-scored in
+// direct form.
+static int run_xf(mmrs_ctx* ctx) {
+    const int64_t U = ctx->n_units;
+    cudaStream_t s = ctx->stream;
+    // tier 0: every candidate in the expanded form (K1x) -> FP32 distances with a bounded ABSOLUTE error on d^2
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key_tc.p, 0xff, U * 8, s));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
+    CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
+    for (const auto& cl : ctx->classes) {
+        if (!cl.work_count) continue;
+        if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, (const UnitDesc*)ctx->d_units.p,
+                          (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
+                          (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key_tc.p,
+                          nullptr, true))
+            return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
+        CUDA_TRY(ctx, cudaGetLastError());
+        ctx->launches += 1;
+    }
+    return rescore_window(ctx, (const unsigned long long*)ctx->d_key_tc.p, 4e-6f, (float)ctx->xf_abs, 2, 16, 1);
+}
+
+// The dense sweep of one size class: K1b (k_sweep_big) for units beyond K1's shared-memory staging, else K1e-partial
+// for the partial cost, K1e where the class takes it, or K1. t32 != NULL: rigid candidates.
+static int sweep_class(mmrs_ctx* ctx, const mmrs_ctx::SweepClass& cl, const float2* t32) {
+    cudaStream_t s = ctx->stream;
+    const UnitDesc* units = (const UnitDesc*)ctx->d_units.p;
+    const WorkItem* work = (const WorkItem*)ctx->d_work.p + cl.work_begin;
+    const float4* lay = (const float4*)ctx->d_lay.p;
+    const float2* cs32 = (const float2*)ctx->d_cs32.p;
+    float* dist32 = (float*)ctx->d_dist32.p;
+    unsigned long long* key = (unsigned long long*)ctx->d_key.p;
+    if (cl.big) {
+        const int grid = (int)std::min<size_t>(cl.work_count, (size_t)ctx->n_sm * 2);
+        ENSURE(ctx->d_big_rows, (size_t)grid * kWarpsPerCta * ctx->big_scratch_per_warp * 4);
+        auto big = t32 ? k_sweep_big<true> : k_sweep_big<false>;
+        big<<<grid, kThreads, 0, s>>>(units, work, (int)cl.work_count, lay, cs32, dist32, key, (float*)ctx->d_big_rows.p,
+                                      ctx->big_scratch_per_warp, t32);
+    } else if (ctx->partial || cl.eb) {
+        if (!ctx->eb_ran) {   // one counter of the pair distances the early-break kernels evaluate in this run
+            ENSURE(ctx->d_eb_pairs, 8);
+            CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
+            ctx->eb_ran = true;
+        }
+        unsigned long long* pairs = (unsigned long long*)ctx->d_eb_pairs.p;
+        if (ctx->partial) {   // K1e-partial (every class: big units are refused at upload)
+            if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<true>));
+            else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<false>));
+            auto ebp = t32 ? k_sweep_ebp<true> : k_sweep_ebp<false>;
+            ebp<<<(unsigned)cl.work_count, cl.ebp_warps * 32, cl.smem_ebp, s>>>(units, work, lay, cs32, dist32, key, pairs,
+                                                                                  t32, ctx->eb_env != 0 ? 1 : 0);
+        } else {
+            if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<true>));
+            else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<false>));
+            auto eb = t32 ? k_sweep_eb<true> : k_sweep_eb<false>;
+            eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(units, work, lay, cs32, dist32, key, pairs, t32);
+        }
+        ctx->eb_cands += cl.live;
+    } else if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units, work, lay, cs32, dist32,
+                             key, nullptr, false, t32)) {
+        return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
+    }
+    CUDA_TRY(ctx, cudaGetLastError());
+    ctx->launches += 1;
+    return MMRS_OK;
+}
+
 extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_sweep_run: ctx is NULL");
     if (!ctx->ready) return set_err(ctx, MMRS_ERR_STATE, "mmrs_sweep_run: no batch uploaded");
@@ -1210,235 +1371,27 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key.p, 0xff, U * 8, s));
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_nitems.p, 0, 16, s));
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[0], s));
-    const bool tc = ctx->use_tc && !ctx->h_work_tc.empty();
-    const bool xf = !tc && ctx->use_xf && !ctx->h_work.empty();
-    const bool prune = !tc && !xf && ctx->use_prune && !ctx->h_work_lb.empty();
+    // the planned tier, or the dense sweep when the tier has no work
+    const bool has_work = ctx->tier == kTierTc      ? !ctx->h_work_tc.empty()
+                          : ctx->tier == kTierXf    ? !ctx->h_work.empty()
+                          : ctx->tier == kTierPrune ? !ctx->h_work_lb.empty()
+                                                    : true;
+    ctx->tier_ran = has_work ? ctx->tier : kTierDense;
     ctx->eb_ran = false;
     ctx->eb_cands = 0;
-    ctx->xf_ran = xf;
-    ctx->tc_ran = tc || xf;
-    ctx->prune_ran = prune;
-    if (prune) {
-        // tier 0: lower bounds of every candidate (rows-only passes over R strided points of each set)
-        const UnitDesc* lbu = (const UnitDesc*)ctx->d_units_lb.p;
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_dist32.p, 0, (size_t)ctx->total_cands * 4, s));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
-        if (ctx->lb_R == 128) {
-            CUDA_TRY(ctx, RAISE_SMEM((k_lb<4, 2>)));
-            k_lb<4, 2><<<(unsigned)ctx->h_work_lb.size(), kThreads, ctx->smem_lb, s>>>(
-                lbu, (const WorkItem*)ctx->d_work_lb.p, (const float4*)ctx->d_lay_lb.p, (const float2*)ctx->d_cs32.p,
-                (float*)ctx->d_dist32.p);
-        } else {
-            CUDA_TRY(ctx, RAISE_SMEM((k_lb<1, 8>)));
-            k_lb<1, 8><<<(unsigned)ctx->h_work_lb.size(), kThreads, ctx->smem_lb, s>>>(
-                lbu, (const WorkItem*)ctx->d_work_lb.p, (const float4*)ctx->d_lay_lb.p, (const float2*)ctx->d_cs32.p,
-                (float*)ctx->d_dist32.p);
-        }
-        CUDA_TRY(ctx, cudaGetLastError());
-        // the candidate with the smallest bound is scored first: its exact FP32 distance bounds the minimum from above
-        k_lb_argmin<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p, (int*)ctx->d_l1_count.p,
-                                                (unsigned*)ctx->d_l1_base.p, (int2*)ctx->d_l1_items.p);
-        CUDA_TRY(ctx, cudaGetLastError());
-        ListArgs la;
-        la.items = (const int2*)ctx->d_l1_items.p;
-        la.n_items = nullptr;  // k_lb_argmin's list: exactly one item per unit
-        la.cap = (unsigned)U;
-        la.chunk = 1;
-        la.rmax = (const unsigned*)ctx->d_rmax.p;
-        la.diag = (unsigned*)ctx->d_l1_n.p + 2;
-        auto rescore = [&]() {   // one launch per size class; each scores the list items of its own units
-            const long long grid = ((long long)la.cap + la.chunk - 1) / la.chunk;
-            for (const auto& cl : ctx->classes) {
-                if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)grid, cl.smem, s, units, nullptr,
-                                  (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p,
-                                  (unsigned long long*)ctx->d_key.p, &la))
-                    return false;
-                ctx->launches += 1;
-            }
-            return true;
-        };
-        if (!rescore()) return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[1], s));
-        // survivors: bound <= that distance + twice the FP32 window; everything else cannot be the arg-min
-        k_shortlist<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p,
-                                                (const unsigned long long*)ctx->d_key.p, (const unsigned*)ctx->d_rmax.p,
-                                                4e-6f, 4e-6f, ctx->l1_cap, (int*)ctx->d_l1_count.p,
-                                                (unsigned*)ctx->d_l1_base.p, (int2*)ctx->d_l1_items.p,
-                                                (unsigned*)ctx->d_l1_n.p, 0, nullptr);
-        CUDA_TRY(ctx, cudaGetLastError());
-        la.n_items = (const unsigned*)ctx->d_l1_n.p;
-        la.cap = ctx->l1_cap;
-        la.chunk = 32;
-        if (!rescore()) return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[2], s));
-        ctx->launches += 3;
-    } else if (tc) {
-        // tier 0: every candidate on the tensor cores (bf16x3, FP32 accumulate) -> approximate dist32 + per-unit minimum
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key_tc.p, 0xff, U * 8, s));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
-        CUDA_TRY(ctx, RAISE_SMEM(k_tc_sweep));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
-        const char* trace_path = std::getenv("MMRS_TC_TRACE");  // experiments: per-tile clock stamps of CTA 0
-        long long* d_trace = nullptr;
-        if (trace_path && *trace_path) {
-            ENSURE(ctx->d_tmp, (8 * 256 + 64 * 8) * 8);
-            d_trace = (long long*)ctx->d_tmp.p;
-            CUDA_TRY(ctx, cudaMemsetAsync(d_trace, 0, (8 * 256 + 64 * 8) * 8, s));
-        }
-        k_tc_sweep<<<(unsigned)ctx->h_work_tc.size(), kTcThreads, ctx->smem_tc, s>>>(
-            units, (const WorkItem*)ctx->d_work_tc.p, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-            (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key_tc.p, d_trace);
-        CUDA_TRY(ctx, cudaGetLastError());
-        if (d_trace) {
-            std::vector<long long> h(8 * 256 + 64 * 8);
-            CUDA_TRY(ctx, cudaMemcpyAsync(h.data(), d_trace, h.size() * 8, cudaMemcpyDeviceToHost, s));
-            CUDA_TRY(ctx, cudaStreamSynchronize(s));
-            if (FILE* f = std::fopen(trace_path, "w")) {
-                std::fprintf(f, "tile wg issuer_ready issuer_committed epi_woken epi_released\n");
-                for (int g = 0; g < 2; ++g)
-                    for (int t = 0; t < 256; ++t)
-                        std::fprintf(f, "%d %d %lld %lld %lld %lld\n", t, g, h[(g * 4 + 0) * 256 + t], h[(g * 4 + 1) * 256 + t],
-                                     h[(g * 4 + 2) * 256 + t], h[(g * 4 + 3) * 256 + t]);
-                std::fprintf(f, "fine stamps (wg 0, quarter 0): tile start ld0_done fold0_done wait1_done wait3_done fold3_done fenced\n");
-                for (int t = 0; t < 64; ++t) {
-                    std::fprintf(f, "%d", t);
-                    for (int k = 0; k < 7; ++k) std::fprintf(f, " %lld", h[2048 + t * 8 + k] - h[2048 + t * 8]);
-                    std::fprintf(f, " | woken->start %lld, fenced->released %lld\n", h[2048 + t * 8] - h[(0 * 4 + 2) * 256 + t],
-                                 h[(0 * 4 + 3) * 256 + t] - h[2048 + t * 8 + 6]);
-                }
-                std::fclose(f);
-            }
-        }
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[1], s));
-        // tier 1: candidates inside the prefilter's error window of the unit's minimum ...
-        k_shortlist<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p,
-                                                (const unsigned long long*)ctx->d_key_tc.p,
-                                                (const unsigned*)ctx->d_rmax.p, 1e-6f, (float)ctx->tc_abs, ctx->l1_cap,
-                                                (int*)ctx->d_l1_count.p, (unsigned*)ctx->d_l1_base.p,
-                                                (int2*)ctx->d_l1_items.p, (unsigned*)ctx->d_l1_n.p, 1, nullptr);
-        CUDA_TRY(ctx, cudaGetLastError());
-        // ... are re-scored with the exact FP32 arithmetic of the dense sweep (tier 2)
-        ListArgs la;
-        la.items = (const int2*)ctx->d_l1_items.p;
-        la.n_items = (const unsigned*)ctx->d_l1_n.p;
-        la.cap = ctx->l1_cap;
-        la.chunk = 8;
-        la.rmax = (const unsigned*)ctx->d_rmax.p;
-        la.diag = (unsigned*)ctx->d_l1_n.p + 1;
-        for (const auto& cl : ctx->classes) {
-            if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)(((long long)ctx->l1_cap + la.chunk - 1) / la.chunk), cl.smem, s,
-                              units, nullptr, (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p,
-                              (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p, &la))
-                return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-            ctx->launches += 1;
-        }
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[2], s));
-        ctx->launches += 2;
-    } else if (xf) {
-        // tier 0: every candidate in the expanded form (K1x) -> FP32 distances with a bounded ABSOLUTE error on d^2
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_key_tc.p, 0xff, U * 8, s));
-        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_l1_n.p, 0, 16, s));
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[0], s));
-        for (const auto& cl : ctx->classes) {
-            if (!cl.work_count) continue;
-            if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units,
-                              (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
-                              (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key_tc.p,
-                              nullptr, true))
-                return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-            CUDA_TRY(ctx, cudaGetLastError());
-            ctx->launches += 1;
-        }
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[1], s));
-        // tier 1: the candidates inside the tier's error window of the unit's minimum ...
-        k_shortlist<<<(unsigned)U, 256, 0, s>>>(units, (const float*)ctx->d_dist32.p,
-                                                (const unsigned long long*)ctx->d_key_tc.p,
-                                                (const unsigned*)ctx->d_rmax.p, 4e-6f, (float)ctx->xf_abs, ctx->l1_cap,
-                                                (int*)ctx->d_l1_count.p, (unsigned*)ctx->d_l1_base.p,
-                                                (int2*)ctx->d_l1_items.p, (unsigned*)ctx->d_l1_n.p, 2, nullptr);
-        CUDA_TRY(ctx, cudaGetLastError());
-        // ... are re-scored in direct form (tier 2): from here on the run works on exact FP32 values
-        ListArgs la;
-        la.items = (const int2*)ctx->d_l1_items.p;
-        la.n_items = (const unsigned*)ctx->d_l1_n.p;
-        la.cap = ctx->l1_cap;
-        la.chunk = 16;
-        la.rmax = (const unsigned*)ctx->d_rmax.p;
-        la.diag = (unsigned*)ctx->d_l1_n.p + 1;
-        for (const auto& cl : ctx->classes) {
-            if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)(((long long)ctx->l1_cap + la.chunk - 1) / la.chunk), cl.smem, s,
-                              units, nullptr, (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p,
-                              (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p, &la))
-                return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-            ctx->launches += 1;
-        }
-        CUDA_TRY(ctx, cudaGetLastError());
-        CUDA_TRY(ctx, cudaEventRecord(ctx->ev_tc[2], s));
-        ctx->launches += 1;
-    } else if (!ctx->h_work.empty()) {
-        for (const auto& cl : ctx->classes) {   // one launch per size class (register tile / chunked / exact tiling)
-            if (!cl.work_count) continue;
-            if (cl.big) {
-                const int grid = (int)std::min<size_t>(cl.work_count, (size_t)ctx->n_sm * 2);
-                ENSURE(ctx->d_big_rows, (size_t)grid * kWarpsPerCta * ctx->big_scratch_per_warp * 4);
-                auto big = t32 ? k_sweep_big<true> : k_sweep_big<false>;
-                big<<<grid, kThreads, 0, s>>>(units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (int)cl.work_count,
-                                              (const float4*)ctx->d_lay.p, (const float2*)ctx->d_cs32.p,
-                                              (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                                              (float*)ctx->d_big_rows.p, ctx->big_scratch_per_warp, t32);
-                CUDA_TRY(ctx, cudaGetLastError());
-                ctx->launches += 1;
-                continue;
-            }
-            if (ctx->partial) {   // K1e-partial (every class: big units are refused at upload)
-                if (!ctx->eb_ran) {
-                    ENSURE(ctx->d_eb_pairs, 8);
-                    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
-                    ctx->eb_ran = true;
-                }
-                if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<true>));
-                else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<false>));
-                auto ebp = t32 ? k_sweep_ebp<true> : k_sweep_ebp<false>;
-                ebp<<<(unsigned)cl.work_count, cl.ebp_warps * 32, cl.smem_ebp, s>>>(
-                    units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
-                    (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                    (unsigned long long*)ctx->d_eb_pairs.p, t32, ctx->eb_env != 0 ? 1 : 0);
-                CUDA_TRY(ctx, cudaGetLastError());
-                ctx->eb_cands += cl.live;
-                ctx->launches += 1;
-                continue;
-            }
-            if (cl.eb) {
-                if (!ctx->eb_ran) {
-                    ENSURE(ctx->d_eb_pairs, 8);
-                    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
-                    ctx->eb_ran = true;
-                }
-                if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<true>));
-                else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<false>));
-                auto eb = t32 ? k_sweep_eb<true> : k_sweep_eb<false>;
-                eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(
-                    units, (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
-                    (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                    (unsigned long long*)ctx->d_eb_pairs.p, t32);
-                CUDA_TRY(ctx, cudaGetLastError());
-                ctx->eb_cands += cl.live;
-                ctx->launches += 1;
-                continue;
-            }
-            if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units,
-                              (const WorkItem*)ctx->d_work.p + cl.work_begin, (const float4*)ctx->d_lay.p,
-                              (const float2*)ctx->d_cs32.p, (float*)ctx->d_dist32.p, (unsigned long long*)ctx->d_key.p,
-                              nullptr, false, t32))
-                return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
-            CUDA_TRY(ctx, cudaGetLastError());
-            ctx->launches += 1;
-        }
+    int rc = MMRS_OK;
+    switch (ctx->tier_ran) {
+        case kTierPrune: rc = run_prune(ctx); break;
+        case kTierTc: rc = run_tc(ctx); break;
+        case kTierXf: rc = run_xf(ctx); break;
+        case kTierDense:
+            for (const auto& cl : ctx->classes)   // one launch per size class (register tile / chunked / exact tiling)
+                if (cl.work_count && (rc = sweep_class(ctx, cl, t32)) != MMRS_OK) break;
+            break;
     }
+    if (rc != MMRS_OK) return rc;
+    // after K1t / K1x, K2 passes a unit whose tier-1 list overflowed (never re-scored in FP32) on as an overflow
+    const bool listed = ctx->tier_ran == kTierTc || ctx->tier_ran == kTierXf;
     if (ctx->part_active == 2) {
         // candidate axis: the global FP32 minimum of every unit = min over ranks of the packed (distance, index) keys
         NcclApi& nc = nccl_api();
@@ -1451,26 +1404,18 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
                                             (const unsigned long long*)ctx->d_key.p, rbits,
                                             (float)ctx->opt_rel, (float)ctx->opt_abs, ctx->pool_cap,
                                             (int*)ctx->d_sl_count.p, (unsigned*)ctx->d_sl_base.p, (int2*)ctx->d_items.p,
-                                            (unsigned*)ctx->d_nitems.p, 0, (tc || xf) ? (const int*)ctx->d_l1_count.p : nullptr);
+                                            (unsigned*)ctx->d_nitems.p, 0, listed ? (const int*)ctx->d_l1_count.p : nullptr);
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
     {
         ExactPlan ep;
-        if (ctx->partial) {
-            if (int rc = exact_plan_partial(ctx, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
-            CUDA_TRY(ctx, RAISE_SMEM(k_exact_partial));
-            k_exact_partial<<<ep.grid, 256, ep.smem, s>>>(
-                units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p, (const double2*)ctx->d_cs64.p,
-                (const unsigned char*)ctx->d_zero.p, (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p,
-                ctx->pool_cap, (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, ep.mins, t64);
-        } else {
-            if (int rc = exact_plan(ctx, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
-            CUDA_TRY(ctx, RAISE_SMEM(k_exact));
-            k_exact<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
-                                                  (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
-                                                  (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
-                                                  (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, t64);
-        }
+        if (int rc = exact_plan(ctx, ctx->partial, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
+        CUDA_TRY(ctx, ctx->partial ? RAISE_SMEM(k_exact<true>) : RAISE_SMEM(k_exact<false>));
+        auto k3 = ctx->partial ? k_exact<true> : k_exact<false>;
+        k3<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
+                                         (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
+                                         (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
+                                         (double*)ctx->d_sl_dist.p, ctx->max_pts, ep.scratch, ep.mins, t64);
         CUDA_TRY(ctx, cudaGetLastError());
         k_select<<<(unsigned)((U + 7) / 8), 256, 0, s>>>(units, (int)U, (const double2*)ctx->d_cs64.p,
                                                          (const int2*)ctx->d_items.p,
@@ -1528,24 +1473,25 @@ static int download_impl(mmrs_ctx* ctx, mmrs_unit_result* out, mmrs_rigid_result
                                   ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     if (std::getenv("MMRS_TRACE")) {  // device time of this run on stderr
+        static const char* const kTierLabel[] = {"dense;", "tc:", "pruned:", "expanded:"};
         float t[4] = {0, 0, 0, 0}, a = 0, b = 0;
         cudaEventElapsedTime(&t[0], ctx->ev[0], ctx->ev[1]);
         cudaEventElapsedTime(&t[1], ctx->ev[1], ctx->ev[2]);
         cudaEventElapsedTime(&t[2], ctx->ev[2], ctx->ev[3]);
-        if (ctx->tc_ran || ctx->prune_ran) {
+        if (ctx->tier_ran != kTierDense) {
             cudaEventElapsedTime(&a, ctx->ev_tc[0], ctx->ev_tc[1]);
             cudaEventElapsedTime(&b, ctx->ev_tc[1], ctx->ev_tc[2]);
         }
         long long scored = 0;
         int worst = 0;
-        if (ctx->tc_ran || ctx->prune_ran) {
+        if (ctx->tier_ran != kTierDense) {
             std::vector<int> cnt((size_t)U);
             cudaMemcpy(cnt.data(), ctx->d_l1_count.p, (size_t)U * 4, cudaMemcpyDeviceToHost);
             for (int c : cnt) scored += c > 0 ? c : 0, worst = std::max(worst, c);
         }
         std::fprintf(stderr, "[mmrs]   run: %lld units, %lld candidates, sweep %.2f ms (%s tier0 %.2f + tier1 %.2f; %lld scored exactly, "
                      "largest unit list %d), shortlist %.2f, recheck %.2f\n",
-                     (long long)U, ctx->total_cands, t[0], ctx->prune_ran ? "pruned:" : ctx->xf_ran ? "expanded:" : ctx->tc_ran ? "tc:" : "dense;", a, b, scored,
+                     (long long)U, ctx->total_cands, t[0], kTierLabel[ctx->tier_ran], a, b, scored,
                      worst, t[1], t[2]);
     }
     if (ctx->part_active == 1 && !ctx->comm && ctx->exchange) {
@@ -1769,22 +1715,13 @@ static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test,
     const int max_n = (int)std::max(n_test, n_ref);
     ExactPlan ep;
     const int want_grid = (int)std::min<int64_t>(n_angles, (int64_t)ctx->n_sm * 8);
-    if (partial) {
-        if (int rc = exact_plan_partial(ctx, max_n, want_grid, &ep)) return rc;
-        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense_partial));
-        k_exact_dense_partial<<<ep.grid, 256, ep.smem, s>>>(
-            (const UnitDesc*)(base + o_unit), 0, (const double*)base, (const double*)(base + (size_t)n_test * 16),
-            (const double2*)(base + o_cs), (const unsigned char*)(base + o_zero), 0, (int)n_angles, (double*)(base + o_out),
-            max_n, ep.scratch, ep.mins, txy ? (const double2*)(base + o_t) : nullptr, true);
-    } else {
-        if (int rc = exact_plan(ctx, max_n, want_grid, &ep)) return rc;
-        CUDA_TRY(ctx, RAISE_SMEM(k_exact_dense));
-        k_exact_dense<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
-                                                    (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
-                                                    (const unsigned char*)(base + o_zero), 0, (int)n_angles,
-                                                    (double*)(base + o_out), max_n, ep.scratch,
-                                                    txy ? (const double2*)(base + o_t) : nullptr, true);
-    }
+    if (int rc = exact_plan(ctx, partial, max_n, want_grid, &ep)) return rc;
+    CUDA_TRY(ctx, partial ? RAISE_SMEM(k_exact_dense<true>) : RAISE_SMEM(k_exact_dense<false>));
+    auto k3 = partial ? k_exact_dense<true> : k_exact_dense<false>;
+    k3<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
+                                     (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
+                                     (const unsigned char*)(base + o_zero), 0, (int)n_angles, (double*)(base + o_out),
+                                     max_n, ep.scratch, ep.mins, txy ? (const double2*)(base + o_t) : nullptr, true);
     CUDA_TRY(ctx, cudaGetLastError());
     CUDA_TRY(ctx, cudaMemcpyAsync(dist_out, base + o_out, b_out, cudaMemcpyDeviceToHost, s));
     CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1846,7 +1783,7 @@ extern "C" int mmrs_sweep_prefilter_info(mmrs_ctx* ctx, double out[6]) {
     if (!ctx->ran) return set_err(ctx, MMRS_ERR_STATE, "mmrs_sweep_prefilter_info: nothing has been run");
     for (int i = 0; i < 6; ++i) out[i] = 0.0;
     out[5] = ctx->tc_abs;
-    if (!ctx->tc_ran && !ctx->prune_ran && ctx->eb_ran) {   // the dense sweep ran K1e: [3] pairs evaluated, [4] candidates
+    if (ctx->tier_ran == kTierDense && ctx->eb_ran) {   // the dense sweep ran K1e: [3] pairs evaluated, [4] candidates
         ENTER_DEVICE(ctx);
         CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev[3]));
         unsigned long long pairs = 0;
@@ -1855,7 +1792,7 @@ extern "C" int mmrs_sweep_prefilter_info(mmrs_ctx* ctx, double out[6]) {
         out[4] = (double)ctx->eb_cands;
         return MMRS_OK;
     }
-    if ((!ctx->tc_ran && !ctx->prune_ran) || ctx->n_units == 0) return MMRS_OK;
+    if (ctx->tier_ran == kTierDense || ctx->n_units == 0) return MMRS_OK;
     ENTER_DEVICE(ctx);
     CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev[3]));
     float a = 0.f, b = 0.f;
@@ -1865,8 +1802,8 @@ extern "C" int mmrs_sweep_prefilter_info(mmrs_ctx* ctx, double out[6]) {
     CUDA_TRY(ctx, cudaMemcpy(h, ctx->d_l1_n.p, 8, cudaMemcpyDeviceToHost));
     float err;
     std::memcpy(&err, &h[1], 4);
-    out[0] = ctx->prune_ran ? 2.0 : ctx->xf_ran ? 3.0 : 1.0;
-    if (ctx->xf_ran) out[5] = ctx->xf_abs;
+    out[0] = (double)ctx->tier_ran;
+    if (ctx->tier_ran == kTierXf) out[5] = ctx->xf_abs;
     out[1] = a;
     out[2] = b;
     out[3] = (double)h[0];

@@ -1442,6 +1442,7 @@ __global__ void k_shortlist(const UnitDesc* __restrict__ units, const float* __r
 //   translate  : rigid candidates only: x' = rx + tx, y' = ry + ty (__dadd_rn; + 0.0 is exact, so a zero translation
 //                is the rotation-only cost bit for bit)
 //   distances  : process_utils.rs:84-121, both directions, sqrt, max
+//                (PARTIAL: the (q + 1)-th largest row minimum of each direction instead of the largest)
 // One CTA per (unit, candidate) item; grid-stride over the item list.
 // t64 != NULL: rigid candidates, c = i n_trans + j -> angle i of the unit's grid, translation j of its translation grid.
 // =============================================================================
@@ -1455,114 +1456,6 @@ __device__ __forceinline__ double block_max(double v, double* s_red) {
     return r;
 }
 
-// s_rot / s_ref: the CTA's staging of the rotated test set / the reference set — shared memory, or (units too large for
-// it) a per-CTA scratch row in global memory for the rotated points and the caller's reference array itself (copy_ref = false).
-__device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* __restrict__ test_xy,
-                                             const double* __restrict__ ref_xy, double cosv, double sinv, bool identity,
-                                             double2* s_rot, const double2* s_ref_in, double* s_red, bool copy_ref = true,
-                                             bool rigid = false, double2 t = double2{0.0, 0.0}) {
-    double2* s_ref_w = const_cast<double2*>(s_ref_in);
-    const double2* s_ref = copy_ref ? s_ref_in : reinterpret_cast<const double2*>(ref_xy + 2 * ud.ref_off);
-    for (int i = threadIdx.x; i < ud.n; i += blockDim.x) {
-        const double px = test_xy[2 * (ud.test_off + i)], py = test_xy[2 * (ud.test_off + i) + 1];
-        double rx = px, ry = py;
-        if (!identity) {
-            const double x = __dsub_rn(px, ud.cx), y = __dsub_rn(py, ud.cy);
-            rx = __dadd_rn(__dsub_rn(__dmul_rn(x, cosv), __dmul_rn(y, sinv)), ud.cx);
-            ry = __dadd_rn(__dadd_rn(__dmul_rn(x, sinv), __dmul_rn(y, cosv)), ud.cy);
-        }
-        if (rigid) rx = __dadd_rn(rx, t.x), ry = __dadd_rn(ry, t.y);
-        s_rot[i] = make_double2(rx, ry);
-    }
-    if (copy_ref)
-        for (int j = threadIdx.x; j < ud.m; j += blockDim.x)
-            s_ref_w[j] = make_double2(ref_xy[2 * (ud.ref_off + j)], ref_xy[2 * (ud.ref_off + j) + 1]);
-    __syncthreads();
-    const double INF = __longlong_as_double(0x7ff0000000000000LL);
-    // forward: reference -> rotated
-    double lmax = 0.0;
-    for (int i = threadIdx.x; i < ud.m; i += blockDim.x) {
-        const double2 a = s_ref[i];
-        double mn = INF;
-        for (int j = 0; j < ud.n; ++j) {
-            const double2 b = s_rot[j];
-            const double dx = __dsub_rn(a.x, b.x), dy = __dsub_rn(a.y, b.y);
-            const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
-            if (d2 < mn) mn = d2;
-        }
-        if (isfinite(mn) && mn > lmax) lmax = mn;
-    }
-    const double fwd = block_max(lmax, s_red);
-    // backward: rotated -> reference
-    lmax = 0.0;
-    for (int i = threadIdx.x; i < ud.n; i += blockDim.x) {
-        const double2 a = s_rot[i];
-        double mn = INF;
-        for (int j = 0; j < ud.m; ++j) {
-            const double2 b = s_ref[j];
-            const double dx = __dsub_rn(a.x, b.x), dy = __dsub_rn(a.y, b.y);
-            const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
-            if (d2 < mn) mn = d2;
-        }
-        if (isfinite(mn) && mn > lmax) lmax = mn;
-    }
-    const double bwd = block_max(lmax, s_red);
-    return fmax(__dsqrt_rn(fwd), __dsqrt_rn(bwd));
-}
-
-__global__ void __launch_bounds__(256)
-    k_exact(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
-            const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
-            const int2* __restrict__ items, const unsigned* __restrict__ n_items, unsigned pool_cap,
-            double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch, const double2* __restrict__ t64) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    double* s_red = reinterpret_cast<double*>(smem_raw);
-    // g_scratch != NULL: the point sets do not fit shared memory — rotated points in this CTA's global scratch row
-    double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
-    double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
-    const unsigned total = min(*n_items, pool_cap);
-    for (unsigned it = blockIdx.x; it < total; it += gridDim.x) {
-        const int2 item = items[it];
-        if (item.x < 0) continue;  // uniform per CTA
-        const UnitDesc ud = units[item.x];
-        const int c = item.y;
-        const int i = t64 ? c / ud.n_trans : c;
-        const double2 cs = cs64[ud.cand_off + i];
-        const bool identity = zero_flag[ud.cand_off + i] != 0;
-        const double2 t = t64 ? t64[ud.t_off + (c - i * ud.n_trans)] : make_double2(0.0, 0.0);
-        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr,
-                                    t64 != nullptr, t);
-        if (threadIdx.x == 0) sl_dist[it] = d;
-        __syncthreads();
-    }
-}
-
-// Dense variant: every candidate [c0, c0+count) of one unit (shortlist overflow
-// path and mmrs_eval_exact). t64 != NULL: rigid candidates; paired = true (mmrs_eval_exact_rigid): candidate c takes
-// angle c and translation t64[c] instead of the grid product.
-__global__ void __launch_bounds__(256)
-    k_exact_dense(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
-                  const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
-                  const unsigned char* __restrict__ zero_flag, long long cs_off, int count, double* __restrict__ out,
-                  int max_n, double2* __restrict__ g_scratch, const double2* __restrict__ t64, bool paired) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    double* s_red = reinterpret_cast<double*>(smem_raw);
-    double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
-    double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
-    const UnitDesc ud = units[unit];
-    for (int c = blockIdx.x; c < count; c += gridDim.x) {
-        const int i = (t64 && !paired) ? c / ud.n_trans : c;
-        const double2 cs = cs64[cs_off + i];
-        const bool identity = zero_flag[cs_off + i] != 0;
-        const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
-        const double d = exact_cost(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, g_scratch == nullptr,
-                                    t64 != nullptr, t);
-        if (threadIdx.x == 0) out[c] = d;
-        __syncthreads();
-    }
-}
-
-// ---- K3 for the partial cost --------------------------------------------------------------------------------------
 // (q + 1)-th largest of the n non-negative values v (duplicates counted), by the whole CTA: the v_i with
 // #{v_j > v_i} <= q < #{v_j >= v_i}. Every i that satisfies this holds the same value, so the result does not depend
 // on the order of the threads.
@@ -1581,12 +1474,13 @@ __device__ __forceinline__ double block_kth_largest(const double* v, int n, int 
     return block_max(sel, s_red);
 }
 
-// exact_cost with the partial cost: each directed value is the (q + 1)-th largest row minimum (a non-finite minimum
-// counts as 0) instead of the largest. s_min: n (or m) doubles of the CTA (shared memory or a global scratch row).
-__device__ __forceinline__ double exact_cost_partial(const UnitDesc& ud, const double* __restrict__ test_xy,
-                                                     const double* __restrict__ ref_xy, double cosv, double sinv,
-                                                     bool identity, double2* s_rot, const double2* s_ref_in, double* s_red,
-                                                     double* s_min, bool copy_ref, bool rigid, double2 t) {
+// Stages the transformed test set in s_rot and, with copy_ref, the reference set in s_ref_in; returns where the
+// reference set is read from. s_rot / s_ref_in: shared memory, or (units too large for it) a per-CTA scratch row in
+// global memory for the transformed points and the caller's reference array itself (copy_ref = false).
+__device__ __forceinline__ const double2* exact_stage(const UnitDesc& ud, const double* __restrict__ test_xy,
+                                                      const double* __restrict__ ref_xy, double cosv, double sinv,
+                                                      bool identity, double2* s_rot, const double2* s_ref_in,
+                                                      bool copy_ref, bool rigid, double2 t) {
     double2* s_ref_w = const_cast<double2*>(s_ref_in);
     const double2* s_ref = copy_ref ? s_ref_in : reinterpret_cast<const double2*>(ref_xy + 2 * ud.ref_off);
     for (int i = threadIdx.x; i < ud.n; i += blockDim.x) {
@@ -1604,8 +1498,21 @@ __device__ __forceinline__ double exact_cost_partial(const UnitDesc& ud, const d
         for (int j = threadIdx.x; j < ud.m; j += blockDim.x)
             s_ref_w[j] = make_double2(ref_xy[2 * (ud.ref_off + j)], ref_xy[2 * (ud.ref_off + j) + 1]);
     __syncthreads();
+    return s_ref;
+}
+
+// The cost of one candidate. Each directed value is the largest row minimum (a non-finite minimum is skipped) or,
+// PARTIAL, the (q + 1)-th largest (a non-finite minimum counts as 0); s_min: n (or m) doubles of the CTA (shared memory
+// or a global scratch row) that hold the row minima of the partial cost.
+template <bool PARTIAL>
+__device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* __restrict__ test_xy,
+                                             const double* __restrict__ ref_xy, double cosv, double sinv, bool identity,
+                                             double2* s_rot, const double2* s_ref_in, double* s_red, double* s_min,
+                                             bool copy_ref, bool rigid, double2 t) {
+    const double2* s_ref = exact_stage(ud, test_xy, ref_xy, cosv, sinv, identity, s_rot, s_ref_in, copy_ref, rigid, t);
     const double INF = __longlong_as_double(0x7ff0000000000000LL);
     auto directed = [&](const double2* rows, int nr, const double2* set, int ns, int q) {
+        double lmax = 0.0;
         for (int i = threadIdx.x; i < nr; i += blockDim.x) {
             const double2 a = rows[i];
             double mn = INF;
@@ -1615,8 +1522,10 @@ __device__ __forceinline__ double exact_cost_partial(const UnitDesc& ud, const d
                 const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
                 if (d2 < mn) mn = d2;
             }
-            s_min[i] = isfinite(mn) ? mn : 0.0;
+            if (PARTIAL) s_min[i] = isfinite(mn) ? mn : 0.0;
+            else if (isfinite(mn) && mn > lmax) lmax = mn;
         }
+        if (!PARTIAL) return block_max(lmax, s_red);
         __syncthreads();
         return block_kth_largest(s_min, nr, q, s_red);   // ends with a barrier: s_min may be reused
     };
@@ -1625,16 +1534,18 @@ __device__ __forceinline__ double exact_cost_partial(const UnitDesc& ud, const d
     return fmax(__dsqrt_rn(fwd), __dsqrt_rn(bwd));
 }
 
-// k_exact / k_exact_dense for the partial cost; g_min != NULL: the CTA's row minima in a global scratch row (with
-// g_scratch), else shared memory after the two staged sets.
+// PARTIAL: g_min != NULL puts the CTA's row minima in a global scratch row (with g_scratch), else shared memory after
+// the two staged sets.
+template <bool PARTIAL>
 __global__ void __launch_bounds__(256)
-    k_exact_partial(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
-                    const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
-                    const int2* __restrict__ items, const unsigned* __restrict__ n_items, unsigned pool_cap,
-                    double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min,
-                    const double2* __restrict__ t64) {
+    k_exact(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
+            const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
+            const int2* __restrict__ items, const unsigned* __restrict__ n_items, unsigned pool_cap,
+            double* __restrict__ sl_dist, int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min,
+            const double2* __restrict__ t64) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* s_red = reinterpret_cast<double*>(smem_raw);
+    // g_scratch != NULL: the point sets do not fit shared memory — rotated points in this CTA's global scratch row
     double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
     double2* s_ref = g_scratch ? nullptr : s_rot + max_n;
     double* s_min = g_min ? g_min + (size_t)blockIdx.x * max_n : reinterpret_cast<double*>(s_ref + max_n);
@@ -1648,19 +1559,23 @@ __global__ void __launch_bounds__(256)
         const double2 cs = cs64[ud.cand_off + i];
         const bool identity = zero_flag[ud.cand_off + i] != 0;
         const double2 t = t64 ? t64[ud.t_off + (c - i * ud.n_trans)] : make_double2(0.0, 0.0);
-        const double d = exact_cost_partial(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
-                                            g_scratch == nullptr, t64 != nullptr, t);
+        const double d = exact_cost<PARTIAL>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+                                             g_scratch == nullptr, t64 != nullptr, t);
         if (threadIdx.x == 0) sl_dist[it] = d;
         __syncthreads();
     }
 }
 
+// Dense variant: every candidate [c0, c0+count) of one unit (shortlist overflow
+// path and mmrs_eval_exact). t64 != NULL: rigid candidates; paired = true (mmrs_eval_exact_rigid): candidate c takes
+// angle c and translation t64[c] instead of the grid product.
+template <bool PARTIAL>
 __global__ void __launch_bounds__(256)
-    k_exact_dense_partial(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
-                          const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
-                          const unsigned char* __restrict__ zero_flag, long long cs_off, int count, double* __restrict__ out,
-                          int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min,
-                          const double2* __restrict__ t64, bool paired) {
+    k_exact_dense(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
+                  const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
+                  const unsigned char* __restrict__ zero_flag, long long cs_off, int count, double* __restrict__ out,
+                  int max_n, double2* __restrict__ g_scratch, double* __restrict__ g_min, const double2* __restrict__ t64,
+                  bool paired) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double* s_red = reinterpret_cast<double*>(smem_raw);
     double2* s_rot = g_scratch ? g_scratch + (size_t)blockIdx.x * max_n : reinterpret_cast<double2*>(smem_raw + 64);
@@ -1672,8 +1587,8 @@ __global__ void __launch_bounds__(256)
         const double2 cs = cs64[cs_off + i];
         const bool identity = zero_flag[cs_off + i] != 0;
         const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
-        const double d = exact_cost_partial(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
-                                            g_scratch == nullptr, t64 != nullptr, t);
+        const double d = exact_cost<PARTIAL>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+                                             g_scratch == nullptr, t64 != nullptr, t);
         if (threadIdx.x == 0) out[c] = d;
         __syncthreads();
     }
