@@ -82,12 +82,11 @@ struct mmrs_ctx {
         size_t smem = 0;
         size_t work_begin = 0, work_count = 0;  // range of h_work / d_work
         long long cost = 0;                     // padded pair evaluations per candidate, summed over the class
-        size_t smem_eb = 0;                     // shared memory of a K1e CTA (k_sweep_eb) of this class
+        int eb_warps = 0;                       // warps per CTA of the early-break kernel (k_sweep_eb): 8 for K1e,
+                                                // 8, 4, 2 or 1 for K1e-partial
+        size_t smem_eb = 0;                     // its shared memory per CTA
         bool eb = false;                        // the dense sweep of this class runs K1e (decided per grid set)
         long long live = 0;                     // candidates of this class swept by this rank
-        size_t stage = 0, ebp_warp = 0;         // partial cost: largest staging image / per-warp block of the class
-        int ebp_warps = 0;                      // warps per CTA of the partial kernel (8, 4, 2 or 1)
-        size_t smem_ebp = 0;
     };
     std::vector<SweepClass> classes;
     std::vector<int> class_of_unit;

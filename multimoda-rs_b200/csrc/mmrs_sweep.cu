@@ -424,6 +424,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
     ctx->classes.clear();
     ctx->class_of_unit.assign(U, -1);
     ctx->big_scratch_per_warp = 0;
+    std::vector<size_t> ebp_stage, ebp_warp;   // partial cost, per class: the largest staging and per-warp block
     long long lay_off = 0;
     for (int64_t u = 0; u < U; ++u) {
         UnitDesc& d = units[u];
@@ -449,14 +450,11 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             d.n_chunks = cc.n_chunks;
             d.n_tail = cc.tailp ? d.n - 32 * cc.ta : 0;
             d.m_pairs = (d.m + 1) / 2;
-            const long long a_elems = (long long)d.n_chunks * ((cc.ta + 1) / 2) * 32,
-                            b_elems = cc.tailp ? 16 * (cc.ta + 1) : d.m_pairs,   // exact tiling pads the B block (k_prep)
-                            nb_elems = (b_elems + 1) / 2,                        // squared norms of the reference points
-                            t_elems = (d.n_tail + 1) / 2;
-            lay_off += a_elems + b_elems + nb_elems + t_elems;
-            // shared memory of a CTA of this unit: mbarrier + key, the staging image, then per warp either the chunked
-            // column minima (MULTI) or the tail pass's column seeds (exact tiling)
-            size_t smem = 16 + (size_t)(a_elems + b_elems + nb_elems + t_elems) * 16;
+            const StageLayout sl = stage_layout(cc.ta, d.n_chunks, d.n_tail, d.m_pairs);
+            const size_t stage = 16 + (size_t)sl.total() * 16;   // mbarrier + key, then the staging image
+            // shared memory of a K1 CTA of this unit: the staging, then per warp either the chunked column minima (MULTI)
+            // or the tail pass's column seeds (exact tiling)
+            size_t smem = stage;
             if (d.n_chunks > 1) smem += (size_t)kWarpsPerCta * ((2 * d.m_pairs + 3) & ~3) * 4;
             if (cc.tailp) smem += (size_t)kWarpsPerCta * 32 * (cc.ta + 1) * 4;
             static const bool force_big = std::getenv("MMRS_FORCE_BIG") && std::getenv("MMRS_FORCE_BIG")[0] == '1';
@@ -464,14 +462,13 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             if (big) {
                 // does not fit K1's shared-memory staging: K1b streams the reference set through shared memory in blocks
                 // (k_sweep_big; register tile 16, the whole staging image stays in global memory / L2)
-                lay_off -= a_elems + b_elems + nb_elems + t_elems;
                 d.ta = kBigTA;
                 d.n_chunks = (d.n + 32 * kBigTA - 1) / (32 * kBigTA);
                 d.n_tail = 0;
-                lay_off += (long long)d.n_chunks * (kBigTA / 2) * 32 + d.m_pairs + (d.m_pairs + 1) / 2;
                 smem = 0;
                 ctx->big_scratch_per_warp = std::max<long long>(ctx->big_scratch_per_warp, (long long)d.n_chunks * 32 * kBigTA);
             }
+            lay_off += stage_layout(d.ta, d.n_chunks, d.n_tail, d.m_pairs).total();
             int k = 0;
             for (; k < (int)ctx->classes.size(); ++k) {
                 const auto& c = ctx->classes[k];
@@ -480,34 +477,36 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             if (k == (int)ctx->classes.size()) {
                 mmrs_ctx::SweepClass c;
                 c.ta = big ? kBigTA : cc.ta, c.multi = d.n_chunks > 1, c.tailp = !big && cc.tailp, c.big = big;
+                c.eb_warps = kWarpsPerCta;
                 ctx->classes.push_back(c);
+                ebp_stage.push_back(0), ebp_warp.push_back(0);
             }
-            ctx->classes[k].smem = std::max(ctx->classes[k].smem, smem);
-            if (!big)   // K1e: the same staging image plus, per warp, A' and the row / column hints
-                ctx->classes[k].smem_eb = std::max(ctx->classes[k].smem_eb, 16 + (size_t)(a_elems + b_elems + nb_elems + t_elems) * 16 +
-                                                                              (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m));
-            ctx->classes[k].cost += (long long)d.n_chunks * 32 * d.ta * d.m;
+            auto& cl = ctx->classes[k];
+            cl.smem = std::max(cl.smem, smem);
+            cl.cost += (long long)d.n_chunks * 32 * d.ta * d.m;
             ctx->class_of_unit[u] = k;
             if (ctx->partial && big)
                 return set_err(ctx, MMRS_ERR_ARG, "partial cost: unit " + std::to_string(u) +
                                                       " is beyond the shared-memory staging (more than ~4 000 points per set)");
             if (ctx->partial) {
-                auto& cl = ctx->classes[k];
-                cl.stage = std::max(cl.stage, 16 + (size_t)(a_elems + b_elems + nb_elems + t_elems) * 16);
-                cl.ebp_warp = std::max(cl.ebp_warp, (size_t)ebp_warp_bytes(d.n, d.m, d.q_bwd, d.q_fwd));
+                ebp_stage[k] = std::max(ebp_stage[k], stage);
+                ebp_warp[k] = std::max(ebp_warp[k], (size_t)ebp_warp_bytes(d.n, d.m, d.q_bwd, d.q_fwd));
+            } else if (!big) {   // K1e: the same staging image plus, per warp, A' and the row / column hints
+                cl.smem_eb = std::max(cl.smem_eb, stage + (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m));
             }
         }
     }
     if (ctx->partial) {
-        // K1e-partial: 8 warps per CTA where the staging image and 8 per-warp blocks fit the 227 KB a CTA may have,
-        // else 4, 2 or 1 (the chunked 2 020-point units take 4)
-        for (auto& cl : ctx->classes) {
-            cl.ebp_warps = 0;
-            for (int wp = kWarpsPerCta; wp >= 1 && !cl.ebp_warps; wp /= 2)
-                if (cl.stage + wp * cl.ebp_warp <= (size_t)kMaxDynSmem) cl.ebp_warps = wp;
-            if (!cl.ebp_warps)
+        // K1e-partial: 8 warps per CTA where the largest staging image and 8 of the largest per-warp blocks fit the
+        // 227 KB a CTA may have, else 4, 2 or 1 (the chunked 2 020-point units take 4)
+        for (size_t k = 0; k < ctx->classes.size(); ++k) {
+            auto& cl = ctx->classes[k];
+            cl.eb_warps = 0;
+            for (int wp = kWarpsPerCta; wp >= 1 && !cl.eb_warps; wp /= 2)
+                if (ebp_stage[k] + wp * ebp_warp[k] <= (size_t)kMaxDynSmem) cl.eb_warps = wp;
+            if (!cl.eb_warps)
                 return set_err(ctx, MMRS_ERR_ARG, "partial cost: a unit does not fit the shared memory of one warp");
-            cl.smem_ebp = cl.stage + cl.ebp_warps * cl.ebp_warp;
+            cl.smem_eb = ebp_stage[k] + cl.eb_warps * ebp_warp[k];
         }
     }
     {   // tensor-core prefilter: every non-empty unit must fit its operand layout
@@ -900,8 +899,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             cl.work_begin = ctx->h_work.size();
             const long long eb_slots = (long long)ctx->n_sm * 3 * 4 * kWarpsPerCta;
             const long long run = std::max(kEbMinRun, std::min(kEbMaxRun, (cl.live + eb_slots - 1) / eb_slots));
-            // K1e-partial: K1e's run per warp, ebp_warps warps per CTA
-            const int tile_k = ctx->partial ? (int)(cl.ebp_warps * run) : cl.eb ? (int)(kWarpsPerCta * run) : tile;
+            const int tile_k = ctx->partial || cl.eb ? (int)(cl.eb_warps * run) : tile;
             for (int64_t u = 0; u < U; ++u) {
                 const UnitDesc& d = units[u];
                 if (d.flags || ctx->class_of_unit[u] != (int)k) continue;
@@ -1331,18 +1329,13 @@ static int sweep_class(mmrs_ctx* ctx, const mmrs_ctx::SweepClass& cl, const floa
             ctx->eb_ran = true;
         }
         unsigned long long* pairs = (unsigned long long*)ctx->d_eb_pairs.p;
-        if (ctx->partial) {   // K1e-partial (every class: big units are refused at upload)
-            if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<true>));
-            else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_ebp<false>));
-            auto ebp = t32 ? k_sweep_ebp<true> : k_sweep_ebp<false>;
-            ebp<<<(unsigned)cl.work_count, cl.ebp_warps * 32, cl.smem_ebp, s>>>(units, work, lay, cs32, dist32, key, pairs,
-                                                                                  t32, ctx->eb_env != 0 ? 1 : 0);
-        } else {
-            if (t32) CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<true>));
-            else CUDA_TRY(ctx, RAISE_SMEM(k_sweep_eb<false>));
-            auto eb = t32 ? k_sweep_eb<true> : k_sweep_eb<false>;
-            eb<<<(unsigned)cl.work_count, kThreads, cl.smem_eb, s>>>(units, work, lay, cs32, dist32, key, pairs, t32);
-        }
+        // K1e-partial for the partial cost (every class: big units are refused at upload), else K1e
+        if (ctx->partial) CUDA_TRY(ctx, t32 ? RAISE_SMEM((k_sweep_eb<true, true>)) : RAISE_SMEM((k_sweep_eb<false, true>)));
+        else CUDA_TRY(ctx, t32 ? RAISE_SMEM((k_sweep_eb<true, false>)) : RAISE_SMEM((k_sweep_eb<false, false>)));
+        auto eb = ctx->partial ? (t32 ? k_sweep_eb<true, true> : k_sweep_eb<false, true>)
+                               : (t32 ? k_sweep_eb<true, false> : k_sweep_eb<false, false>);
+        eb<<<(unsigned)cl.work_count, cl.eb_warps * 32, cl.smem_eb, s>>>(units, work, lay, cs32, dist32, key, pairs, t32,
+                                                                          ctx->eb_env != 0 ? 1 : 0);
         ctx->eb_cands += cl.live;
     } else if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units, work, lay, cs32, dist32,
                              key, nullptr, false, t32)) {

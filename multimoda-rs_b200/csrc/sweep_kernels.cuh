@@ -9,9 +9,16 @@
 //                     a register-tiled min-over-M / max-over-N with packed
 //                     f32x2 arithmetic (FADD2/FMUL2/FFMA2), 3-input FMNMX and
 //                     warp REDUX; fused per-unit arg-min on a packed
-//                     (distance, index) 64-bit key with atomicMin.
-//   K1e k_sweep_eb    the dense sweep with early-break directed passes: every candidate's FP32 distance,
+//                     (distance, index) 64-bit key with atomicMin. Also re-scores
+//                     candidate lists (LIST) and runs the expanded-form tier K1x (XF).
+//   K1e k_sweep_eb<RIGID, false>
+//                     the dense sweep with early-break directed passes: every candidate's FP32 distance,
 //                     bit-identical to K1, from ~1 % of the pair distances (default wherever it fits)
+//   K1e-partial k_sweep_eb<RIGID, true>
+//                     the same passes for the partial (rank-K) cost: per direction the q + 1 largest exact minima
+//   K1b k_sweep_big   the FP32 sweep for units beyond K1's shared-memory staging (reference set streamed in blocks)
+//   K1p k_prep_lb, k_lb, k_lb_argmin
+//                     exact lower-bound pruning tier: candidates bounded above the best are never scored
 //   K2  k_shortlist   candidates within the FP32 error window of the minimum
 //   K3  k_exact       the reference's f64 arithmetic, literally, on those
 //   K4  k_select      leftmost f64 arg-min + tie count per unit
@@ -121,25 +128,32 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t phase) {
 // Tail block (exact tiling, UnitDesc.n_tail > 0; after the NB block): the n mod 32 test points that do not fill a
 // register slot, two per float4 (x0, y0, x1, y1). K1 scores them in a short pass of its own instead of a padded slot.
 // =============================================================================
+// Block sizes of one unit's staging image in float4. The B block of exact tiling (n_tail > 0) is padded to 16 (TA + 1)
+// float4 so that the tail pass can address its reference points lane + 32 q without clamping.
+struct StageLayout {
+    int a, b, nb, t;   // A, B, NB (float2 per pair of reference points, rounded up to float4) and tail blocks
+    __host__ __device__ int total() const { return a + b + nb + t; }
+};
+__host__ __device__ inline StageLayout stage_layout(int ta, int n_chunks, int n_tail, int m_pairs) {
+    const int b = n_tail > 0 ? 16 * (ta + 1) : m_pairs;
+    return StageLayout{n_chunks * ((ta + 1) / 2) * 32, b, (b + 1) / 2, (n_tail + 1) / 2};
+}
+
 __global__ void k_prep(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy,
                        const double* __restrict__ ref_xy, float4* __restrict__ lay, unsigned* __restrict__ rmax_bits) {
     const UnitDesc ud = units[blockIdx.x];
     if (ud.n <= 0 || ud.m <= 0) return;
     const int TA = ud.ta;
     const int half = (TA + 1) / 2, pairs = TA / 2;
-    const int a_elems = ud.n_chunks * half * 32;
+    const StageLayout sl = stage_layout(TA, ud.n_chunks, ud.n_tail, ud.m_pairs);
     // exact tiling (n_tail > 0): the register slots hold the first 32 TA points only, the rest is the tail block
     const int n_main = ud.n - ud.n_tail;
-    // exact tiling: the B block is padded to 16 (TA + 1) float4 so that the tail pass can address its reference points
-    // lane + 32 q without clamping (indices past the end repeat the last point)
-    const int b_elems = ud.n_tail > 0 ? 16 * (TA + 1) : ud.m_pairs;
-    const int nb_elems = (b_elems + 1) / 2;   // NB block: |b|^2 of the FP32 reference points, float2 per pair of points
     float4* A = lay + ud.lay_off;
-    float4* B = A + a_elems;
-    float2* NB = reinterpret_cast<float2*>(B + b_elems);
-    float4* T = B + b_elems + nb_elems;
+    float4* B = A + sl.a;
+    float2* NB = reinterpret_cast<float2*>(B + sl.b);
+    float4* T = B + sl.b + sl.nb;
     float rmax = 0.f;
-    for (int e = threadIdx.x; e < a_elems; e += blockDim.x) {
+    for (int e = threadIdx.x; e < sl.a; e += blockDim.x) {
         int l = e & 31, ck = e >> 5;
         int c = ck / half, k = ck - c * half;
         int i0 = c * 32 * TA + 2 * k * 32 + l, i1 = (k < pairs) ? i0 + 32 : i0;
@@ -155,7 +169,7 @@ __global__ void k_prep(const UnitDesc* __restrict__ units, const double* __restr
         A[e] = v;
         rmax = fmaxf(rmax, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
     }
-    for (int j = threadIdx.x; j < b_elems; j += blockDim.x) {
+    for (int j = threadIdx.x; j < sl.b; j += blockDim.x) {
         const int j0 = min(2 * j, ud.m - 1), j1 = min(2 * j + 1, ud.m - 1);
         const double* p0 = ref_xy + 2 * (ud.ref_off + j0);
         const double* p1 = ref_xy + 2 * (ud.ref_off + j1);
@@ -166,7 +180,7 @@ __global__ void k_prep(const UnitDesc* __restrict__ units, const double* __restr
         NB[j] = make_float2((float)((double)v.x * v.x + (double)v.y * v.y), (float)((double)v.z * v.z + (double)v.w * v.w));
         rmax = fmaxf(rmax, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
     }
-    if (threadIdx.x == 0 && (b_elems & 1)) NB[b_elems] = make_float2(0.f, 0.f);   // padding of the odd float4
+    if (threadIdx.x == 0 && (sl.b & 1)) NB[sl.b] = make_float2(0.f, 0.f);   // padding of the odd float4
     // tail block: float4 t = tail points 2t and 2t+1 as (x0, y0, x1, y1) (an odd count repeats the last point)
     for (int t = threadIdx.x; t < (ud.n_tail + 1) / 2; t += blockDim.x) {
         const int i0 = n_main + min(2 * t, ud.n_tail - 1), i1 = n_main + min(2 * t + 1, ud.n_tail - 1);
@@ -565,8 +579,9 @@ __global__ void __launch_bounds__(kThreads, 2)
 }
 
 // =============================================================================
-// K1e: the dense sweep with EARLY-BREAK directed passes. Same work items, staging image (one TMA bulk copy) and outputs
-// (dist32, the packed (distance, index) key) as K1, but a candidate no longer costs all N M pair distances:
+// K1e (k_sweep_eb<RIGID, false>): the dense sweep with EARLY-BREAK directed passes. Same work items, staging image (one
+// TMA bulk copy) and outputs (dist32, the packed (distance, index) key) as K1, but a candidate no longer costs all N M
+// pair distances:
 //     H^2 = max( max_a min_b d^2 , max_b min_a d^2 ),
 // and once L, an exactly computed row or column minimum of THIS candidate, is known, a row that meets one b with
 // d^2 <= L cannot raise the maximum and stops there. Per warp, over a contiguous run of the tile's candidates:
@@ -627,172 +642,50 @@ __device__ __forceinline__ int eb_warp_argmax(unsigned v, int idx) {
     return __shfl_sync(0xffffffffu, idx, __ffs(__ballot_sync(0xffffffffu, v == m)) - 1);
 }
 
-// RIGID = true: rigid candidates, c = i n_trans + j (see k_sweep): A'[k] = R a_k + t, the translation added once with
-// __fadd_rn when the row is materialised; the column pass reads the same A', so K1e stays bit-identical to K1.
-template <bool RIGID = false>
-__global__ void __launch_bounds__(kThreads, 3)
-    k_sweep_eb(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
-               const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
-               unsigned long long* __restrict__ pairs_out, const float2* __restrict__ t32) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
-    unsigned long long* s_key = reinterpret_cast<unsigned long long*>(smem_raw + 8);
-    float4* sA = reinterpret_cast<float4*>(smem_raw + 16);
-    const WorkItem w = work[blockIdx.x];
-    const UnitDesc ud = units[w.unit];
-    const int lane = threadIdx.x & 31, wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-    const int TA = ud.ta, S = (TA + 1) / 2, N = ud.n, M = ud.m, n_main = N - ud.n_tail;
-    const int a_elems = ud.n_chunks * S * 32;
-    const int b_elems = ud.n_tail > 0 ? 16 * (TA + 1) : ud.m_pairs;
-    const int nb_elems = (b_elems + 1) / 2, t_elems = (ud.n_tail + 1) / 2;
-    const float4* sB4 = sA + a_elems;
-    const float2* sB = reinterpret_cast<const float2*>(sB4);                              // reference point j
-    const float2* sT = reinterpret_cast<const float2*>(sB4 + b_elems + nb_elems);         // tail point t
-    unsigned char* my = reinterpret_cast<unsigned char*>(sA + a_elems + b_elems + nb_elems + t_elems) + wid * eb_warp_bytes(N, M);
-    float2* sR = reinterpret_cast<float2*>(my);                                           // A': rotated test points
-    unsigned short* hr = reinterpret_cast<unsigned short*>(sR + N);                       // row hints
-    unsigned short* hc = hr + N;                                                          // column hints
-    if (threadIdx.x == 0) {
-        mbar_init(bar, 1);
-        *s_key = ~0ull;
-        const uint32_t bytes = (uint32_t)(a_elems + b_elems + nb_elems + t_elems) * 16u;
-        mbar_expect_tx(bar, bytes);
-        tma_bulk_g2s(sA, lay + ud.lay_off, bytes, bar);
-    }
-    __syncthreads();
-    mbar_wait(bar, 0);
-
-    // test point i of the staging image (K0's layout: register slots, then the exact-tiling tail block)
-    auto test_pt = [&](int i) -> float2 {
-        if (i >= n_main) return sT[i - n_main];
-        const int c = i / (32 * TA), r = i - c * 32 * TA;
-        const float4 v = sA[(c * S + (r >> 6)) * 32 + (r & 31)];
-        return (r & 32) ? make_float2(v.y, v.w) : make_float2(v.x, v.z);
-    };
-    // this warp's contiguous run of candidates: neighbouring angles keep the hints valid
-    const int per = (w.count + kWarpsPerCta - 1) / kWarpsPerCta;
-    const int c_begin = w.begin + min(w.count, wid * per), c_end = w.begin + min(w.count, (wid + 1) * per);
-    unsigned long long best = ~0ull;
-    unsigned pairs = 0;
-    if (c_begin < c_end) {
-        // first candidate: hints on the index diagonal, seeds at the points farthest from the rotation centre
-        unsigned far_a = 0u, far_b = 0u;
-        int ia = 0, ib = 0;
-        for (int i = lane; i < N; i += 32) {
-            const float2 p = test_pt(i);
-            const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
-            if (r2 > far_a) far_a = r2, ia = i;
-            hr[i] = (unsigned short)(((long long)i * M) / N);
-        }
-        for (int j = lane; j < M; j += 32) {
-            const float2 p = sB[j];
-            const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
-            if (r2 > far_b) far_b = r2, ib = j;
-            hc[j] = (unsigned short)(((long long)j * N) / M);
-        }
-        int ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
-        for (int c = c_begin; c < c_end; ++c) {
-            float2 tr = make_float2(0.f, 0.f);
-            int ia = c;
-            if (RIGID) {
-                ia = c / ud.n_trans;
-                tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
-            }
-            const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
-            __syncwarp();   // the previous candidate is done with A' and the hints
-            for (int i = lane; i < N; i += 32) {
-                const float2 p = test_pt(i);
-                float2 r = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
-                if (RIGID) r = make_float2(__fadd_rn(r.x, tr.x), __fadd_rn(r.y, tr.y));
-                sR[i] = r;
-            }
-            __syncwarp();
-            int arg;
-            unsigned L = eb_warp_min(sB, M, sR[ra], hr[ra], 0u, false, lane, arg, pairs);
-            const int h_ra = arg;
-            const unsigned lc = eb_warp_min(sR, N, sB[cb], hc[cb], 0u, false, lane, arg, pairs);
-            __syncwarp();
-            if (lane == 0) hr[ra] = (unsigned short)h_ra, hc[cb] = (unsigned short)arg;
-            L = max(L, lc);
-            __syncwarp();
-            // rows: test point i against the reference points
-            for (int g = 0; g < N; g += 32) {
-                const int i = g + lane;
-                bool open = false;
-                if (i < N) {
-                    const float2 a = sR[i];
-                    const int h = hr[i];
-                    open = true;
-                    for (int t = 0; t < kEbTries && t < M; ++t) {
-                        const int j = eb_zig(h, t, M);
-                        ++pairs;
-                        if (__float_as_uint(eb_d2(a, sB[j])) <= L) {
-                            hr[i] = (unsigned short)j;
-                            open = false;
-                            break;
-                        }
-                    }
-                }
-                for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
-                    const int ii = g + __ffs(open_mask) - 1;
-                    const unsigned mn = eb_warp_min(sB, M, sR[ii], hr[ii], L, true, lane, arg, pairs);
-                    if (mn > L) L = mn, ra = ii;
-                    __syncwarp();
-                    if (lane == 0) hr[ii] = (unsigned short)arg;
-                }
-            }
-            // columns: reference point j against A'
-            for (int g = 0; g < M; g += 32) {
-                const int j = g + lane;
-                bool open = false;
-                if (j < M) {
-                    const float2 b = sB[j];
-                    const int h = hc[j];
-                    open = true;
-                    for (int t = 0; t < kEbTries && t < N; ++t) {
-                        const int i = eb_zig(h, t, N);
-                        ++pairs;
-                        if (__float_as_uint(eb_d2(sR[i], b)) <= L) {
-                            hc[j] = (unsigned short)i;
-                            open = false;
-                            break;
-                        }
-                    }
-                }
-                for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
-                    const int jj = g + __ffs(open_mask) - 1;
-                    const unsigned mn = eb_warp_min(sR, N, sB[jj], hc[jj], L, true, lane, arg, pairs);
-                    if (mn > L) L = mn, cb = jj;
-                    __syncwarp();
-                    if (lane == 0) hc[jj] = (unsigned short)arg;
-                }
-            }
-            const float d = sqrtf(__uint_as_float(L));
-            if (lane == 0) {
-                dist32[ud.dist_off + c] = d;
-                best = min(best, ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)c);
+// Rows g .. g + 31 of one direction of the early-break passes (call it with the full warp): rows R[i] against the n_set
+// points of P, with the rows' hints h; open: row g + lane takes part. Lane l first tries kEbTries positions of the
+// zig-zag around the hint of row g + l; the rows still open are then finished one at a time by the whole warp. A row
+// stops at its first d^2 <= L and keeps that position as its hint; a row that scans to its end has an exact minimum
+// mn > L, and L becomes exact(mn, i).
+template <class Exact>
+__device__ __forceinline__ void eb_rows(const float2* R, int g, bool open, const float2* P, int n_set, unsigned short* h,
+                                        unsigned& L, Exact exact, int lane, unsigned& pairs) {
+    if (open) {
+        const int i = g + lane;
+        const float2 a = R[i];
+        const int h0 = h[i];
+        for (int t = 0; t < kEbTries && t < n_set; ++t) {
+            const int j = eb_zig(h0, t, n_set);
+            ++pairs;
+            if (__float_as_uint(eb_d2(a, P[j])) <= L) {
+                h[i] = (unsigned short)j;
+                open = false;
+                break;
             }
         }
     }
-    const unsigned warp_pairs = __reduce_add_sync(0xffffffffu, pairs);
-    if (lane == 0 && pairs_out && warp_pairs) atomicAdd(pairs_out, (unsigned long long)warp_pairs);
-    if (lane == 0 && best != ~0ull) atomicMin(s_key, best);
-    __syncthreads();
-    if (threadIdx.x == 0 && *s_key != ~0ull) atomicMin(&key[w.unit], *s_key);
+    for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
+        const int ii = g + __ffs(open_mask) - 1;
+        int arg;
+        const unsigned mn = eb_warp_min(P, n_set, R[ii], h[ii], L, true, lane, arg, pairs);
+        __syncwarp();
+        if (lane == 0) h[ii] = (unsigned short)arg;
+        if (mn > L) L = exact(mn, ii);
+    }
 }
 
 // =============================================================================
-// K1e-partial (k_sweep_ebp): the early-break sweep for the PARTIAL cost (include/mmrs_b200.h "partial cost"). In each
-// direction the directed value is the (q + 1)-th largest row minimum instead of the largest, so the q worst points of
-// each set do not count. Same work items, staging image and outputs as K1e; per warp, over its contiguous run:
+// K1e-partial (k_sweep_eb<RIGID, true>): the early-break sweep for the PARTIAL cost (include/mmrs_b200.h "partial
+// cost"). In each direction the directed value is the (q + 1)-th largest row minimum instead of the largest, so the q
+// worst points of each set do not count. Same work items, staging image and outputs as K1e; per warp, over its
+// contiguous run:
 //   lists   per direction the q + 1 largest EXACT minima found so far (float bits + point index) in per-warp shared
 //           memory; kth = the smallest of them when the list is full, else 0; L = max(kth_rows, kth_cols);
 //   seed    the rows of the previous candidate's list in the direction that defined its value (the run's first
 //           candidate: the q + 1 points farthest from the centre, both directions), each scanned to its end by one
 //           lane; they enter the list and are marked so that the main pass skips them;
-//   rows    exactly K1e's passes: zig-zag tries from the hints, then the warp finishes the open rows; a row stops at
-//           the first d^2 <= L; a row that scans to its end has an exact minimum > L and enters its list (replacing
-//           the smallest entry when full); L is recomputed;
+//   rows    K1e's pass (eb_rows) with the seeded rows left out: a row that scans to its end has an exact minimum > L
+//           and enters its list (replacing the smallest entry when full); L is recomputed;
 //   columns the same with the reference points as rows.
 // Exactness (F = max(V_r, V_c), V the true (q + 1)-th largest FP32 minimum of a direction): L is always the (q + 1)-th
 // largest of a subset of exact minima, so L <= F; a row that was not collected has a minimum <= L at that time <=
@@ -850,95 +743,118 @@ __device__ __forceinline__ unsigned eb_lane_min(const float2* P, int n, float2 a
     return best;
 }
 
-// RIGID: as in k_sweep_eb. Warps per CTA = blockDim.x / 32 (the host picks 8, 4, 2 or 1 per size class).
-template <bool RIGID>
-__global__ void __launch_bounds__(kThreads, 2)
-    k_sweep_ebp(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
-                const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
-                unsigned long long* __restrict__ pairs_out, const float2* __restrict__ t32, int early) {
+// RIGID = true: rigid candidates, c = i n_trans + j (see k_sweep): A'[k] = R a_k + t, the translation added once with
+// __fadd_rn when the row is materialised; the column pass reads the same A', so K1e stays bit-identical to K1.
+// PARTIAL = false: K1e, kWarpsPerCta warps per CTA; early is not read.
+// PARTIAL = true: K1e-partial, blockDim.x / 32 warps per CTA (the host picks 8, 4, 2 or 1 per size class).
+template <bool RIGID, bool PARTIAL>
+__global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
+    k_sweep_eb(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
+               const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
+               unsigned long long* __restrict__ pairs_out, const float2* __restrict__ t32, int early) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw);
     unsigned long long* s_key = reinterpret_cast<unsigned long long*>(smem_raw + 8);
     float4* sA = reinterpret_cast<float4*>(smem_raw + 16);
     const WorkItem w = work[blockIdx.x];
     const UnitDesc ud = units[w.unit];
-    const int n_warps = blockDim.x >> 5;
+    const int n_warps = PARTIAL ? blockDim.x >> 5 : kWarpsPerCta;
     const int lane = threadIdx.x & 31, wid = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
     const int TA = ud.ta, S = (TA + 1) / 2, N = ud.n, M = ud.m, n_main = N - ud.n_tail;
-    const int a_elems = ud.n_chunks * S * 32;
-    const int b_elems = ud.n_tail > 0 ? 16 * (TA + 1) : ud.m_pairs;
-    const int nb_elems = (b_elems + 1) / 2, t_elems = (ud.n_tail + 1) / 2;
-    const float4* sB4 = sA + a_elems;
-    const float2* sB = reinterpret_cast<const float2*>(sB4);
-    const float2* sT = reinterpret_cast<const float2*>(sB4 + b_elems + nb_elems);
-    unsigned char* my = reinterpret_cast<unsigned char*>(sA + a_elems + b_elems + nb_elems + t_elems) +
-                        wid * ebp_warp_bytes(N, M, ud.q_bwd, ud.q_fwd);
-    float2* sR = reinterpret_cast<float2*>(my);
-    unsigned short* hint[2];
-    hint[0] = reinterpret_cast<unsigned short*>(sR + N);   // rows: test point i against the reference points
-    hint[1] = hint[0] + N;                                 // columns: reference point j against A'
-    unsigned* lp = reinterpret_cast<unsigned*>(my + eb_warp_bytes(N, M));
-    EbList lst[2];
-    lst[0].cap = ud.q_bwd + 1, lst[1].cap = ud.q_fwd + 1;
-    lst[0].val = lp;
-    lst[0].idx = reinterpret_cast<int*>(lp + lst[0].cap);
-    lst[1].val = lp + 2 * lst[0].cap;
-    lst[1].idx = reinterpret_cast<int*>(lst[1].val + lst[1].cap);
-    unsigned* bits[2];
-    bits[0] = lp + 2 * (lst[0].cap + lst[1].cap);
-    bits[1] = bits[0] + (N + 31) / 32;
+    const StageLayout sl = stage_layout(TA, ud.n_chunks, ud.n_tail, ud.m_pairs);
+    const float2* sB = reinterpret_cast<const float2*>(sA + sl.a);                        // reference point j
+    const float2* sT = reinterpret_cast<const float2*>(sA + sl.a + sl.b + sl.nb);         // tail point t
+    unsigned char* my = reinterpret_cast<unsigned char*>(sA + sl.a + sl.b + sl.nb + sl.t) +
+                        wid * (PARTIAL ? ebp_warp_bytes(N, M, ud.q_bwd, ud.q_fwd) : eb_warp_bytes(N, M));
+    float2* sR = reinterpret_cast<float2*>(my);                                           // A': rotated test points
+    // direction 0, rows: A' against the reference points; direction 1, columns: the reference points against A'
+    const float2* pts[2] = {sR, sB};
     const int n_rows[2] = {N, M};
+    unsigned short* hint[2];
+    hint[0] = reinterpret_cast<unsigned short*>(sR + N);
+    hint[1] = hint[0] + N;
+    EbList lst[2];       // PARTIAL: the lists of the two directions
+    unsigned* bits[2];   // PARTIAL: the seeded rows of the two directions
+    if constexpr (PARTIAL) {
+        unsigned* lp = reinterpret_cast<unsigned*>(my + eb_warp_bytes(N, M));
+        lst[0].cap = ud.q_bwd + 1, lst[1].cap = ud.q_fwd + 1;
+        lst[0].val = lp;
+        lst[0].idx = reinterpret_cast<int*>(lp + lst[0].cap);
+        lst[1].val = lp + 2 * lst[0].cap;
+        lst[1].idx = reinterpret_cast<int*>(lst[1].val + lst[1].cap);
+        bits[0] = lp + 2 * (lst[0].cap + lst[1].cap);
+        bits[1] = bits[0] + (N + 31) / 32;
+    }
     if (threadIdx.x == 0) {
         mbar_init(bar, 1);
         *s_key = ~0ull;
-        const uint32_t bytes = (uint32_t)(a_elems + b_elems + nb_elems + t_elems) * 16u;
+        const uint32_t bytes = (uint32_t)sl.total() * 16u;
         mbar_expect_tx(bar, bytes);
         tma_bulk_g2s(sA, lay + ud.lay_off, bytes, bar);
     }
     __syncthreads();
     mbar_wait(bar, 0);
 
+    // test point i of the staging image (K0's layout: register slots, then the exact-tiling tail block)
     auto test_pt = [&](int i) -> float2 {
         if (i >= n_main) return sT[i - n_main];
         const int c = i / (32 * TA), r = i - c * 32 * TA;
         const float4 v = sA[(c * S + (r >> 6)) * 32 + (r & 31)];
         return (r & 32) ? make_float2(v.y, v.w) : make_float2(v.x, v.z);
     };
-    // direction 0: rows = A' against the reference points; direction 1: columns = reference points against A'
-    auto row_pt = [&](int dir, int r) -> float2 { return dir ? sB[r] : sR[r]; };
-    auto set_of = [&](int dir) -> const float2* { return dir ? sR : sB; };
+    // this warp's contiguous run of candidates: neighbouring angles keep the hints valid
     const int per = (w.count + n_warps - 1) / n_warps;
     const int c_begin = w.begin + min(w.count, wid * per), c_end = w.begin + min(w.count, (wid + 1) * per);
     unsigned long long best = ~0ull;
     unsigned pairs = 0;
     if (c_begin < c_end) {
-        bool seed[2] = {true, true};
+        int ra = 0, cb = 0;            // K1e: the row and the column that defined the previous candidate's value
+        bool seed[2] = {true, true};   // PARTIAL: the directions whose lists seed the next candidate
+        if constexpr (PARTIAL) {
 #pragma unroll
-        for (int dir = 0; dir < 2; ++dir) {
-            const int n = n_rows[dir];
-            for (int k = lane; k < (n + 31) / 32; k += 32) bits[dir][k] = 0u;
-            for (int r = lane; r < n; r += 32)
-                hint[dir][r] = (unsigned short)(((long long)r * n_rows[1 - dir]) / n);
-            __syncwarp();
-            // first candidate's seeds: the q + 1 points farthest from the rotation centre (unrotated)
-            EbList& l = lst[dir];
-            for (int k = 0; k < l.cap; ++k) {
-                unsigned far = 0u;
-                int at = 0;
-                for (int r = lane; r < n; r += 32) {
-                    if ((bits[dir][r >> 5] >> (r & 31)) & 1u) continue;
-                    const float2 p = dir ? sB[r] : test_pt(r);
-                    const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y) + 1u;   // > 0: not yet taken
-                    if (r2 > far) far = r2, at = r;
-                }
-                const int r = eb_warp_argmax(far, at);
-                if (lane == 0) {
-                    l.idx[k] = r;
-                    bits[dir][r >> 5] |= 1u << (r & 31);
-                }
+            for (int dir = 0; dir < 2; ++dir) {
+                const int n = n_rows[dir];
+                for (int k = lane; k < (n + 31) / 32; k += 32) bits[dir][k] = 0u;
+                for (int r = lane; r < n; r += 32)
+                    hint[dir][r] = (unsigned short)(((long long)r * n_rows[1 - dir]) / n);
                 __syncwarp();
+                // first candidate's seeds: the q + 1 points farthest from the rotation centre (unrotated)
+                EbList& l = lst[dir];
+                for (int k = 0; k < l.cap; ++k) {
+                    unsigned far = 0u;
+                    int at = 0;
+                    for (int r = lane; r < n; r += 32) {
+                        if ((bits[dir][r >> 5] >> (r & 31)) & 1u) continue;
+                        const float2 p = dir ? sB[r] : test_pt(r);
+                        const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y) + 1u;   // > 0: not yet taken
+                        if (r2 > far) far = r2, at = r;
+                    }
+                    const int r = eb_warp_argmax(far, at);
+                    if (lane == 0) {
+                        l.idx[k] = r;
+                        bits[dir][r >> 5] |= 1u << (r & 31);
+                    }
+                    __syncwarp();
+                }
+                l.cnt = l.cap;
             }
-            l.cnt = l.cap;
+        } else {
+            // first candidate: hints on the index diagonal, seeds at the points farthest from the rotation centre
+            unsigned far_a = 0u, far_b = 0u;
+            int ia = 0, ib = 0;
+            for (int i = lane; i < N; i += 32) {
+                const float2 p = test_pt(i);
+                const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
+                if (r2 > far_a) far_a = r2, ia = i;
+                hint[0][i] = (unsigned short)(((long long)i * M) / N);
+            }
+            for (int j = lane; j < M; j += 32) {
+                const float2 p = sB[j];
+                const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
+                if (r2 > far_b) far_b = r2, ib = j;
+                hint[1][j] = (unsigned short)(((long long)j * N) / M);
+            }
+            ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
         }
         for (int c = c_begin; c < c_end; ++c) {
             float2 tr = make_float2(0.f, 0.f);
@@ -956,90 +872,92 @@ __global__ void __launch_bounds__(kThreads, 2)
                 sR[i] = r;
             }
             __syncwarp();
-            // seeds: the listed rows of the seeded directions, one lane each, scanned to the end
+            unsigned L;
+            if constexpr (PARTIAL) {
+                // seeds: the listed rows of the seeded directions, one lane each, scanned to the end
 #pragma unroll
-            for (int dir = 0; dir < 2; ++dir) {
-                EbList& l = lst[dir];
-                if (!seed[dir]) {
-                    l.cnt = 0;
-                    l.kth = 0u;
-                    continue;
+                for (int dir = 0; dir < 2; ++dir) {
+                    EbList& l = lst[dir];
+                    if (!seed[dir]) {
+                        l.cnt = 0;
+                        l.kth = 0u;
+                        continue;
+                    }
+                    for (int k = lane; k < l.cnt; k += 32) {
+                        const int r = l.idx[k];
+                        int arg;
+                        l.val[k] = eb_lane_min(pts[1 - dir], n_rows[1 - dir], pts[dir][r], arg, pairs);
+                        hint[dir][r] = (unsigned short)arg;
+                        atomicOr(&bits[dir][r >> 5], 1u << (r & 31));
+                    }
+                    ebl_refresh(l, lane);
                 }
-                for (int k = lane; k < l.cnt; k += 32) {
-                    const int r = l.idx[k];
-                    int arg;
-                    l.val[k] = eb_lane_min(set_of(dir), n_rows[1 - dir], row_pt(dir, r), arg, pairs);
-                    hint[dir][r] = (unsigned short)arg;
-                    atomicOr(&bits[dir][r >> 5], 1u << (r & 31));
-                }
-                ebl_refresh(l, lane);
-            }
-            unsigned L = max(lst[0].kth, lst[1].kth);
+                L = max(lst[0].kth, lst[1].kth);
 #pragma unroll
-            for (int dir = 0; dir < 2; ++dir) {
-                const int n = n_rows[dir], n_set = n_rows[1 - dir];
-                const float2* P = set_of(dir);
-                unsigned short* h = hint[dir];
-                EbList& l = lst[dir];
-                for (int g = 0; g < n; g += 32) {
-                    const int i = g + lane;
-                    bool open = i < n && !((bits[dir][i >> 5] >> (i & 31)) & 1u);
-                    if (!early) {
+                for (int dir = 0; dir < 2; ++dir) {
+                    const float2* R = pts[dir];
+                    const float2* P = pts[1 - dir];
+                    const int n = n_rows[dir], n_set = n_rows[1 - dir];
+                    unsigned short* h = hint[dir];
+                    const unsigned* seeded = bits[dir];
+                    for (int g = 0; g < n; g += 32) {
+                        const int i = g + lane;
+                        const bool open = i < n && !((seeded[i >> 5] >> (i & 31)) & 1u);
+                        if (early) {
+                            eb_rows(R, g, open, P, n_set, h, L,
+                                    [&](unsigned mn, int r) {
+                                        ebl_insert(lst[dir], mn, r, lane);
+                                        return max(lst[0].kth, lst[1].kth);
+                                    },
+                                    lane, pairs);
+                            continue;
+                        }
                         // every open row scanned to its end by its lane; the exact minima > L enter the list in lane order
                         unsigned mn = ~0u;
                         if (open) {
                             int arg;
-                            mn = eb_lane_min(P, n_set, row_pt(dir, i), arg, pairs);
+                            mn = eb_lane_min(P, n_set, R[i], arg, pairs);
                             h[i] = (unsigned short)arg;
                         }
                         for (unsigned m = __ballot_sync(0xffffffffu, open); m; m &= m - 1) {
                             const int src = __ffs(m) - 1;
                             const unsigned v = __shfl_sync(0xffffffffu, mn, src);
                             if (v > L) {
-                                ebl_insert(l, v, g + src, lane);
+                                ebl_insert(lst[dir], v, g + src, lane);
                                 L = max(lst[0].kth, lst[1].kth);
                             }
                         }
-                        continue;
-                    }
-                    if (open) {
-                        const float2 a = row_pt(dir, i);
-                        const int h0 = h[i];
-                        for (int t = 0; t < kEbTries && t < n_set; ++t) {
-                            const int j = eb_zig(h0, t, n_set);
-                            ++pairs;
-                            if (__float_as_uint(eb_d2(a, P[j])) <= L) {
-                                h[i] = (unsigned short)j;
-                                open = false;
-                                break;
-                            }
-                        }
-                    }
-                    for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
-                        const int ii = g + __ffs(open_mask) - 1;
-                        int arg;
-                        const unsigned mn = eb_warp_min(P, n_set, row_pt(dir, ii), h[ii], L, true, lane, arg, pairs);
-                        __syncwarp();
-                        if (lane == 0) h[ii] = (unsigned short)arg;
-                        if (mn > L) {
-                            ebl_insert(l, mn, ii, lane);
-                            L = max(lst[0].kth, lst[1].kth);
-                        }
                     }
                 }
+            } else {
+                // seeds: the exact minima of the row and the column that defined the previous candidate's value
+                int arg;
+                L = eb_warp_min(sB, M, sR[ra], hint[0][ra], 0u, false, lane, arg, pairs);
+                const int h_ra = arg;
+                const unsigned lc = eb_warp_min(sR, N, sB[cb], hint[1][cb], 0u, false, lane, arg, pairs);
+                __syncwarp();
+                if (lane == 0) hint[0][ra] = (unsigned short)h_ra, hint[1][cb] = (unsigned short)arg;
+                L = max(L, lc);
+                __syncwarp();
+                for (int g = 0; g < N; g += 32)   // rows: test point i against the reference points
+                    eb_rows(sR, g, g + lane < N, sB, M, hint[0], L, [&](unsigned mn, int i) { ra = i; return mn; }, lane, pairs);
+                for (int g = 0; g < M; g += 32)   // columns: reference point j against A'
+                    eb_rows(sB, g, g + lane < M, sR, N, hint[1], L, [&](unsigned mn, int j) { cb = j; return mn; }, lane, pairs);
             }
             const float d = sqrtf(__uint_as_float(L));
             if (lane == 0) {
                 dist32[ud.dist_off + c] = d;
                 best = min(best, ((unsigned long long)__float_as_uint(d) << 32) | (unsigned)c);
             }
-            // the next candidate seeds the direction that defined this value (ties: rows) from this list
-            seed[0] = lst[0].kth >= lst[1].kth;
-            seed[1] = !seed[0];
-            __syncwarp();
+            if constexpr (PARTIAL) {
+                // the next candidate seeds the direction that defined this value (ties: rows) from this list
+                seed[0] = lst[0].kth >= lst[1].kth;
+                seed[1] = !seed[0];
+                __syncwarp();
 #pragma unroll
-            for (int dir = 0; dir < 2; ++dir)
-                for (int k = lane; k < (n_rows[dir] + 31) / 32; k += 32) bits[dir][k] = 0u;
+                for (int dir = 0; dir < 2; ++dir)
+                    for (int k = lane; k < (n_rows[dir] + 31) / 32; k += 32) bits[dir][k] = 0u;
+            }
         }
     }
     const unsigned warp_pairs = __reduce_add_sync(0xffffffffu, pairs);
