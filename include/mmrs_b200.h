@@ -302,6 +302,39 @@ int mmrs_eval_exact_partial(mmrs_ctx* ctx, const double* test_xy, int64_t n_test
                             double cx, double cy, int32_t mode, const double* angles, const double* txy /* NULL: none */,
                             int64_t n_cand, double inlier_fraction, double* dist_out);
 
+/* ---- mean cost: modified Hausdorff distance, every point's closest-point distance averaged (opt-in) ------------
+ * Both costs above are decided by one or a few extreme points. The modified Hausdorff distance (Dubuisson and Jain,
+ * ICPR 1994) averages each point's closest-point distance in each direction and takes the larger direction, so every
+ * point counts and there is no parameter. Like the rigid and partial costs, this is this library's own extension,
+ * restated by the tests.
+ *
+ * For a candidate: A, the n finite transformed test points; B, the m finite reference points (non-finite points are
+ *   dropped, as everywhere).
+ * Row value of a point p against a set Q: v(p) = sqrt(min_{x in Q} (dx*dx + dy*dy)), reference arithmetic (unfused,
+ *   IEEE sqrt); a non-finite minimum counts as 0.
+ * fwd = (v(b_0) + v(b_1) + ... + v(b_{m-1})) / m: a sequential left-to-right f64 sum in point order, then one
+ *   division. bwd: the same over A against B, divided by n. Cost (f64): fmax(fwd, bwd). The summation order is part of
+ *   the definition.
+ * The transform (mode 0 / 1 rotation, plus the optional translation grid) and the selection (leftmost arg-min, tie
+ *   margin, R_eff for rigid runs) are those of the rotation-only and rigid sweeps. An empty set costs 0
+ *   (MMRS_FLAG_EMPTY).
+ * Limits (MMRS_ERR_ARG, checked before any device work): no unit beyond the shared-memory staging (more than ~4 000
+ *   points per set); opts.prune > 0 or opts.prefilter 2 / 3. The context's prune default and any partition across
+ *   ranks are not used, as for rigid runs; MMRS_EARLY_BREAK does not apply (every pair is evaluated).
+ * FP32 -> f64: the sweep's FP32 value of a candidate is within 5e-7 R + 3.6e-7 d of its f64 cost (R: Rmax, or R_eff
+ *   for rigid runs), inside the FP32 window of the full cost, which is used unchanged.                             */
+
+/* mmrs_sweep_upload (tgrids == NULL) or mmrs_rigid_sweep_upload with the mean cost. The cost stays with the uploaded
+ * points: mmrs_sweep_regrid / mmrs_rigid_sweep_regrid, mmrs_sweep_run and the download calls work on it unchanged; a
+ * later plain or partial upload clears it.                                                                        */
+int mmrs_mean_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* batch, const mmrs_tgrid* tgrids /* NULL: rotation only */,
+                           int64_t n_tgrids, const int32_t* tgrid_of_unit, const mmrs_sweep_opts* opts);
+/* f64 mean cost of explicit candidates k = (angles[k], txy[2k], txy[2k+1]) for one unit (txy == NULL: no
+ * translation), on the finite points of each set.                                                              */
+int mmrs_eval_exact_mean(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
+                         double cx, double cy, int32_t mode, const double* angles, const double* txy /* NULL: none */,
+                         int64_t n_cand, double* dist_out);
+
 /* ---- geometry blob -------------------------------------------------------------
  * Geometries cross the boundary as one f64 stream (u32 ids are exact in f64):
  *   n_frames,

@@ -36,6 +36,10 @@ constexpr int kFlagRemote = 0x400;  // internal UnitDesc.flags bit: another rank
 // re-scores a list with the exact FP32 sweep. The values are the codes mmrs_sweep_prefilter_info reports in out[0].
 enum Tier : int { kTierDense = 0, kTierTc = 1, kTierPrune = 2, kTierXf = 3 };
 
+// What a candidate's cost is (include/mmrs_b200.h): the symmetric Hausdorff distance, the partial (rank-K) distance or
+// the mean (modified Hausdorff) distance. Partial and mean runs are solo: the dense sweep on one device, no tier.
+enum Cost : int { kCostFull = 0, kCostPartial = 1, kCostMean = 2 };
+
 struct WorkItem {
     int unit;
     int begin;  // first candidate
@@ -153,9 +157,9 @@ struct mmrs_ctx {
     std::vector<double> h_tmax;             // per unit: largest |t| of its translation grid
     mmrs::DevBuf d_t64, d_t32, d_tmax, d_reff;   // translation tables; per unit R_eff = Rmax + max |t| (float bits)
 
-    // partial (rank-K) cost (mmrs_partial_sweep_upload): set with the points, kept across regrids
-    bool partial = false;
-    double inlier_fraction = 1.0;
+    // the cost (mmrs_partial_sweep_upload, mmrs_mean_sweep_upload): set with the points, kept across regrids
+    mmrs::Cost cost = mmrs::kCostFull;
+    double inlier_fraction = 1.0;   // partial cost
 
     // partition of every batched sweep across ranks (mmrs_ctx_comm_init / mmrs_ctx_set_shard / mmrs_ctx_set_partition)
     int shard_rank = 0, shard_world = 1;

@@ -266,24 +266,43 @@ static cudaError_t raise_smem_once(K kernel, std::once_flag& once, cudaError_t& 
         return raise_smem_once(kernel, once, result);            \
     }())
 
-template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false>
+template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false, bool MEAN = false>
 static void launch_sweep_k(int grid, size_t smem, cudaStream_t s, const UnitDesc* units, const WorkItem* work,
                            const float4* lay, const float2* cs32, float* dist32, unsigned long long* key,
                            const ListArgs& l, const float2* t32 = nullptr) {
-    RAISE_SMEM((k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID>));
-    k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID><<<grid, kThreads, smem, s>>>(units, work, lay, cs32, dist32, key, l.items,
-                                                                            l.n_items, l.cap, l.chunk, l.rmax, l.diag, t32);
+    RAISE_SMEM((k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID, MEAN>));
+    k_sweep<TA, MULTI, LIST, TAILP, XF, RIGID, MEAN><<<grid, kThreads, smem, s>>>(
+        units, work, lay, cs32, dist32, key, l.items, l.n_items, l.cap, l.chunk, l.rmax, l.diag, t32);
 }
 // xf: the expanded-form tier K1x (dense launches only; a list is always re-scored in direct form)
 // t32 != NULL: rigid candidates (dense direct-form launches only)
+// mean: the mean cost (dense direct-form launches only, rotation only or rigid)
 template <int TA>
 static void launch_sweep_ta(bool multi, bool tailp, bool xf, int grid, size_t smem, cudaStream_t s, const UnitDesc* units,
                             const WorkItem* work, const float4* lay, const float2* cs32, float* dist32,
-                            unsigned long long* key, const ListArgs* l, const float2* t32) {
+                            unsigned long long* key, const ListArgs* l, const float2* t32, bool mean) {
     const ListArgs none{};
     const ListArgs& la = l ? *l : none;
 #define GO(M, L, T, X) launch_sweep_k<TA, M, L, T, X>(grid, smem, s, units, work, lay, cs32, dist32, key, la)
 #define GO_RIGID(M, T) launch_sweep_k<TA, M, false, T, false, true>(grid, smem, s, units, work, lay, cs32, dist32, key, la, t32)
+#define GO_MEAN(M, T, R) launch_sweep_k<TA, M, false, T, false, R, true>(grid, smem, s, units, work, lay, cs32, dist32, key, la, t32)
+    if (mean) {
+        if constexpr (TA % 2 == 0 && TA >= 4) {
+            if (tailp) {
+                if (t32) GO_MEAN(false, true, true);
+                else GO_MEAN(false, true, false);
+                return;
+            }
+        }
+        if (multi) {
+            if (t32) GO_MEAN(true, false, true);
+            else GO_MEAN(true, false, false);
+        } else {
+            if (t32) GO_MEAN(false, false, true);
+            else GO_MEAN(false, false, false);
+        }
+        return;
+    }
     if (t32) {
         if constexpr (TA % 2 == 0 && TA >= 4) {
             if (tailp) {
@@ -315,14 +334,16 @@ static void launch_sweep_ta(bool multi, bool tailp, bool xf, int grid, size_t sm
     }
 #undef GO
 #undef GO_RIGID
+#undef GO_MEAN
 }
 static bool launch_sweep(int TA, bool multi, bool tailp, int grid, size_t smem, cudaStream_t s, const UnitDesc* units,
                          const WorkItem* work, const float4* lay, const float2* cs32, float* dist32,
-                         unsigned long long* key, const ListArgs* l = nullptr, bool xf = false, const float2* t32 = nullptr) {
+                         unsigned long long* key, const ListArgs* l = nullptr, bool xf = false, const float2* t32 = nullptr,
+                         bool mean = false) {
     switch (TA) {
-#define CASE(T)                                                                                        \
-    case T:                                                                                            \
-        launch_sweep_ta<T>(multi, tailp, xf, grid, smem, s, units, work, lay, cs32, dist32, key, l, t32); \
+#define CASE(T)                                                                                              \
+    case T:                                                                                                  \
+        launch_sweep_ta<T>(multi, tailp, xf, grid, smem, s, units, work, lay, cs32, dist32, key, l, t32, mean); \
         return true;
         CASE(2) CASE(3) CASE(4) CASE(5) CASE(6) CASE(7) CASE(8) CASE(9) CASE(10) CASE(11) CASE(12) CASE(13) CASE(14)
             CASE(15) CASE(16) CASE(17) CASE(18)
@@ -364,6 +385,8 @@ static int partial_q(double f, int n) {
     if (n <= 0) return 0;
     return n - (int)std::max(1.0, std::ceil(f * (double)n));
 }
+
+static const char* cost_name(Cost c) { return c == kCostMean ? "mean cost" : c == kCostPartial ? "partial cost" : "cost"; }
 
 // ---- upload ----------------------------------------------------------------------------
 // Points part of an upload: validates the offsets, chooses the register tile, lays every unit out in the
@@ -435,7 +458,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
         d.cx = b->centre_xy[2 * u];
         d.cy = b->centre_xy[2 * u + 1];
         d.lay_off = lay_off;
-        if (ctx->partial) {
+        if (ctx->cost == kCostPartial) {
             const int q_f = partial_q(ctx->inlier_fraction, d.m), q_b = partial_q(ctx->inlier_fraction, d.n);
             if (q_f > kPartialMaxQ || q_b > kPartialMaxQ)
                 return set_err(ctx, MMRS_ERR_ARG, "partial cost: unit " + std::to_string(u) + " leaves out " +
@@ -452,10 +475,10 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             d.m_pairs = (d.m + 1) / 2;
             const StageLayout sl = stage_layout(cc.ta, d.n_chunks, d.n_tail, d.m_pairs);
             const size_t stage = 16 + (size_t)sl.total() * 16;   // mbarrier + key, then the staging image
-            // shared memory of a K1 CTA of this unit: the staging, then per warp either the chunked column minima (MULTI)
-            // or the tail pass's column seeds (exact tiling)
+            // shared memory of a K1 CTA of this unit: the staging, then per warp either the chunked column minima (MULTI;
+            // the mean cost: every class but exact tiling) or the tail pass's column seeds (exact tiling)
             size_t smem = stage;
-            if (d.n_chunks > 1) smem += (size_t)kWarpsPerCta * ((2 * d.m_pairs + 3) & ~3) * 4;
+            if (d.n_chunks > 1 || (ctx->cost == kCostMean && !cc.tailp)) smem += (size_t)kWarpsPerCta * ((2 * d.m_pairs + 3) & ~3) * 4;
             if (cc.tailp) smem += (size_t)kWarpsPerCta * 32 * (cc.ta + 1) * 4;
             static const bool force_big = std::getenv("MMRS_FORCE_BIG") && std::getenv("MMRS_FORCE_BIG")[0] == '1';
             const bool big = smem > (size_t)kMaxDynSmem || (force_big && d.n >= 64);
@@ -485,10 +508,10 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             cl.smem = std::max(cl.smem, smem);
             cl.cost += (long long)d.n_chunks * 32 * d.ta * d.m;
             ctx->class_of_unit[u] = k;
-            if (ctx->partial && big)
-                return set_err(ctx, MMRS_ERR_ARG, "partial cost: unit " + std::to_string(u) +
+            if (ctx->cost != kCostFull && big)
+                return set_err(ctx, MMRS_ERR_ARG, std::string(cost_name(ctx->cost)) + ": unit " + std::to_string(u) +
                                                       " is beyond the shared-memory staging (more than ~4 000 points per set)");
-            if (ctx->partial) {
+            if (ctx->cost == kCostPartial) {
                 ebp_stage[k] = std::max(ebp_stage[k], stage);
                 ebp_warp[k] = std::max(ebp_warp[k], (size_t)ebp_warp_bytes(d.n, d.m, d.q_bwd, d.q_fwd));
             } else if (!big) {   // K1e: the same staging image plus, per warp, A' and the row / column hints
@@ -496,7 +519,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             }
         }
     }
-    if (ctx->partial) {
+    if (ctx->cost == kCostPartial) {
         // K1e-partial: 8 warps per CTA where the largest staging image and 8 of the largest per-warp blocks fit the
         // 227 KB a CTA may have, else 4, 2 or 1 (the chunked 2 020-point units take 4)
         for (size_t k = 0; k < ctx->classes.size(); ++k) {
@@ -537,7 +560,7 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
         ctx->lb_R = biggest >= 1024 ? 128 : 32;  // rows per lower-bound pass: k_lb<1,8> or k_lb<4,2>
         // the bound tier's staging images are only built for a batch that may use it (opts / context default / MMRS_PRUNE)
         const char* prune_env = std::getenv("MMRS_PRUNE");
-        const bool may_prune = !ctx->rigid && !ctx->partial && ((prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1);
+        const bool may_prune = !ctx->rigid && ctx->cost == kCostFull && ((prune_env && *prune_env) ? (*prune_env != '0') : ctx->opt_prune == 1);
         ctx->lb_shape_ok = ok && biggest > 0 && may_prune;
         ctx->h_units_lb.assign(2 * (size_t)U, UnitDesc{});
         long long off = 0;
@@ -622,7 +645,7 @@ static inline void tgrid_offset(const mmrs_tgrid& t, int64_t j, double* tx, doub
 }
 
 // The tier of the uploaded grids, in order of precedence: the tensor-core prefilter K1t, the expanded form K1x, then
-// lower-bound pruning K1p. solo (rigid or partial candidates) and the candidate-axis partition take the dense sweep.
+// lower-bound pruning K1p. solo (rigid candidates, the partial or the mean cost) and the candidate-axis partition take the dense sweep.
 // Sizes the tier's candidate list and builds its work list.
 static int plan_tier(mmrs_ctx* ctx, bool solo, long long live) {
     const int64_t U = ctx->n_units;
@@ -727,7 +750,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         ctx->grid_of_unit[u] = g;
     }
     ctx->rigid = tgrids != nullptr;
-    const bool solo = ctx->rigid || ctx->partial;   // the dense sweep on this device alone: no tier, no partition
+    const bool solo = ctx->rigid || ctx->cost != kCostFull;   // the dense sweep on this device alone: no tier, no partition
     std::vector<long long> tgrid_off(1, 0);
     if (ctx->rigid) {
         if (n_tgrids < 1) return set_err(ctx, MMRS_ERR_ARG, "rigid sweep: n_tgrids must be >= 1");
@@ -880,9 +903,10 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
         }
     // K1e per size class (MMRS_EARLY_BREAK: 0 = K1 everywhere, 1 = K1e wherever its shared memory fits). A class beyond
     // the per-warp A' and hints (sets above ~1 000 points, the chunked 2 020-point units among them) keeps K1.
-    // A partial run takes K1e-partial in every class (MMRS_EARLY_BREAK=0 only switches its early break off).
+    // A partial run takes K1e-partial in every class (MMRS_EARLY_BREAK=0 only switches its early break off), a mean run
+    // the mean K1 in every class.
     for (auto& cl : ctx->classes)
-        cl.eb = !ctx->partial && ctx->eb_env != 0 && !cl.big && cl.smem_eb <= (ctx->eb_env == 1 ? (size_t)kMaxDynSmem : kEbAutoSmem);
+        cl.eb = ctx->cost == kCostFull && ctx->eb_env != 0 && !cl.big && cl.smem_eb <= (ctx->eb_env == 1 ? (size_t)kMaxDynSmem : kEbAutoSmem);
     // work list: one CTA = one unit x one tile of candidates (8 warps, one candidate per warp per pass; K1e: one
     // contiguous run per warp, as long as the batch still gives ~4 waves of 3 CTAs per SM)
     {
@@ -899,7 +923,7 @@ static int apply_grids(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, c
             cl.work_begin = ctx->h_work.size();
             const long long eb_slots = (long long)ctx->n_sm * 3 * 4 * kWarpsPerCta;
             const long long run = std::max(kEbMinRun, std::min(kEbMaxRun, (cl.live + eb_slots - 1) / eb_slots));
-            const int tile_k = ctx->partial || cl.eb ? (int)(cl.eb_warps * run) : tile;
+            const int tile_k = ctx->cost == kCostPartial || cl.eb ? (int)(cl.eb_warps * run) : tile;
             for (int64_t u = 0; u < U; ++u) {
                 const UnitDesc& d = units[u];
                 if (d.flags || ctx->class_of_unit[u] != (int)k) continue;
@@ -972,9 +996,10 @@ static int check_tgrids(mmrs_ctx* ctx, const char* fn, int64_t n_units, const mm
     return MMRS_OK;
 }
 
-// Upload of a rotation-only batch (tgrids == NULL) or of a rigid one; inlier_fraction < 1: the partial cost.
+// Upload of a rotation-only batch (tgrids == NULL) or of a rigid one, with its cost (the partial cost: inlier_fraction).
 static int upload_impl(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_sweep_opts* o, const mmrs_tgrid* tgrids,
-                       int64_t n_tgrids, const int32_t* tgrid_of_unit, const char* fn, double inlier_fraction = 1.0) {
+                       int64_t n_tgrids, const int32_t* tgrid_of_unit, const char* fn, Cost cost = kCostFull,
+                       double inlier_fraction = 1.0) {
     if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (!b || b->n_units < 0 || (b->n_units > 0 && (!b->test_off || !b->ref_off || !b->centre_xy || !b->grids)) ||
         (b->n_grids < 1 && b->n_units > 0))
@@ -986,17 +1011,17 @@ static int upload_impl(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_swee
         if (o && (o->prefilter == 2 || o->prefilter == 3))
             return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3 is not supported with a translation grid");
     }
-    const bool partial = inlier_fraction < 1.0;
-    if (partial) {
-        if (o && o->prune > 0) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prune is not supported with the partial cost");
+    if (cost != kCostFull) {
+        const std::string with = std::string(" is not supported with the ") + cost_name(cost);
+        if (o && o->prune > 0) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prune" + with);
         if (o && (o->prefilter == 2 || o->prefilter == 3))
-            return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3 is not supported with the partial cost");
+            return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": prefilter 2 / 3" + with);
     }
     ENTER_DEVICE(ctx);
     ctx->ready = false;
     ctx->ran = false;
     ctx->rigid = tgrids != nullptr;
-    ctx->partial = partial;
+    ctx->cost = cost;
     ctx->inlier_fraction = inlier_fraction;
     ctx->n_units = b->n_units;
     ctx->mode = b->mode;
@@ -1062,7 +1087,14 @@ extern "C" int mmrs_partial_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* 
                        inlier_fraction < 1.0 ? "mmrs_partial_sweep_upload"
                        : tgrids              ? "mmrs_rigid_sweep_upload"
                                              : "mmrs_sweep_upload",
-                       inlier_fraction);
+                       inlier_fraction < 1.0 ? kCostPartial : kCostFull, inlier_fraction);
+}
+
+extern "C" int mmrs_mean_sweep_upload(mmrs_ctx* ctx, const mmrs_sweep_batch* b, const mmrs_tgrid* tgrids,
+                                      int64_t n_tgrids, const int32_t* tgrid_of_unit, const mmrs_sweep_opts* o) {
+    if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, "mmrs_mean_sweep_upload: ctx is NULL");
+    if (!tgrids && (n_tgrids || tgrid_of_unit)) return set_err(ctx, MMRS_ERR_ARG, "mmrs_mean_sweep_upload: bad translation grids");
+    return upload_impl(ctx, b, o, tgrids, n_tgrids, tgrid_of_unit, "mmrs_mean_sweep_upload", kCostMean);
 }
 
 static int regrid_impl(mmrs_ctx* ctx, const mmrs_grid* grids, int64_t n_grids, const int32_t* grid_of_unit,
@@ -1105,21 +1137,40 @@ extern "C" int mmrs_rigid_sweep_regrid(mmrs_ctx* ctx, const mmrs_grid* grids, in
 struct ExactPlan {
     int smem, grid;
     double2* scratch;
-    double* mins = nullptr;   // partial cost: the CTAs' row minima in global memory (with scratch)
+    double* mins = nullptr;   // partial and mean costs: the CTAs' row minima in global memory (with scratch)
 };
-// The partial cost also keeps the row minima of one direction (max_pts doubles per CTA).
-static int exact_plan(mmrs_ctx* ctx, bool partial, int max_pts, int want_grid, ExactPlan* p) {
-    const long long smem = 64 + 2LL * max_pts * 16 + (partial ? (long long)max_pts * 8 : 0);
+// The partial and mean costs also keep the row minima of one direction (max_pts doubles per CTA).
+static int exact_plan(mmrs_ctx* ctx, Cost cost, int max_pts, int want_grid, ExactPlan* p) {
+    const bool mins = cost != kCostFull;
+    const long long smem = 64 + 2LL * max_pts * 16 + (mins ? (long long)max_pts * 8 : 0);
     if (smem <= kMaxDynSmem) {
         *p = ExactPlan{(int)smem, want_grid, nullptr};
         return MMRS_OK;
     }
     const int grid = std::max(1, std::min(want_grid, ctx->n_sm * 2));
     const size_t rot = (size_t)grid * max_pts * 16;
-    ENSURE(ctx->d_exact_scratch, partial ? (size_t)grid * max_pts * 24 : rot);
+    ENSURE(ctx->d_exact_scratch, mins ? (size_t)grid * max_pts * 24 : rot);
     char* base = (char*)ctx->d_exact_scratch.p;
-    *p = ExactPlan{64, grid, (double2*)base, partial ? (double*)(base + rot) : nullptr};
+    *p = ExactPlan{64, grid, (double2*)base, mins ? (double*)(base + rot) : nullptr};
     return MMRS_OK;
+}
+
+// K3 of a cost (k_exact<COST>, and k_exact_dense<COST> for a whole unit), its shared-memory limit raised once.
+using ExactKernel = decltype(&k_exact<kCostFull>);
+using ExactDenseKernel = decltype(&k_exact_dense<kCostFull>);
+static cudaError_t exact_kernel(Cost c, ExactKernel* k) {
+    switch (c) {
+        case kCostPartial: *k = k_exact<kCostPartial>; return RAISE_SMEM(k_exact<kCostPartial>);
+        case kCostMean: *k = k_exact<kCostMean>; return RAISE_SMEM(k_exact<kCostMean>);
+        default: *k = k_exact<kCostFull>; return RAISE_SMEM(k_exact<kCostFull>);
+    }
+}
+static cudaError_t exact_kernel(Cost c, ExactDenseKernel* k) {
+    switch (c) {
+        case kCostPartial: *k = k_exact_dense<kCostPartial>; return RAISE_SMEM(k_exact_dense<kCostPartial>);
+        case kCostMean: *k = k_exact_dense<kCostMean>; return RAISE_SMEM(k_exact_dense<kCostMean>);
+        default: *k = k_exact_dense<kCostFull>; return RAISE_SMEM(k_exact_dense<kCostFull>);
+    }
 }
 
 // f64 recheck of every candidate of `unit` (shortlist overflow): leftmost arg-min on the host
@@ -1128,9 +1179,9 @@ static int full_f64_unit(mmrs_ctx* ctx, int64_t u, UnitResultDev& r) {
     const UnitDesc& d = ctx->h_units[u];
     ENSURE(ctx->d_tmp, (size_t)d.n_cand * 8);
     ExactPlan ep;
-    if (int rc = exact_plan(ctx, ctx->partial, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
-    CUDA_TRY(ctx, ctx->partial ? RAISE_SMEM(k_exact_dense<true>) : RAISE_SMEM(k_exact_dense<false>));
-    auto k3 = ctx->partial ? k_exact_dense<true> : k_exact_dense<false>;
+    if (int rc = exact_plan(ctx, ctx->cost, ctx->max_pts, std::min(d.n_cand, ctx->n_sm * 8), &ep)) return rc;
+    ExactDenseKernel k3;
+    CUDA_TRY(ctx, exact_kernel(ctx->cost, &k3));
     k3<<<ep.grid, 256, ep.smem, ctx->stream>>>((const UnitDesc*)ctx->d_units.p, (int)u, (const double*)ctx->d_test.p,
                                                (const double*)ctx->d_ref.p, (const double2*)ctx->d_cs64.p,
                                                (const unsigned char*)ctx->d_zero.p, d.cand_off, d.n_cand,
@@ -1307,7 +1358,8 @@ static int run_xf(mmrs_ctx* ctx) {
 }
 
 // The dense sweep of one size class: K1b (k_sweep_big) for units beyond K1's shared-memory staging, else K1e-partial
-// for the partial cost, K1e where the class takes it, or K1. t32 != NULL: rigid candidates.
+// for the partial cost, K1e where the class takes it, or K1 (its mean form for the mean cost). t32 != NULL: rigid
+// candidates.
 static int sweep_class(mmrs_ctx* ctx, const mmrs_ctx::SweepClass& cl, const float2* t32) {
     cudaStream_t s = ctx->stream;
     const UnitDesc* units = (const UnitDesc*)ctx->d_units.p;
@@ -1322,7 +1374,7 @@ static int sweep_class(mmrs_ctx* ctx, const mmrs_ctx::SweepClass& cl, const floa
         auto big = t32 ? k_sweep_big<true> : k_sweep_big<false>;
         big<<<grid, kThreads, 0, s>>>(units, work, (int)cl.work_count, lay, cs32, dist32, key, (float*)ctx->d_big_rows.p,
                                       ctx->big_scratch_per_warp, t32);
-    } else if (ctx->partial || cl.eb) {
+    } else if (ctx->cost == kCostPartial || cl.eb) {
         if (!ctx->eb_ran) {   // one counter of the pair distances the early-break kernels evaluate in this run
             ENSURE(ctx->d_eb_pairs, 8);
             CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_eb_pairs.p, 0, 8, s));
@@ -1330,15 +1382,16 @@ static int sweep_class(mmrs_ctx* ctx, const mmrs_ctx::SweepClass& cl, const floa
         }
         unsigned long long* pairs = (unsigned long long*)ctx->d_eb_pairs.p;
         // K1e-partial for the partial cost (every class: big units are refused at upload), else K1e
-        if (ctx->partial) CUDA_TRY(ctx, t32 ? RAISE_SMEM((k_sweep_eb<true, true>)) : RAISE_SMEM((k_sweep_eb<false, true>)));
+        const bool partial = ctx->cost == kCostPartial;
+        if (partial) CUDA_TRY(ctx, t32 ? RAISE_SMEM((k_sweep_eb<true, true>)) : RAISE_SMEM((k_sweep_eb<false, true>)));
         else CUDA_TRY(ctx, t32 ? RAISE_SMEM((k_sweep_eb<true, false>)) : RAISE_SMEM((k_sweep_eb<false, false>)));
-        auto eb = ctx->partial ? (t32 ? k_sweep_eb<true, true> : k_sweep_eb<false, true>)
+        auto eb = partial ? (t32 ? k_sweep_eb<true, true> : k_sweep_eb<false, true>)
                                : (t32 ? k_sweep_eb<true, false> : k_sweep_eb<false, false>);
         eb<<<(unsigned)cl.work_count, cl.eb_warps * 32, cl.smem_eb, s>>>(units, work, lay, cs32, dist32, key, pairs, t32,
                                                                           ctx->eb_env != 0 ? 1 : 0);
         ctx->eb_cands += cl.live;
     } else if (!launch_sweep(cl.ta, cl.multi, cl.tailp, (int)cl.work_count, cl.smem, s, units, work, lay, cs32, dist32,
-                             key, nullptr, false, t32)) {
+                             key, nullptr, false, t32, ctx->cost == kCostMean)) {
         return set_err(ctx, MMRS_ERR_ARG, "no sweep kernel for this register tile");
     }
     CUDA_TRY(ctx, cudaGetLastError());
@@ -1402,9 +1455,9 @@ extern "C" int mmrs_sweep_run(mmrs_ctx* ctx) {
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev[2], s));
     {
         ExactPlan ep;
-        if (int rc = exact_plan(ctx, ctx->partial, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
-        CUDA_TRY(ctx, ctx->partial ? RAISE_SMEM(k_exact<true>) : RAISE_SMEM(k_exact<false>));
-        auto k3 = ctx->partial ? k_exact<true> : k_exact<false>;
+        if (int rc = exact_plan(ctx, ctx->cost, ctx->max_pts, ctx->n_sm * 8, &ep)) return rc;
+        ExactKernel k3;
+        CUDA_TRY(ctx, exact_kernel(ctx->cost, &k3));
         k3<<<ep.grid, 256, ep.smem, s>>>(units, (const double*)ctx->d_test.p, (const double*)ctx->d_ref.p,
                                          (const double2*)ctx->d_cs64.p, (const unsigned char*)ctx->d_zero.p,
                                          (const int2*)ctx->d_items.p, (const unsigned*)ctx->d_nitems.p, ctx->pool_cap,
@@ -1647,16 +1700,15 @@ extern "C" int mmrs_last_timings(mmrs_ctx* ctx, float ms_out[4], int32_t* launch
 
 // ---- explicit-angle exact evaluation ----------------------------------------------------
 // txy == NULL: rotation only; otherwise candidate k is (angles[k], txy[2k], txy[2k+1]).
-// inlier_fraction < 1: the partial cost, on the finite points of each set (as the sweep uploads them).
+// The partial (inlier_fraction) and mean costs: on the finite points of each set (as the sweep uploads them).
 static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy, int64_t n_ref,
                            double cx, double cy, int32_t mode, const double* angles, const double* txy, int64_t n_angles,
-                           double* dist_out, const char* fn, double inlier_fraction = 1.0) {
+                           double* dist_out, const char* fn, Cost cost = kCostFull, double inlier_fraction = 1.0) {
     if (!ctx) return set_err(nullptr, MMRS_ERR_ARG, std::string(fn) + ": ctx is NULL");
     if (n_test < 0 || n_ref < 0 || n_angles < 0 || (n_angles > 0 && (!angles || !dist_out)))
         return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad arguments");
-    const bool partial = inlier_fraction < 1.0;
     std::vector<double> f_test, f_ref;
-    if (partial) {
+    if (cost != kCostFull) {
         if ((n_test > 0 && !test_xy) || (n_ref > 0 && !ref_xy)) return set_err(ctx, MMRS_ERR_ARG, std::string(fn) + ": bad arguments");
         auto finite = [](const double* xy, int64_t n, std::vector<double>& out) {
             for (int64_t i = 0; i < n; ++i)
@@ -1708,9 +1760,9 @@ static int eval_exact_impl(mmrs_ctx* ctx, const double* test_xy, int64_t n_test,
     const int max_n = (int)std::max(n_test, n_ref);
     ExactPlan ep;
     const int want_grid = (int)std::min<int64_t>(n_angles, (int64_t)ctx->n_sm * 8);
-    if (int rc = exact_plan(ctx, partial, max_n, want_grid, &ep)) return rc;
-    CUDA_TRY(ctx, partial ? RAISE_SMEM(k_exact_dense<true>) : RAISE_SMEM(k_exact_dense<false>));
-    auto k3 = partial ? k_exact_dense<true> : k_exact_dense<false>;
+    if (int rc = exact_plan(ctx, cost, max_n, want_grid, &ep)) return rc;
+    ExactDenseKernel k3;
+    CUDA_TRY(ctx, exact_kernel(cost, &k3));
     k3<<<ep.grid, 256, ep.smem, s>>>((const UnitDesc*)(base + o_unit), 0, (const double*)base,
                                      (const double*)(base + (size_t)n_test * 16), (const double2*)(base + o_cs),
                                      (const unsigned char*)(base + o_zero), 0, (int)n_angles, (double*)(base + o_out),
@@ -1743,7 +1795,14 @@ extern "C" int mmrs_eval_exact_partial(mmrs_ctx* ctx, const double* test_xy, int
     if (!std::isfinite(inlier_fraction) || !(inlier_fraction > 0.0) || inlier_fraction > 1.0)
         return set_err(ctx, MMRS_ERR_ARG, "mmrs_eval_exact_partial: inlier_fraction must be finite with 0 < f <= 1");
     return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, txy, n_cand, dist_out,
-                           "mmrs_eval_exact_partial", inlier_fraction);
+                           "mmrs_eval_exact_partial", inlier_fraction < 1.0 ? kCostPartial : kCostFull, inlier_fraction);
+}
+
+extern "C" int mmrs_eval_exact_mean(mmrs_ctx* ctx, const double* test_xy, int64_t n_test, const double* ref_xy,
+                                    int64_t n_ref, double cx, double cy, int32_t mode, const double* angles,
+                                    const double* txy, int64_t n_cand, double* dist_out) {
+    return eval_exact_impl(ctx, test_xy, n_test, ref_xy, n_ref, cx, cy, mode, angles, txy, n_cand, dist_out,
+                           "mmrs_eval_exact_mean", kCostMean);
 }
 
 // ---- FP32 peak probe ------------------------------------------------------------------------

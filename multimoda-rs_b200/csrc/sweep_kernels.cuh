@@ -10,7 +10,7 @@
 //                     f32x2 arithmetic (FADD2/FMUL2/FFMA2), 3-input FMNMX and
 //                     warp REDUX; fused per-unit arg-min on a packed
 //                     (distance, index) 64-bit key with atomicMin. Also re-scores
-//                     candidate lists (LIST) and runs the expanded-form tier K1x (XF).
+//                     candidate lists (LIST), runs the expanded-form tier K1x (XF) and scores the mean cost (MEAN).
 //   K1e k_sweep_eb<RIGID, false>
 //                     the dense sweep with early-break directed passes: every candidate's FP32 distance,
 //                     bit-identical to K1, from ~1 % of the pair distances (default wherever it fits)
@@ -20,7 +20,7 @@
 //   K1p k_prep_lb, k_lb, k_lb_argmin
 //                     exact lower-bound pruning tier: candidates bounded above the best are never scored
 //   K2  k_shortlist   candidates within the FP32 error window of the minimum
-//   K3  k_exact       the reference's f64 arithmetic, literally, on those
+//   K3  k_exact<COST> the reference's f64 arithmetic, literally, on those (full, partial or mean cost)
 //   K4  k_select      leftmost f64 arg-min + tie count per unit
 //
 // Replaces (reference paths): search_range + hausdorff_distance +
@@ -233,7 +233,15 @@ __global__ void k_cs32(const double2* __restrict__ cs64, float2* __restrict__ cs
 // RIGID = true: rigid candidates (dense launches, direct form). Candidate c = i n_trans + j is angle i of the unit's
 //               grid and translation j of its translation grid (t32, FP32); every rotated test point gets the
 //               translation added once (one FADD2 per packed pair and coordinate, one FADD for the unpaired point).
-template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false>
+// MEAN = true : the mean cost (include/mmrs_b200.h "mean cost"; dense direct-form launches). Same pairs, staging, tail
+//               pass and chunk walk; only the reductions change. Each lane sums sqrtf of its completed row minima in
+//               f64 (per chunk; lane 0 also takes the tail pass's REDUX'ed minima); the final column minima go, like a
+//               chunked unit's intermediate ones, from lane 0 to the warp's shared row, and after the walk each lane
+//               sums sqrtf of every 32nd. Then a fixed shuffle tree, one division per direction, one rounding to FP32.
+//               Every padding duplicate of the staging image stays out of both sums: register slots at or past
+//               n - n_tail, the last chunk's padding, the repeated last point of an odd tail and column indices at or
+//               past m (an odd m's repeated last reference point, the B-block padding of exact tiling).
+template <int TA, bool MULTI, bool LIST, bool TAILP, bool XF, bool RIGID = false, bool MEAN = false>
 __global__ void __launch_bounds__(kThreads, 2)
     k_sweep(const UnitDesc* __restrict__ units, const WorkItem* __restrict__ work, const float4* __restrict__ lay,
             const float2* __restrict__ cs32, float* __restrict__ dist32, unsigned long long* __restrict__ key,
@@ -243,6 +251,7 @@ __global__ void __launch_bounds__(kThreads, 2)
     static_assert(!(TAILP && MULTI), "the tail pass is for single-chunk units");
     static_assert(!(XF && LIST), "the expanded form is a dense tier; lists are re-scored in direct form");
     static_assert(!(RIGID && (XF || LIST)), "rigid candidates run the dense direct-form sweep");
+    static_assert(!(MEAN && (XF || LIST)), "the mean cost runs the dense direct-form sweep");
     constexpr int SB = TA + 1;         // TAILP: reference points per lane of the tail pass (M <= 32 SB)
     constexpr int H = TA / 2;          // packed pairs of test points per lane
     constexpr bool TAIL = (TA & 1);    // plus one unpaired point when TA is odd
@@ -298,7 +307,7 @@ __global__ void __launch_bounds__(kThreads, 2)
     float4* sB = sA + a_elems;
     const float2* sNB = reinterpret_cast<const float2*>(sB + b_elems);
     const float4* sT = sB + b_elems + nb_elems;
-    unsigned* s_col = reinterpret_cast<unsigned*>(sB + b_elems + nb_elems + t_elems);  // MULTI: [warp][b_pts rounded up to 4]; TAILP: [warp][32 SB]
+    unsigned* s_col = reinterpret_cast<unsigned*>(sB + b_elems + nb_elems + t_elems);  // MULTI, MEAN: [warp][b_pts rounded up to 4]; TAILP: [warp][32 SB]
 
     if (threadIdx.x == 0) {
         *s_key = ~0ull;
@@ -334,6 +343,7 @@ __global__ void __launch_bounds__(kThreads, 2)
         const uint64_t C2 = pk(cs.x, cs.x), S2 = pk(cs.y, cs.y), NS2 = pk(-cs.y, -cs.y);
         const uint64_t TX2 = pk(tr.x, tr.x), TY2 = pk(tr.y, tr.y);
         unsigned rowmax = 0u, colmax = 0u;  // bit patterns of non-negative floats order like unsigned ints
+        double rsum = 0.0;                  // MEAN: this lane's sum of row values
         bool gave_up = false;
 
         if (TAILP) {
@@ -381,7 +391,14 @@ __global__ void __launch_bounds__(kThreads, 2)
                 }
                 const unsigned m0 = __reduce_min_sync(0xffffffffu, __float_as_uint(r0));
                 const unsigned m1 = __reduce_min_sync(0xffffffffu, __float_as_uint(r1));
-                rowmax = max(rowmax, max(m0, m1));
+                if constexpr (MEAN) {
+                    if (lane == 0) {   // an odd tail repeats its last point as tail point 2t + 1
+                        rsum += (double)sqrtf(__uint_as_float(m0));
+                        if (2 * t + 1 < ud.n_tail) rsum += (double)sqrtf(__uint_as_float(m1));
+                    }
+                } else {
+                    rowmax = max(rowmax, max(m0, m1));
+                }
             }
             __syncwarp();  // the previous candidate's main loop is done reading the seeds
 #pragma unroll
@@ -471,7 +488,7 @@ __global__ void __launch_bounds__(kThreads, 2)
                 }
                 const unsigned r0 = __reduce_min_sync(0xffffffffu, __float_as_uint(c0));
                 const unsigned r1 = __reduce_min_sync(0xffffffffu, __float_as_uint(c1));
-                if (LASTC) {
+                if (LASTC && !MEAN) {
                     colmax = max(colmax, max(r0, r1));  // these are the column minima
                 } else if (lane == 0) {
                     *reinterpret_cast<uint2*>(col_out) = make_uint2(r0, r1);
@@ -531,6 +548,13 @@ __global__ void __launch_bounds__(kThreads, 2)
                 walk(T_{}, T_{});
             }
             if (LIST && gave_up) break;  // the row minima are incomplete: only the column bound counts
+            if constexpr (MEAN) {   // row[k] is test point ch 32 TA + 32 k + lane; from n - n_tail on, padding
+                const int i0 = ch * 32 * TA + lane, n_main = ud.n - ud.n_tail;
+#pragma unroll
+                for (int k = 0; k < TA; ++k)
+                    if (i0 + 32 * k < n_main) rsum += (double)sqrtf(row[k]);
+                continue;
+            }
             if (XF) {   // row minima of r -> squared distances: + |a|^2 (the odd scalar slot is already a distance)
 #pragma unroll
                 for (int k = 0; k < H; ++k) {
@@ -546,8 +570,23 @@ __global__ void __launch_bounds__(kThreads, 2)
             rowmax = max(rowmax, __float_as_uint(rm));
         }
         if (MULTI) __syncwarp();  // the next candidate reuses my_col
-        const unsigned h2 = __reduce_max_sync(0xffffffffu, max(rowmax, colmax));
-        const float d = sqrtf(__uint_as_float(h2));
+        float d;
+        if constexpr (MEAN) {
+            __syncwarp();   // lane 0 stored the column minima
+            double csum = 0.0;
+            for (int j = lane; j < ud.m; j += 32) csum += (double)sqrtf(__uint_as_float(my_col[j]));
+            __syncwarp();   // the next candidate reuses my_col
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                rsum += __shfl_xor_sync(0xffffffffu, rsum, o);
+                csum += __shfl_xor_sync(0xffffffffu, csum, o);
+            }
+            // an FP32 overflow of d^2 makes a term, and so the cost, +inf, as it makes the full cost's maximum
+            d = (float)fmax(csum / (double)ud.m, rsum / (double)ud.n);
+        } else {
+            const unsigned h2 = __reduce_max_sync(0xffffffffu, max(rowmax, colmax));
+            d = sqrtf(__uint_as_float(h2));
+        }
         if (lane == 0) {
             // A candidate that gave up holds only a proven LOWER BOUND (above the unit's window): it is stored as such
             // (mmrs_b200.h: dist32 of pruned / given-up candidates is a bound) but enters neither the error diagnostic
@@ -1360,7 +1399,8 @@ __global__ void k_shortlist(const UnitDesc* __restrict__ units, const float* __r
 //   translate  : rigid candidates only: x' = rx + tx, y' = ry + ty (__dadd_rn; + 0.0 is exact, so a zero translation
 //                is the rotation-only cost bit for bit)
 //   distances  : process_utils.rs:84-121, both directions, sqrt, max
-//                (PARTIAL: the (q + 1)-th largest row minimum of each direction instead of the largest)
+//                (partial cost: the (q + 1)-th largest row minimum of each direction instead of the largest; mean
+//                cost: the mean row value sqrt(minimum) of each direction)
 // One CTA per (unit, candidate) item; grid-stride over the item list.
 // t64 != NULL: rigid candidates, c = i n_trans + j -> angle i of the unit's grid, translation j of its translation grid.
 // =============================================================================
@@ -1419,10 +1459,12 @@ __device__ __forceinline__ const double2* exact_stage(const UnitDesc& ud, const 
     return s_ref;
 }
 
-// The cost of one candidate. Each directed value is the largest row minimum (a non-finite minimum is skipped) or,
-// PARTIAL, the (q + 1)-th largest (a non-finite minimum counts as 0); s_min: n (or m) doubles of the CTA (shared memory
-// or a global scratch row) that hold the row minima of the partial cost.
-template <bool PARTIAL>
+// The cost of one candidate. Each directed value is the largest row minimum (a non-finite minimum is skipped); for the
+// partial cost the (q + 1)-th largest (a non-finite minimum counts as 0); for the mean cost the sum of the row values
+// sqrt(minimum) (a non-finite minimum counts as 0), sequential in point order on thread 0, over the count. s_min: n
+// (or m) doubles of the CTA (shared memory or a global scratch row) that hold the row minima of the partial cost, the
+// row values of the mean cost.
+template <Cost COST>
 __device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* __restrict__ test_xy,
                                              const double* __restrict__ ref_xy, double cosv, double sinv, bool identity,
                                              double2* s_rot, const double2* s_ref_in, double* s_red, double* s_min,
@@ -1440,21 +1482,32 @@ __device__ __forceinline__ double exact_cost(const UnitDesc& ud, const double* _
                 const double d2 = __dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy));
                 if (d2 < mn) mn = d2;
             }
-            if (PARTIAL) s_min[i] = isfinite(mn) ? mn : 0.0;
+            if (COST == kCostPartial) s_min[i] = isfinite(mn) ? mn : 0.0;
+            else if (COST == kCostMean) s_min[i] = isfinite(mn) ? __dsqrt_rn(mn) : 0.0;
             else if (isfinite(mn) && mn > lmax) lmax = mn;
         }
-        if (!PARTIAL) return block_max(lmax, s_red);
+        if (COST == kCostFull) return block_max(lmax, s_red);
         __syncthreads();
-        return block_kth_largest(s_min, nr, q, s_red);   // ends with a barrier: s_min may be reused
+        if (COST == kCostPartial) return block_kth_largest(s_min, nr, q, s_red);   // ends with a barrier: s_min may be reused
+        if (threadIdx.x == 0) {
+            double s = 0.0;
+            for (int i = 0; i < nr; ++i) s = __dadd_rn(s, s_min[i]);
+            s_red[0] = __ddiv_rn(s, (double)nr);
+        }
+        __syncthreads();
+        const double mean = s_red[0];
+        __syncthreads();   // s_min and s_red may be reused
+        return mean;
     };
     const double fwd = directed(s_ref, ud.m, s_rot, ud.n, ud.q_fwd);   // reference -> transformed
     const double bwd = directed(s_rot, ud.n, s_ref, ud.m, ud.q_bwd);   // transformed -> reference
+    if (COST == kCostMean) return fmax(fwd, bwd);
     return fmax(__dsqrt_rn(fwd), __dsqrt_rn(bwd));
 }
 
-// PARTIAL: g_min != NULL puts the CTA's row minima in a global scratch row (with g_scratch), else shared memory after
-// the two staged sets.
-template <bool PARTIAL>
+// Partial and mean costs: g_min != NULL puts the CTA's row minima in a global scratch row (with g_scratch), else shared
+// memory after the two staged sets.
+template <Cost COST>
 __global__ void __launch_bounds__(256)
     k_exact(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy, const double* __restrict__ ref_xy,
             const double2* __restrict__ cs64, const unsigned char* __restrict__ zero_flag,
@@ -1477,7 +1530,7 @@ __global__ void __launch_bounds__(256)
         const double2 cs = cs64[ud.cand_off + i];
         const bool identity = zero_flag[ud.cand_off + i] != 0;
         const double2 t = t64 ? t64[ud.t_off + (c - i * ud.n_trans)] : make_double2(0.0, 0.0);
-        const double d = exact_cost<PARTIAL>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+        const double d = exact_cost<COST>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
                                              g_scratch == nullptr, t64 != nullptr, t);
         if (threadIdx.x == 0) sl_dist[it] = d;
         __syncthreads();
@@ -1487,7 +1540,7 @@ __global__ void __launch_bounds__(256)
 // Dense variant: every candidate [c0, c0+count) of one unit (shortlist overflow
 // path and mmrs_eval_exact). t64 != NULL: rigid candidates; paired = true (mmrs_eval_exact_rigid): candidate c takes
 // angle c and translation t64[c] instead of the grid product.
-template <bool PARTIAL>
+template <Cost COST>
 __global__ void __launch_bounds__(256)
     k_exact_dense(const UnitDesc* __restrict__ units, int unit, const double* __restrict__ test_xy,
                   const double* __restrict__ ref_xy, const double2* __restrict__ cs64,
@@ -1505,7 +1558,7 @@ __global__ void __launch_bounds__(256)
         const double2 cs = cs64[cs_off + i];
         const bool identity = zero_flag[cs_off + i] != 0;
         const double2 t = !t64 ? make_double2(0.0, 0.0) : paired ? t64[c] : t64[ud.t_off + (c - i * ud.n_trans)];
-        const double d = exact_cost<PARTIAL>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
+        const double d = exact_cost<COST>(ud, test_xy, ref_xy, cs.x, cs.y, identity, s_rot, s_ref, s_red, s_min,
                                              g_scratch == nullptr, t64 != nullptr, t);
         if (threadIdx.x == 0) out[c] = d;
         __syncthreads();

@@ -93,7 +93,8 @@ EXPORTS = [
     "mmrs_align_centerline", "mmrs_sweep_prefilter_info", "mmrs_ctx_set_prune", "mmrs_contour_metrics",
     "mmrs_comm_unique_id", "mmrs_ctx_comm_init", "mmrs_ctx_set_partition", "mmrs_ctx_comm_info",
     "mmrs_rigid_sweep_batched", "mmrs_rigid_sweep_upload", "mmrs_rigid_sweep_regrid", "mmrs_rigid_sweep_download",
-    "mmrs_eval_exact_rigid", "mmrs_partial_sweep_upload", "mmrs_eval_exact_partial",
+    "mmrs_eval_exact_rigid", "mmrs_partial_sweep_upload", "mmrs_eval_exact_partial", "mmrs_mean_sweep_upload",
+    "mmrs_eval_exact_mean",
 ]
 
 _lib = None
@@ -145,6 +146,10 @@ def lib():
                                                 C.c_double, C.POINTER(SweepOpts)]
         L.mmrs_eval_exact_partial.argtypes = [C.c_void_p, c_dp, C.c_int64, c_dp, C.c_int64, C.c_double, C.c_double,
                                               C.c_int32, c_dp, c_dp, C.c_int64, C.c_double, c_dp]
+        L.mmrs_mean_sweep_upload.argtypes = [C.c_void_p, C.POINTER(SweepBatch), C.POINTER(TGrid), C.c_int64, c_i32p,
+                                             C.POINTER(SweepOpts)]
+        L.mmrs_eval_exact_mean.argtypes = [C.c_void_p, c_dp, C.c_int64, c_dp, C.c_int64, C.c_double, C.c_double,
+                                           C.c_int32, c_dp, c_dp, C.c_int64, c_dp]
         _lib = L
     return _lib
 
@@ -348,6 +353,36 @@ class Context:
                                                   float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
                                                   None if tt is None else tt.ctypes.data_as(c_dp), len(a),
                                                   float(inlier_fraction), out.ctypes.data_as(c_dp)))
+        return out
+
+    # -- mean cost (modified Hausdorff distance, mmrs_b200.h "mean cost") -------------------------------------------
+    def mean_upload(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids=None, grid_of_unit=None,
+                    tgrid_of_unit=None, mode=0, **opts):
+        """mmrs_mean_sweep_upload: rigid_upload (tgrids given) or sweep_upload (tgrids=None) with the mean cost.
+        Run with sweep_run; download with sweep_download, or rigid_download after a rigid upload."""
+        b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
+        o = self._opts(**opts)
+        if tgrids is None:
+            tarr, n_t, ptou = None, 0, None
+        else:
+            tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+            n_t = len(tgrids)
+        self._check(lib().mmrs_mean_sweep_upload(self._p, C.byref(b), tarr, n_t, ptou, C.byref(o)))
+        self._n_units = U
+
+    def eval_exact_mean(self, test_xy, ref_xy, centre, mode, angles, txy=None):
+        """f64 mean cost of the candidates (angles[k], txy[k]) (txy=None: rotation only; mmrs_eval_exact_mean)."""
+        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
+        tt = None
+        if txy is not None:
+            tt = _f64(txy).reshape(-1, 2)
+            if len(tt) != len(a):
+                raise ValueError("eval_exact_mean: angles and txy differ in length")
+        out = np.empty(len(a), dtype=np.float64)
+        self._check(lib().mmrs_eval_exact_mean(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r),
+                                               float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
+                                               None if tt is None else tt.ctypes.data_as(c_dp), len(a),
+                                               out.ctypes.data_as(c_dp)))
         return out
 
     def plan(self):

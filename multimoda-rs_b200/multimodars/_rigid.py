@@ -56,7 +56,8 @@ def _finite_number(v, name):
 
 
 def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rotation_deg=90.0, step_translation=0.05,
-                              range_translation=0.25, centre=None, bruteforce=False, inlier_fraction=1.0):
+                              range_translation=0.25, centre=None, bruteforce=False, inlier_fraction=1.0,
+                              cost="hausdorff"):
     """Best rigid transform (rotation about `centre`, then translation) of `test` onto `reference`.
 
     Candidates: rotations on the grid of the rotation sweep (coarse-to-fine like find_best_rotation, or one stage
@@ -70,6 +71,9 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
     inlier_fraction: f < 1 scores the partial (rank-K) Hausdorff distance instead (include/mmrs_b200.h "partial
     cost"): in each direction the worst n - max(1, ceil(f n)) points of a set do not count, so a few artefact points
     (a side-branch bulge, a calcification) do not decide the transform. 1.0 is the full distance.
+    cost: "hausdorff" (the symmetric Hausdorff distance, or its partial form above) or "mean": the modified Hausdorff
+    distance (include/mmrs_b200.h "mean cost"), the larger of the two directions' mean closest-point distances, so
+    every point counts. "mean" takes inlier_fraction = 1 only. range_translation = 0 searches the rotation only.
     Returns a structured array, one row per pair: angle_rad, rotation_deg, tx, ty, distance, n_ties."""
     tests, refs = _as_sets(test, "test"), _as_sets(reference, "reference")
     if len(tests) != len(refs):
@@ -93,6 +97,10 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
     frac = _finite_number(inlier_fraction, "inlier_fraction")
     if not 0.0 < frac <= 1.0:
         raise ValueError("inlier_fraction must satisfy 0 < inlier_fraction <= 1")
+    if not isinstance(cost, str) or cost not in ("hausdorff", "mean"):
+        raise ValueError(f"cost must be 'hausdorff' or 'mean', got {cost!r}")
+    if cost == "mean" and frac != 1.0:
+        raise ValueError("cost='mean' takes inlier_fraction = 1 only (a trimmed mean is not supported)")
     half_n = int(math.floor(range_t / step_t + 1e-9))
     if half_n > 1000:
         raise ValueError(f"range_translation / step_translation = {half_n} translations per side; at most 1000")
@@ -119,7 +127,10 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
     ctx = get_context()
     res = None
     for k, (step, window) in enumerate(stages):
-        if k == 0 and frac < 1.0:
+        if k == 0 and cost == "mean":
+            ctx.mean_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
+                            mode=1)
+        elif k == 0 and frac < 1.0:
             ctx.partial_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
                                mode=1, inlier_fraction=frac)
         elif k == 0:   # stage 0 centred on 0; stage k > 0 on the previous stage's angle, clipped to +-range_rotation_deg
