@@ -276,18 +276,21 @@ class Context:
     # -- rigid candidates (angle grid x translation grid, mmrs_b200.h "rigid candidates") -------------------------
     @staticmethod
     def _tgrids(tgrids, tgrid_of_unit):
+        """(array, count, tgrid_of_unit pointer) of the C calls; tgrids=None (rotation only): (None, 0, None)."""
+        if tgrids is None:
+            return None, 0, None
         tarr = (TGrid * max(len(tgrids), 1))(*tgrids)
         tou = None if tgrid_of_unit is None else np.ascontiguousarray(tgrid_of_unit, dtype=np.int32)
-        return tarr, tou, None if tou is None else tou.ctypes.data_as(c_i32p)
+        return tarr, len(tgrids), None if tou is None else tou.ctypes.data_as(c_i32p)   # the pointer keeps tou alive
 
     def rigid_sweep_batched(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids, grid_of_unit=None,
                             tgrid_of_unit=None, mode=0, **opts):
         """mmrs_rigid_sweep_batched: host arrays in, structured result array (RIGID_RESULT_DTYPE) out."""
         b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
-        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        tarr, n_t, ptou = self._tgrids(tgrids, tgrid_of_unit)
         o = self._opts(**opts)
         out = np.zeros(U, dtype=RIGID_RESULT_DTYPE)
-        self._check(lib().mmrs_rigid_sweep_batched(self._p, C.byref(b), tarr, len(tgrids), ptou, C.byref(o),
+        self._check(lib().mmrs_rigid_sweep_batched(self._p, C.byref(b), tarr, n_t, ptou, C.byref(o),
                                                    out.ctypes.data_as(C.c_void_p)))
         self._n_units = U
         return out
@@ -295,34 +298,40 @@ class Context:
     def rigid_upload(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids, grid_of_unit=None,
                      tgrid_of_unit=None, mode=0, **opts):
         b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
-        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        tarr, n_t, ptou = self._tgrids(tgrids, tgrid_of_unit)
         o = self._opts(**opts)
-        self._check(lib().mmrs_rigid_sweep_upload(self._p, C.byref(b), tarr, len(tgrids), ptou, C.byref(o)))
+        self._check(lib().mmrs_rigid_sweep_upload(self._p, C.byref(b), tarr, n_t, ptou, C.byref(o)))
         self._n_units = U
 
     def rigid_regrid(self, grids, tgrids, grid_of_unit=None, tgrid_of_unit=None, tie_margin=0.0):
         garr = (Grid * max(len(grids), 1))(*grids)
         gou = None if grid_of_unit is None else np.ascontiguousarray(grid_of_unit, dtype=np.int32)
-        tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
+        tarr, n_t, ptou = self._tgrids(tgrids, tgrid_of_unit)
         self._check(lib().mmrs_rigid_sweep_regrid(self._p, garr, len(grids), None if gou is None else gou.ctypes.data_as(c_i32p),
-                                                  tarr, len(tgrids), ptou, float(tie_margin)))
+                                                  tarr, n_t, ptou, float(tie_margin)))
 
     def rigid_download(self):
         out = np.zeros(self._n_units, dtype=RIGID_RESULT_DTYPE)
         self._check(lib().mmrs_rigid_sweep_download(self._p, out.ctypes.data_as(C.c_void_p)))
         return out
 
+    def _eval(self, fn, name, test_xy, ref_xy, centre, mode, angles, txy, *cost_args):
+        """mmrs_eval_exact_<cost>: f64 cost of the candidates (angles[k], txy[k]); txy=None passes NULL."""
+        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
+        tt = None
+        if txy is not None:
+            tt = _f64(txy).reshape(-1, 2)
+            if len(tt) != len(a):
+                raise ValueError(f"{name}: angles and txy differ in length")
+        out = np.empty(len(a), dtype=np.float64)
+        self._check(fn(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r), float(centre[0]),
+                       float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
+                       None if tt is None else tt.ctypes.data_as(c_dp), len(a), *cost_args, out.ctypes.data_as(c_dp)))
+        return out
+
     def eval_exact_rigid(self, test_xy, ref_xy, centre, mode, angles, txy):
         """f64 cost of the rigid candidates (angles[k], txy[k]) (mmrs_eval_exact_rigid)."""
-        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
-        tt = _f64(txy).reshape(-1, 2)
-        if len(tt) != len(a):
-            raise ValueError("eval_exact_rigid: angles and txy differ in length")
-        out = np.empty(len(a), dtype=np.float64)
-        self._check(lib().mmrs_eval_exact_rigid(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r),
-                                                float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
-                                                tt.ctypes.data_as(c_dp), len(a), out.ctypes.data_as(c_dp)))
-        return out
+        return self._eval(lib().mmrs_eval_exact_rigid, "eval_exact_rigid", test_xy, ref_xy, centre, mode, angles, txy)
 
     # -- partial cost (rank-K Hausdorff distance, mmrs_b200.h "partial cost") -------------------------------------
     def partial_upload(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids=None, grid_of_unit=None,
@@ -331,29 +340,15 @@ class Context:
         Run with sweep_run; download with sweep_download, or rigid_download after a rigid upload."""
         b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
         o = self._opts(**opts)
-        if tgrids is None:
-            tarr, n_t, ptou = None, 0, None
-        else:
-            tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
-            n_t = len(tgrids)
+        tarr, n_t, ptou = self._tgrids(tgrids, tgrid_of_unit)
         self._check(lib().mmrs_partial_sweep_upload(self._p, C.byref(b), tarr, n_t, ptou, float(inlier_fraction),
                                                     C.byref(o)))
         self._n_units = U
 
     def eval_exact_partial(self, test_xy, ref_xy, centre, mode, angles, txy=None, inlier_fraction=1.0):
         """f64 partial cost of the candidates (angles[k], txy[k]) (txy=None: rotation only; mmrs_eval_exact_partial)."""
-        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
-        tt = None
-        if txy is not None:
-            tt = _f64(txy).reshape(-1, 2)
-            if len(tt) != len(a):
-                raise ValueError("eval_exact_partial: angles and txy differ in length")
-        out = np.empty(len(a), dtype=np.float64)
-        self._check(lib().mmrs_eval_exact_partial(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r),
-                                                  float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
-                                                  None if tt is None else tt.ctypes.data_as(c_dp), len(a),
-                                                  float(inlier_fraction), out.ctypes.data_as(c_dp)))
-        return out
+        return self._eval(lib().mmrs_eval_exact_partial, "eval_exact_partial", test_xy, ref_xy, centre, mode, angles,
+                          txy, float(inlier_fraction))
 
     # -- mean cost (modified Hausdorff distance, mmrs_b200.h "mean cost") -------------------------------------------
     def mean_upload(self, test_xy, test_off, ref_xy, ref_off, centre_xy, grids, tgrids=None, grid_of_unit=None,
@@ -362,28 +357,13 @@ class Context:
         Run with sweep_run; download with sweep_download, or rigid_download after a rigid upload."""
         b, U = self._batch(test_xy, test_off, ref_xy, ref_off, centre_xy, grids, grid_of_unit, mode)
         o = self._opts(**opts)
-        if tgrids is None:
-            tarr, n_t, ptou = None, 0, None
-        else:
-            tarr, tou, ptou = self._tgrids(tgrids, tgrid_of_unit)
-            n_t = len(tgrids)
+        tarr, n_t, ptou = self._tgrids(tgrids, tgrid_of_unit)
         self._check(lib().mmrs_mean_sweep_upload(self._p, C.byref(b), tarr, n_t, ptou, C.byref(o)))
         self._n_units = U
 
     def eval_exact_mean(self, test_xy, ref_xy, centre, mode, angles, txy=None):
         """f64 mean cost of the candidates (angles[k], txy[k]) (txy=None: rotation only; mmrs_eval_exact_mean)."""
-        t, r, a = _f64(test_xy).reshape(-1, 2), _f64(ref_xy).reshape(-1, 2), _f64(angles).reshape(-1)
-        tt = None
-        if txy is not None:
-            tt = _f64(txy).reshape(-1, 2)
-            if len(tt) != len(a):
-                raise ValueError("eval_exact_mean: angles and txy differ in length")
-        out = np.empty(len(a), dtype=np.float64)
-        self._check(lib().mmrs_eval_exact_mean(self._p, t.ctypes.data_as(c_dp), len(t), r.ctypes.data_as(c_dp), len(r),
-                                               float(centre[0]), float(centre[1]), int(mode), a.ctypes.data_as(c_dp),
-                                               None if tt is None else tt.ctypes.data_as(c_dp), len(a),
-                                               out.ctypes.data_as(c_dp)))
-        return out
+        return self._eval(lib().mmrs_eval_exact_mean, "eval_exact_mean", test_xy, ref_xy, centre, mode, angles, txy)
 
     def plan(self):
         p = (C.c_int64 * 5)()

@@ -4,7 +4,7 @@ The reference aligns centroids and then searches the rotation only (align_within
 A side branch, a calcification or a catheter artefact moves a centroid, so the Hausdorff-optimal rotation is then
 found about the wrong offset. `find_best_rigid_transform` searches a translation grid alongside the rotation sweep:
 every candidate (theta, tx, ty) is scored by the symmetric Hausdorff distance on the GPU (mmrs_rigid_sweep_*,
-include/mmrs_b200.h "rigid candidates"). This has no reference counterpart; tests/rigid_oracle.py restates it."""
+include/mmrs_b200.h "rigid candidates"). This has no reference counterpart; tests/cost_oracle.py restates it."""
 from __future__ import annotations
 
 import math
@@ -127,15 +127,12 @@ def find_best_rigid_transform(test, reference, step_rotation_deg=0.5, range_rota
     ctx = get_context()
     res = None
     for k, (step, window) in enumerate(stages):
-        if k == 0 and cost == "mean":
-            ctx.mean_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
-                            mode=1)
-        elif k == 0 and frac < 1.0:
-            ctx.partial_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
-                               mode=1, inlier_fraction=frac)
-        elif k == 0:   # stage 0 centred on 0; stage k > 0 on the previous stage's angle, clipped to +-range_rotation_deg
-            ctx.rigid_upload(test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg],
-                             mode=1)
+        if k == 0:   # stage 0 centred on 0; stage k > 0 on the previous stage's angle, clipped to +-range_rotation_deg
+            args = (test_xy, test_off, ref_xy, ref_off, cen, [nat.make_grid(step, window, None, range_r)], [tg])
+            if cost == "mean":
+                ctx.mean_upload(*args, mode=1)
+            else:   # inlier_fraction = 1 is the full cost, as rigid_upload
+                ctx.partial_upload(*args, mode=1, inlier_fraction=frac)
         else:
             grids = [nat.make_grid(step, window, float(a), range_r) for a in res["best_angle"]]
             ctx.rigid_regrid(grids, [tg], grid_of_unit=np.arange(U, dtype=np.int32))

@@ -8,7 +8,7 @@ distances evaluated per candidate, for K1e (default) and K1 (MMRS_EARLY_BREAK=0)
 (b) a config-3-shaped batch (1 596 units, N = M = 510) through find_best_rigid_transform, coarse-to-fine 0.01 deg over
     +-180 deg, 11^2 translations (wall-clock of the whole call: three stages, uploads and downloads included);
 (c) the (a) units with half_n = 0 against the rotation-only sweep on the same grid;
-plus the CPU f64 restatement (tests/rigid_oracle.py) on a few candidates as a baseline. Needs a CUDA device."""
+plus the CPU f64 restatement (tests/cost_oracle.py) on a few candidates as a baseline. Needs a CUDA device."""
 from __future__ import annotations
 
 import json
@@ -116,18 +116,18 @@ def main():
         print(out["cases"][-1], flush=True)
     set_eb(None)
     # CPU baseline: the f64 restatement (numpy, one thread) on a few candidates of two bench units
-    from tests import rigid_oracle as ro
+    from tests import cost_oracle as co
 
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     t0 = time.perf_counter()
     k = 0
     for u in (0, U // 2):
         for a in (0.1, -0.7):
-            ro.costs_at_angle(txy[toff[u]:toff[u + 1]], rxy[roff[u]:roff[u + 1]], cen[u], 0, a, offs)
+            co.costs_at_angle(txy[toff[u]:toff[u + 1]], rxy[roff[u]:roff[u + 1]], cen[u], 0, a, offs, "full")
             k += T
     dt = time.perf_counter() - t0
-    out["cpu_oracle"] = {"what": "tests/rigid_oracle.py costs_at_angle (numpy f64, 1 process)", "candidates": k,
-                         "s": dt, "evals_per_s": k / dt, "points": [n, n]}
+    out["cpu_oracle"] = {"what": "tests/cost_oracle.py costs_at_angle, full cost (numpy f64, 1 process)",
+                         "candidates": k, "s": dt, "evals_per_s": k / dt, "points": [n, n]}
     print(out["cpu_oracle"], flush=True)
     out["gpu_after"] = gpu_info()
     out_path.parent.mkdir(parents=True, exist_ok=True)

@@ -1,6 +1,6 @@
 """The mean cost (include/mmrs_b200.h "mean cost") on the GPU.
 
-1. mmrs_eval_exact_mean against the f64 restatement in tests/mean_oracle.py, bit for bit.
+1. mmrs_eval_exact_mean against the f64 restatement in tests/cost_oracle.py, bit for bit.
 2. The sweep against the oracle over every K1 size class (padded odd and even register tiles, exact tiling with even
    and odd tails, n = 32 TA +- 1, odd m, tiny and duplicated sets, the chunked 2 020-point class, rigid batches):
    selection, f64 distance and ties exactly, and every candidate's FP32 value within the documented bound of its f64
@@ -13,9 +13,8 @@ import pytest
 import multimodars as mm
 from multimodars import _native as nat
 from oracle import oracle_py as ora
-from tests import mean_oracle as mo
-from tests import rigid_oracle as ro
-from tests.test_sweep_gpu import contour, make_units
+from tests import cost_oracle as co
+from tests.test_sweep_gpu import contour, make_units, pack
 
 pytestmark = pytest.mark.gpu
 
@@ -34,15 +33,9 @@ def ctx():
     print(f"\nmean cost: largest |d32 - d64| / R_eff = {WORST['ratio']:.3e}")
 
 
-def _pack(tests, refs):
-    toff = np.concatenate([[0], np.cumsum([len(t) for t in tests])])
-    roff = np.concatenate([[0], np.cumsum([len(r) for r in refs])])
-    return np.concatenate(tests), toff, np.concatenate(refs), roff
-
-
 def mean_run(ctx, tests, refs, cents, grid, tg=None, mode=0, **opts):
     """One mean sweep with keep_dist32: (results, dist32 per unit (None for an empty set))."""
-    txy, toff, rxy, roff = _pack(tests, refs)
+    txy, toff, rxy, roff = pack(tests, refs)
     ctx.mean_upload(txy, toff, rxy, roff, cents, [grid], None if tg is None else [tg], mode=mode, keep_dist32=True,
                     **opts)
     ctx.sweep_run()
@@ -52,17 +45,12 @@ def mean_run(ctx, tests, refs, cents, grid, tg=None, mode=0, **opts):
     return res, d32
 
 
-def _finite(a):
-    a = np.asarray(a, dtype=np.float64).reshape(-1, 2)
-    return a[np.isfinite(a).all(axis=1)]
-
-
 def check_oracle(ctx, tests, refs, cents, res, d32, grid_params, mode, tg=None):
-    offs = np.zeros((1, 2)) if tg is None else ro.offsets_of(tg)
+    offs = np.zeros((1, 2)) if tg is None else co.offsets_of(tg)
     T = len(offs)
     angles, _ = ora.search_grid(*grid_params)
     for u in range(len(tests)):
-        idx, costs = mo.search(tests[u], refs[u], cents[u], mode, angles, offs)
+        idx, costs = co.search(tests[u], refs[u], cents[u], mode, angles, offs, "mean")
         flat = costs.reshape(-1)
         assert res["best_idx"][u] == idx, (u, res["best_idx"][u], idx)
         assert res["best_angle"][u] == angles[idx // T]
@@ -74,7 +62,7 @@ def check_oracle(ctx, tests, refs, cents, res, d32, grid_params, mode, tg=None):
                                   None if tg is None else np.tile(offs, (len(angles), 1)))
         assert np.array_equal(d64, flat), u
         if d32[u] is not None:
-            pts = np.concatenate([_finite(tests[u]), _finite(refs[u])])
+            pts = np.concatenate([co.finite(tests[u]), co.finite(refs[u])])
             r_eff = np.abs(pts - cents[u]).max() + np.hypot(offs[:, 0], offs[:, 1]).max()
             err = np.abs(d32[u].astype(np.float64) - flat)
             assert (err <= ABS_BOUND * r_eff + REL_BOUND * flat).all(), (u, len(tests[u]), len(refs[u]), err.max(), r_eff)
@@ -95,16 +83,16 @@ def test_eval_exact_mean_against_oracle(ctx, mode):
              (rng.normal(0, 1, (3, 2)), rng.normal(0, 1, (1, 2))),
              (a_dup, rng.normal(0, 1, (30, 2))),                           # duplicated points
              (nf, nf_r),                                                   # non-finite points dropped
-             mo.crafted_order_case()]                                      # sequential order differs from pairwise
+             co.crafted_order_case()]                                      # sequential order differs from pairwise
     angles = np.array([0.0, 0.3, -1.1, 2.5])
     txy = np.array([[0.0, 0.0], [0.1, -0.2], [0.0, 0.05], [-0.3, 0.01]])
     for test, ref in pairs:
         cen = (0.1, -0.1)
         got = ctx.eval_exact_mean(test, ref, cen, mode, angles)
-        want = np.array([mo.cost(test, ref, cen, mode, a) for a in angles])
+        want = np.array([co.candidate_cost(test, ref, cen, mode, a, (0.0, 0.0), "mean") for a in angles])
         assert np.array_equal(got, want), (got, want)
         got = ctx.eval_exact_mean(test, ref, cen, mode, angles, txy)
-        want = np.array([mo.cost(test, ref, cen, mode, a, t) for a, t in zip(angles, txy)])
+        want = np.array([co.candidate_cost(test, ref, cen, mode, a, t, "mean") for a, t in zip(angles, txy)])
         assert np.array_equal(got, want), (got, want)
     empty = np.zeros((0, 2))
     assert (ctx.eval_exact_mean(empty, pairs[0][1], (0, 0), mode, angles) == 0.0).all()
@@ -166,7 +154,7 @@ def test_regrid_keeps_the_cost_and_plain_upload_clears_it(ctx):
     fine = ctx.sweep_download()
     for u in range(3):
         angles, _ = ora.search_grid(0.01, 0.5, float(coarse["best_angle"][u]), 180.0)
-        idx, costs = mo.search(tests[u], refs[u], cents[u], 0, angles, np.zeros((1, 2)))
+        idx, costs = co.search(tests[u], refs[u], cents[u], 0, angles, np.zeros((1, 2)), "mean")
         assert fine["best_idx"][u] == idx and fine["best_dist"][u] == costs.reshape(-1)[idx]
     ctx.sweep_upload(txy, toff, rxy, roff, cents, [nat.make_grid(1.0, 180.0)], keep_dist32=True)
     ctx.sweep_run()
@@ -182,7 +170,7 @@ def test_planted_rotation_and_translation_recovered(ctx):
     cen = ref.mean(axis=0)
     g = nat.make_grid(0.5, 20.0)
     tg = nat.make_tgrid(0.05, 3)
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     i_star, j_star = 23, 3 * 7 + 5
     theta = nat.grid_angle(g, i_star)
     c, s = np.cos(theta), np.sin(theta)
@@ -226,17 +214,17 @@ def test_find_best_rigid_transform_mean_against_oracle():
     rng = np.random.default_rng(370)
     tests, refs, _, *_ = make_units(rng, [(80, 90), (64, 64)])
     kw = dict(step_rotation_deg=0.5, range_rotation_deg=10.0, step_translation=0.05)
-    offs = ro.tgrid_offsets(0.0, 0.0, 0.05, 1)
+    offs = co.tgrid_offsets(0.0, 0.0, 0.05, 1)
     for brute in (False, True):
         out = mm.find_best_rigid_transform(tests, refs, range_translation=0.05, bruteforce=brute, cost="mean", **kw)
         for u in range(2):
             cen = (np.cumsum(refs[u][:, 0])[-1] / len(refs[u]), np.cumsum(refs[u][:, 1])[-1] / len(refs[u]))
-            a, j, tx, ty, d = mo.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, offs, bruteforce=brute)
+            a, j, tx, ty, d = co.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, offs, "mean", bruteforce=brute)
             assert out["angle_rad"][u] == a and out["tx"][u] == tx and out["ty"][u] == ty and out["distance"][u] == d
     rot = mm.find_best_rigid_transform(tests, refs, range_translation=0.0, cost="mean", **kw)   # rotation only
     for u in range(2):
         cen = (np.cumsum(refs[u][:, 0])[-1] / len(refs[u]), np.cumsum(refs[u][:, 1])[-1] / len(refs[u]))
-        a, j, tx, ty, d = mo.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, np.zeros((1, 2)))
+        a, j, tx, ty, d = co.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, np.zeros((1, 2)), "mean")
         assert rot["angle_rad"][u] == a and rot["tx"][u] == 0.0 and rot["ty"][u] == 0.0 and rot["distance"][u] == d
     same = mm.find_best_rigid_transform(tests, refs, range_translation=0.05, **kw)
     full = mm.find_best_rigid_transform(tests, refs, range_translation=0.05, cost="hausdorff", **kw)

@@ -3,7 +3,7 @@
 1. inlier_fraction = 1 is the plain rotation-only / rigid sweep, field for field and dist32 bit for bit; in a batch
    with f < 1, units whose q is 0 in both directions match the plain sweep.
 2. Early break on (K1e-partial) equals early break off (every row scanned to its end), dist32 bit for bit.
-3. Results against the f64 restatement in tests/partial_oracle.py and mmrs_eval_exact_partial.
+3. Results against the f64 restatement in tests/cost_oracle.py and mmrs_eval_exact_partial.
 4. A planted transform is recovered despite a 3-point bulge. 5. find_best_rigid_transform(inlier_fraction=...).
 6. Error cases."""
 import numpy as np
@@ -13,9 +13,8 @@ import bench
 import multimodars as mm
 from multimodars import _native as nat
 from oracle import oracle_py as ora
-from tests import partial_oracle as po
-from tests import rigid_oracle as ro
-from tests.test_sweep_gpu import contour, make_units
+from tests import cost_oracle as co
+from tests.test_sweep_gpu import contour, make_units, pack, same_bits
 
 pytestmark = pytest.mark.gpu
 
@@ -30,12 +29,6 @@ def ctx():
     c.close()
 
 
-def _pack(tests, refs):
-    toff = np.concatenate([[0], np.cumsum([len(t) for t in tests])])
-    roff = np.concatenate([[0], np.cumsum([len(r) for r in refs])])
-    return np.concatenate(tests), toff, np.concatenate(refs), roff
-
-
 def n_cands(tests, refs, grids, tgrids, gou=None):
     T = 1 if tgrids is None else (2 * tgrids[0].half_n + 1) ** 2
     return [0 if grids[0 if gou is None else gou[u]].degenerate else grids[0 if gou is None else gou[u]].n_cand * T
@@ -44,7 +37,7 @@ def n_cands(tests, refs, grids, tgrids, gou=None):
 
 def partial(ctx, tests, refs, cents, grids, f, tgrids=None, gou=None, mode=0, **opts):
     """One partial sweep with keep_dist32: (results, dist32 per unit (None for an empty set), prefilter_info)."""
-    txy, toff, rxy, roff = _pack(tests, refs)
+    txy, toff, rxy, roff = pack(tests, refs)
     ctx.partial_upload(txy, toff, rxy, roff, cents, grids, tgrids, grid_of_unit=gou, mode=mode, inlier_fraction=f,
                        keep_dist32=True, **opts)
     ctx.sweep_run()
@@ -55,7 +48,7 @@ def partial(ctx, tests, refs, cents, grids, f, tgrids=None, gou=None, mode=0, **
 
 
 def plain(ctx, tests, refs, cents, grids, tgrids=None, gou=None, mode=0):
-    txy, toff, rxy, roff = _pack(tests, refs)
+    txy, toff, rxy, roff = pack(tests, refs)
     if tgrids is None:
         res = ctx.sweep_batched(txy, toff, rxy, roff, cents, grids, grid_of_unit=gou, mode=mode, keep_dist32=True)
     else:
@@ -63,13 +56,6 @@ def plain(ctx, tests, refs, cents, grids, tgrids=None, gou=None, mode=0):
                                       keep_dist32=True)
     nc = n_cands(tests, refs, grids, tgrids, gou)
     return res, [ctx.dist32(u, int(nc[u])) if len(tests[u]) and len(refs[u]) else None for u in range(len(tests))]
-
-
-def same_bits(a, b, what):
-    for u, (x, y) in enumerate(zip(a, b)):
-        if x is not None:
-            bad = np.flatnonzero(x.view(np.uint32) != y.view(np.uint32))
-            assert bad.size == 0, (what, u, bad[:8], x[bad[:8]], y[bad[:8]])
 
 
 def bench_units(k, rng_deg=None):
@@ -203,7 +189,8 @@ def test_on_off_rigid_and_hierarchical(ctx, monkeypatch):
     # the regridded stage scores the partial cost: compare the fine winner with the oracle
     for u in range(4):
         angles, _ = ora.search_grid(0.01, 2.0, float(coarse["best_angle"][u]), 180.0)
-        assert fine["best_dist"][u] == po.cost(tests[u], refs[u], cents[u], 0, angles[fine["best_idx"][u]], (0, 0), 0.95)
+        assert fine["best_dist"][u] == co.candidate_cost(tests[u], refs[u], cents[u], 0, angles[fine["best_idx"][u]],
+                                                         (0, 0), "partial", 0.95)
 
 
 def test_on_off_chunked_units_and_q255(ctx, monkeypatch):
@@ -213,17 +200,17 @@ def test_on_off_chunked_units_and_q255(ctx, monkeypatch):
     on_vs_off(ctx, monkeypatch, tests, refs, cents, [nat.make_grid(0.05, 2.0)], 0.95)
     t2, r2, c2, *_ = make_units(rng, [(1275, 1275), (600, 1275)])
     f = 1.0 - 255.0 / 1275.0                      # K = ceil(f n) = 1020 -> q = 255 for n = 1275
-    assert po.q_of(1275, f) == 255
+    assert co.q_of(1275, f) == 255
     on_vs_off(ctx, monkeypatch, t2, r2, c2, [nat.make_grid(1.0, 30.0)], f)
 
 
 # ---- 3. against the oracle ------------------------------------------------------------------------------------------
 def check_oracle(ctx, tests, refs, cents, res, d32, grid_params, f, mode, tg=None):
-    offs = np.zeros((1, 2)) if tg is None else ro.offsets_of(tg)
+    offs = np.zeros((1, 2)) if tg is None else co.offsets_of(tg)
     T = len(offs)
     for u in range(len(tests)):
         angles, _ = ora.search_grid(*grid_params)
-        idx, costs = po.search(tests[u], refs[u], cents[u], mode, angles, offs, f)
+        idx, costs = co.search(tests[u], refs[u], cents[u], mode, angles, offs, "partial", f)
         flat = costs.reshape(-1)
         assert res["best_idx"][u] == idx, (u, res["best_idx"][u], idx)
         assert res["best_angle"][u] == angles[idx // T]
@@ -259,7 +246,7 @@ def test_circle_ties_and_self_match(ctx):
     g = nat.make_grid(4.0, 180.0)                   # every angle maps the circle onto itself
     res, d32, _ = partial(ctx, [circ], [circ.copy()], np.zeros((1, 2)), [g], 0.9, mode=1, tie_margin=1e-9)
     angles, _ = ora.search_grid(4.0, 180.0, None, 180.0)
-    idx, costs = po.search(circ, circ, (0.0, 0.0), 1, angles, np.zeros((1, 2)), 0.9)
+    idx, costs = co.search(circ, circ, (0.0, 0.0), 1, angles, np.zeros((1, 2)), "partial", 0.9)
     assert res["best_idx"][0] == idx and res["best_dist"][0] == costs.reshape(-1)[idx]
     assert res["n_ties"][0] > 1
 
@@ -272,7 +259,7 @@ def test_bulge_does_not_decide_the_transform(ctx, rigid):
     cen = cents[0]
     g = nat.make_grid(0.5, 20.0)
     tg = nat.make_tgrid(0.05, 3) if rigid else None
-    offs = ro.offsets_of(tg) if rigid else np.zeros((1, 2))
+    offs = co.offsets_of(tg) if rigid else np.zeros((1, 2))
     i_star, j_star = 17, (3 * 7 + 5 if rigid else 0)
     theta = nat.grid_angle(g, i_star)
     c, s = np.cos(theta), np.sin(theta)
@@ -284,7 +271,7 @@ def test_bulge_does_not_decide_the_transform(ctx, rigid):
         v = test[k] - test.mean(axis=0)
         test[k] += 0.5 * v / np.linalg.norm(v)
     f = 1.0 - 4.0 / len(test)                         # q >= 3 in both directions
-    assert po.q_of(len(test), f) >= 3 and po.q_of(len(ref), f) >= 3
+    assert co.q_of(len(test), f) >= 3 and co.q_of(len(ref), f) >= 3
     tgs = None if tg is None else [tg]
     res, _, _ = partial(ctx, [test], [ref], cen[None], [g], f, tgs, mode=1)
     full, _, _ = partial(ctx, [test], [ref], cen[None], [g], 1.0, tgs, mode=1)
@@ -301,10 +288,10 @@ def test_find_best_rigid_transform_partial_against_oracle():
     tests, refs, _, *_ = make_units(rng, [(80, 90), (64, 64)])
     out = mm.find_best_rigid_transform(tests, refs, step_rotation_deg=0.5, range_rotation_deg=10.0,
                                        step_translation=0.05, range_translation=0.05, inlier_fraction=0.95)
-    offs = ro.tgrid_offsets(0.0, 0.0, 0.05, 1)
+    offs = co.tgrid_offsets(0.0, 0.0, 0.05, 1)
     for u in range(2):
         cen = (np.cumsum(refs[u][:, 0])[-1] / len(refs[u]), np.cumsum(refs[u][:, 1])[-1] / len(refs[u]))
-        a, j, tx, ty, d = po.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, offs, 0.95)
+        a, j, tx, ty, d = co.coarse_to_fine(tests[u], refs[u], cen, 1, 0.5, 10.0, offs, "partial", 0.95)
         assert out["angle_rad"][u] == a and out["tx"][u] == tx and out["ty"][u] == ty and out["distance"][u] == d
     same = mm.find_best_rigid_transform(tests, refs, step_rotation_deg=0.5, range_rotation_deg=10.0,
                                         step_translation=0.05, range_translation=0.05)

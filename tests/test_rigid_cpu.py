@@ -11,7 +11,7 @@ from scipy.spatial.distance import directed_hausdorff
 
 import multimodars as mm
 from multimodars import _native as nat
-from tests import rigid_oracle as ro
+from tests import cost_oracle as co
 
 ROOT = Path(__file__).resolve().parent.parent
 
@@ -22,8 +22,8 @@ def test_rigid_search_against_scipy(mode):
     test, ref = rng.normal(0, 1, (23, 2)), rng.normal(0.1, 1.1, (19, 2))
     centre = (0.2, -0.1)
     angles = [0.0, 0.3, -1.2]
-    offs = ro.tgrid_offsets(0.05, -0.02, 0.1, 2)
-    idx, costs = ro.rigid_search(test, ref, centre, mode, angles, offs)
+    offs = co.tgrid_offsets(0.05, -0.02, 0.1, 2)
+    idx, costs = co.search(test, ref, centre, mode, angles, offs, "full")
     want = np.empty_like(costs)
     for i, a in enumerate(angles):
         for j, (tx, ty) in enumerate(offs):
@@ -39,23 +39,24 @@ def test_rigid_search_against_scipy(mode):
 
 
 def test_rigid_search_empty_and_non_finite():
-    offs = ro.tgrid_offsets(0.0, 0.0, 0.1, 1)
-    idx, costs = ro.rigid_search(np.zeros((0, 2)), np.ones((3, 2)), (0, 0), 1, [0.1, 0.2], offs)
+    offs = co.tgrid_offsets(0.0, 0.0, 0.1, 1)
+    idx, costs = co.search(np.zeros((0, 2)), np.ones((3, 2)), (0, 0), 1, [0.1, 0.2], offs, "full")
     assert idx == 0 and (costs == 0.0).all()
     rng = np.random.default_rng(9)
     a, b = rng.normal(size=(10, 2)), rng.normal(size=(8, 2))
     a_nan = np.concatenate([a, [[np.nan, 1.0], [np.inf, 0.0]]])
-    assert np.array_equal(ro.rigid_search(a_nan, b, (0, 0), 1, [0.4], offs)[1], ro.rigid_search(a, b, (0, 0), 1, [0.4], offs)[1])
+    assert np.array_equal(co.search(a_nan, b, (0, 0), 1, [0.4], offs, "full")[1],
+                          co.search(a, b, (0, 0), 1, [0.4], offs, "full")[1])
 
 
 def test_translation_grid_formula():
     tg = nat.make_tgrid(0.07, 3, t0=(0.3, -0.2))
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     assert offs.shape == (49, 2)
     for j in (0, 5, 7, 24, 48):
         jy, jx = divmod(j, 7)
         assert offs[j, 0] == 0.3 + float(jx - 3) * 0.07 and offs[j, 1] == -0.2 + float(jy - 3) * 0.07
-    assert np.array_equal(ro.offsets_of(nat.make_tgrid(0.5, 0)), [[0.0, 0.0]])   # half_n = 0: c == i
+    assert np.array_equal(co.offsets_of(nat.make_tgrid(0.5, 0)), [[0.0, 0.0]])   # half_n = 0: c == i
 
 
 def test_struct_mirrors_match_header():

@@ -2,7 +2,7 @@
 
 1. A zero translation grid is the rotation-only sweep, field for field and dist32 bit for bit, under K1 and K1e.
 2. K1e equals K1 on rigid runs, dist32 bit for bit.
-3. Results against the f64 restatement in tests/rigid_oracle.py; every FP32 distance within 1e-5 relative of
+3. Results against the f64 restatement in tests/cost_oracle.py; every FP32 distance within 1e-5 relative of
    mmrs_eval_exact_rigid.
 4. A known transform is recovered exactly. 5. Ties. 6. find_best_rigid_transform against the oracle's
    coarse-to-fine. 7. Error cases."""
@@ -13,8 +13,8 @@ import bench
 import multimodars as mm
 from multimodars import _native as nat
 from oracle import oracle_py as ora
-from tests import rigid_oracle as ro
-from tests.test_sweep_gpu import contour, make_units
+from tests import cost_oracle as co
+from tests.test_sweep_gpu import contour, make_units, pack, same_bits
 
 pytestmark = pytest.mark.gpu
 
@@ -28,18 +28,12 @@ def ctx():
     c.close()
 
 
-def _pack(tests, refs):
-    toff = np.concatenate([[0], np.cumsum([len(t) for t in tests])])
-    roff = np.concatenate([[0], np.cumsum([len(r) for r in refs])])
-    return np.concatenate(tests), toff, np.concatenate(refs), roff
-
-
 def _d32(ctx, tests, refs, n_cand):
     return [ctx.dist32(u, int(n_cand[u])) if len(tests[u]) and len(refs[u]) else None for u in range(len(tests))]
 
 
 def rigid(ctx, tests, refs, cents, grids, tgrids, gou=None, tou=None, mode=0, **opts):
-    txy, toff, rxy, roff = _pack(tests, refs)
+    txy, toff, rxy, roff = pack(tests, refs)
     res = ctx.rigid_sweep_batched(txy, toff, rxy, roff, cents, grids, tgrids, grid_of_unit=gou, tgrid_of_unit=tou,
                                   mode=mode, keep_dist32=True, **opts)
     U = len(tests)
@@ -50,16 +44,9 @@ def rigid(ctx, tests, refs, cents, grids, tgrids, gou=None, tou=None, mode=0, **
     return res, _d32(ctx, tests, refs, n_cand), ctx.prefilter_info()
 
 
-def same_bits(a, b, what):
-    for u, (x, y) in enumerate(zip(a, b)):
-        if x is not None:
-            bad = np.flatnonzero(x.view(np.uint32) != y.view(np.uint32))
-            assert bad.size == 0, (what, u, bad[:8], x[bad[:8]], y[bad[:8]])
-
-
 # ---- 1. zero translation == the rotation-only sweep -------------------------------------------------------------
 def zero_vs_rotation(ctx, monkeypatch, tests, refs, cents, grids, gou=None, mode=0):
-    txy, toff, rxy, roff = _pack(tests, refs)
+    txy, toff, rxy, roff = pack(tests, refs)
     z = nat.make_tgrid(0.0, 0)
     for flag in ("0", "1"):
         monkeypatch.setenv("MMRS_EARLY_BREAK", flag)
@@ -160,11 +147,11 @@ def test_k1e_equals_k1_rigid(ctx, monkeypatch, half_n):
 
 # ---- 3. against the oracle -----------------------------------------------------------------------------------------
 def check_oracle(ctx, tests, refs, cents, res, d32, grid_params, tg, mode):
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     worst = 0.0
     for u in range(len(tests)):
         angles, fb = ora.search_grid(*grid_params)
-        idx, costs = ro.rigid_search(tests[u], refs[u], cents[u], mode, angles, offs)
+        idx, costs = co.search(tests[u], refs[u], cents[u], mode, angles, offs, "full")
         T = len(offs)
         assert res["best_idx"][u] == idx
         assert res["angle_idx"][u] == idx // T and res["trans_idx"][u] == idx % T
@@ -202,7 +189,7 @@ def test_empty_set_and_degenerate_grid(ctx):
     grids = [nat.make_grid(2.0, 10.0), nat.make_grid(0.0, 10.0, center=0.3)]
     res, d32, _ = rigid(ctx, tests, refs, cents, grids, [tg], gou=np.array([0, 0, 1], np.int32))
     assert res["best_idx"][1] == 0 and res["best_dist"][1] == 0.0 and res["flags"][1] & nat.FLAG_EMPTY
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     assert res["trans_idx"][1] == 0 and res["best_tx"][1] == offs[0, 0] and res["best_ty"][1] == offs[0, 1]
     assert res["best_idx"][2] == -1 and res["best_angle"][2] == 0.3 and res["flags"][2] & nat.FLAG_DEGENERATE
     assert res["angle_idx"][2] == -1 and res["trans_idx"][2] == -1
@@ -217,7 +204,7 @@ def test_known_transform_is_recovered(ctx):
     cen = np.array([4.5, 4.5])
     g = nat.make_grid(1.0, 30.0)
     tg = nat.make_tgrid(0.05, 5)
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     i_star, j_star = 37, 7 * 11 + 2
     theta = nat.grid_angle(g, i_star)
     c, s = np.cos(theta), np.sin(theta)
@@ -238,14 +225,14 @@ def test_circle_ties_pick_the_lowest_flattened_index(ctx):
     tg = nat.make_tgrid(0.1, 1)
     res, _, _ = rigid(ctx, [circ], [circ.copy()], np.zeros((1, 2)), [g], [tg], mode=1, tie_margin=1e-9)
     angles, _ = ora.search_grid(4.0, 180.0, None, 180.0)
-    idx, costs = ro.rigid_search(circ, circ, (0.0, 0.0), 1, angles, ro.offsets_of(tg))
+    idx, costs = co.search(circ, circ, (0.0, 0.0), 1, angles, co.offsets_of(tg), "full")
     assert res["best_idx"][0] == idx
     best = costs.reshape(-1)[idx]
     flat = costs.reshape(-1)
     T = 9
     lim = best + 1e-9 * max(1.0, 2.0 + 0.1 * np.sqrt(2))
     cs = np.array([[np.cos(a), np.sin(a)] for a in angles])
-    offs = ro.offsets_of(tg)
+    offs = co.offsets_of(tg)
     want = 1 + sum(1 for c in range(len(flat)) if c != idx and flat[c] <= lim and
                    (not np.array_equal(cs[c // T], cs[idx // T]) or not np.array_equal(offs[c % T], offs[idx % T])))
     assert want > 1
@@ -261,10 +248,11 @@ def test_find_best_rigid_transform_against_oracle(bruteforce):
     step, rng_deg = (2.0, 20.0) if bruteforce else (0.5, 20.0)
     out = mm.find_best_rigid_transform(tests, refs, step_rotation_deg=step, range_rotation_deg=rng_deg,
                                        step_translation=0.05, range_translation=0.1, bruteforce=bruteforce)
-    offs = ro.tgrid_offsets(0.0, 0.0, 0.05, 2)
+    offs = co.tgrid_offsets(0.0, 0.0, 0.05, 2)
     for u in range(2):
         cen = (np.cumsum(refs[u][:, 0])[-1] / len(refs[u]), np.cumsum(refs[u][:, 1])[-1] / len(refs[u]))
-        a, j, tx, ty, d = ro.rigid_coarse_to_fine(tests[u], refs[u], cen, 1, step, rng_deg, offs, bruteforce=bruteforce)
+        a, j, tx, ty, d = co.coarse_to_fine(tests[u], refs[u], cen, 1, step, rng_deg, offs, "full",
+                                            bruteforce=bruteforce)
         assert out["angle_rad"][u] == a and out["tx"][u] == tx and out["ty"][u] == ty and out["distance"][u] == d
 
 

@@ -38,9 +38,22 @@ def make_units(rng, sizes, centre=(4.5, 4.5)):
         refs.append(contour(rng, m, r0=rng.uniform(1.5, 3.0), e=rng.uniform(0.05, 0.35)))
         tests.append(contour(rng, n, r0=rng.uniform(1.5, 3.0), e=rng.uniform(0.05, 0.35), rot=rot))
         cents.append(np.array(centre) + rng.normal(0, 0.05, 2))
+    return (tests, refs, np.array(cents), *pack(tests, refs))
+
+
+def pack(tests, refs):
+    """Per-unit point sets -> (test_xy, test_off, ref_xy, ref_off) of one batch."""
     toff = np.concatenate([[0], np.cumsum([len(t) for t in tests])])
     roff = np.concatenate([[0], np.cumsum([len(r) for r in refs])])
-    return tests, refs, np.array(cents), np.concatenate(tests), toff, np.concatenate(refs), roff
+    return np.concatenate(tests), toff, np.concatenate(refs), roff
+
+
+def same_bits(a, b, what):
+    """Per-unit FP32 distance arrays equal bit for bit (None: a unit without distances)."""
+    for u, (x, y) in enumerate(zip(a, b)):
+        if x is not None:
+            bad = np.flatnonzero(x.view(np.uint32) != y.view(np.uint32))
+            assert bad.size == 0, (what, u, bad[:8], x[bad[:8]], y[bad[:8]])
 
 
 def check_against_oracle(ctx, tests, refs, cents, res, step, rng_deg, mode, center=None, limes=None, check_dist32=True):
