@@ -624,9 +624,10 @@ __global__ void __launch_bounds__(kThreads, 2)
 //     H^2 = max( max_a min_b d^2 , max_b min_a d^2 ),
 // and once L, an exactly computed row or column minimum of THIS candidate, is known, a row that meets one b with
 // d^2 <= L cannot raise the maximum and stops there. Per warp, over a contiguous run of the tile's candidates:
-//   rotate  the N test points into a per-warp shared-memory row A'[N];
-//   seed    L = max(exact minimum of row ra, exact minimum of column cb), where ra / cb defined the previous
-//           candidate's maximum (the warp's first candidate: the points farthest from the rotation centre);
+//   rotate  the N test points into a per-warp shared-memory row A'[N], two per lane and staging slot;
+//   seed    L = the exact minimum of row ra or of column cb, whichever last raised the previous candidate's L (the
+//           warp's first candidate, and every RIGID candidate: the larger of both; ra / cb start at the points
+//           farthest from the rotation centre);
 //   rows    lane l takes rows l, l + 32, ...: kEbTries positions of a zig-zag scan around the row's hint (the index
 //           where it stopped for the previous candidate); rows still open are then finished one at a time by the
 //           whole warp (32 positions per round, one REDUX.MIN), stopping at the first round whose minimum is <= L;
@@ -648,7 +649,8 @@ __device__ __forceinline__ float eb_d2(float2 a, float2 b) {
     return __fmaf_rn(dx, dx, __fmul_rn(dy, dy));
 }
 // t-th position (t < n: every index exactly once) of a scan over n points that starts at h and zig-zags outward:
-// h, h + 1, h - 1, h + 2, ... modulo n (contours are closed)
+// h, h + 1, h - 1, h + 2, ... modulo n (contours are closed). Position t + 2k lies k further out on the same side as t,
+// so the scans below step from one position to the next instead of calling this for every t.
 __device__ __forceinline__ int eb_zig(int h, int t, int n) {
     int j = h + ((t & 1) ? (t + 1) >> 1 : -(t >> 1));
     j = j < 0 ? j + n : j;
@@ -661,16 +663,20 @@ __device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a
                                                 int& arg, unsigned& pairs) {
     unsigned best = ~0u, m = ~0u;
     int bj = h;
+    // lane l scans positions t = l, l + 32, ...: each round moves 16 further out on the lane's side of the zig-zag, +16
+    // (odd t) or -16 = + (n - 16) (even t), wrapped once; a second round exists only for n > 32, where 0 < n - 16 < n
+    int j = eb_zig(h, lane, n);
+    const int step = (lane & 1) ? 16 : n - 16;
     for (int t0 = 0; t0 < n; t0 += 32) {
-        const int t = t0 + lane;
-        if (t < n) {
-            const int j = eb_zig(h, t, n);
+        if (t0 + lane < n) {
             const unsigned d = __float_as_uint(eb_d2(a, P[j]));
             if (d < best) best = d, bj = j;
             ++pairs;
         }
         m = __reduce_min_sync(0xffffffffu, best);
         if (early && m <= L) break;
+        j += step;
+        j = j >= n ? j - n : j;
     }
     arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
     return m;
@@ -692,9 +698,16 @@ __device__ __forceinline__ void eb_rows(const float2* R, int g, bool open, const
     if (open) {
         const int i = g + lane;
         const float2 a = R[i];
-        const int h0 = h[i];
+        int j = h[i];   // zig-zag position t: h, then steps of +1, -2, +3, each wrapped once
+#pragma unroll
         for (int t = 0; t < kEbTries && t < n_set; ++t) {
-            const int j = eb_zig(h0, t, n_set);
+            if (t & 1) {
+                j += t;
+                j = j >= n_set ? j - n_set : j;
+            } else if (t) {
+                j -= t;
+                j = j < 0 ? j + n_set : j;
+            }
             ++pairs;
             if (__float_as_uint(eb_d2(a, P[j])) <= L) {
                 h[i] = (unsigned short)j;
@@ -847,8 +860,8 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
     unsigned long long best = ~0ull;
     unsigned pairs = 0;
     if (c_begin < c_end) {
-        int ra = 0, cb = 0;            // K1e: the row and the column that defined the previous candidate's value
-        bool seed[2] = {true, true};   // PARTIAL: the directions whose lists seed the next candidate
+        int ra = 0, cb = 0;            // K1e: the row and the column that last raised L
+        bool seed[2] = {true, true};   // the directions that seed the next candidate (PARTIAL: from their lists)
         if constexpr (PARTIAL) {
 #pragma unroll
             for (int dir = 0; dir < 2; ++dir) {
@@ -895,20 +908,40 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
             }
             ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
         }
+        int ia = c_begin, it = 0;   // candidate c's angle and (RIGID) translation, c = ia n_trans + it: stepped, not divided
+        if (RIGID) ia = c_begin / ud.n_trans, it = c_begin - ia * ud.n_trans;
         for (int c = c_begin; c < c_end; ++c) {
             float2 tr = make_float2(0.f, 0.f);
-            int ia = c;
-            if (RIGID) {
-                ia = c / ud.n_trans;
-                tr = __ldg(&t32[ud.t_off + (c - ia * ud.n_trans)]);
-            }
+            if (RIGID) tr = __ldg(&t32[ud.t_off + it]);
             const float2 cs = __ldg(&cs32[ud.cand_off + ia]);
+            if (!RIGID || ++it == ud.n_trans) it = 0, ++ia;
             __syncwarp();   // the previous candidate is done with A', the hints and the lists
-            for (int i = lane; i < N; i += 32) {
-                const float2 p = test_pt(i);
-                float2 r = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
-                if (RIGID) r = make_float2(__fadd_rn(r.x, tr.x), __fadd_rn(r.y, tr.y));
-                sR[i] = r;
+            // A': the A block in its own slot order, two points (x0, x1, y0, y1) per float4, rotated with K1's packed
+            // sequence (each half the scalar x' = fma(y, -s, x c), y' = fma(x, s, y c), + t); then the tail block
+            {
+                const uint64_t C2 = pk(cs.x, cs.x), S2 = pk(cs.y, cs.y), NS2 = pk(-cs.y, -cs.y);
+                const uint64_t TX2 = pk(tr.x, tr.x), TY2 = pk(tr.y, tr.y);
+                const float4* a4 = sA + lane;
+                for (int c0 = 0; c0 < n_main; c0 += 32 * TA) {           // chunk: test points c0 .. c0 + 32 TA - 1
+                    for (int k = 0; k < TA; k += 2, a4 += 32) {          // slot k / 2: points i, and i + 32 if k + 1 < TA
+                        const float4 v = *a4;
+                        const uint64_t X2 = pk(v.x, v.y), Y2 = pk(v.z, v.w);
+                        uint64_t PX = fma2(Y2, NS2, mul2(X2, C2)), PY = fma2(X2, S2, mul2(Y2, C2));
+                        if (RIGID) PX = add2(PX, TX2), PY = add2(PY, TY2);
+                        float x0, x1, y0, y1;
+                        upk(PX, x0, x1);
+                        upk(PY, y0, y1);
+                        const int i = c0 + 32 * k + lane;
+                        if (i < n_main) sR[i] = make_float2(x0, y0);
+                        if (k + 1 < TA && i + 32 < n_main) sR[i + 32] = make_float2(x1, y1);
+                    }
+                }
+                if (lane < N - n_main) {   // the tail block (exact tiling): fewer than 32 points
+                    const float2 p = sT[lane];
+                    float2 r = make_float2(__fmaf_rn(p.y, -cs.y, __fmul_rn(p.x, cs.x)), __fmaf_rn(p.x, cs.y, __fmul_rn(p.y, cs.x)));
+                    if (RIGID) r = make_float2(__fadd_rn(r.x, tr.x), __fadd_rn(r.y, tr.y));
+                    sR[n_main + lane] = r;
+                }
             }
             __syncwarp();
             unsigned L;
@@ -969,19 +1002,29 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                     }
                 }
             } else {
-                // seeds: the exact minima of the row and the column that defined the previous candidate's value
-                int arg;
-                L = eb_warp_min(sB, M, sR[ra], hint[0][ra], 0u, false, lane, arg, pairs);
-                const int h_ra = arg;
-                const unsigned lc = eb_warp_min(sR, N, sB[cb], hint[1][cb], 0u, false, lane, arg, pairs);
+                // seed: the exact minimum of the row ra or the column cb, whichever last raised the previous
+                // candidate's L (the run's first candidate: both)
+                int h_ra = 0, h_cb = 0;
+                L = 0u;
+                if (seed[0]) L = eb_warp_min(sB, M, sR[ra], hint[0][ra], 0u, false, lane, h_ra, pairs);
+                const unsigned lc = seed[1] ? eb_warp_min(sR, N, sB[cb], hint[1][cb], 0u, false, lane, h_cb, pairs) : 0u;
                 __syncwarp();
-                if (lane == 0) hint[0][ra] = (unsigned short)h_ra, hint[1][cb] = (unsigned short)arg;
+                if (lane == 0) {
+                    if (seed[0]) hint[0][ra] = (unsigned short)h_ra;
+                    if (seed[1]) hint[1][cb] = (unsigned short)h_cb;
+                }
+                bool by_row = seed[0] && !(lc > L);   // the direction that last raised L (both seeded and tied: rows)
                 L = max(L, lc);
                 __syncwarp();
                 for (int g = 0; g < N; g += 32)   // rows: test point i against the reference points
-                    eb_rows(sR, g, g + lane < N, sB, M, hint[0], L, [&](unsigned mn, int i) { ra = i; return mn; }, lane, pairs);
+                    eb_rows(sR, g, g + lane < N, sB, M, hint[0], L, [&](unsigned mn, int i) { ra = i, by_row = true; return mn; }, lane, pairs);
                 for (int g = 0; g < M; g += 32)   // columns: reference point j against A'
-                    eb_rows(sB, g, g + lane < M, sR, N, hint[1], L, [&](unsigned mn, int j) { cb = j; return mn; }, lane, pairs);
+                    eb_rows(sB, g, g + lane < M, sR, N, hint[1], L, [&](unsigned mn, int j) { cb = j, by_row = false; return mn; }, lane, pairs);
+                // rotation only: seed one direction. RIGID keeps both: a run steps through the translations and jumps
+                // back across the whole translation grid at each new angle, and a single seed leaves L lower there
+                // often enough to cost more pairs than the second seed scan (4 277 against 4 184 per candidate on the
+                // bench units, 361 angles x 121 translations)
+                seed[0] = RIGID || by_row, seed[1] = RIGID || !by_row;
             }
             const float d = sqrtf(__uint_as_float(L));
             if (lane == 0) {

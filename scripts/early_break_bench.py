@@ -78,9 +78,8 @@ def run_case(ctx, name, batch, grid, n, m):
     return out
 
 
-def main():
-    out_path = Path(sys.argv[1]) if len(sys.argv) > 1 else None
-    ctx = nat.Context(0)
+def make_cases():
+    """The workload classes: (name, batch, grid, n, m)."""
     txy, toff, rxy, roff, cen, U, n = bench.make_units(n_pairs=1)   # pair 0: 398 frame pairs, N = M = 520
     bench_batch = (txy, toff, rxy, roff, cen)
     rng = np.random.default_rng(2026)
@@ -89,7 +88,7 @@ def main():
     circ = np.stack([2.0 * np.cos(phi), 2.0 * np.sin(phi)], 1)
     cfg4 = bench.synthetic_pullback(9, 2000, bench.SEED + 40)
     cfg4 = [np.concatenate([f, f[:20]]) - f.mean(0) for f in cfg4]   # N = M = 2 020
-    cases = [
+    return [
         ("bench units, 0.01 deg over +-180", bench_batch, nat.make_grid(0.01, 180.0), 520, 520),
         ("398 random contour pairs, 0.01 deg over +-180", pack(rand[::2], rand[1::2]), nat.make_grid(0.01, 180.0), 520, 520),
         ("circle on circle x 64, 0.01 deg over +-180", pack([circ] * 64, [circ] * 64), nat.make_grid(0.01, 180.0), 520, 520),
@@ -99,7 +98,12 @@ def main():
         ("bench units, 40 candidates (between-pullback shape)", bench_batch, nat.make_grid(0.5, 10.0), 520, 520),
         ("config-4 size, 8 frame pairs, 0.05 deg over +-180", pack(cfg4[1:], cfg4[:-1]), nat.make_grid(0.05, 180.0), 2020, 2020),
     ]
-    rows = [run_case(ctx, *c) for c in cases]
+
+
+def main():
+    out_path = Path(sys.argv[1]) if len(sys.argv) > 1 else None
+    ctx = nat.Context(0)
+    rows = [run_case(ctx, *c) for c in make_cases()]
     doc = {"gpu": gpu_info(), "reps": REPS, "timing": "sweep-kernel device time (CUDA events), median of the reps",
            "rows": rows}
     if out_path:
