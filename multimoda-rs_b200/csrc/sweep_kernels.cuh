@@ -628,18 +628,22 @@ __global__ void __launch_bounds__(kThreads, 2)
 //   seed    L = the exact minimum of row ra or of column cb, whichever last raised the previous candidate's L (the
 //           warp's first candidate, and every RIGID candidate: the larger of both; ra / cb start at the points
 //           farthest from the rotation centre);
-//   rows    lane l takes rows l, l + 32, ...: kEbTries positions of a zig-zag scan around the row's hint (the index
-//           where it stopped for the previous candidate); rows still open are then finished one at a time by the
-//           whole warp (32 positions per round, one REDUX.MIN), stopping at the first round whose minimum is <= L;
-//           a row that runs to its end has an exact minimum > L, which becomes L;
+//   hints   a row's hint is the index where it stopped for the previous candidate; on the run's first candidate, which
+//           starts anywhere in the angle range, it is the nearest of every kEbColdStride-th point of the other set
+//           (eb_cold_hints, after A' is written);
+//   rows    lane l takes rows l, l + 32, ...: kEbTries positions of a zig-zag scan around the row's hint; rows still
+//           open are then finished one at a time by the whole warp (32 positions per round, one REDUX.MIN), stopping
+//           at the first round whose minimum is <= L; a row that runs to its end has an exact minimum > L, which
+//           becomes L;
 //   columns the same with the reference points as rows and A' as the set.
 // Every pair distance is K1's operation sequence (x' = fma(y, -s, x c), y' = fma(x, s, y c), d^2 = fma(dx, dx, dy dy)),
 // pinned against contraction; the column pass reads the same A' (|a - b|^2 and |b - a|^2 round alike). L only ever
-// holds exact minima of the current candidate: earlier candidates decide the ORDER of the scans, never a threshold. So
-// the final L is max over every row and column minimum, and dist32 is bit-identical to K1's. An overflowed d^2 = inf
-// never passes <= L: that row scans to its exact minimum, as K1 computes it.
+// holds exact minima of the current candidate: earlier candidates and the subsample decide the ORDER of the scans,
+// never a threshold. So the final L is max over every row and column minimum, and dist32 is bit-identical to K1's. An
+// overflowed d^2 = inf never passes <= L: that row scans to its exact minimum, as K1 computes it.
 // =============================================================================
 constexpr int kEbTries = 4;   // zig-zag positions a lane tries on its own before the warp takes its row over
+constexpr int kEbColdStride = 16;   // a run's first hints: the nearest of every kEbColdStride-th point
 
 // per-warp shared memory of K1e: A'[n] (float2), then the row hints [n] and column hints [m] (16-bit indices)
 __host__ __device__ constexpr int eb_warp_bytes(int n, int m) { return (8 * n + 2 * (n + m) + 15) & ~15; }
@@ -680,6 +684,24 @@ __device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a
     }
     arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
     return m;
+}
+// Hints of rows R[0 .. n) for the first candidate of a run: each row's nearest point among P[0], P[kEbColdStride], ...
+// of the n_set points of P (one lane per row, no early stop; the warp's lanes read the same P[j]: a broadcast). The
+// hint is a multiple of the stride below n_set whatever the distances are (a NaN d^2 may win, which is harmless: the
+// hint only orders the scans).
+__device__ __forceinline__ void eb_cold_hints(const float2* R, int n, const float2* P, int n_set, unsigned short* h,
+                                              int lane, unsigned& pairs) {
+    for (int i = lane; i < n; i += 32) {
+        const float2 a = R[i];
+        unsigned best = ~0u;
+        int bj = 0;
+        for (int j = 0; j < n_set; j += kEbColdStride) {
+            const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+            if (d < best) best = d, bj = j;
+        }
+        h[i] = (unsigned short)bj;
+        pairs += (unsigned)((n_set + kEbColdStride - 1) / kEbColdStride);
+    }
 }
 // Index of the largest v over the warp (v: non-negative float bits; ties -> lowest lane).
 __device__ __forceinline__ int eb_warp_argmax(unsigned v, int idx) {
@@ -867,8 +889,6 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
             for (int dir = 0; dir < 2; ++dir) {
                 const int n = n_rows[dir];
                 for (int k = lane; k < (n + 31) / 32; k += 32) bits[dir][k] = 0u;
-                for (int r = lane; r < n; r += 32)
-                    hint[dir][r] = (unsigned short)(((long long)r * n_rows[1 - dir]) / n);
                 __syncwarp();
                 // first candidate's seeds: the q + 1 points farthest from the rotation centre (unrotated)
                 EbList& l = lst[dir];
@@ -891,20 +911,18 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                 l.cnt = l.cap;
             }
         } else {
-            // first candidate: hints on the index diagonal, seeds at the points farthest from the rotation centre
+            // first candidate: seeds at the points farthest from the rotation centre
             unsigned far_a = 0u, far_b = 0u;
             int ia = 0, ib = 0;
             for (int i = lane; i < N; i += 32) {
                 const float2 p = test_pt(i);
                 const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
                 if (r2 > far_a) far_a = r2, ia = i;
-                hint[0][i] = (unsigned short)(((long long)i * M) / N);
             }
             for (int j = lane; j < M; j += 32) {
                 const float2 p = sB[j];
                 const unsigned r2 = __float_as_uint(p.x * p.x + p.y * p.y);
                 if (r2 > far_b) far_b = r2, ib = j;
-                hint[1][j] = (unsigned short)(((long long)j * N) / M);
             }
             ra = eb_warp_argmax(far_a, ia), cb = eb_warp_argmax(far_b, ib);
         }
@@ -944,6 +962,11 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                 }
             }
             __syncwarp();
+            if (c == c_begin) {   // the run's first candidate: no previous hints to start from
+                eb_cold_hints(sR, N, sB, M, hint[0], lane, pairs);
+                eb_cold_hints(sB, M, sR, N, hint[1], lane, pairs);
+                __syncwarp();
+            }
             unsigned L;
             if constexpr (PARTIAL) {
                 // seeds: the listed rows of the seeded directions, one lane each, scanned to the end
