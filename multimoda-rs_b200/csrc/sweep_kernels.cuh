@@ -631,10 +631,11 @@ __global__ void __launch_bounds__(kThreads, 2)
 //   hints   a row's hint is the index where it stopped for the previous candidate; on the run's first candidate, which
 //           starts anywhere in the angle range, it is the nearest of every kEbColdStride-th point of the other set
 //           (eb_cold_hints, after A' is written);
-//   rows    lane l takes rows l, l + 32, ...: kEbTries positions of a zig-zag scan around the row's hint; rows still
-//           open are then finished one at a time by the whole warp (32 positions per round, one REDUX.MIN), stopping
-//           at the first round whose minimum is <= L; a row that runs to its end has an exact minimum > L, which
-//           becomes L;
+//   rows    lane l takes rows l, l + 32, ...: first every row tests its hint against the seeded L in one lane-parallel
+//           loop, then the rows that missed try kEbTries - 1 more positions of a zig-zag scan around the hint; rows
+//           still open are then finished one at a time by the whole warp (32 positions per round, one REDUX.MIN),
+//           stopping at the first round whose minimum is <= L; a row that runs to its end has an exact minimum > L,
+//           which becomes L (eb_pass; the run's first candidate takes the groups one at a time, eb_rows);
 //   columns the same with the reference points as rows and A' as the set.
 // Every pair distance is K1's operation sequence (x' = fma(y, -s, x c), y' = fma(x, s, y c), d^2 = fma(dx, dx, dy dy)),
 // pinned against contraction; the column pass reads the same A' (|a - b|^2 and |b - a|^2 round alike). L only ever
@@ -661,10 +662,10 @@ __device__ __forceinline__ int eb_zig(int h, int t, int n) {
     return j >= n ? j - n : j;
 }
 // Minimum of d^2(a, P[j]) over the n points of P, the whole warp together along the zig-zag from h (call it with the
-// full warp, warp-uniform arguments). early: stop after the first round whose running minimum is <= L. Returns the bit
+// full warp, warp-uniform arguments), stopping after the first round whose running minimum is <= L. Returns the bit
 // pattern of the minimum found (the exact minimum whenever it is > L) and, in arg, where it was found.
-__device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a, int h, unsigned L, bool early, int lane,
-                                                int& arg, unsigned& pairs) {
+__device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a, int h, unsigned L, int lane, int& arg,
+                                                unsigned& pairs) {
     unsigned best = ~0u, m = ~0u;
     int bj = h;
     // lane l scans positions t = l, l + 32, ...: each round moves 16 further out on the lane's side of the zig-zag, +16
@@ -678,10 +679,34 @@ __device__ __forceinline__ unsigned eb_warp_min(const float2* P, int n, float2 a
             ++pairs;
         }
         m = __reduce_min_sync(0xffffffffu, best);
-        if (early && m <= L) break;
+        if (m <= L) break;
         j += step;
         j = j >= n ? j - n : j;
     }
+    arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
+    return m;
+}
+// The exact minimum of d^2(a, P[j]) over the n points of P (the seeds), the same positions per lane as eb_warp_min but
+// without stopping: the full rounds unguarded, then the tail round, and one REDUX at the end. arg: where the lowest lane
+// among equal minima first found it, as eb_warp_min.
+__device__ __forceinline__ unsigned eb_warp_exact(const float2* P, int n, float2 a, int h, int lane, int& arg,
+                                                  unsigned& pairs) {
+    unsigned best = ~0u;
+    int bj = h;
+    int j = eb_zig(h, lane, n);
+    const int step = (lane & 1) ? 16 : n - 16, full = n & ~31;
+    for (int t0 = 0; t0 < full; t0 += 32) {
+        const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+        if (d < best) best = d, bj = j;
+        j += step;
+        j = j >= n ? j - n : j;
+    }
+    if (lane < n - full) {
+        const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+        if (d < best) best = d, bj = j;
+    }
+    pairs += (unsigned)(full >> 5) + (lane < n - full);
+    const unsigned m = __reduce_min_sync(0xffffffffu, best);
     arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
     return m;
 }
@@ -713,7 +738,8 @@ __device__ __forceinline__ int eb_warp_argmax(unsigned v, int idx) {
 // points of P, with the rows' hints h; open: row g + lane takes part. Lane l first tries kEbTries positions of the
 // zig-zag around the hint of row g + l; the rows still open are then finished one at a time by the whole warp. A row
 // stops at its first d^2 <= L and keeps that position as its hint; a row that scans to its end has an exact minimum
-// mn > L, and L becomes exact(mn, i).
+// mn > L, and L becomes exact(mn, i). Each group's tries see the latest L: the pass of K1e-partial, whose L rises with
+// every insert into a full list, and of a K1e run's first candidate, whose hints are only the subsample's.
 template <class Exact>
 __device__ __forceinline__ void eb_rows(const float2* R, int g, bool open, const float2* P, int n_set, unsigned short* h,
                                         unsigned& L, Exact exact, int lane, unsigned& pairs) {
@@ -741,10 +767,81 @@ __device__ __forceinline__ void eb_rows(const float2* R, int g, bool open, const
     for (unsigned open_mask = __ballot_sync(0xffffffffu, open); open_mask; open_mask &= open_mask - 1) {
         const int ii = g + __ffs(open_mask) - 1;
         int arg;
-        const unsigned mn = eb_warp_min(P, n_set, R[ii], h[ii], L, true, lane, arg, pairs);
+        const unsigned mn = eb_warp_min(P, n_set, R[ii], h[ii], L, lane, arg, pairs);
         __syncwarp();
         if (lane == 0) h[ii] = (unsigned short)arg;
         if (mn > L) L = exact(mn, ii);
+    }
+}
+// Positions T0 .. T1 - 1 of the zig-zag around the hint (steps +1, -2, +3, each wrapped once) of every row of the lane
+// that is open in this block, against L; a row that stops leaves the mask and keeps that position as its hint.
+template <int T0, int T1>
+__device__ __forceinline__ void eb_tries(const float2* R, int b0, const float2* P, int n_set, unsigned short* h,
+                                         unsigned L, unsigned& open, int lane, unsigned& pairs) {
+    for (unsigned m = open; m; m &= m - 1) {
+        const int k = __ffs(m) - 1, i = b0 + 32 * k + lane;
+        const float2 a = R[i];
+        int j = h[i];
+#pragma unroll
+        for (int t = 0; t < T1 && t < n_set; ++t) {
+            if (t & 1) {
+                j += t;
+                j = j >= n_set ? j - n_set : j;
+            } else if (t) {
+                j -= t;
+                j = j < 0 ? j + n_set : j;
+            }
+            if (t < T0) continue;
+            ++pairs;
+            if (__float_as_uint(eb_d2(a, P[j])) <= L) {
+                if (t) h[i] = (unsigned short)j;
+                open &= ~(1u << k);
+                break;
+            }
+        }
+    }
+}
+// One direction of the early-break passes (call it with the full warp): rows R[0 .. n) against the n_set points of P,
+// with the rows' hints h. Lane l takes rows l, l + 32, ..., in blocks of 32 groups of 32 rows, one bit per group in the
+// lane's mask of open rows:
+//   1. every row of the lane tests the position at its hint against L, with no warp-synchronous operation in the loop
+//      and no store (a row that stops there keeps its hint);
+//   2. the open rows try the next kEbTries - 1 positions of the zig-zag (steps +1, -2, +3, each wrapped once) against
+//      the current L; a row that stops keeps that position as its hint;
+//   3. the rows still open are finished one at a time by the whole warp; a row that scans to its end has an exact
+//      minimum mn > L, and L becomes exact(mn, i). Whenever that raises L, the rows still open first test their
+//      hints again, against the new L.
+// L only ever rises. A row that stops against an earlier L stops at a d^2 <= that L <= the final L, so it cannot raise
+// the maximum; a row that does not stop is finished against the current L; the order of the rows is free.
+template <class Exact>
+__device__ __forceinline__ void eb_pass(const float2* R, int n, const float2* P, int n_set, unsigned short* h,
+                                        unsigned& L, Exact exact, int lane, unsigned& pairs) {
+    for (int b0 = 0; b0 < n; b0 += 32 * 32) {
+        const int n_l = min(32, (n - b0 - lane + 31) >> 5);   // rows of this lane in the block
+        unsigned open = 0u;
+#pragma unroll 4
+        for (int k = 0; k < n_l; ++k) {
+            const int i = b0 + 32 * k + lane;
+            ++pairs;
+            open |= (unsigned)(__float_as_uint(eb_d2(R[i], P[h[i]])) > L) << k;
+        }
+        eb_tries<1, kEbTries>(R, b0, P, n_set, h, L, open, lane, pairs);
+        for (unsigned any = __ballot_sync(0xffffffffu, open); any; any = __ballot_sync(0xffffffffu, open)) {
+            const int src = __ffs(any) - 1;
+            const int ii = b0 + 32 * (__ffs(__shfl_sync(0xffffffffu, open, src)) - 1) + src;
+            if (lane == src) open &= open - 1;
+            int arg;
+            const unsigned mn = eb_warp_min(P, n_set, R[ii], h[ii], L, lane, arg, pairs);
+            __syncwarp();
+            if (lane == 0) h[ii] = (unsigned short)arg;
+            if (mn > L) {
+                const unsigned L0 = L;
+                L = exact(mn, ii);
+                // the rows still open missed their hints against a lower L: test the hints again before the warp takes
+                // the rows
+                if (L != L0) eb_tries<0, 1>(R, b0, P, n_set, h, L, open, lane, pairs);
+            }
+        }
     }
 }
 
@@ -758,7 +855,7 @@ __device__ __forceinline__ void eb_rows(const float2* R, int g, bool open, const
 //   seed    the rows of the previous candidate's list in the direction that defined its value (the run's first
 //           candidate: the q + 1 points farthest from the centre, both directions), each scanned to its end by one
 //           lane; they enter the list and are marked so that the main pass skips them;
-//   rows    K1e's pass (eb_rows) with the seeded rows left out: a row that scans to its end has an exact minimum > L
+//   rows    K1e's per-group pass (eb_rows) with the seeded rows left out: a row that scans to its end has an exact minimum > L
 //           and enters its list (replacing the smallest entry when full); L is recomputed;
 //   columns the same with the reference points as rows.
 // Exactness (F = max(V_r, V_c), V the true (q + 1)-th largest FP32 minimum of a direction): L is always the (q + 1)-th
@@ -1029,8 +1126,8 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                 // candidate's L (the run's first candidate: both)
                 int h_ra = 0, h_cb = 0;
                 L = 0u;
-                if (seed[0]) L = eb_warp_min(sB, M, sR[ra], hint[0][ra], 0u, false, lane, h_ra, pairs);
-                const unsigned lc = seed[1] ? eb_warp_min(sR, N, sB[cb], hint[1][cb], 0u, false, lane, h_cb, pairs) : 0u;
+                if (seed[0]) L = eb_warp_exact(sB, M, sR[ra], hint[0][ra], lane, h_ra, pairs);
+                const unsigned lc = seed[1] ? eb_warp_exact(sR, N, sB[cb], hint[1][cb], lane, h_cb, pairs) : 0u;
                 __syncwarp();
                 if (lane == 0) {
                     if (seed[0]) hint[0][ra] = (unsigned short)h_ra;
@@ -1039,10 +1136,18 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                 bool by_row = seed[0] && !(lc > L);   // the direction that last raised L (both seeded and tied: rows)
                 L = max(L, lc);
                 __syncwarp();
-                for (int g = 0; g < N; g += 32)   // rows: test point i against the reference points
-                    eb_rows(sR, g, g + lane < N, sB, M, hint[0], L, [&](unsigned mn, int i) { ra = i, by_row = true; return mn; }, lane, pairs);
-                for (int g = 0; g < M; g += 32)   // columns: reference point j against A'
-                    eb_rows(sB, g, g + lane < M, sR, N, hint[1], L, [&](unsigned mn, int j) { cb = j, by_row = false; return mn; }, lane, pairs);
+                // rows: test point i against the reference points; columns: reference point j against A'. The run's
+                // first candidate keeps the per-group pass: with hints from the subsample many of its rows miss, and
+                // there batching the first tries against the seed costs more than it saves (DESIGN §4 K1e, round 9)
+                const auto row = [&](unsigned mn, int i) { ra = i, by_row = true; return mn; };
+                const auto col = [&](unsigned mn, int j) { cb = j, by_row = false; return mn; };
+                if (c == c_begin) {
+                    for (int g = 0; g < N; g += 32) eb_rows(sR, g, g + lane < N, sB, M, hint[0], L, row, lane, pairs);
+                    for (int g = 0; g < M; g += 32) eb_rows(sB, g, g + lane < M, sR, N, hint[1], L, col, lane, pairs);
+                } else {
+                    eb_pass(sR, N, sB, M, hint[0], L, row, lane, pairs);
+                    eb_pass(sB, M, sR, N, hint[1], L, col, lane, pairs);
+                }
                 // rotation only: seed one direction. RIGID keeps both: a run steps through the translations and jumps
                 // back across the whole translation grid at each new angle, and a single seed leaves L lower there
                 // often enough to cost more pairs than the second seed scan (4 277 against 4 184 per candidate on the
