@@ -14,7 +14,7 @@ struct UnitDesc {
     long long test_off, ref_off;  // point offsets into the f64 (x,y) arrays
     int n, m;                     // test / reference point counts
     double cx, cy;                // rotation centre
-    long long lay_off;            // float4 offset of this unit's staging block (A then B)
+    long long lay_off;            // float4 offset of this unit's staging block (A, B, NB, tail, K1e's grid block)
     int n_chunks;                 // A is stored as n_chunks x (TA/2) x 32 float4
     int m_pairs;                  // B is stored as m_pairs float4 (bx0,by0,bx1,by1)
     long long cand_off;           // offset of this unit's grid in the cos/sin tables
@@ -29,6 +29,7 @@ struct UnitDesc {
     long long t_off;              // rigid runs: offset of this unit's translation grid in the t64 / t32 tables
     int n_trans;                  // translations per angle (1 without a translation grid): candidate c = i n_trans + j
     short q_fwd, q_bwd;           // partial cost: points that do not count, reference -> test (q(m)) / test -> reference (q(n))
+    int eb_grid;                  // K1e: the staging image carries the grid block (sweep_kernels.cuh, K0), else full seed scans
 };
 constexpr int kFlagRemote = 0x400;  // internal UnitDesc.flags bit: another rank owns this unit (never leaves the library)
 

@@ -491,7 +491,14 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
                 smem = 0;
                 ctx->big_scratch_per_warp = std::max<long long>(ctx->big_scratch_per_warp, (long long)d.n_chunks * 32 * kBigTA);
             }
-            lay_off += stage_layout(d.ta, d.n_chunks, d.n_tail, d.m_pairs).total();
+            // K1e: the same staging image plus, per warp, A' and the row / column hints; and the grid block where it does
+            // not move the unit across a shared-memory rule of K1e (3 CTAs per SM in auto mode, the opt-in maximum with
+            // MMRS_EARLY_BREAK=1): a unit without grids seeds by full scans and keeps K1e wherever it had it
+            const size_t smem_eb = stage + (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m);
+            const size_t smem_eb_grid = smem_eb + (size_t)eb_grid_f4(d.n, d.m, true) * 16;
+            d.eb_grid = ctx->cost == kCostFull && !big &&
+                        (smem_eb_grid <= kEbAutoSmem || (smem_eb > kEbAutoSmem && smem_eb_grid <= (size_t)kMaxDynSmem));
+            lay_off += stage_layout(d.ta, d.n_chunks, d.n_tail, d.m_pairs).total() + eb_grid_f4(d.n, d.m, d.eb_grid);
             int k = 0;
             for (; k < (int)ctx->classes.size(); ++k) {
                 const auto& c = ctx->classes[k];
@@ -514,8 +521,8 @@ static int upload_points(mmrs_ctx* ctx, const mmrs_sweep_batch* b_in) {
             if (ctx->cost == kCostPartial) {
                 ebp_stage[k] = std::max(ebp_stage[k], stage);
                 ebp_warp[k] = std::max(ebp_warp[k], (size_t)ebp_warp_bytes(d.n, d.m, d.q_bwd, d.q_fwd));
-            } else if (!big) {   // K1e: the same staging image plus, per warp, A' and the row / column hints
-                cl.smem_eb = std::max(cl.smem_eb, stage + (size_t)kWarpsPerCta * eb_warp_bytes(d.n, d.m));
+            } else if (!big) {
+                cl.smem_eb = std::max(cl.smem_eb, d.eb_grid ? smem_eb_grid : smem_eb);
             }
         }
     }

@@ -139,8 +139,113 @@ __host__ __device__ inline StageLayout stage_layout(int ta, int n_chunks, int n_
     return StageLayout{n_chunks * ((ta + 1) / 2) * 32, b, (b + 1) / 2, (n_tail + 1) / 2};
 }
 
+// Grid block (after the tail block of a unit with UnitDesc.eb_grid, else empty; read by K1e only, which stages it with
+// the rest): a uniform G x G grid over the reference set in its own frame, then one over the test set unrotated. Per set
+// of k points:
+//   float4 (x0, y0, ix, iy): origin and inverse cell sizes (ix = 0: no grid, K1e scans the whole set),
+//   float4 (r, 0, 0, 0)    : r >= max |x| + max |y| over the set (rounded up), for K1e's distance margin,
+//   u16 start[G^2 + 1]     : CSR offsets of the cells (cell = row cy * G + cx),
+//   u16 idx[k]             : point indices sorted by cell, in index order within a cell,
+// padded to 16 bytes. A point's cell on each axis is clamp(floorf(fl(fl(v - v0) * iv)), 0, G - 1) (eb_cell), the
+// expression K1e evaluates on its query bounds: it is monotone in v, so every point with a coordinate inside a query
+// interval lies in a cell the query visits.
+#ifndef MMRS_EB_GRID
+#define MMRS_EB_GRID 16   // cells per axis of the grid over a set of 256 to 1 023 points (half below, twice above)
+#endif
+constexpr int kEbGridMinPts = 64, kEbGridMaxPts = 4096;   // sets outside this range get no grid (header only)
+constexpr int kEbGridMaxG = 2 * MMRS_EB_GRID;
+// no grid above this coordinate magnitude: d^2 of two such points, and K1e's query bounds, stay finite
+constexpr float kEbGridMaxCoord = 1.152921504606846976e18f;   // 2^60
+__host__ __device__ constexpr int eb_grid_g(int k) { return k < 256 ? MMRS_EB_GRID / 2 : k < 1024 ? MMRS_EB_GRID : 2 * MMRS_EB_GRID; }
+__host__ __device__ constexpr bool eb_grid_sized(int k) { return k >= kEbGridMinPts && k <= kEbGridMaxPts; }
+// float4 of one set's grid, and of a unit's grid block (reference set first)
+__host__ __device__ constexpr int eb_grid_set_f4(int k) {
+    return eb_grid_sized(k) ? 2 + (2 * (eb_grid_g(k) * eb_grid_g(k) + 1) + 2 * k + 15) / 16 : 2;
+}
+__host__ __device__ constexpr int eb_grid_f4(int n, int m, bool on) { return on ? eb_grid_set_f4(m) + eb_grid_set_f4(n) : 0; }
+__device__ __forceinline__ float eb_cell(float v, float v0, float iv) { return floorf(__fmul_rn(__fsub_rn(v, v0), iv)); }
+
+// One set's grid, built by one warp. pt(i): the FP32 point i exactly as staged.
+template <class Pt>
+__device__ __forceinline__ void eb_grid_build(Pt pt, int k, float4* out, unsigned short* s_cur, int lane) {
+    float x_lo = INFINITY, x_hi = -INFINITY, y_lo = INFINITY, y_hi = -INFINITY, ax = 0.f, ay = 0.f;
+    bool finite = true;
+    for (int i = lane; i < k; i += 32) {
+        const float2 p = pt(i);
+        x_lo = fminf(x_lo, p.x), x_hi = fmaxf(x_hi, p.x), y_lo = fminf(y_lo, p.y), y_hi = fmaxf(y_hi, p.y);
+        ax = fmaxf(ax, fabsf(p.x)), ay = fmaxf(ay, fabsf(p.y));
+        finite = finite && fabsf(p.x) <= 3.402823466e38f && fabsf(p.y) <= 3.402823466e38f;
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+        x_lo = fminf(x_lo, __shfl_xor_sync(0xffffffffu, x_lo, o)), x_hi = fmaxf(x_hi, __shfl_xor_sync(0xffffffffu, x_hi, o));
+        y_lo = fminf(y_lo, __shfl_xor_sync(0xffffffffu, y_lo, o)), y_hi = fmaxf(y_hi, __shfl_xor_sync(0xffffffffu, y_hi, o));
+        ax = fmaxf(ax, __shfl_xor_sync(0xffffffffu, ax, o)), ay = fmaxf(ay, __shfl_xor_sync(0xffffffffu, ay, o));
+    }
+    const int G = eb_grid_g(k);
+    const float ix = __fdiv_rn((float)G, __fsub_rn(x_hi, x_lo)), iy = __fdiv_rn((float)G, __fsub_rn(y_hi, y_lo));
+    // no grid: a set outside the size range, a coordinate that is not finite in FP32, zero (or denormal) extent on an
+    // axis (ix not a finite positive number), or coordinates large enough for d^2 to overflow
+    const bool on = __all_sync(0xffffffffu, finite) && eb_grid_sized(k) && ix > 0.f && ix <= 3.402823466e38f && iy > 0.f &&
+                    iy <= 3.402823466e38f && fmaxf(ax, ay) <= kEbGridMaxCoord;
+    if (lane == 0) {
+        out[0] = make_float4(x_lo, y_lo, on ? ix : 0.f, iy);
+        out[1] = make_float4(__fadd_ru(ax, ay), 0.f, 0.f, 0.f);
+    }
+    if (!on) return;
+    const float gm1 = (float)(G - 1);
+    unsigned short* start = reinterpret_cast<unsigned short*>(out + 2);
+    unsigned short* idx = start + G * G + 1;
+    auto cell_of = [&](int i) {
+        const float2 p = pt(i);
+        const int cx = (int)fminf(fmaxf(eb_cell(p.x, x_lo, ix), 0.f), gm1), cy = (int)fminf(fmaxf(eb_cell(p.y, y_lo, iy), 0.f), gm1);
+        return cy * G + cx;
+    };
+    for (int c = lane; c < G * G; c += 32) s_cur[c] = 0;
+    __syncwarp();
+    // counts: per chunk of 32 points, the lowest lane of each cell adds the chunk's points in that cell
+    for (int c0 = 0; c0 < k; c0 += 32) {
+        const int i = c0 + lane, c = i < k ? cell_of(i) : -1;
+        const unsigned same = __match_any_sync(0xffffffffu, c);
+        if (c >= 0 && lane == __ffs(same) - 1) s_cur[c] += (unsigned short)__popc(same);
+        __syncwarp();
+    }
+    // exclusive scan: the cell starts (G^2 may be below 32: G = 4)
+    int carry = 0;
+    for (int c0 = 0; c0 < G * G; c0 += 32) {
+        const int c = c0 + lane;
+        const int v = c < G * G ? s_cur[c] : 0;
+        int s = v;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, s, o);
+            if (lane >= o) s += t;
+        }
+        if (c < G * G) {
+            s_cur[c] = (unsigned short)(carry + s - v);
+            start[c] = (unsigned short)(carry + s - v);
+        }
+        carry += __shfl_sync(0xffffffffu, s, 31);
+    }
+    if (lane == 0) start[G * G] = (unsigned short)k;
+    __syncwarp();
+    // fill, in index order within a cell
+    for (int c0 = 0; c0 < k; c0 += 32) {
+        const int i = c0 + lane, c = i < k ? cell_of(i) : -1;
+        const unsigned same = __match_any_sync(0xffffffffu, c);
+        const int pos = c >= 0 ? s_cur[c] + __popc(same & ((1u << lane) - 1u)) : 0;
+        __syncwarp();
+        if (c >= 0) {
+            idx[pos] = (unsigned short)i;
+            if (lane == __ffs(same) - 1) s_cur[c] += (unsigned short)__popc(same);
+        }
+        __syncwarp();
+    }
+}
+
 __global__ void k_prep(const UnitDesc* __restrict__ units, const double* __restrict__ test_xy,
                        const double* __restrict__ ref_xy, float4* __restrict__ lay, unsigned* __restrict__ rmax_bits) {
+    __shared__ unsigned short s_cur[2][kEbGridMaxG * kEbGridMaxG];
     const UnitDesc ud = units[blockIdx.x];
     if (ud.n <= 0 || ud.m <= 0) return;
     const int TA = ud.ta;
@@ -193,6 +298,19 @@ __global__ void k_prep(const UnitDesc* __restrict__ units, const double* __restr
     }
     unsigned rb = __reduce_max_sync(0xffffffffu, __float_as_uint(rmax));
     if ((threadIdx.x & 31) == 0) atomicMax(&rmax_bits[blockIdx.x], rb);
+    // K1e's grids: warp 0 over the reference set, warp 1 over the test set, from the same FP32 values as staged above
+    if (!ud.eb_grid) return;
+    const int wid = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float4* Gb = T + sl.t;
+    if (wid == 0) {
+        const double* r = ref_xy + 2 * ud.ref_off;
+        eb_grid_build([&](int j) { return make_float2((float)(r[2 * j] - ud.cx), (float)(r[2 * j + 1] - ud.cy)); }, ud.m, Gb,
+                      s_cur[0], lane);
+    } else if (wid == 1) {
+        const double* t = test_xy + 2 * ud.test_off;
+        eb_grid_build([&](int i) { return make_float2((float)(t[2 * i] - ud.cx), (float)(t[2 * i + 1] - ud.cy)); }, ud.n,
+                      Gb + eb_grid_set_f4(ud.m), s_cur[1], lane);
+    }
 }
 
 // f64 (cos, sin) table -> FP32 table for K1.
@@ -710,6 +828,45 @@ __device__ __forceinline__ unsigned eb_warp_exact(const float2* P, int n, float2
     arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
     return m;
 }
+// The same exact minimum (the seeds), visiting only the cells of P's grid gr (K0's grid block) that can hold it. q is a
+// in the grid's frame: a itself for the rows (the reference set's grid), R(-theta)(a - t) for the columns (the test set's
+// grid, unrotated); r bounds the coordinate magnitudes of a, q and the set, rotated or not. U = d^2 at the hint bounds
+// the minimum; every point outside the square of half-width rho = sqrt(U) (1 + 1.2e-6) + 2e-6 r around q has a
+// computed d^2 > U (DESIGN §4 K1e, "grid seed"), so it cannot hold the minimum and is skipped. The lanes take the
+// visited cells' points, one contiguous CSR range, 32 at a time and reduce once at the end. A unit without a grid block
+// (on = false), a set without cells (ix = 0) and a bound that is not finite scan the whole set.
+__device__ __forceinline__ unsigned eb_grid_exact(bool on, const float4* gr, const float2* P, int n, float2 a, float2 q,
+                                                  float r, int h, int lane, int& arg, unsigned& pairs) {
+    const float4 o = on ? gr[0] : make_float4(0.f, 0.f, 0.f, 0.f);
+    if (o.z == 0.f) return eb_warp_exact(P, n, a, h, lane, arg, pairs);
+    const int G = eb_grid_g(n);
+    const float gm1 = (float)(G - 1);
+    const unsigned short* start = reinterpret_cast<const unsigned short*>(gr + 2);
+    const unsigned short* idx = start + G * G + 1;
+    const float U = eb_d2(a, P[h]);
+    pairs += lane == 0;
+    const float rho = __fmaf_ru(__fsqrt_ru(U), 1.0f + 1.2e-6f, __fmul_ru(2e-6f, r));
+    // a NaN bound (U or rho not finite) clamps to the whole axis: lo to 0, hi to G - 1
+    const int x0 = (int)fminf(fmaxf(eb_cell(__fsub_rn(q.x, rho), o.x, o.z), 0.f), gm1);
+    const int x1 = (int)fmaxf(fminf(eb_cell(__fadd_rn(q.x, rho), o.x, o.z), gm1), 0.f);
+    const int y0 = (int)fminf(fmaxf(eb_cell(__fsub_rn(q.y, rho), o.y, o.w), 0.f), gm1);
+    const int y1 = (int)fmaxf(fminf(eb_cell(__fadd_rn(q.y, rho), o.y, o.w), gm1), 0.f);
+    unsigned best = lane == 0 ? __float_as_uint(U) : ~0u;   // the hint's pair takes part: the minimum is never above U
+    int bj = h;
+    // cells (x0, y0) .. (x1, y1) in row-major order: one contiguous CSR range that holds every cell of the square (and the
+    // cells of the rows in between outside it: extra points never change a minimum), scanned with one loop
+    const int e = start[y1 * G + x1 + 1];
+#pragma unroll 2
+    for (int k = start[y0 * G + x0] + lane; k < e; k += 32) {
+        const int j = idx[k];
+        const unsigned d = __float_as_uint(eb_d2(a, P[j]));
+        if (d < best) best = d, bj = j;
+        ++pairs;
+    }
+    const unsigned m = __reduce_min_sync(0xffffffffu, best);
+    arg = __shfl_sync(0xffffffffu, bj, __ffs(__ballot_sync(0xffffffffu, best == m)) - 1);
+    return m;
+}
 // Hints of rows R[0 .. n) for the first candidate of a run: each row's nearest point among P[0], P[kEbColdStride], ...
 // of the n_set points of P (one lane per row, no early stop; the warp's lanes read the same P[j]: a broadcast). The
 // hint is a multiple of the stride below n_set whatever the distances are (a NaN d^2 may win, which is harmless: the
@@ -935,7 +1092,11 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
     const StageLayout sl = stage_layout(TA, ud.n_chunks, ud.n_tail, ud.m_pairs);
     const float2* sB = reinterpret_cast<const float2*>(sA + sl.a);                        // reference point j
     const float2* sT = reinterpret_cast<const float2*>(sA + sl.a + sl.b + sl.nb);         // tail point t
-    unsigned char* my = reinterpret_cast<unsigned char*>(sA + sl.a + sl.b + sl.nb + sl.t) +
+    const float4* gB = sA + sl.total();                                                   // K1e: the grid block
+    const float4* gA = gB + eb_grid_set_f4(M);
+    const bool grid = !PARTIAL && ud.eb_grid;       // K1e-partial does not stage the grids
+    const int g4 = eb_grid_f4(N, M, grid);
+    unsigned char* my = reinterpret_cast<unsigned char*>(sA + sl.total() + g4) +
                         wid * (PARTIAL ? ebp_warp_bytes(N, M, ud.q_bwd, ud.q_fwd) : eb_warp_bytes(N, M));
     float2* sR = reinterpret_cast<float2*>(my);                                           // A': rotated test points
     // direction 0, rows: A' against the reference points; direction 1, columns: the reference points against A'
@@ -959,7 +1120,7 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
     if (threadIdx.x == 0) {
         mbar_init(bar, 1);
         *s_key = ~0ull;
-        const uint32_t bytes = (uint32_t)sl.total() * 16u;
+        const uint32_t bytes = (uint32_t)(sl.total() + g4) * 16u;
         mbar_expect_tx(bar, bytes);
         tma_bulk_g2s(sA, lay + ud.lay_off, bytes, bar);
     }
@@ -1126,8 +1287,16 @@ __global__ void __launch_bounds__(kThreads, PARTIAL ? 2 : 3)
                 // candidate's L (the run's first candidate: both)
                 int h_ra = 0, h_cb = 0;
                 L = 0u;
-                if (seed[0]) L = eb_warp_exact(sB, M, sR[ra], hint[0][ra], lane, h_ra, pairs);
-                const unsigned lc = seed[1] ? eb_warp_exact(sR, N, sB[cb], hint[1][cb], lane, h_cb, pairs) : 0u;
+                // through the grids: rows against the reference set's, columns against the test set's at R(-theta)(b - t)
+                const float r = grid ? __fadd_ru(__fadd_ru(gA[1].x, gB[1].x), __fadd_ru(fabsf(tr.x), fabsf(tr.y))) : 0.f;
+                if (seed[0]) L = eb_grid_exact(grid, gB, sB, M, sR[ra], sR[ra], r, hint[0][ra], lane, h_ra, pairs);
+                unsigned lc = 0u;
+                if (seed[1]) {
+                    const float2 b = sB[cb];
+                    const float bx = RIGID ? __fsub_rn(b.x, tr.x) : b.x, by = RIGID ? __fsub_rn(b.y, tr.y) : b.y;
+                    const float2 q = make_float2(__fmaf_rn(by, cs.y, __fmul_rn(bx, cs.x)), __fmaf_rn(bx, -cs.y, __fmul_rn(by, cs.x)));
+                    lc = eb_grid_exact(grid, gA, sR, N, b, q, r, hint[1][cb], lane, h_cb, pairs);
+                }
                 __syncwarp();
                 if (lane == 0) {
                     if (seed[0]) hint[0][ra] = (unsigned short)h_ra;
